@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # reference CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs to DIR/*.npy
 
 One "step" = one pass of the hot path (forward + MSE loss + backward, all parameter gradients)
 over one batch of B synthetic snapshots.  Default workload: BASELINE.json's headline config --
@@ -65,7 +66,36 @@ def parse():
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of the cpu_baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the spmm / reference_call_pattern / cfg2 side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (loss, out, hidden, every parameter "
+                         "gradient; rank 0's) as DIR/<name>.npy, float32, at most 64 MB in all (see dump_outputs)")
     return ap.parse_args()
+
+
+DUMP_BUDGET_BYTES = 60_000_000     # data of all .npy files together; their headers stay well inside 64 MB
+
+
+def dump_outputs(dirname: str, arrays: dict) -> dict:
+    """writes every tensor of ``arrays`` as ``dirname/<name>.npy`` in float32.  The smallest arrays are written whole; an array
+    that would overrun what is left of DUMP_BUDGET_BYTES is written as a fixed sample of its flattened elements: one element
+    drawn (seed 0) from each of k equal strides.  The sample depends only on the array's size, so two runs, or two builds,
+    with the same arguments compare element for element.  Returns {name: (full shape, elements written)}."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    left = DUMP_BUDGET_BYTES // 4
+    written = {}
+    items = sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    for i, (name, t) in enumerate(items):
+        a = t.detach()
+        n = a.numel()
+        k = min(n, max(1, left // (len(items) - i)))
+        if k < n:
+            idx = np.arange(k, dtype=np.int64) * n // k + np.random.default_rng(0).integers(0, n // k, size=k)
+            a = a.reshape(-1)[torch.from_numpy(idx).to(a.device)]
+        np.save(os.path.join(dirname, name + ".npy"), a.float().cpu().numpy())
+        left -= k
+        written[name] = (tuple(t.shape), k)
+    return written
 
 
 # ------------------------------------------------------------------------------------------------
@@ -459,13 +489,16 @@ def main():
     loss_h = [torch.zeros(1).pin_memory(), torch.zeros(1).pin_memory()]
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)  # > 126 MB L2
     the_model = sm.model if sharded else model
+    results = [None, None]    # (loss, out, hid) of the last step on each input buffer; the graphs' static outputs once captured
 
     def raw_step(b=0):
         xd, yd = bufs[b]
         ex.zero()     # per-step gradients: the flat buffer holds this step's contribution only (and feeds the exchange at N > 1)
         if sharded:
-            return sm.fused_step(None, None, micro_batch=args.micro_batch, local_inputs=(xd, yd), sync=False)[0]
-        return model.fused_step(xd, yd, *graph_args, micro_batch=args.micro_batch)[0]
+            results[b] = sm.fused_step(None, None, micro_batch=args.micro_batch, local_inputs=(xd, yd), sync=False)
+        else:
+            results[b] = model.fused_step(xd, yd, *graph_args, micro_batch=args.micro_batch)
+        return results[b][0]
 
     # warm-up (eager) -- also builds and caches the static-graph plan (K1), excluded from timing
     lib.regt_launch_count(1)
@@ -641,6 +674,14 @@ def main():
     if dist is not None:
         dist.all_reduce(e2e_ms, op=dist.ReduceOp.MAX)
     e2e_ms = float(e2e_ms)
+
+    # ---------------- what the last timed step returned, before the eager steps below overwrite the gradients ----------
+    if args.dump_outputs and rank == 0:
+        _, out_d, hid_d = results[(K - 1) & 1]
+        arrays = {"loss": loss_d, "out": out_d, "hidden": hid_d}
+        arrays.update({"grad." + n: p.grad for n, p in the_model.named_parameters() if p.grad is not None})
+        for name, (shape, k) in dump_outputs(args.dump_outputs, arrays).items():
+            print(f"dump {name}: shape {list(shape)}, {k} elements written", file=sys.stderr)
 
     # ---------------- per-kernel breakdown for the roofline (rank 0, eager, events per launch) -----
     roofline, breakdown, step_roof = None, None, None

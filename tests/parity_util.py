@@ -55,6 +55,19 @@ def oracle_step(w, B, dtype=torch.float64, seed=1234):
     return dict(out=out, hid=hid, loss=loss, grads=grads, state=copy.deepcopy(m.state_dict()))
 
 
+def shipped_checkpoint_state(fname, seed=0):
+    """a state_dict with the tensor names, shapes and dtype of the upstream project's checkpoint ``fname``
+    (pretrained/occrate/RegionalTemporalGCN/, 3 MB each, not redistributed here), filled with seeded values.  The layout is
+    stored in tests/golden/shipped_checkpoints.json: it is the one the three files were loaded with, strict, into the
+    oracle while they were at hand (26 float32 tensors, 766 577 parameters in model_in6_out1_epoch50.pt)."""
+    import json
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "shipped_checkpoints.json")) as f:
+        spec = json.load(f)[fname]
+    g = torch.Generator().manual_seed(seed)
+    dtype = getattr(torch, spec["dtype"])
+    return spec, {k: torch.rand(s, generator=g, dtype=dtype) - 0.5 for k, s in spec["shapes"].items()}
+
+
 def to_dev(args, device):
     return tuple(None if a is None else a.to(device) for a in args)
 

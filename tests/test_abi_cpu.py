@@ -111,9 +111,8 @@ def test_reference_state_dict_keys():
                  f"tgnn._base_tgcn.linear_{g}.weight", f"tgnn._base_tgcn.linear_{g}.bias"}
     assert keys == want and len(keys) == 26
     assert tuple(m.state_dict()["tgnn.linear.weight"].shape) == (256, 1280)
-    ref = "/root/reference/pretrained/occrate/RegionalTemporalGCN/model_in6_out1_epoch50.pt"
-    if os.path.exists(ref):
-        m.load_state_dict(torch.load(ref, map_location="cpu"), strict=True)
+    from parity_util import shipped_checkpoint_state
+    m.load_state_dict(shipped_checkpoint_state("model_in6_out1_epoch50.pt")[1], strict=True)
 
 
 def test_run_py_keeps_the_reference_flags():

@@ -9,8 +9,6 @@ from oracle import regt_oracle as O
 from oracle import dense_check as D
 from regt_b200 import workloads as W
 
-REF_CKPT = "/root/reference/pretrained/occrate/RegionalTemporalGCN"
-
 
 def test_laplacian_known_answer_upstream():
     """Known-answer vector of PyG's own test-suite for get_laplacian(normalization='sym')
@@ -68,14 +66,19 @@ def test_scatter_formulation_matches_dense_restatement(model, adv):
     assert np.abs(hid.detach().numpy() - h2).max() < 1e-12
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_CKPT), reason="reference checkpoints only exist in the build container")
 @pytest.mark.parametrize("fname,nn_,od", [("model_in6_out1_epoch50.pt", 104, 1), ("model_in6_out3_epoch50.pt", 105, 3),
                                           ("model_in6_out36_epoch50.pt", 105, 36)])
 def test_shipped_checkpoints_load_strict(fname, nn_, od):
-    sd = torch.load(os.path.join(REF_CKPT, fname), map_location="cpu")
+    """the layout of the upstream checkpoints (tensor names, shapes, dtype; tests/golden/shipped_checkpoints.json) loads strict
+    into the oracle built with that checkpoint's constructor arguments."""
+    from parity_util import shipped_checkpoint_state
+    spec, sd = shipped_checkpoint_state(fname)
+    assert (spec["num_nodes"], spec["periods"], spec["output_dim"]) == (nn_, 6, od)
     m = O.RegionalTemporalGCN(8, nn_, 6, od)
     m.load_state_dict(sd, strict=True)
-    assert len(sd) == 26
+    assert len(sd) == 26 and all(v.dtype == torch.float32 for v in sd.values())
+    if fname == "model_in6_out1_epoch50.pt":
+        assert sum(v.numel() for v in sd.values()) == 766_577
     full, rei, rea, N = W.tpims_graph()
     x = torch.rand(N, 8, 6, generator=torch.Generator().manual_seed(1))
     out, hid = m(x, full, *rei, *rea)
