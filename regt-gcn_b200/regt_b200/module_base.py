@@ -64,13 +64,16 @@ class RegTModelBase(nn.Module):
     def _param_dict(self) -> Dict[str, torch.Tensor]:
         raise NotImplementedError
 
-    def _prec(self) -> int:
+    def _prec(self, T: Optional[int] = None) -> int:
         """``precision="auto"`` (the default): fp32-equivalent arithmetic on the fastest path that offers it -- the 3xTF32
-        tensor-core kernels when the hidden width allows (hidden % 32 == 0; the reference's 256 does), else the FFMA kernels.
-        Both meet the same 1e-5 parity bound; ``bf16`` (stated tolerance) is opt-in only."""
+        tensor-core kernels when the hidden width allows (hidden % 32 == 0; the reference's 256 does) and the input has at
+        most 64 periods (``T``, the tf32x3 kernels' limit), else the FFMA kernels, which take any period count.
+        Both meet the same 1e-5 parity bound; ``bf16`` (stated tolerance) is opt-in only.  An explicit precision is
+        used as given: tf32x3 with T > 64 is refused by the kernels."""
         prec = self.precision
         if prec == "auto":
-            prec = "tf32x3" if (self._hidden % 32 == 0 and self._mode != _lib.MODE_TGCN) else "fp32"
+            fits = self._hidden % 32 == 0 and self._mode != _lib.MODE_TGCN and (T is None or T <= 64)
+            prec = "tf32x3" if fits else "fp32"
         try:
             return _lib.PRECISIONS[prec]
         except KeyError:
@@ -100,7 +103,7 @@ class RegTModelBase(nn.Module):
     def _run(self, x: torch.Tensor, plan):
         xb, batched = self._as_batched(x)
         xb = xb.to(torch.float32).contiguous()
-        out, hid = engine.model_apply(self._mode, self._prec(), plan, self._hidden, self.output_dim, xb,
+        out, hid = engine.model_apply(self._mode, self._prec(xb.shape[3]), plan, self._hidden, self.output_dim, xb,
                                       self._param_dict(), None, True)
         if not batched:
             out, hid = out[0], hid[0]
@@ -127,20 +130,21 @@ class RegTModelBase(nn.Module):
                     p.grad = torch.zeros_like(p)
             grads[k] = p.grad
         B = xb.shape[0]
+        prec = self._prec(xb.shape[3])
         if micro_batch:
             mb = min(B, micro_batch)
         else:   # whole batch if its saved planes fit, else the largest divisor of B that does (decided once per shape)
             key = (B, xb.shape[1], xb.shape[3])
             if getattr(self, "_mb_key", None) != key:
                 ws = getattr(self, "_ws", None)
-                self._mb = engine.auto_micro_batch(self._mode, self._prec(), plan, B, xb.shape[1], xb.shape[3], self._hidden,
+                self._mb = engine.auto_micro_batch(self._mode, prec, plan, B, xb.shape[1], xb.shape[3], self._hidden,
                                                    self.output_dim, 0 if ws is None else ws.numel())
                 self._mb_key = key
             mb = self._mb
         loss = None
         outs, hids = [], []
         for b0 in range(0, B, mb):
-            st = engine.build_state(self._mode, self._prec(), plan, xb[b0:b0 + mb], self._hidden, self.output_dim,
+            st = engine.build_state(self._mode, prec, plan, xb[b0:b0 + mb], self._hidden, self.output_dim,
                                     params, yb[b0:b0 + mb], None, True, getattr(self, "_ws", None), fuse_head=True,
                                     loss_nodes=loss_nodes)
             self._ws = st.workspace

@@ -155,20 +155,27 @@ def get_plan(N: int, device: torch.device, edge_index: torch.Tensor, edge_weight
                     _content_key([edge_index, edge_weight, *reg_edge_index, *reg_edge_weight]))
         plan = _CONTENT.get(ckey)
         if plan is not None:
+            # also by identity: a CUDA-graph capture of a step with these tensors must find the plan without the device
+            # work of hashing (or building) it, even when their content was first seen through other tensors
+            _remember(key, plan, edge_index, edge_weight, reg_edge_index, reg_edge_weight)
             return plan
     plan = GraphPlanTensors(device, N)
     build_gcn(plan, edge_index, edge_weight)
     if need_cheb:
         build_cheb(plan, reg_edge_index, reg_edge_weight)
-    if len(_CACHE) > 64:
-        _CACHE.clear()
+    _remember(key, plan, edge_index, edge_weight, reg_edge_index, reg_edge_weight)
     if len(_CONTENT) > 16:
         _CONTENT.clear()
-    # keep the key tensors alive so data_ptr() cannot be recycled while the entry lives
-    _CACHE[key] = (plan, edge_index, edge_weight, list(reg_edge_index), list(reg_edge_weight))
     if ckey is not None:
         _CONTENT[ckey] = plan
     return plan
+
+
+def _remember(key, plan, edge_index, edge_weight, reg_edge_index, reg_edge_weight) -> None:
+    if len(_CACHE) > 64:
+        _CACHE.clear()
+    # keep the key tensors alive so data_ptr() cannot be recycled while the entry lives
+    _CACHE[key] = (plan, edge_index, edge_weight, list(reg_edge_index), list(reg_edge_weight))
 
 
 _PARTS: dict = {}     # (rowptr ptr, col ptr, versions, N, width) -> (rowptr, col, blk_ptr, nblk): the staged SpMM's row partition

@@ -486,7 +486,7 @@ class RegionShardedModel:
         """inference: full-N ``(out, out_hidden)`` on every rank (all-gather of the regional outputs)."""
         from . import engine
         xl, _ = self.local_inputs(x, None)
-        out, hid = engine.model_apply(self.model._mode, self.model._prec(), self.plan, self.model._hidden,
+        out, hid = engine.model_apply(self.model._mode, self.model._prec(xl.shape[3]), self.plan, self.model._hidden,
                                       self.model.output_dim, xl, self.model._param_dict(), None, True)
         if self.shard.world > 1:
             both = all_gather_nodes(torch.cat([out, hid], dim=2), self.shard, self.group)
