@@ -13,8 +13,8 @@
  *    least regt_workspace_bytes() bytes (256-byte aligned);
  *  - every function returns 0 on success, <0 on error; regt_last_error() returns a
  *    thread-local message for the last failure on the calling thread;
- *  - work is enqueued on `stream`; nothing synchronises the device except the two
- *    regt_*_plan_build calls (they return counts to the host);
+ *  - work is enqueued on `stream`; nothing synchronises the device except the
+ *    regt_gcn_plan_build / regt_cheb_plan_build calls (they return counts to the host);
  *  - thread-compatible: no global state except the thread-local error string.
  */
 #ifndef REGT_B200_H
@@ -194,9 +194,44 @@ int regt_head_forward(const regt_args* a);
  * (g.head_*, loss) is then finalised by the regt_cell_backward that must follow, beside the cell
  * kernel on a second stream.                                                             */
 int regt_head_backward(const regt_args* a);
-/* autograd of the cell (run.py:190): all parameter gradients of the cell.  No gradient
- * wrt x is produced (x is data in the reference: batch.x never requires grad).          */
+/* autograd of the cell (run.py:190): all parameter gradients of the cell.  The gradient wrt x
+ * is not part of this call (x is data in the reference's loop: batch.x never requires grad);
+ * regt_cell_backward_x below computes it from what this call leaves in the workspace.    */
 int regt_cell_backward(const regt_args* a);
+
+/* ---- gradient wrt x (csrc/input_grad.cu) ----------------------------------------------
+ * What autograd gives PyG's modules for an x that requires grad (saliency, input perturbation,
+ * an upstream layer feeding models.utils.TGCN).  Per row (b, n, t) the gate-gradient plane
+ * D = [Dz | Dr | Dc | Dpre] of the cell backward is contracted with the collapsed weights into
+ *   dS = Dzr (A_zr W_zr) + Dc (A_c W_c),  dXd = Dpre M0,  dU_seg = Dpre M1[r_seg]  (F wide each),
+ * then  dx = dXd + A_hat^T dS + sum_r C_r^T dU  (the graphs are directed: neither transpose
+ * equals its operator).  The transposed operator is one CSR by input node j over the stacked
+ * source rows [dXd (N) | dS (N) | dU (nseg)] of a snapshot; row j holds, in this fixed order, the
+ * identity entry (dXd row j, weight 1), then the A_hat entries with g_col = j, then the regional
+ * entries with c_col = j, each group in canonical CSR order: sums are deterministic.          */
+typedef struct regt_xgrad_plan {
+  int32_t N;              /* nodes                                                          */
+  int32_t nnz;            /* N + nnz_gcn + nnz_cheb                                         */
+  int32_t n_src;          /* 2 N + nseg: stacked source rows of one snapshot                */
+  int32_t _pad;
+  const int32_t* rowptr;  /* [N+1]                                                          */
+  const int32_t* col;     /* [nnz] stacked source row                                       */
+  const float* val;       /* [nnz] 1 (identity), g_val or c_val of the entry                */
+} regt_xgrad_plan;
+
+/* Built once per static graph from a regt_graph_plan (stable counting sort by column, on the
+ * device; all sizes come from the plan, so it does not synchronise).  Outputs: rowptr [N+1],
+ * col / val [N + nnz_gcn + nnz_cheb].                                                         */
+size_t regt_xgrad_plan_workspace_bytes(const regt_graph_plan* p);
+int regt_xgrad_plan_build(const regt_graph_plan* p, int32_t* rowptr, int32_t* col, float* val, void* workspace,
+                          size_t workspace_bytes, regt_stream_t stream);
+/* d_x [B,N,F,T] f32 (overwritten) = gradient wrt x of the loss whose gradients the preceding
+ * regt_cell_backward (same args, same workspace) consumed.  Reads the workspace, allocates nothing:
+ * scratch is at least regt_cell_backward_x_scratch_bytes(a, xp) bytes (256-byte aligned).
+ * Refused: precision bf16 (its kernels keep no D plane), region shards (x_rows != N: halo rows
+ * belong to other ranks), inference = 1 (no backward ran).                                    */
+size_t regt_cell_backward_x_scratch_bytes(const regt_args* a, const regt_xgrad_plan* xp);
+int regt_cell_backward_x(const regt_args* a, const regt_xgrad_plan* xp, float* d_x, void* scratch, size_t scratch_bytes);
 
 /* ---- exchange step over NVLink peer memory (csrc/peer.cu) ------------------------------
  * SURVEY 8e: one sum all-reduce of the flat shared-weight gradient buffer per step.  The

@@ -15,6 +15,8 @@ int cell_forward_g(const regt_args* a, const Layout& L, cudaStream_t st);
 int cell_backward_g(const regt_args* a, const Layout& L, cudaStream_t st);
 int cell_forward_f(const regt_args* a, const Layout& L, cudaStream_t st);
 int cell_backward_f(const regt_args* a, const Layout& L, cudaStream_t st);
+size_t cell_backward_x_scratch_bytes(const regt_args* a, const regt_xgrad_plan* xp);
+int cell_backward_x(const regt_args* a, const Layout& L, const regt_xgrad_plan* xp, float* d_x, void* scratch, cudaStream_t st);
 
 Layout make_layout(const regt_args* a, void* base) {
   Layout L{};
@@ -157,6 +159,36 @@ extern "C" int regt_cell_backward(const regt_args* a) {
     return cell_f_usable(a) ? cell_backward_f(a, L, st) : cell_backward_g(a, L, st);
   }
   return cell_backward_tc(a, L, st);
+}
+
+static int validate_x(const regt_args* a, const regt_xgrad_plan* xp, const char* who) {
+  REGT_CHECK(a != nullptr, "%s: args is NULL", who);
+  REGT_CHECK(a->precision != REGT_PREC_BF16, "%s: precision bf16 keeps no gate-gradient plane; use fp32 or tf32x3", who);
+  REGT_CHECK(a->x_rows == 0 || a->x_rows == a->N,
+             "%s: region shards (x_rows=%d != N=%d) are not supported: their halo rows belong to other ranks", who, a->x_rows, a->N);
+  REGT_CHECK(!a->inference, "%s: the forward ran with inference=1 (no activations were saved)", who);
+  if (validate(a, who)) return -1;
+  REGT_CHECK(xp && xp->N == a->N && xp->n_src == 2 * a->N + a->plan.nseg && xp->rowptr && xp->col && xp->val,
+             "%s: transposed plan missing or built for another graph", who);
+  return 0;
+}
+
+extern "C" size_t regt_cell_backward_x_scratch_bytes(const regt_args* a, const regt_xgrad_plan* xp) {
+  if (!a || !xp) return 0;
+  return cell_backward_x_scratch_bytes(a, xp);
+}
+
+extern "C" int regt_cell_backward_x(const regt_args* a, const regt_xgrad_plan* xp, float* d_x, void* scratch,
+                                    size_t scratch_bytes) {
+  if (validate_x(a, xp, "regt_cell_backward_x")) return -1;
+  REGT_CHECK(d_x, "regt_cell_backward_x: d_x is NULL");
+  REGT_CHECK(scratch && scratch_bytes >= cell_backward_x_scratch_bytes(a, xp), "regt_cell_backward_x: scratch missing or too small");
+  if (a->precision == REGT_PREC_TF32X3)
+    REGT_CHECK(a->H % 32 == 0, "precision tf32x3 needs hidden %% 32 == 0 (got %d); use precision fp32", a->H);
+  Layout L = make_layout(a, a->workspace);
+  cudaStream_t st = (cudaStream_t)a->stream;
+  prof_mark("<begin>", st);
+  return cell_backward_x(a, L, xp, d_x, scratch, st);
 }
 
 extern "C" int regt_head_forward(const regt_args* a) {

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.normpath(os.path.join(HERE, "..", ".."))
 OUT = os.path.join(HERE, "..", "lib")
-SOURCES = ["api_core.cu", "plan.cu", "spmm.cu", "weights.cu", "cell.cu", "cell_g.cu", "cell_f.cu", "head.cu", "head_f.cu", "api.cu", "cell_tc.cu", "head_tc.cu", "gemm_tc.cu", "gemm_tma.cu", "peer.cu", "loop.cu", "umma_selftest.cu"]
+SOURCES = ["api_core.cu", "plan.cu", "spmm.cu", "weights.cu", "cell.cu", "cell_g.cu", "cell_f.cu", "head.cu", "head_f.cu", "input_grad.cu", "api.cu", "cell_tc.cu", "head_tc.cu", "gemm_tc.cu", "gemm_tma.cu", "peer.cu", "loop.cu", "umma_selftest.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-I", os.path.join(ROOT, "include"), "-I", HERE]
 

@@ -251,9 +251,83 @@ __global__ void k_seg_ptr(const int32_t* __restrict__ rowptr, const int32_t* __r
   seg_ptr[n] = (k < nnz) ? segid[k] : *nseg;
 }
 
+// ---------------- transposed operator of the input gradient (regt_xgrad_plan) ---------------
+// row_of[e] = i for every entry e in [ptr[i], ptr[i+1]): destination row of an A_hat entry, segment of a regional entry
+__global__ void k_row_of(const int32_t* __restrict__ ptr, int n, int32_t* __restrict__ row_of) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  for (int e = ptr[i]; e < ptr[i + 1]; ++e) row_of[e] = i;
+}
+// entry ids: [0, N) identity, [N, N + ng) A_hat entries, then the regional entries; key = the input node they read
+__global__ void k_xg_keys(int N, int ng, int nc, const int32_t* __restrict__ g_col, const int32_t* __restrict__ c_col,
+                          int32_t* __restrict__ key) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= N + ng + nc) return;
+  key[i] = i < N ? i : (i < N + ng ? g_col[i - N] : c_col[i - N - ng]);
+}
+__global__ void k_xg_fill(const int32_t* __restrict__ sorted, int N, int ng, int nc, const int32_t* __restrict__ g_dst,
+                          const float* __restrict__ g_val, const int32_t* __restrict__ c_seg, const float* __restrict__ c_val,
+                          int32_t* __restrict__ col, float* __restrict__ val) {
+  int k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= N + ng + nc) return;
+  const int id = sorted[k];
+  if (id < N) {
+    col[k] = id;
+    val[k] = 1.0f;
+  } else if (id < N + ng) {
+    col[k] = N + g_dst[id - N];
+    val[k] = g_val[id - N];
+  } else {
+    col[k] = 2 * N + c_seg[id - N - ng];
+    val[k] = c_val[id - N - ng];
+  }
+}
+
 }  // namespace regt
 
 using namespace regt;
+
+extern "C" size_t regt_xgrad_plan_workspace_bytes(const regt_graph_plan* p) {
+  if (!p) return 0;
+  const size_t n = (size_t)p->N + p->nnz_gcn + p->nnz_cheb;
+  return 3 * align_up(n * 4, 256) + align_up((size_t)(p->N + 1) * 4, 256) + align_up((size_t)p->nnz_gcn * 4 + 4, 256) +
+         align_up((size_t)p->nnz_cheb * 4 + 4, 256) + 256;
+}
+
+extern "C" int regt_xgrad_plan_build(const regt_graph_plan* p, int32_t* rowptr, int32_t* col, float* val, void* workspace,
+                                     size_t workspace_bytes, regt_stream_t stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  REGT_CHECK(p && rowptr && col && val, "xgrad_plan: NULL argument");
+  REGT_CHECK(p->N > 0 && p->nnz_gcn >= 0 && p->nnz_cheb >= 0 && p->nseg >= 0 &&
+                 (long long)p->N + p->nnz_gcn + p->nnz_cheb < (1ll << 31) && 2ll * p->N + p->nseg < (1ll << 31),
+             "xgrad_plan: bad sizes");
+  REGT_CHECK(p->nnz_gcn == 0 || (p->g_rowptr && p->g_col && p->g_val), "xgrad_plan: gcn CSR missing");
+  REGT_CHECK(p->nnz_cheb == 0 || (p->seg_eptr && p->c_col && p->c_val), "xgrad_plan: regional CSR missing");
+  REGT_CHECK(workspace && workspace_bytes >= regt_xgrad_plan_workspace_bytes(p), "xgrad_plan: workspace too small");
+  const int N = p->N, ng = p->nnz_gcn, nc = p->nnz_cheb, n = N + ng + nc;
+  Carver c(workspace);
+  int32_t* key = c.take<int32_t>(n);
+  int32_t* tmp = c.take<int32_t>(n);
+  int32_t* sorted = c.take<int32_t>(n);
+  int32_t* cnt = c.take<int32_t>(N + 1);
+  int32_t* g_dst = c.take<int32_t>(ng + 1);
+  int32_t* c_seg = c.take<int32_t>(nc + 1);
+  if (ng > 0) {
+    k_row_of<<<cdiv(N, 256), 256, 0, st>>>(p->g_rowptr, N, g_dst);
+    REGT_LAUNCH_CHECK();
+  }
+  if (nc > 0) {
+    k_row_of<<<cdiv(p->nseg, 256), 256, 0, st>>>(p->seg_eptr, p->nseg, c_seg);
+    REGT_LAUNCH_CHECK();
+  }
+  k_xg_keys<<<cdiv(n, 256), 256, 0, st>>>(N, ng, nc, p->g_col, p->c_col, key);
+  REGT_LAUNCH_CHECK();
+  // stable by entry id: identity, then A_hat entries, then regional entries, each in canonical CSR order
+  if (bucket_sort(key, n, N, rowptr, sorted, cnt, tmp, st)) return -1;
+  k_xg_fill<<<cdiv(n, 256), 256, 0, st>>>(sorted, N, ng, nc, g_dst, p->g_val, c_seg, p->c_val, col, val);
+  REGT_LAUNCH_CHECK();
+  return 0;
+}
 
 extern "C" size_t regt_plan_workspace_bytes(int64_t N, int64_t E) {
   // generous: ~16 int32/float arrays of (E+N) entries + a few of N

@@ -26,6 +26,11 @@ class GraphPlan(C.Structure):
                 ("rseg_ptr", vp), ("rseg_list", vp)]
 
 
+class XgradPlan(C.Structure):
+    _fields_ = [("N", C.c_int32), ("nnz", C.c_int32), ("n_src", C.c_int32), ("_pad", C.c_int32),
+                ("rowptr", vp), ("col", vp), ("val", vp)]
+
+
 class Params(C.Structure):
     _fields_ = [("attention", vp), ("conv_w", vp * 3), ("conv_b", vp * 3), ("lin_w", vp * 3), ("lin_b", vp * 3),
                 ("cheb_w0", vp), ("cheb_w1", vp), ("cheb_b", vp), ("comb_w", vp), ("comb_b", vp),
@@ -51,6 +56,8 @@ EXPORTS = ["regt_version", "regt_last_error", "regt_launch_count", "regt_plan_wo
            "regt_gcn_plan_build", "regt_cheb_plan_build", "regt_spmm_f8", "regt_spmm_partition_capacity", "regt_spmm_partition",
            "regt_spmm_f8_blocked", "regt_gather_rows", "regt_scatter_rows", "regt_workspace_bytes",
            "regt_cell_forward", "regt_head_forward", "regt_head_backward", "regt_cell_backward",
+           "regt_xgrad_plan_workspace_bytes", "regt_xgrad_plan_build", "regt_cell_backward_x_scratch_bytes",
+           "regt_cell_backward_x",
            "regt_profile", "regt_profile_begin", "regt_profile_read",
            "regt_comm_region_bytes", "regt_comm_data_offset", "regt_comm_alloc", "regt_comm_free", "regt_comm_export",
            "regt_comm_import", "regt_comm_unimport", "regt_peer_allreduce_f32", "regt_peer_push_max_floats", "regt_comm_error",
@@ -108,6 +115,14 @@ def load() -> C.CDLL:
         fn = getattr(lib, name)
         fn.restype = C.c_int
         fn.argtypes = [C.POINTER(Args)]
+    lib.regt_xgrad_plan_workspace_bytes.restype = C.c_size_t
+    lib.regt_xgrad_plan_workspace_bytes.argtypes = [C.POINTER(GraphPlan)]
+    lib.regt_xgrad_plan_build.restype = C.c_int
+    lib.regt_xgrad_plan_build.argtypes = [C.POINTER(GraphPlan), vp, vp, vp, vp, C.c_size_t, vp]
+    lib.regt_cell_backward_x_scratch_bytes.restype = C.c_size_t
+    lib.regt_cell_backward_x_scratch_bytes.argtypes = [C.POINTER(Args), C.POINTER(XgradPlan)]
+    lib.regt_cell_backward_x.restype = C.c_int
+    lib.regt_cell_backward_x.argtypes = [C.POINTER(Args), C.POINTER(XgradPlan), vp, vp, C.c_size_t]
     lib.regt_profile.restype = C.c_int
     lib.regt_profile.argtypes = [C.c_int, vp]
     lib.regt_profile_begin.restype = C.c_int

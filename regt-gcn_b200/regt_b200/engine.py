@@ -180,6 +180,33 @@ def run_backward(st: StepState, grads: Dict[str, Optional[torch.Tensor]], d_out:
         _lib.check(lib.regt_cell_backward(C.byref(a)), "regt_cell_backward")
 
 
+def run_backward_x(st: StepState) -> torch.Tensor:
+    """gradient wrt x [B,N,F,T] of the loss whose gradients the preceding ``run_backward`` on ``st`` consumed."""
+    lib = _lib.load()
+    a = st.args
+    plan = st.keep[1]
+    x = st.keep[0]
+    with torch.cuda.device(x.device):
+        xp = plan.xgrad_struct()
+        nbytes = lib.regt_cell_backward_x_scratch_bytes(C.byref(a), C.byref(xp))
+        scratch = torch.empty(nbytes, device=x.device, dtype=torch.uint8)
+        d_x = torch.empty_like(x)
+        a.stream = _stream()
+        _lib.check(lib.regt_cell_backward_x(C.byref(a), C.byref(xp), d_x.data_ptr(), scratch.data_ptr(), nbytes),
+                   "regt_cell_backward_x")
+    return d_x
+
+
+def _check_input_grad(precision: int, plan: GraphPlanTensors, x: torch.Tensor) -> None:
+    """refuse, at the forward, an x that requires grad where the kernels cannot differentiate through it."""
+    if precision == _lib.PREC_BF16:
+        raise RuntimeError("regt_b200: the gradient wrt x is not available in precision bf16 (its kernels keep no "
+                           "gate-gradient plane); use precision fp32 or tf32x3")
+    if x.shape[1] != plan.N:
+        raise RuntimeError("regt_b200: the gradient wrt x is not available on region shards (x has halo rows owned by "
+                           "other ranks)")
+
+
 class _ModelFn(torch.autograd.Function):
     """(x, *params) -> (out, out_hidden); everything runs in the C-ABI kernels."""
 
@@ -215,15 +242,19 @@ class _ModelFn(torch.autograd.Function):
         if ctx.h_ext_grad:
             d_h_ext = torch.empty(st.args.B, st.args.N, st.args.T, st.args.H, device=st.out_hidden.device)
         run_backward(st, grads, d_out, d_hidden, False, ctx.head, d_h_ext)
+        d_x = run_backward_x(st) if ctx.needs_input_grad[6] else None
         ctx.st = None
-        return (None, None, None, None, None, None, None, d_h_ext) + tuple(grads[k] for k in ctx.keys)
+        return (None, None, None, None, None, None, d_x, d_h_ext) + tuple(grads[k] for k in ctx.keys)
 
 
 def model_apply(mode: int, precision: int, plan: GraphPlanTensors, H: int, O: int, x: torch.Tensor,
                 params: Dict[str, torch.Tensor], h_ext: Optional[torch.Tensor] = None, head: bool = True):
     keys = keys_for(mode, head)
-    needs_grad = torch.is_grad_enabled() and (any(params[k].requires_grad for k in keys) or
-                                              (h_ext is not None and h_ext.requires_grad))
+    x_grad = torch.is_grad_enabled() and x.requires_grad
+    if x_grad:
+        _check_input_grad(precision, plan, x)
+    needs_grad = x_grad or torch.is_grad_enabled() and (any(params[k].requires_grad for k in keys) or
+                                                        (h_ext is not None and h_ext.requires_grad))
     if not needs_grad:
         # run.py:208-216 / predict.py:151-172 (torch.no_grad()): forward only -- the fused kernels keep no activations
         st = build_state(mode, precision, plan, x, H, O, params, None, h_ext, head, inference=True)

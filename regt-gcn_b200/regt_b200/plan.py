@@ -27,6 +27,7 @@ class GraphPlanTensors:
         self.R = 1
         self.nnz_gcn = self.nnz_cheb = self.nseg = 0
         self.t = {}
+        self.xg = None          # transposed operator of the input gradient (xgrad_struct), built on first use
 
     def c_struct(self) -> _lib.GraphPlan:
         p = _lib.GraphPlan()
@@ -34,6 +35,33 @@ class GraphPlanTensors:
         for k in ("g_rowptr", "g_col", "g_val", "c_rowptr", "c_col", "c_val", "c_reg", "seg_ptr", "seg_eptr",
                   "seg_reg", "seg_node", "rseg_ptr", "rseg_list"):
             setattr(p, k, _ptr(self.t.get(k)))
+        return p
+
+    def xgrad_struct(self) -> _lib.XgradPlan:
+        """the ``regt_xgrad_plan`` of this graph (A_hat^T and the regional operators transposed, one CSR by input node).
+        Built on the first backward that asks for the gradient wrt x and kept with the plan, so the identity and the
+        content entries of the plan cache both reach it."""
+        if self.xg is None:
+            if torch.cuda.is_current_stream_capturing():
+                raise RuntimeError("regt_b200: the transposed graph operator of the input gradient is built on the first "
+                                   "backward that needs it; run one such backward outside CUDA-graph capture first")
+            lib = _lib.load()
+            ps = self.c_struct()
+            n = self.N + self.nnz_gcn + self.nnz_cheb
+            dev = self.device
+            rowptr = torch.empty(self.N + 1, device=dev, dtype=torch.int32)
+            col = torch.empty(n, device=dev, dtype=torch.int32)
+            val = torch.empty(n, device=dev, dtype=torch.float32)
+            wsb = lib.regt_xgrad_plan_workspace_bytes(C.byref(ps))
+            with torch.cuda.device(dev):
+                ws = torch.empty(wsb, device=dev, dtype=torch.uint8)
+                rc = lib.regt_xgrad_plan_build(C.byref(ps), rowptr.data_ptr(), col.data_ptr(), val.data_ptr(), ws.data_ptr(),
+                                               wsb, _stream_ptr())
+                _lib.check(rc, "regt_xgrad_plan_build")
+            self.xg = dict(nnz=n, n_src=2 * self.N + self.nseg, rowptr=rowptr, col=col, val=val)
+        p = _lib.XgradPlan()
+        p.N, p.nnz, p.n_src = self.N, self.xg["nnz"], self.xg["n_src"]
+        p.rowptr, p.col, p.val = (self.xg[k].data_ptr() for k in ("rowptr", "col", "val"))
         return p
 
 
