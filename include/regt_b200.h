@@ -285,21 +285,15 @@ int regt_profile_read(char* names, size_t names_len, float* ms, int max_n);
 
 /* ---- TEST HOOKS ------------------------------------------------------------------------------------------------
  * Not part of the reference-facing boundary: no reference call site maps to these.  They expose the internal
- * tensor-core building blocks (3xTF32 GEMMs of gemm_tc.cu / gemm_tma.cu, the hand-built UMMA operand layouts of
+ * tensor-core building blocks (3xTF32 GEMMs of gemm_tma.cu, the hand-built UMMA operand layouts of
  * tc_common.cuh) to tests/test_gpu_gemm.py and tests/test_gpu_umma.py so that each is pinned against an fp64 matmul on
  * its own.  Integrators do not bind them.
- *   gemm_nt*:  C[M][N]   = A[M][K] . Bt[N][K]^T                       (scratch: 2 * ceil128(N) * ceil32(K) floats)
- *   gemm_tn*:  Cp[z]     = sum over the rows of split z of A[r][:K]^T . B[r][:N]      (+ a second, 32-wide operand B2)
+ *   gemm_nt_tma:  C[M][N]   = A[M][K] . Bt[N][K]^T                    (scratch: 2 * ceil128(N) * ceil32(K) floats)
+ *   gemm_tn_tma:  Cp[z]     = sum over the rows of split z of A[r][:K]^T . B[r][:N]      (+ a second, 32-wide operand B2)
  *   gemm_tn_multi: the four-gate-block form of the cell backward, A = D [M][4H]
  *   gemm_kt: the same contraction over transposed tiles A^T [ntile][4H][128], B^T [ntile][H][128], F^T [ntile][32][128]
  *            (what the fused cell backward of cell_f.cu writes); H = 128 or 64
  *   umma_selftest: one 128 x N x K MMA on operand tiles written by CUDA-core threads (fmt 1 = bf16, 2 = tf32)         */
-int regt_debug_gemm_nt(const float* A, int64_t lda, const float* Bt, int64_t ldb, float* C, int64_t ldc, int64_t M,
-                       int32_t N, int32_t K, regt_stream_t stream);
-int regt_debug_gemm_tn(const float* A, int64_t lda, const float* B, int64_t ldb, float* Cp, int64_t M, int32_t K,
-                       int32_t N, int32_t splits, regt_stream_t stream);
-int regt_debug_gemm_tn2(const float* A, int64_t lda, const float* B, int64_t ldb, float* Cp, int64_t M, int32_t K,
-                        int32_t N, int32_t splits, const float* B2, int64_t ldb2, float* Cp2, regt_stream_t stream);
 int regt_debug_gemm_nt_tma(const float* A, int64_t lda, const float* Bt, int64_t ldb, float* C, int64_t ldc, int64_t M,
                            int32_t N, int32_t K, float* scratch, regt_stream_t stream);
 int regt_debug_gemm_tn_tma(const float* A, int64_t lda, const float* B, int64_t ldb, float* Cp, int64_t M, int32_t K,

@@ -6,25 +6,13 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.normpath(os.path.join(HERE, "..", ".."))
 OUT = os.path.join(HERE, "..", "lib")
-SOURCES = ["api_core.cu", "plan.cu", "spmm.cu", "weights.cu", "cell.cu", "cell_g.cu", "cell_f.cu", "head.cu", "head_f.cu", "input_grad.cu", "api.cu", "cell_tc.cu", "head_tc.cu", "gemm_tc.cu", "gemm_tma.cu", "peer.cu", "loop.cu", "umma_selftest.cu"]
+SOURCES = ["api_core.cu", "plan.cu", "spmm.cu", "weights.cu", "cell.cu", "cell_g.cu", "cell_f.cu", "head.cu", "head_f.cu", "input_grad.cu", "api.cu", "cell_tc.cu", "head_tc.cu", "gemm_tma.cu", "peer.cu", "loop.cu", "umma_selftest.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-I", os.path.join(ROOT, "include"), "-I", HERE]
 
 
 def lib_path() -> str:
     return os.path.normpath(os.path.join(OUT, "libregt_b200.so"))
-
-
-def build_variant(name: str, defs) -> str:
-    """experiment builds: lib/variants/<name>/libregt_b200.so compiled with extra -D switches
-    (select at run time with REGT_B200_LIB=<path>)."""
-    out = os.path.join(OUT, "variants", name)
-    os.makedirs(out, exist_ok=True)
-    nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-    srcs = [os.path.join(HERE, s) for s in SOURCES]
-    target = os.path.join(out, "libregt_b200.so")
-    subprocess.check_call([nvcc, *NVCC_FLAGS, *[f"-D{d}" for d in defs], "-shared", "-o", target, *srcs, "-lcudart", "-lcuda"])
-    return target
 
 
 def build(verbose: bool = False, force: bool = False) -> str:

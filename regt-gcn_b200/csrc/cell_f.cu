@@ -29,19 +29,6 @@
 
 #include "cell_tc.cuh"
 
-// build-time switch (tools/build_variants.py, A/B on B200): 1 = h of the next step is computed under the candidate MMAs and
-// waits in registers (32 more live registers per epilogue thread), 0 = computed after them
-#ifndef REGT_F_PRE
-#define REGT_F_PRE 1
-#endif
-// timing experiments only (results are wrong with either): what the recompute of h and the E0 stores cost
-#ifndef REGT_XP_SKIP_H16
-#define REGT_XP_SKIP_H16 0
-#endif
-#ifndef REGT_XP_SKIP_E0_STORES
-#define REGT_XP_SKIP_E0_STORES 0
-#endif
-
 namespace regt {
 using namespace tc;
 
@@ -89,12 +76,7 @@ struct FCfg {
   static constexpr int WP_TILE = 3 * 2 * SW_TILE;
   static constexpr int FIXED = ((TAIL + 1023) & ~1023) + 2 * S_TILE + 4 * 8 * HH * 4 + XU_TILE + WP_TILE;   // + M1 cache (M1C, declared below)
   static constexpr int NS_FIT = (SMEM_MAX - 2048 - FIXED) / STAGE;
-#ifdef REGT_F_NS_CAP
-  static constexpr int NS0 = NS_FIT < 2 * NSTEP ? NS_FIT : 2 * NSTEP;
-  static constexpr int NS = NS0 < REGT_F_NS_CAP ? NS0 : REGT_F_NS_CAP;   // TEST HOOK: shallower ring
-#else
   static constexpr int NS = NS_FIT < 2 * NSTEP ? NS_FIT : 2 * NSTEP;   // ring depth
-#endif
   static constexpr int SMEM = 1024 + NS * STAGE + FIXED;
   static constexpr int CWF = HH / 4;                  // columns per epilogue thread
   static constexpr int M1C = 4 * REGT_F * HH * 4;     // bytes of the 4-slot cache of per-region M1 blocks
@@ -642,17 +624,12 @@ __global__ void __launch_bounds__(NTHR, 1) k_cell_fwd_f(FArgs a) {
       tc_fence_before();
       mbar_arrive(&bar_a2);
       F_TS(0, 4)
-#if REGT_F_PRE
       if (s + 1 < S) Pcompute(s + 1);      // under the candidate MMAs (h of the next step waits in registers)
-#endif
       // ---- candidate GEMM done: A is free -> h of the next step goes in first (its z-gate MMAs start), then E2 under them ----
       F_TS(0, 5)
       mbar_wait(&bar_c, ph);
       tc_fence_after();
       F_TS(0, 6)
-#if !REGT_F_PRE
-      if (s + 1 < S) Pcompute(s + 1);
-#endif
       if (s + 1 < S) Pstore();
       F_TS(0, 7)
 #pragma unroll
@@ -789,18 +766,9 @@ __global__ void __launch_bounds__(NTHR, 1) k_cell_fwd_f(FArgs a) {
 // Lane = row makes every store of one column a contiguous 128-byte line -- and a [column][row] tile is exactly the K-major
 // operand the row contraction wants (K = rows): gemm_tma.cu reads these tiles with plain TMA boxes and no transposing
 // converters.  v2 issued those lines as 192 scalar st.global per thread and step: 8.5 of the 17.7 us of phase E0 were spent
-// stalled on the store path (timing experiment REGT_XP_SKIP_E0_STORES, tools/f_phases.py).  Staging the lines in per-warp
+// stalled on the store path (timed with the stores removed, tools/f_phases.py).  Staging the lines in per-warp
 // shared-memory slots for the bulk-copy engine (cp.async.bulk shared -> global) measured slower (33.3 vs 29.8 us per step: a put
 // waits for the engine to have read the slot used two puts ago); what did help is in profiles/r02_fused_phases.md.
-#ifndef REGT_F_PREFETCH
-#define REGT_F_PREFETCH 2      // L2 prefetch of the next step's planes by the producer lane: 0 off, 1 a step ahead, 2 late (see k_cell_bwd_f)
-#endif
-#ifndef REGT_F_LDCS
-#define REGT_F_LDCS 1          // backward: Z and H~ (read once) with the streaming load operator
-#endif
-#ifndef REGT_F_STCS
-#define REGT_F_STCS 1          // backward plane stores with the streaming (evict-first) cache operator
-#endif
 template <int HH>
 struct BCfg {   // shared-memory plan of the backward: ring | resident tail | M1 cache
   using C = FCfg<HH>;
@@ -981,23 +949,13 @@ __global__ void __launch_bounds__(NTHR, 1) k_cell_bwd_f(FArgs a) {
         float4 zq[2], rq[2], cq[2], gq[2];
 #pragma unroll
         for (int i = 0; i < 2; ++i) {
-#if REGT_F_LDCS
-          zq[i] = __ldcs(reinterpret_cast<const float4*>(zt + piece(r, c + 4 * i)));
+          zq[i] = __ldcs(reinterpret_cast<const float4*>(zt + piece(r, c + 4 * i)));   // Z and H~ are read once: streaming loads
           cq[i] = __ldcs(reinterpret_cast<const float4*>(ct + piece(r, c + 4 * i)));
-#else
-          zq[i] = __ldg(reinterpret_cast<const float4*>(zt + piece(r, c + 4 * i)));
-          cq[i] = __ldg(reinterpret_cast<const float4*>(ct + piece(r, c + 4 * i)));
-#endif
           rq[i] = __ldg(reinterpret_cast<const float4*>(rt + piece(r, c + 4 * i)));
           gq[i] = __ldg(reinterpret_cast<const float4*>(gt + piece(r, c + 4 * i)));
         }
         float h[8];
-#if REGT_XP_SKIP_H16
-#pragma unroll
-        for (int i = 0; i < 8; ++i) h[i] = consts[C::C_C0 + c + i] + f.x[i & 7];
-#else
         hcols<HH, 8>(a, consts, mc, ri, f, t, c, h);
-#endif
         if (j == 0) { F_TS(1, 9) }
         float dc[8], gz[8];
         float dpc = 0.f;
@@ -1022,18 +980,10 @@ __global__ void __launch_bounds__(NTHR, 1) k_cell_bwd_f(FArgs a) {
             gz[i + e] = gg * z[e];
             DZ(8 * j + i + e) = dzv;
             if (!(hh > 0.f)) ng |= 1u << (i + e);
-#if !REGT_XP_SKIP_E0_STORES
             o_h[(i + e) * 32] = hh;                                           // re-read in E1: not streamed
-#if REGT_F_STCS
-            __stcs(o_hr + (i + e) * 32, hh * rg[e]);
+            __stcs(o_hr + (i + e) * 32, hh * rg[e]);                          // the other planes: streaming (evict-first) stores
             __stcs(o_dz + (i + e) * 32, dzv);
             __stcs(o_dc + (i + e) * 32, dc[i + e]);
-#else
-            o_hr[(i + e) * 32] = hh * rg[e];
-            o_dz[(i + e) * 32] = dzv;
-            o_dc[(i + e) * 32] = dc[i + e];
-#endif
-#endif
           }
         }
         neg |= ng << (8 * j);
@@ -1089,11 +1039,7 @@ __global__ void __launch_bounds__(NTHR, 1) k_cell_bwd_f(FArgs a) {
           for (int e = 0; e < 4; ++e) {
             dr[i + e] = v[i + e] * hh[i + e] * rg[e] * (1.0f - rg[e]);
             v[i + e] *= rg[e];
-#if REGT_F_STCS
             __stcs(o_dr + (i + e) * 32, dr[i + e]);
-#else
-            o_dr[(i + e) * 32] = dr[i + e];
-#endif
           }
         }
         st_f32x8(t1c + c, v);
@@ -1122,11 +1068,7 @@ __global__ void __launch_bounds__(NTHR, 1) k_cell_bwd_f(FArgs a) {
         for (int i = 0; i < 8; ++i) {
           float d = v[i] + u[i];
           if (a.mode == REGT_MODE_REGIONAL && ((neg >> (8 * j + i)) & 1u)) d *= 0.01f;
-#if REGT_F_STCS
           __stcs(o_dh + i * 32, d);
-#else
-          o_dh[i * 32] = d;
-#endif
         }
       }
       tc_fence_before();
@@ -1163,18 +1105,12 @@ __global__ void __launch_bounds__(NTHR, 1) k_cell_bwd_f(FArgs a) {
       if (t == 0) bulk_prefetch_l2(reinterpret_cast<const uint8_t*>(a.G) + (size_t)qt * TB, TB);
       prefetch_feats(a, t, qt);
     };
-    // REGT_F_PREFETCH 1: a whole step ahead (as the weight stages are issued) -- measured harmful: at 148 x 576 KB of plane
-    // traffic per step the lines are evicted again before their step comes and DRAM reads double (ncu: 7.6 GB against 3.3 GB
-    // per launch).  2 (default): when the dHR MMAs of step s complete (bar_1), i.e. 6-8 us before E0 of step s + 1 reads them.
-#if REGT_F_PREFETCH == 1
-    if (S > 0) prefetch_step(0);
-#endif
+    // L2 prefetch of the next step's planes when the dHR MMAs of step s complete (bar_1), i.e. 6-8 us before E0 of step s + 1
+    // reads them.  A whole step ahead (as the weight stages are issued) measured harmful: at 148 x 576 KB of plane traffic per
+    // step the lines are evicted again before their step comes and DRAM reads double (ncu: 7.6 GB against 3.3 GB per launch).
     long long gs = 0;
     for (int s = 0; s < S; ++s) {
-#if REGT_F_PREFETCH == 1
-      if (s + 1 < S) prefetch_step(s + 1);
-#endif
-      bool pf_pending = (REGT_F_PREFETCH == 2) && (s + 1 < S);
+      bool pf_pending = s + 1 < S;
       for (int i = 0; i < C::NSTEP; ++i, ++gs) {
         const int st = (int)(gs % NS);
         if (gs >= NS) {

@@ -1,5 +1,5 @@
 // REGT_PREC_TF32X3 for any hidden width that is a multiple of 32: the regional temporal GCN cell with
-// every H x H contraction on the sm_100a tensor cores through the generic 3xTF32 GEMMs of gemm_tc.cu
+// every H x H contraction on the sm_100a tensor cores through the generic 3xTF32 GEMMs of gemm_tma.cu
 // (fp32-equivalent accuracy), forward AND backward.  Unlike the fused H = 64 kernels of cell_tc.cu the
 // gate pre-activations make one round trip through HBM, which is what lets the same code serve H = 128
 // (configs 4, 5) and H = 256 (configs 1, 3): no weight set has to fit one SM's shared memory or TMEM.
@@ -32,18 +32,13 @@ int launch_prep(const regt_args* a, const Layout& L, cudaStream_t st);
 int launch_chain(const regt_args* a, const Layout& L, cudaStream_t st);
 int launch_spmm_rows(const int32_t* rowptr, const int32_t* col, const float* val, const float* x, float* y, int B,
                      int n_out, int n_in, int width, cudaStream_t st);
-int launch_gemm_nt_tf32x3(const float* A, long long lda, const float* Bt, long long ldb, float* C, long long ldc, long long M,
-                          int N, int K, cudaStream_t st);
-int launch_gemm_tn_tf32x3(const float* A, long long lda, const float* B, long long ldb, float* Cp, long long M, int K, int N,
-                          int splits, cudaStream_t st, const float* B2 = nullptr, long long ldb2 = 0, float* Cp2 = nullptr,
-                          long long c2_split = 0, int relu_b = 0);
 int launch_gemm_nt_tma(const float* A, long long lda, const float* Bt, long long ldb, float* C, long long ldc, long long M, int N,
                        int K, float* scratch, cudaStream_t st);
 int launch_gemm_tn_tma(const float* A, long long lda, long long M, int Ktot, int nseg, const int* seg_k0, const int* seg_b,
                        float* const* seg_C, const float* const* Bs, const long long* ldbs, int N, int splits, const float* B2,
                        long long ldb2, float* C2, long long c2_split, cudaStream_t st, int relu_b);
-int launch_gemm_tn_auto(const float* A, long long lda, const float* B, long long ldb, float* Cp, long long M, int K, int N, int splits,
-                        cudaStream_t st, const float* B2, long long ldb2, float* Cp2, long long c2_split, int relu_b);
+int launch_gemm_tn(const float* A, long long lda, const float* B, long long ldb, float* Cp, long long M, int K, int N, int splits,
+                   cudaStream_t st, const float* B2, long long ldb2, float* Cp2, long long c2_split, int relu_b);
 int launch_attn_accum(const float* Hn, const float* probs, int T, int H, long long BN, float* out_hidden, cudaStream_t st);
 int launch_dprobs(const float* G, const float* Hn, int T, int H, long long BN, float* part, float* dprobs, cudaStream_t st);
 int launch_fwide_wgrads(const regt_args* a, const Layout& L, int splits, cudaStream_t st);
@@ -446,9 +441,9 @@ int cell_backward_g(const regt_args* a, const Layout& L, cudaStream_t st) {
     const long long lds[2] = {H, H};
     if (launch_gemm_tn_tma(L.D, 4 * H, rows, 4 * H, 3, k0, sb, cs, bs, lds, H, splits, L.Feat, 32, pF, fsplit, st, 0)) return -1;
   } else {
-    if (launch_gemm_tn_auto(L.D, 4 * H, L.h, H, pB, rows, 2 * H, H, splits, st, L.Feat, 32, pF, fsplit, 0)) return -1;
-    if (launch_gemm_tn_auto(L.D + 2 * H, 4 * H, L.hR, H, pBh, rows, H, H, splits, st, L.Feat, 32, pF + (size_t)2 * H * 32, fsplit, 0)) return -1;
-    if (launch_gemm_tn_auto(L.D + 3 * H, 4 * H, nullptr, 0, nullptr, rows, H, 0, splits, st, L.Feat, 32, pF + (size_t)3 * H * 32, fsplit, 0)) return -1;
+    if (launch_gemm_tn(L.D, 4 * H, L.h, H, pB, rows, 2 * H, H, splits, st, L.Feat, 32, pF, fsplit, 0)) return -1;
+    if (launch_gemm_tn(L.D + 2 * H, 4 * H, L.hR, H, pBh, rows, H, H, splits, st, L.Feat, 32, pF + (size_t)2 * H * 32, fsplit, 0)) return -1;
+    if (launch_gemm_tn(L.D + 3 * H, 4 * H, nullptr, 0, nullptr, rows, H, 0, splits, st, L.Feat, 32, pF + (size_t)3 * H * 32, fsplit, 0)) return -1;
   }
   if (launch_reduce_splits(pB, L.dB, 2ll * H * H, splits, 0, st)) return -1;
   if (launch_reduce_splits(pBh, L.dB + (size_t)2 * H * H, (long long)H * H, splits, 0, st)) return -1;

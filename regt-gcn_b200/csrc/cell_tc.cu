@@ -4,119 +4,80 @@
 // the 256 epilogue threads owns row r (= TMEM lane r) and one half of the H columns, and walks the
 // periods of its item, so the period-attention sum  sum_t probs[t] * H'_t  stays in registers.
 // Per period:
-//   P   CUDA cores : h = act(X_t M0 + U_t M1[r] + c0)  -> bf16 / tf32(hi,lo) SW128 operand tile in smem
+//   P   CUDA cores : h = act(X_t M0 + U_t M1[r] + c0)  -> bf16 SW128 operand tile in smem
 //   M1  tcgen05.mma: [S_t | h] x Wzr  -> TMEM cols [0,2H)          (weights resident in smem)
 //   E1  CUDA cores : Z,R = sigmoid(. + czr) (tcgen05.ld), save Z,R; h*R -> operand tile
 //   M2  tcgen05.mma: [S_t | h*R] x Wc -> TMEM cols [2H,3H)
 //   E2  CUDA cores : H~ = tanh(. + cc), save H~;  acc += probs[t] * (Z h + (1-Z) H~)
-// Precision: REGT_PREC_BF16 = bf16 operands, fp32 accumulate; REGT_PREC_TF32X3 = three tf32 products
-// (hi*hi + lo*hi + hi*lo) per contraction, fp32-equivalent accuracy.
+// Precision: REGT_PREC_BF16 = bf16 operands, fp32 accumulate.
 // Reference arithmetic replaced: models/utils.py:168-188 + models/RegionalTemporalGCN.py:134-148.
-#include <stdlib.h>
-
 #include "cell_tc.cuh"
 #include "gemm_simt.cuh"
 
-// build-time switches of the pipeline experiments (tools/build_variants.py + tools/gpu_ab.sh; measured on
-// B200 at config 2, profiles/r01_ab_variants.txt; defaults = the fastest measured)
-#ifndef REGT_FWD_PIPE
-#define REGT_FWD_PIPE 0      // 1: software-pipelined forward epilogue (bf16), 0: one phase after the other (A/B: 38 vs 46 us)
-#endif
-#ifndef REGT_BWD_H_UNDER_M2
-#define REGT_BWD_H_UNDER_M2 0  // 1: h of step s+1 is produced while M2 of step s runs (A/B: no gain)
-#endif
-#ifndef REGT_BWD_EARLY_E0
-#define REGT_BWD_EARLY_E0 1  // 1: M1 starts as soon as the Dh tile is stored (A/B: 62.7 vs 65.5 us)
-#endif
-#ifndef REGT_CW
-#define REGT_CW 32
-#endif
+// Pipeline variants measured on B200 at config 2 and dropped (profiles/r01_ab_variants.txt): a software-pipelined forward
+// epilogue (47.0 against 38.5 us), h of step s+1 produced under M2 of step s in the backward (no gain), 16 columns per
+// epilogue thread, one mbarrier arrival per warp.
 
 namespace regt {
 using namespace tc;
 constexpr int F = REGT_F;
-constexpr int CW = REGT_CW;                    // columns owned by one epilogue thread
+constexpr int CW = 32;                     // columns owned by one epilogue thread
 constexpr int NEPI_WARPS = 4 * (64 / CW);  // 4 lane quarters x column groups (hidden = 64)
 constexpr int NEPI = NEPI_WARPS * 32;      // epilogue threads
 constexpr int WARP_MMA = NEPI_WARPS;       // issues every tcgen05.mma (one elected lane) + bulk prefetches
 constexpr int WARP_LOAD = NEPI_WARPS + 1;  // builds the F-wide operand tile of the NEXT period (off the critical path)
 constexpr int NTHREADS = NEPI + 64;
 
-// Gate nonlinearities.  tf32x3 (fp32-parity) mode: exp + reciprocal (2 MUFU each, ~1e-7 relative).
-// bf16 mode: the single-MUFU tanh.approx.f32 (max relative error 2^-11, below the bf16 operand
+// Gate nonlinearities: the single-MUFU tanh.approx.f32 (max relative error 2^-11, below the bf16 operand
 // rounding of 2^-9), sigmoid(v) = 0.5 tanh(v/2) + 0.5 -- the kernel is MUFU-bound otherwise.
-template <int FMT>
 __device__ __forceinline__ float fast_tanh(float v) {
-  if constexpr (FMT == FMT_BF16) {
-    float r;
-    asm("tanh.approx.f32 %0, %1;" : "=f"(r) : "f"(v));
-    return r;
-  } else {
-    return 1.0f - __fdividef(2.0f, 1.0f + __expf(2.0f * v));
-  }
+  float r;
+  asm("tanh.approx.f32 %0, %1;" : "=f"(r) : "f"(v));
+  return r;
 }
-template <int FMT>
-__device__ __forceinline__ float fast_sigmoid(float v) {
-  if constexpr (FMT == FMT_BF16) return fmaf(0.5f, fast_tanh<FMT>(0.5f * v), 0.5f);
-  else return __fdividef(1.0f, 1.0f + __expf(-v));
-}
-__device__ __forceinline__ uint32_t tf32_rn_bits(float a) {
-  uint32_t u;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(u) : "f"(a));
-  return u;
-}
+__device__ __forceinline__ float fast_sigmoid(float v) { return fmaf(0.5f, fast_tanh(0.5f * v), 0.5f); }
 
 // ------------------------------------------------------------------------------------------
 // weight image: fp32 collapsed weights (k_prep) -> swizzled operand tiles
 // ------------------------------------------------------------------------------------------
-template <int FMT, int HH>
-__device__ __forceinline__ void put_w(uint8_t* tile0, int split_stride, bool chunk_tile, int rows, int r, int c, float v) {
-  using Cfg = TcCfg<FMT, HH>;
-  const uint32_t off = chunk_tile ? chunk_off(r, (c * Cfg::ES) >> 4, rows) + ((c * Cfg::ES) & 15)
-                                  : sw128_off(r, c * Cfg::ES, rows);
-  if constexpr (FMT == FMT_TF32) {
-    const float hi = __uint_as_float(tf32_rn_bits(v));
-    *reinterpret_cast<float*>(tile0 + off) = hi;
-    *reinterpret_cast<float*>(tile0 + split_stride + off) = v - hi;
-  } else {
-    *reinterpret_cast<__nv_bfloat16*>(tile0 + off) = __float2bfloat16(v);
-  }
+__device__ __forceinline__ void put_w(uint8_t* tile0, bool chunk_tile, int rows, int r, int c, float v) {
+  const uint32_t off = chunk_tile ? chunk_off(r, (c * 2) >> 4, rows) + ((c * 2) & 15) : sw128_off(r, c * 2, rows);
+  *reinterpret_cast<__nv_bfloat16*>(tile0 + off) = __float2bfloat16(v);
 }
 
 // Wzr [F+H][2H], Wc [F+H][H] (rows 0..F-1: S part, rows F..: h part), lin_w[g] [H][2H]
-template <int FMT, int HH>
+template <int HH>
 __global__ void k_pack_tc(const float* __restrict__ Wzr, const float* __restrict__ Wc, const float* __restrict__ czr,
                           const float* __restrict__ cc, const float* __restrict__ c0, const float* __restrict__ M0t,
                           const float* __restrict__ M1t, const float* __restrict__ probs, int T,
                           const float* __restrict__ lw0, const float* __restrict__ lw1, const float* __restrict__ lw2,
                           uint8_t* __restrict__ img_f, uint8_t* __restrict__ img_b) {
-  using Cfg = TcCfg<FMT, HH>;
-  constexpr int SKE = 16 * 2 / Cfg::ES;  // elements of the padded S part (8 tf32 / 16 bf16)
+  using Cfg = TcCfg<HH>;
+  constexpr int SKE = 16;  // elements of the padded S part
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   constexpr int n_zr_h = 2 * HH * HH, n_zr_s = 2 * HH * SKE, n_c_h = HH * HH, n_c_s = HH * SKE;
   int j = i;
   if (j < n_zr_h) {
     const int n = j / HH, k = j % HH;
-    put_w<FMT, HH>(img_f, Cfg::FWD_SPLIT, false, 2 * HH, n, k, Wzr[(size_t)(F + k) * 2 * HH + n]);
+    put_w(img_f, false, 2 * HH, n, k, Wzr[(size_t)(F + k) * 2 * HH + n]);
     return;
   }
   j -= n_zr_h;
   if (j < n_zr_s) {
     const int n = j / SKE, f = j % SKE;
-    put_w<FMT, HH>(img_f + Cfg::WZR_H, Cfg::FWD_SPLIT, true, 2 * HH, n, f, f < F ? Wzr[(size_t)f * 2 * HH + n] : 0.f);
+    put_w(img_f + Cfg::WZR_H, true, 2 * HH, n, f, f < F ? Wzr[(size_t)f * 2 * HH + n] : 0.f);
     return;
   }
   j -= n_zr_s;
   if (j < n_c_h) {
     const int n = j / HH, k = j % HH;
-    put_w<FMT, HH>(img_f + Cfg::WZR_H + Cfg::WZR_S, Cfg::FWD_SPLIT, false, HH, n, k, Wc[(size_t)(F + k) * HH + n]);
+    put_w(img_f + Cfg::WZR_H + Cfg::WZR_S, false, HH, n, k, Wc[(size_t)(F + k) * HH + n]);
     return;
   }
   j -= n_c_h;
   if (j < n_c_s) {
     const int n = j / SKE, f = j % SKE;
-    put_w<FMT, HH>(img_f + Cfg::WZR_H + Cfg::WZR_S + Cfg::WC_H, Cfg::FWD_SPLIT, true, HH, n, f,
-                   f < F ? Wc[(size_t)f * HH + n] : 0.f);
+    put_w(img_f + Cfg::WZR_H + Cfg::WZR_S + Cfg::WC_H, true, HH, n, f, f < F ? Wc[(size_t)f * HH + n] : 0.f);
     return;
   }
   j -= n_c_s;
@@ -137,107 +98,64 @@ __global__ void k_pack_tc(const float* __restrict__ Wzr, const float* __restrict
     const int g = j / (HH * HH), rem = j % (HH * HH);
     const int k = rem / HH, n = rem % HH;
     const float* lw = g == 0 ? lw0 : (g == 1 ? lw1 : lw2);
-    put_w<FMT, HH>(img_b + g * Cfg::BT, Cfg::BWD_SPLIT, false, HH, k, n, lw[(size_t)n * 2 * HH + HH + k]);
+    put_w(img_b + g * Cfg::BT, false, HH, k, n, lw[(size_t)n * 2 * HH + HH + k]);
     return;
   }
   j -= 3 * HH * HH;
   if (j < HH * 16) {  // B0[n][k]: k < 8 -> M0[n][k], k >= 8 -> M1[0][n][k-8]   (forward and backward images)
     const int n = j / 16, k = j % 16;
     const float v = k < F ? (M0t ? M0t[k * HH + n] : 0.f) : (M1t ? M1t[(k - F) * HH + n] : 0.f);
-    put_w<FMT, HH>(img_f + Cfg::OFF_W0, Cfg::FWD_SPLIT, true, HH, n, k, v);
-    put_w<FMT, HH>(img_b + 3 * Cfg::BT, Cfg::BWD_SPLIT, true, HH, n, k, v);
+    put_w(img_f + Cfg::OFF_W0, true, HH, n, k, v);
+    put_w(img_b + 3 * Cfg::BT, true, HH, n, k, v);
   }
 }
 
 // ------------------------------------------------------------------------------------------
 // shared device helpers
 // ------------------------------------------------------------------------------------------
-// write CW consecutive columns [c0, c0+CW) of row r into the [128 x HH] SW128 operand tile(s)
-template <int FMT, int HH>
+// write CW consecutive columns [c0, c0+CW) of row r into the [128 x HH] SW128 operand tile
 __device__ __forceinline__ void store_operand(uint8_t* tile, int r, int c0, const float (&v)[CW]) {
-  using Cfg = TcCfg<FMT, HH>;
-  if constexpr (FMT == FMT_TF32) {
 #pragma unroll
-    for (int j = 0; j < CW; j += 4) {
-      float hi[4], lo[4];
-#pragma unroll
-      for (int e = 0; e < 4; ++e) {
-        hi[e] = __uint_as_float(tf32_rn_bits(v[j + e]));
-        lo[e] = v[j + e] - hi[e];
-      }
-      const uint32_t off = sw128_off(r, (c0 + j) * 4, TC_ROWS);
-      *reinterpret_cast<float4*>(tile + off) = make_float4(hi[0], hi[1], hi[2], hi[3]);
-      *reinterpret_cast<float4*>(tile + Cfg::A_TILE + off) = make_float4(lo[0], lo[1], lo[2], lo[3]);
-    }
-  } else {
-#pragma unroll
-    for (int j = 0; j < CW; j += 8) {
-      uint4 p;
-      p.x = pack_bf16(v[j], v[j + 1]);
-      p.y = pack_bf16(v[j + 2], v[j + 3]);
-      p.z = pack_bf16(v[j + 4], v[j + 5]);
-      p.w = pack_bf16(v[j + 6], v[j + 7]);
-      *reinterpret_cast<uint4*>(tile + sw128_off(r, (c0 + j) * 2, TC_ROWS)) = p;
-    }
+  for (int j = 0; j < CW; j += 8) {
+    uint4 p;
+    p.x = pack_bf16(v[j], v[j + 1]);
+    p.y = pack_bf16(v[j + 2], v[j + 3]);
+    p.z = pack_bf16(v[j + 4], v[j + 5]);
+    p.w = pack_bf16(v[j + 6], v[j + 7]);
+    *reinterpret_cast<uint4*>(tile + sw128_off(r, (c0 + j) * 2, TC_ROWS)) = p;
   }
 }
-// write the 8 F-wide values of row r into chunk tile(s): chunk c holds 16 bytes
-template <int FMT, int HH>
-__device__ __forceinline__ void store_small8(uint8_t* tile, int split_stride, int r, int elem0, const float (&v)[8]) {
-  if constexpr (FMT == FMT_TF32) {  // 8 fp32 = 2 chunks, starting at chunk elem0/4
-    float hi[8], lo[8];
-#pragma unroll
-    for (int e = 0; e < 8; ++e) {
-      hi[e] = __uint_as_float(tf32_rn_bits(v[e]));
-      lo[e] = v[e] - hi[e];
-    }
-#pragma unroll
-    for (int c = 0; c < 2; ++c) {
-      const uint32_t off = chunk_off(r, elem0 / 4 + c, TC_ROWS);
-      *reinterpret_cast<float4*>(tile + off) = make_float4(hi[4 * c], hi[4 * c + 1], hi[4 * c + 2], hi[4 * c + 3]);
-      *reinterpret_cast<float4*>(tile + split_stride + off) = make_float4(lo[4 * c], lo[4 * c + 1], lo[4 * c + 2], lo[4 * c + 3]);
-    }
-  } else {  // 8 bf16 = 1 chunk
-    uint4 p;
-    p.x = pack_bf16(v[0], v[1]);
-    p.y = pack_bf16(v[2], v[3]);
-    p.z = pack_bf16(v[4], v[5]);
-    p.w = pack_bf16(v[6], v[7]);
-    *reinterpret_cast<uint4*>(tile + chunk_off(r, elem0 / 8, TC_ROWS)) = p;
-  }
+// write the 8 F-wide values of row r into a chunk tile (8 bf16 = one 16-byte chunk)
+__device__ __forceinline__ void store_small8(uint8_t* tile, int r, int elem0, const float (&v)[8]) {
+  uint4 p;
+  p.x = pack_bf16(v[0], v[1]);
+  p.y = pack_bf16(v[2], v[3]);
+  p.z = pack_bf16(v[4], v[5]);
+  p.w = pack_bf16(v[6], v[7]);
+  *reinterpret_cast<uint4*>(tile + chunk_off(r, elem0 / 8, TC_ROWS)) = p;
 }
 
-// one contraction D[128 x N] (+)= [h-part | S-part] x W  with all precision products
-template <int FMT, int HH>
+// one contraction D[128 x N] = [h-part | S-part] x W
+template <int HH>
 __device__ __forceinline__ void issue_gate_mma(uint32_t tmem_d, uint32_t a_h, uint32_t a_s, uint32_t w_h, uint32_t w_s,
                                                int n_rows_w, uint32_t idesc) {
-  using Cfg = TcCfg<FMT, HH>;
   uint32_t acc = 0;
-  constexpr int NPROD = (FMT == FMT_TF32) ? 3 : 1;
 #pragma unroll
-  for (int p = 0; p < NPROD; ++p) {
-    const int pa = (p == 1) ? 1 : 0, pb = (p == 2) ? 1 : 0;  // hi*hi, lo*hi, hi*lo
-    const uint32_t ah = a_h + pa * Cfg::A_TILE, as = a_s + pa * Cfg::SMF_TILE;
-    const uint32_t wh = w_h + pb * Cfg::FWD_SPLIT, ws = w_s + pb * Cfg::FWD_SPLIT;
-#pragma unroll
-    for (int s = 0; s < HH / Cfg::UK; ++s) {
-      const int kb = s * 32;
-      const uint64_t da = make_desc(ah + (kb >> 7) * TC_ROWS * 128 + (kb & 127), 16, 1024, LAYOUT_SW128);
-      const uint64_t db = make_desc(wh + (kb >> 7) * n_rows_w * 128 + (kb & 127), 16, 1024, LAYOUT_SW128);
-      umma<FMT>(tmem_d, da, db, idesc, acc);
-      acc = 1;
-    }
-    const uint64_t da = make_desc(as, TC_ROWS * 16, 128, LAYOUT_NONE);
-    const uint64_t db = make_desc(ws, n_rows_w * 16, 128, LAYOUT_NONE);
-    umma<FMT>(tmem_d, da, db, idesc, 1);
+  for (int s = 0; s < HH / TcCfg<HH>::UK; ++s) {
+    const int kb = s * 32;
+    const uint64_t da = make_desc(a_h + (kb >> 7) * TC_ROWS * 128 + (kb & 127), 16, 1024, LAYOUT_SW128);
+    const uint64_t db = make_desc(w_h + (kb >> 7) * n_rows_w * 128 + (kb & 127), 16, 1024, LAYOUT_SW128);
+    umma<FMT_BF16>(tmem_d, da, db, idesc, acc);
+    acc = 1;
   }
+  umma<FMT_BF16>(tmem_d, make_desc(a_s, TC_ROWS * 16, 128, LAYOUT_NONE), make_desc(w_s, n_rows_w * 16, 128, LAYOUT_NONE), idesc, 1);
 }
 
 // h[CW] for columns [c0, c0+CW) of row q at period t (regional combine on F-wide features)
 template <int HH>
 __device__ __forceinline__ void compute_h(const TcArgs& a, const float* consts_s, bool valid, long long q, int b, int s0,
                                           int s1, int t, int c0, float (&h)[CW], float (&sv)[8]) {
-  using C = TcCfg<FMT_BF16, HH>;  // constant offsets do not depend on FMT
+  using C = TcCfg<HH>;
   float xv[8];
   {
     const size_t ro = ((size_t)t * a.BN + (valid ? q : 0)) * F;
@@ -301,11 +219,11 @@ __device__ __forceinline__ void compute_h(const TcArgs& a, const float* consts_s
 }
 
 // Saved-plane tile layout: one (t, q-tile) tile is contiguous so the backward can bulk-copy it.
-//   tf32x3 mode: fp32  [T][nqt][HH/4][128][4]      bf16 mode: bf16  [T][nqt][HH/8][128][8]
+//   bf16 planes (Z, R, H~): [T][nqt][HH/8][128][8]      fp32 plane (d h_pre): [T][nqt][HH/4][128][4]
 // Thread r writes 16-byte pieces; a warp instruction covers 512 contiguous bytes.
-template <int FMT, int HH>
+template <typename E, int HH>
 struct PlaneIO {
-  static constexpr bool BF = (FMT == FMT_BF16);
+  static constexpr bool BF = sizeof(E) == 2;
   static constexpr int TILE_BYTES = TC_ROWS * HH * (BF ? 2 : 4);
   __device__ static __forceinline__ uint8_t* tile(void* plane, int nqt, int t, int qt) {
     return reinterpret_cast<uint8_t*>(plane) + ((size_t)t * nqt + qt) * TILE_BYTES;
@@ -377,43 +295,23 @@ __device__ __forceinline__ void load_feats(const TcArgs& a, bool valid, long lon
   uv[0] = u0.x; uv[1] = u0.y; uv[2] = u0.z; uv[3] = u0.w; uv[4] = u1.x; uv[5] = u1.y; uv[6] = u1.z; uv[7] = u1.w;
 }
 
-// forward small tile: S (+ zero pad in bf16) | X | U
-template <int FMT, int HH>
+// forward small tile: S (+ zero pad) | X | U
+template <int HH>
 __device__ __forceinline__ void write_small_fwd(uint8_t* sm, int r, const float (&sv)[8], const float (&xv)[8],
                                                 const float (&uv)[8]) {
-  using Cfg = TcCfg<FMT, HH>;
-  constexpr int EPC = 16 / Cfg::ES;  // elements per chunk
-  store_small8<FMT, HH>(sm, Cfg::SMF_TILE, r, 0, sv);
-  if constexpr (FMT == FMT_BF16) *reinterpret_cast<uint4*>(sm + chunk_off(r, 1, TC_ROWS)) = make_uint4(0, 0, 0, 0);
-  store_small8<FMT, HH>(sm, Cfg::SMF_TILE, r, Cfg::SMF_XU_CHUNK * EPC, xv);
-  store_small8<FMT, HH>(sm, Cfg::SMF_TILE, r, Cfg::SMF_XU_CHUNK * EPC + 8, uv);
+  constexpr int XU = TcCfg<HH>::SMF_XU_CHUNK * 8;   // first element of the X | U part (8 bf16 per chunk)
+  store_small8(sm, r, 0, sv);
+  *reinterpret_cast<uint4*>(sm + chunk_off(r, 1, TC_ROWS)) = make_uint4(0, 0, 0, 0);
+  store_small8(sm, r, XU, xv);
+  store_small8(sm, r, XU + 8, uv);
 }
 
-// h_pre[128 x HH] = [X | U] x [M0 ; M1]   (K = 16), all precision products
-template <int FMT, int HH>
-__device__ __forceinline__ void issue_h_mma(uint32_t tmem_d, uint32_t sm_xu, int sm_split, uint32_t w0, int w_split) {
-  using Cfg = TcCfg<FMT, HH>;
-  const uint32_t idesc = make_idesc(FMT, 128, HH, 0, 0);
-  constexpr int NPROD = (FMT == FMT_TF32) ? 3 : 1;
-  constexpr int KSTEPS = 16 / Cfg::UK;
-  uint32_t acc = 0;
-#pragma unroll
-  for (int p = 0; p < NPROD; ++p) {
-    const int pa = (p == 1) ? 1 : 0, pb = (p == 2) ? 1 : 0;
-#pragma unroll
-    for (int s = 0; s < KSTEPS; ++s) {
-      umma<FMT>(tmem_d, make_desc(sm_xu + pa * sm_split + s * 2 * TC_ROWS * 16, TC_ROWS * 16, 128, LAYOUT_NONE),
-                make_desc(w0 + pb * w_split + s * 2 * HH * 16, HH * 16, 128, LAYOUT_NONE), idesc, acc);
-      acc = 1;
-    }
-  }
+// h_pre[128 x HH] = [X | U] x [M0 ; M1]   (K = 16: one MMA)
+template <int HH>
+__device__ __forceinline__ void issue_h_mma(uint32_t tmem_d, uint32_t sm_xu, uint32_t w0) {
+  umma<FMT_BF16>(tmem_d, make_desc(sm_xu, TC_ROWS * 16, 128, LAYOUT_NONE), make_desc(w0, HH * 16, 128, LAYOUT_NONE),
+                 make_idesc(FMT_BF16, 128, HH, 0, 0), 0);
 }
-
-#define REGT_TS(i)                                                  \
-  if (a.dbg && blockIdx.x == 0 && tid == 0 && dbg_n < 24) {         \
-    a.dbg[dbg_n * 10 + (i)] = clock64();                             \
-    a.dbg[dbg_n * 10 + 9] = 0x5245475444424721ll;                    \
-  }
 
 // ------------------------------------------------------------------------------------------
 // forward
@@ -452,20 +350,19 @@ struct RowInfo {
   }
 };
 
-template <int FMT, int HH>
+template <int HH>
 __global__ void __launch_bounds__(NTHREADS, 1) k_cell_fwd_tc(TcArgs a) {
-  using Cfg = TcCfg<FMT, HH>;
-  constexpr int NBUF = Cfg::PIPE ? 2 : 1;
-  constexpr int SMB = Cfg::NSPLIT * Cfg::SMF_TILE;     // bytes per small-tile buffer
+  using Cfg = TcCfg<HH>;
+  using PIO = PlaneIO<__nv_bfloat16, HH>;
+  constexpr int NBUF = 2;                              // small-tile buffers
+  constexpr int SMB = Cfg::SMF_TILE;                   // bytes per small-tile buffer
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   // align inside the shared window with pointer arithmetic only (an integer round trip would make
   // every later access a generic LD/ST instead of LDS/STS)
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   uint8_t* W = smem;                                   // weight image (tiles + consts)
-  uint8_t* Ah = W + ((Cfg::FWD_IMG + 1023) & ~1023);   // [NSPLIT][128 x HH]
-  constexpr bool PIPE2 = Cfg::PIPE && REGT_FWD_PIPE;   // software-pipelined epilogue: h and h*R tiles are separate
-  uint8_t* Ah2 = PIPE2 ? Ah + Cfg::NSPLIT * Cfg::A_TILE : Ah;   // h*R operand tile (own buffer when pipelined)
-  uint8_t* SMf = Ah2 + Cfg::NSPLIT * Cfg::A_TILE;      // [NBUF] small tiles  S(+pad) | X | U
+  uint8_t* Ah = W + ((Cfg::FWD_IMG + 1023) & ~1023);   // [128 x HH] operand tile: h, then h*R
+  uint8_t* SMf = Ah + Cfg::A_TILE;                     // [NBUF] small tiles  S(+pad) | X | U
   __shared__ uint64_t bar_a, bar_zr, bar_a2, bar_c, bar_img, bar_h;
   __shared__ uint64_t bar_x[2];   // per small-tile buffer, like bar_free: tile written / tile consumed
   // bar_free[b]: completes once per use of small-tile buffer b (the MMAs that read it are done).  The
@@ -474,14 +371,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_cell_fwd_tc(TcArgs a) {
   __shared__ uint64_t bar_free[2];
   __shared__ uint32_t tmem_base_s;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  if (a.dbg && blockIdx.x == 0 && tid == 0) a.dbg[240] = clock64();
 
   if (tid == 0) {
     mbar_init(&bar_free[0], 1);
     mbar_init(&bar_free[1], 1);
-    mbar_init(&bar_a, NEPI_WARPS * ARRIVALS_PER_WARP);
+    mbar_init(&bar_a, NEPI);
     mbar_init(&bar_zr, 1);
-    mbar_init(&bar_a2, NEPI_WARPS * ARRIVALS_PER_WARP);
+    mbar_init(&bar_a2, NEPI);
     mbar_init(&bar_c, 1);
     mbar_init(&bar_img, 1);
     mbar_init(&bar_x[0], 1);
@@ -503,7 +399,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_cell_fwd_tc(TcArgs a) {
   const float* consts = reinterpret_cast<const float*>(W + Cfg::FWD_W);
   const bool hmma = a.hmma != 0;
   const int S = cta_steps(a);
-  int dbg_n = 0;
 
   if (warp < NEPI_WARPS) {
     // ================= epilogue threads: thread = (row r, CW columns) =================
@@ -514,205 +409,92 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_cell_fwd_tc(TcArgs a) {
     RowInfo ri;
     float acc[CW];
     StepIt it;
-    // h of one step: from the tensor-core h_pre (single regional list) or on the CUDA cores
-    auto make_h = [&](const StepIt& st_, uint32_t ph_, float (&h_)[CW]) {
+    for (int s = 0; s < S; ++s) {
+      const uint32_t ph = s & 1;
+      it.set(a, s);
+      const int qt = it.item / a.ntc;
+      if (it.ti == 0) {
+        ri.set(a, it.item, r, !hmma);
+#pragma unroll
+        for (int j = 0; j < CW; ++j) acc[j] = 0.f;
+      }
+      float h[CW];
       if (hmma) {
-        mbar_wait(&bar_h, ph_);
+        mbar_wait(&bar_h, ph);
         tc_fence_after();
-        tmem_ld<CW>(tlane + 3 * HH + c0, h_);
+        tmem_ld<CW>(tlane + 3 * HH + c0, h);
 #pragma unroll
         for (int j = 0; j < CW; ++j) {
-          const float v = h_[j] + consts[Cfg::C_C0 + c0 + j];
-          h_[j] = (a.mode == REGT_MODE_REGIONAL) ? (v > 0.f ? v : 0.01f * v) : v;
+          const float v = h[j] + consts[Cfg::C_C0 + c0 + j];
+          h[j] = (a.mode == REGT_MODE_REGIONAL) ? (v > 0.f ? v : 0.01f * v) : v;
         }
       } else {
         float sv[8];
-        compute_h<HH>(a, consts, ri.valid, ri.q, ri.b, ri.s0, ri.s1, st_.t, c0, h_, sv);
+        compute_h<HH>(a, consts, ri.valid, ri.q, ri.b, ri.s0, ri.s1, it.t, c0, h, sv);
       }
-    };
-    if constexpr (PIPE2) {
-      // Software-pipelined order (two operand tiles: Ah = h, Ah2 = h*R).  Per step s:
-      //   E1r  r gate -> R plane, h*R tile -> M2(s) starts        E1z  z gate -> Z plane (under M2)
-      //   P    h of step s+1 -> h tile -> M1(s+1) starts          E2   candidate, blend (under M1(s+1))
-      // so neither MMA's latency is exposed.
-      float h[CW], hn[CW];
-      if (S > 0) {
-        it.set(a, 0);
-        ri.set(a, it.item, r, !hmma);
-        make_h(it, 0u, hn);
-        store_operand<FMT, HH>(Ah, r, c0, hn);
-        fence_proxy_async();
-        tc_fence_before();
-        mbar_arrive_warp(&bar_a);
-      }
-      for (int s = 0; s < S; ++s) {
-        const uint32_t ph = s & 1;
-        it.set(a, s);
-        const int qt = it.item / a.ntc;
-#pragma unroll
-        for (int j = 0; j < CW; ++j) h[j] = hn[j];
-        if (it.ti == 0) {
-#pragma unroll
-          for (int j = 0; j < CW; ++j) acc[j] = 0.f;
-        }
-        REGT_TS(0)
-        mbar_wait(&bar_zr, ph);
-        tc_fence_after();
-        REGT_TS(1)
-        float z[CW];
-        {
-          float raw[CW], hr[CW];
-          tmem_ld<CW>(tlane + HH + c0, raw);
-#pragma unroll
-          for (int j = 0; j < CW; ++j) {
-            const float rg = fast_sigmoid<FMT>(raw[j] + consts[Cfg::C_CZR + HH + c0 + j]);
-            raw[j] = rg;
-            hr[j] = h[j] * rg;
-          }
-          store_operand<FMT, HH>(Ah2, r, c0, hr);
-          fence_proxy_async();
-          tc_fence_before();
-          mbar_arrive_warp(&bar_a2);
-          PlaneIO<FMT, HH>::store(a.Rp, a.nqt, it.t, qt, r, c0, raw);
-          REGT_TS(2)
-          tmem_ld<CW>(tlane + c0, raw);
-#pragma unroll
-          for (int j = 0; j < CW; ++j) z[j] = fast_sigmoid<FMT>(raw[j] + consts[Cfg::C_CZR + c0 + j]);
-          PlaneIO<FMT, HH>::store(a.Zp, a.nqt, it.t, qt, r, c0, z);
-        }
-        REGT_TS(3)
-        if (s + 1 < S) {   // h of the next step: M1(s) has finished reading the h tile (bar_zr above)
-          StepIt nx;
-          nx.set(a, s + 1);
-          if (nx.ti == 0) ri.set(a, nx.item, r, !hmma);
-          make_h(nx, (uint32_t)((s + 1) & 1), hn);
-          store_operand<FMT, HH>(Ah, r, c0, hn);
-          fence_proxy_async();
-          tc_fence_before();
-          mbar_arrive_warp(&bar_a);
-        }
-        REGT_TS(4)
-        mbar_wait(&bar_c, ph);
-        tc_fence_after();
-        REGT_TS(5)
-        {
-          float raw[CW];
-          tmem_ld<CW>(tlane + 2 * HH + c0, raw);
-          const float pt = consts[Cfg::C_PROBS + it.t];
-#pragma unroll
-          for (int j = 0; j < CW; ++j) {
-            const float hc = fast_tanh<FMT>(raw[j] + consts[Cfg::C_CC + c0 + j]);
-            raw[j] = hc;
-            acc[j] = fmaf(pt, z[j] * h[j] + (1.0f - z[j]) * hc, acc[j]);
-          }
-          PlaneIO<FMT, HH>::store(a.Hcp, a.nqt, it.t, qt, r, c0, raw);
-        }
-        if (it.ti + 1 == a.tp) {   // item done: its partial attention sum, tile layout [chunk][qt][HH/4][128][4]
-          float4* o = reinterpret_cast<float4*>(a.hid_part) + ((size_t)(it.item % a.ntc) * a.nqt + qt) * (HH / 4) * TC_ROWS;
-#pragma unroll
-          for (int j = 0; j < CW; j += 4)
-            o[(size_t)((c0 + j) >> 2) * TC_ROWS + r] = make_float4(acc[j], acc[j + 1], acc[j + 2], acc[j + 3]);
-        }
-        REGT_TS(6)
-        ++dbg_n;
-      }
+      store_operand(Ah, r, c0, h);
+      fence_proxy_async();
       tc_fence_before();
-    } else {
-    for (int s = 0; s < S; ++s) {
-        const uint32_t ph = s & 1;
-        it.set(a, s);
-        const int qt = it.item / a.ntc;
-        if (it.ti == 0) {
-          ri.set(a, it.item, r, !hmma);
-  #pragma unroll
-          for (int j = 0; j < CW; ++j) acc[j] = 0.f;
+      mbar_arrive(&bar_a);
+
+      // ---- E1: gates ----
+      mbar_wait(&bar_zr, ph);
+      tc_fence_after();
+      float z[CW];
+      {
+        float raw[CW];
+        tmem_ld<CW>(tlane + c0, raw);
+#pragma unroll
+        for (int j = 0; j < CW; ++j) z[j] = fast_sigmoid(raw[j] + consts[Cfg::C_CZR + c0 + j]);
+        PIO::store(a.Zp, a.nqt, it.t, qt, r, c0, z);
+        tmem_ld<CW>(tlane + HH + c0, raw);
+        float hr[CW];
+#pragma unroll
+        for (int j = 0; j < CW; ++j) {
+          const float rg = fast_sigmoid(raw[j] + consts[Cfg::C_CZR + HH + c0 + j]);
+          raw[j] = rg;
+          hr[j] = h[j] * rg;
         }
-        float h[CW];
-        REGT_TS(0)
-        if (hmma) {
-          mbar_wait(&bar_h, ph);
-          tc_fence_after();
-          tmem_ld<CW>(tlane + 3 * HH + c0, h);
-  #pragma unroll
-          for (int j = 0; j < CW; ++j) {
-            const float v = h[j] + consts[Cfg::C_C0 + c0 + j];
-            h[j] = (a.mode == REGT_MODE_REGIONAL) ? (v > 0.f ? v : 0.01f * v) : v;
-          }
-        } else {
-          float sv[8];
-          compute_h<HH>(a, consts, ri.valid, ri.q, ri.b, ri.s0, ri.s1, it.t, c0, h, sv);
-        }
-        REGT_TS(1)
-        store_operand<FMT, HH>(Ah, r, c0, h);
-        fence_proxy_async();
-        tc_fence_before();
-        mbar_arrive_warp(&bar_a);
-  
-        // ---- E1: gates ----
-        REGT_TS(2)
-        mbar_wait(&bar_zr, ph);
-        tc_fence_after();
-        REGT_TS(3)
-        float z[CW];
-        {
-          float raw[CW];
-          tmem_ld<CW>(tlane + c0, raw);
-  #pragma unroll
-          for (int j = 0; j < CW; ++j) z[j] = fast_sigmoid<FMT>(raw[j] + consts[Cfg::C_CZR + c0 + j]);
-          PlaneIO<FMT, HH>::store(a.Zp, a.nqt, it.t, qt, r, c0, z);
-          tmem_ld<CW>(tlane + HH + c0, raw);
-          float hr[CW];
-  #pragma unroll
-          for (int j = 0; j < CW; ++j) {
-            const float rg = fast_sigmoid<FMT>(raw[j] + consts[Cfg::C_CZR + HH + c0 + j]);
-            raw[j] = rg;
-            hr[j] = h[j] * rg;
-          }
-          PlaneIO<FMT, HH>::store(a.Rp, a.nqt, it.t, qt, r, c0, raw);
-          store_operand<FMT, HH>(Ah, r, c0, hr);
-        }
-        fence_proxy_async();
-        tc_fence_before();
-        mbar_arrive_warp(&bar_a2);
-  
-        // ---- E2: candidate, blend, attention accumulation ----
-        REGT_TS(4)
-        mbar_wait(&bar_c, ph);
-        tc_fence_after();
-        REGT_TS(5)
-        {
-          float raw[CW];
-          tmem_ld<CW>(tlane + 2 * HH + c0, raw);
-          const float pt = consts[Cfg::C_PROBS + it.t];
-  #pragma unroll
-          for (int j = 0; j < CW; ++j) {
-            const float hc = fast_tanh<FMT>(raw[j] + consts[Cfg::C_CC + c0 + j]);
-            raw[j] = hc;
-            acc[j] = fmaf(pt, z[j] * h[j] + (1.0f - z[j]) * hc, acc[j]);
-          }
-          PlaneIO<FMT, HH>::store(a.Hcp, a.nqt, it.t, qt, r, c0, raw);
-        }
-        if (it.ti + 1 == a.tp) {   // item done: its partial attention sum, tile layout [chunk][qt][HH/4][128][4]
-          float4* o = reinterpret_cast<float4*>(a.hid_part) + ((size_t)(it.item % a.ntc) * a.nqt + qt) * (HH / 4) * TC_ROWS;
-  #pragma unroll
-          for (int j = 0; j < CW; j += 4)
-            o[(size_t)((c0 + j) >> 2) * TC_ROWS + r] = make_float4(acc[j], acc[j + 1], acc[j + 2], acc[j + 3]);
-        }
-        REGT_TS(6)
-        ++dbg_n;
+        PIO::store(a.Rp, a.nqt, it.t, qt, r, c0, raw);
+        store_operand(Ah, r, c0, hr);
       }
+      fence_proxy_async();
       tc_fence_before();
+      mbar_arrive(&bar_a2);
+
+      // ---- E2: candidate, blend, attention accumulation ----
+      mbar_wait(&bar_c, ph);
+      tc_fence_after();
+      {
+        float raw[CW];
+        tmem_ld<CW>(tlane + 2 * HH + c0, raw);
+        const float pt = consts[Cfg::C_PROBS + it.t];
+#pragma unroll
+        for (int j = 0; j < CW; ++j) {
+          const float hc = fast_tanh(raw[j] + consts[Cfg::C_CC + c0 + j]);
+          raw[j] = hc;
+          acc[j] = fmaf(pt, z[j] * h[j] + (1.0f - z[j]) * hc, acc[j]);
+        }
+        PIO::store(a.Hcp, a.nqt, it.t, qt, r, c0, raw);
+      }
+      if (it.ti + 1 == a.tp) {   // item done: its partial attention sum, tile layout [chunk][qt][HH/4][128][4]
+        float4* o = reinterpret_cast<float4*>(a.hid_part) + ((size_t)(it.item % a.ntc) * a.nqt + qt) * (HH / 4) * TC_ROWS;
+#pragma unroll
+        for (int j = 0; j < CW; j += 4)
+          o[(size_t)((c0 + j) >> 2) * TC_ROWS + r] = make_float4(acc[j], acc[j + 1], acc[j + 2], acc[j + 3]);
+      }
     }
+    tc_fence_before();
   } else if (warp == WARP_MMA) {
     // ================= MMA issuer (one elected lane) =================
-    const uint32_t idesc_zr = make_idesc(FMT, 128, 2 * HH, 0, 0), idesc_c = make_idesc(FMT, 128, HH, 0, 0);
-    const uint32_t ah = smem_u32(Ah), ah2 = smem_u32(Ah2), smf = smem_u32(SMf), w = smem_u32(W);
+    const uint32_t idesc_zr = make_idesc(FMT_BF16, 128, 2 * HH, 0, 0), idesc_c = make_idesc(FMT_BF16, 128, HH, 0, 0);
+    const uint32_t ah = smem_u32(Ah), smf = smem_u32(SMf), w = smem_u32(W);
     constexpr int XU = Cfg::SMF_XU_CHUNK * TC_ROWS * 16;             // offset of the X | U chunks
     if (S > 0) {  // the loader has built step 0's tile: h_pre of step 0
       mbar_wait(&bar_x[0], 0);
       tc_fence_after();
       if (lane == 0 && hmma) {
-        issue_h_mma<FMT, HH>(tmem + 3 * HH, smf + XU, Cfg::SMF_TILE, w + Cfg::OFF_W0, Cfg::FWD_SPLIT);
+        issue_h_mma<HH>(tmem + 3 * HH, smf + XU, w + Cfg::OFF_W0);
         umma_commit(&bar_h);
       }
       __syncwarp();
@@ -723,15 +505,15 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_cell_fwd_tc(TcArgs a) {
       mbar_wait(&bar_a, ph);
       tc_fence_after();
       if (lane == 0) {
-        issue_gate_mma<FMT, HH>(tmem, ah, as, w, w + Cfg::WZR_H, 2 * HH, idesc_zr);
+        issue_gate_mma<HH>(tmem, ah, as, w, w + Cfg::WZR_H, 2 * HH, idesc_zr);
         umma_commit(&bar_zr);
       }
       __syncwarp();
       mbar_wait(&bar_a2, ph);
       tc_fence_after();
       if (lane == 0) {
-        issue_gate_mma<FMT, HH>(tmem + 2 * HH, ah2, as, w + Cfg::WZR_H + Cfg::WZR_S,
-                                w + Cfg::WZR_H + Cfg::WZR_S + Cfg::WC_H, HH, idesc_c);
+        issue_gate_mma<HH>(tmem + 2 * HH, ah, as, w + Cfg::WZR_H + Cfg::WZR_S, w + Cfg::WZR_H + Cfg::WZR_S + Cfg::WC_H, HH,
+                           idesc_c);
         umma_commit(&bar_c);
         umma_commit(&bar_free[s % NBUF]);
       }
@@ -740,7 +522,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_cell_fwd_tc(TcArgs a) {
         mbar_wait(&bar_x[(s + 1) % NBUF], (uint32_t)(((s + 1) / NBUF) & 1));
         tc_fence_after();
         if (lane == 0 && hmma) {
-          issue_h_mma<FMT, HH>(tmem + 3 * HH, smf + ((s + 1) % NBUF) * SMB + XU, Cfg::SMF_TILE, w + Cfg::OFF_W0, Cfg::FWD_SPLIT);
+          issue_h_mma<HH>(tmem + 3 * HH, smf + ((s + 1) % NBUF) * SMB + XU, w + Cfg::OFF_W0);
           umma_commit(&bar_h);
         }
         __syncwarp();
@@ -764,15 +546,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_cell_fwd_tc(TcArgs a) {
       if (s >= NBUF) mbar_wait(&bar_free[s % NBUF], (uint32_t)((s / NBUF - 1) & 1));
       uint8_t* sm = SMf + (s % NBUF) * SMB;
 #pragma unroll
-      for (int k = 0; k < 4; ++k) write_small_fwd<FMT, HH>(sm, lane + 32 * k, sv[k], xv[k], uv[k]);
+      for (int k = 0; k < 4; ++k) write_small_fwd<HH>(sm, lane + 32 * k, sv[k], xv[k], uv[k]);
       fence_proxy_async();
       __syncwarp();
       if (lane == 0) mbar_arrive(&bar_x[s % NBUF]);
     }
   }
-  if (a.dbg && blockIdx.x == 0 && tid == 0) a.dbg[241] = clock64();
   __syncthreads();
-  if (a.dbg && blockIdx.x == 0 && tid == 0) a.dbg[242] = clock64();
   if (warp == WARP_MMA) tmem_dealloc(tmem, 256);
 }
 
@@ -850,27 +630,24 @@ static TcArgs make_tcargs(const regt_args* a, const Layout& L, int slots) {
   k.img = L.tc_img_f;
   k.Zp = L.Zp; k.Rp = L.Rp; k.Hcp = L.Hcp; k.hid_part = L.hid_part;
   k.G = L.G; k.dhp = L.dhp_p; k.wpart = L.tc_wpart; k.dprobs_part = L.tc_dpp;
-  k.dbg = getenv("REGT_TC_DEBUG") ? reinterpret_cast<long long*>(L.part) : nullptr;  // scratch reuse (debug only)
   return k;
 }
 
-template <int FMT, int HH>
+template <int HH>
 static int run_fwd_tc(const regt_args* a, const Layout& L, cudaStream_t st, bool forked) {
-  using Cfg = TcCfg<FMT, HH>;
+  using Cfg = TcCfg<HH>;
   static_assert(Cfg::FWD_IMG <= TC_IMG_BYTES && Cfg::BWD_IMG <= TC_IMG_BYTES, "weight image too large");
   const int n_pack = 2 * HH * HH + 2 * HH * 16 + HH * HH + HH * 16 + Cfg::C_FLOATS + 3 * HH * HH + HH * 16;
-  k_pack_tc<FMT, HH><<<cdiv(n_pack, 256), 256, 0, st>>>(L.Wzr, L.Wc, L.czr, L.cc, L.c0, L.M0t, L.M1t, L.probs, a->T,
-                                                       a->p.lin_w[0], a->p.lin_w[1], a->p.lin_w[2], L.tc_img_f,
-                                                       L.tc_img_b);
+  k_pack_tc<HH><<<cdiv(n_pack, 256), 256, 0, st>>>(L.Wzr, L.Wc, L.czr, L.cc, L.c0, L.M0t, L.M1t, L.probs, a->T,
+                                                  a->p.lin_w[0], a->p.lin_w[1], a->p.lin_w[2], L.tc_img_f, L.tc_img_b);
   REGT_LAUNCHED("k_pack_tc", st);
   if (forked && join_side(st)) return -1;   // the feature builder ran beside the weight collapse
   const int slots = num_sms();
   TcArgs k = make_tcargs(a, L, slots);
-  const size_t smem = 1024 + ((Cfg::FWD_IMG + 1023) & ~1023) + ((Cfg::PIPE && REGT_FWD_PIPE) ? 2 : 1) * Cfg::NSPLIT * Cfg::A_TILE +
-                      (Cfg::PIPE ? 2 : 1) * Cfg::NSPLIT * Cfg::SMF_TILE;
-  REGT_CUDA(cudaFuncSetAttribute(k_cell_fwd_tc<FMT, HH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const size_t smem = 1024 + ((Cfg::FWD_IMG + 1023) & ~1023) + Cfg::A_TILE + 2 * Cfg::SMF_TILE;
+  REGT_CUDA(cudaFuncSetAttribute(k_cell_fwd_tc<HH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int grid = min(slots, k.items);
-  k_cell_fwd_tc<FMT, HH><<<grid, NTHREADS, smem, st>>>(k);
+  k_cell_fwd_tc<HH><<<grid, NTHREADS, smem, st>>>(k);
   REGT_LAUNCHED("k_cell_fwd_tc", st);
   if (!head_fusable(a)) {  // otherwise the fused head sums the partials while loading its tiles
     const long long count = (long long)k.BN * HH;
@@ -888,7 +665,7 @@ int cell_forward_tc(const regt_args* a, const Layout& L, cudaStream_t st) {
   cudaStream_t side = fork_side(st);
   if (launch_feat_tc(a->plan, a->x, a->B, a->x_rows > 0 ? a->x_rows : a->N, a->T, L.Xt, L.S, L.U, side ? side : st)) return -1;
   if (launch_prep(a, L, st)) return -1;
-  return run_fwd_tc<FMT_BF16, 64>(a, L, st, side != nullptr);
+  return run_fwd_tc<64>(a, L, st, side != nullptr);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -913,8 +690,8 @@ constexpr int WP_COLS = 192;  // per-CTA partial: [128][192] = accW1 | accW1s | 
 template <int HH>
 __global__ void __launch_bounds__(NTHREADS, 1) k_cell_bwd_tc(TcArgs a) {
   constexpr int FMT = FMT_BF16;
-  using Cfg = TcCfg<FMT, HH>;
-  using PIO = PlaneIO<FMT, HH>;
+  using Cfg = TcCfg<HH>;
+  using PIO = PlaneIO<__nv_bfloat16, HH>;
   constexpr int TILE = Cfg::A_TILE;          // 16 KB
   constexpr int PT = PIO::TILE_BYTES;        // 16 KB
   constexpr int SMT = 4 * TC_ROWS * 16;      // small tile: S | X | U | ones
@@ -937,17 +714,16 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_cell_bwd_tc(TcArgs a) {
   __shared__ uint64_t bar_x[2], bar_sfree[2];
   __shared__ uint32_t tmem_base_s;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  if (a.dbg && blockIdx.x == 0 && tid == 0) a.dbg[240] = clock64();
 
   if (tid == 0) {
     mbar_init(&bar_img, 1);
     mbar_init(&bar_stage, 1);
     mbar_init(&bar_g, 1);
-    mbar_init(&bar_e0, NEPI_WARPS * ARRIVALS_PER_WARP);
+    mbar_init(&bar_e0, NEPI);
     mbar_init(&bar_m1, 1);
-    mbar_init(&bar_e1, NEPI_WARPS * ARRIVALS_PER_WARP);
+    mbar_init(&bar_e1, NEPI);
     mbar_init(&bar_m2, 1);
-    mbar_init(&bar_e2, NEPI_WARPS * ARRIVALS_PER_WARP);
+    mbar_init(&bar_e2, NEPI);
     mbar_init(&bar_w, 1);
     mbar_init(&bar_x[0], 1);
     mbar_init(&bar_x[1], 1);
@@ -968,7 +744,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_cell_bwd_tc(TcArgs a) {
   const float* consts = reinterpret_cast<const float*>(W + Cfg::BWD_W);
   const bool hmma = a.hmma != 0;
   const int S = cta_steps(a);
-  int dbg_n = 0;
 
   if (warp < NEPI_WARPS) {
     const int r = (warp & 3) * 32 + lane;
@@ -977,7 +752,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_cell_bwd_tc(TcArgs a) {
     const uint32_t tlane = tmem + ((uint32_t)((warp & 3) * 32) << 16);
     RowInfo ri;
     StepIt it;
-    float hn[CW];
     float dpr0 = 0.f, dpr1 = 0.f;   // attention-gradient sums of periods lane and 32 + lane
     // h of one step (recomputed, not saved): tensor-core h_pre (single regional list) or CUDA cores
     auto make_h = [&](const StepIt& st_, uint32_t ph_, float (&h_)[CW]) {
@@ -998,26 +772,18 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_cell_bwd_tc(TcArgs a) {
     if (S > 0) {
       it.set(a, 0);
       ri.set(a, it.item, r, !hmma);
-      if (REGT_BWD_H_UNDER_M2) make_h(it, 0u, hn);
     }
     for (int s = 0; s < S; ++s) {
       const uint32_t ph = s & 1;
       it.set(a, s);
       const int qt = it.item / a.ntc;
       float h[CW], dh[CW], rr[CW];
-      if (REGT_BWD_H_UNDER_M2) {
-#pragma unroll
-        for (int j = 0; j < CW; ++j) h[j] = hn[j];
-      } else {
-        if (it.ti == 0 && s > 0) ri.set(a, it.item, r, !hmma);
-        make_h(it, ph, h);
-      }
+      if (it.ti == 0 && s > 0) ri.set(a, it.item, r, !hmma);
+      make_h(it, ph, h);
       const bool row_valid = ri.valid;   // ri moves on to the next item before this step ends
-      REGT_TS(0)
       if (it.ti == 0) mbar_wait(&bar_g, (uint32_t)((s / a.tp) & 1));   // this item's G tile has landed in smem
       const float pt = consts[Cfg::C_PROBS + it.t];
       float dp = 0.f;
-      REGT_TS(1)
       mbar_wait(&bar_stage, ph);
       {
         float z[CW], hc[CW];
@@ -1041,29 +807,20 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_cell_bwd_tc(TcArgs a) {
           }
         }
         if (s > 0) mbar_wait(&bar_w, (uint32_t)((s - 1) & 1));  // previous step's MMAs released the tiles
-        store_operand<FMT, HH>(T_DH, r, c0, hc);
-        if (REGT_BWD_EARLY_E0) {
-          fence_proxy_async();
-          tc_fence_before();
-          mbar_arrive_warp(&bar_e0);        // M1 needs Dh only: it runs under the remaining tile stores
-        }
-        store_operand<FMT, HH>(T_DZ, r, c0, z);
+        store_operand(T_DH, r, c0, hc);
+        fence_proxy_async();
+        tc_fence_before();
+        mbar_arrive(&bar_e0);          // M1 needs Dh only: it runs under the remaining tile stores (62.7 against 65.5 us)
+        store_operand(T_DZ, r, c0, z);
 #pragma unroll
         for (int j = 0; j < CW; ++j) z[j] = h[j] * rr[j];
-        store_operand<FMT, HH>(T_HR, r, c0, z);
-        store_operand<FMT, HH>(T_H, r, c0, h);   // made visible to the tensor core by the fence before bar_e1
-        if (!REGT_BWD_EARLY_E0) {
-          fence_proxy_async();
-          tc_fence_before();
-          mbar_arrive_warp(&bar_e0);
-        }
+        store_operand(T_HR, r, c0, z);
+        store_operand(T_H, r, c0, h);   // made visible to the tensor core by the fence before bar_e1
       }
-      REGT_TS(2)
 
       // ---- E1 ----
       mbar_wait(&bar_m1, ph);
       tc_fence_after();
-      REGT_TS(3)
       {
         float raw[CW];
         tmem_ld<CW>(tlane + c0, raw);
@@ -1073,23 +830,15 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_cell_bwd_tc(TcArgs a) {
           dh[j] = fmaf(dHR, rr[j], dh[j]);
           raw[j] = dHR * h[j] * rr[j] * (1.0f - rr[j]);   // Dr
         }
-        store_operand<FMT, HH>(T_DR, r, c0, raw);
+        store_operand(T_DR, r, c0, raw);
       }
       fence_proxy_async();
       tc_fence_before();
-      mbar_arrive_warp(&bar_e1);
-      if (REGT_BWD_H_UNDER_M2 && s + 1 < S) {   // h of the next step, under M2 of this one (its h_pre MMA was issued right after M1)
-        StepIt nx;
-        nx.set(a, s + 1);
-        if (nx.ti == 0) ri.set(a, nx.item, r, !hmma);
-        make_h(nx, (uint32_t)((s + 1) & 1), hn);
-      }
-      REGT_TS(4)
+      mbar_arrive(&bar_e1);
 
       // ---- E2 ----
       mbar_wait(&bar_m2, ph);
       tc_fence_after();
-      REGT_TS(5)
       {
         float raw[CW];
         tmem_ld<CW>(tlane + 64 + c0, raw);
@@ -1099,13 +848,12 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_cell_bwd_tc(TcArgs a) {
           if (a.mode == REGT_MODE_REGIONAL) v *= (h[j] > 0.f ? 1.0f : 0.01f);
           raw[j] = v;
         }
-        store_operand<FMT, HH>(T_DHP, r, c0, raw);
-        if (a.mode == REGT_MODE_REGIONAL && !hmma) PlaneIO<FMT_TF32, HH>::store(a.dhp, a.nqt, it.t, qt, r, c0, raw);
+        store_operand(T_DHP, r, c0, raw);
+        if (a.mode == REGT_MODE_REGIONAL && !hmma) PlaneIO<float, HH>::store(a.dhp, a.nqt, it.t, qt, r, c0, raw);
       }
       fence_proxy_async();
       tc_fence_before();
-      mbar_arrive_warp(&bar_e2);
-      REGT_TS(6)
+      mbar_arrive(&bar_e2);
 
       // ---- attention gradient partial: fixed-order block reduction ----
 #pragma unroll
@@ -1116,8 +864,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_cell_bwd_tc(TcArgs a) {
         if (it.t < 32) dpr0 += dp;
         else dpr1 += dp;
       }
-      REGT_TS(7)
-      ++dbg_n;
     }
     // ---- attention-gradient partial of this CTA: fixed-order sum over the epilogue warps ----
     {
@@ -1183,7 +929,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_cell_bwd_tc(TcArgs a) {
       mbar_wait(&bar_x[0], 0);
       tc_fence_after();
       if (lane == 0 && hmma) {
-        issue_h_mma<FMT, HH>(tmem + 320, sm0 + XU, 0, w + 3 * Cfg::BT, 0);
+        issue_h_mma<HH>(tmem + 320, sm0 + XU, w + 3 * Cfg::BT);
         umma_commit(&bar_h);
       }
       __syncwarp();
@@ -1215,7 +961,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_cell_bwd_tc(TcArgs a) {
         mbar_wait(&bar_x[(s + 1) & 1], (uint32_t)(((s + 1) >> 1) & 1));
         tc_fence_after();
         if (lane == 0 && hmma) {
-          issue_h_mma<FMT, HH>(tmem + 320, sm0 + ((s + 1) & 1) * SMT + XU, 0, w + 3 * Cfg::BT, 0);
+          issue_h_mma<HH>(tmem + 320, sm0 + ((s + 1) & 1) * SMT + XU, w + 3 * Cfg::BT);
           umma_commit(&bar_h);
         }
         __syncwarp();
@@ -1279,9 +1025,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_cell_bwd_tc(TcArgs a) {
 #pragma unroll
       for (int k = 0; k < 4; ++k) {
         const int row = lane + 32 * k;
-        store_small8<FMT, HH>(sm, 0, row, 0, sv[k]);
-        store_small8<FMT, HH>(sm, 0, row, 8, xv[k]);
-        store_small8<FMT, HH>(sm, 0, row, 16, uv[k]);
+        store_small8(sm, row, 0, sv[k]);
+        store_small8(sm, row, 8, xv[k]);
+        store_small8(sm, row, 16, uv[k]);
         *reinterpret_cast<uint4*>(sm + chunk_off(row, 3, TC_ROWS)) = make_uint4(0x00003F80u, 0, 0, 0);  // bf16 1.0
       }
       fence_proxy_async();
@@ -1289,9 +1035,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_cell_bwd_tc(TcArgs a) {
       if (lane == 0) mbar_arrive(&bar_x[s & 1]);
     }
   }
-  if (a.dbg && blockIdx.x == 0 && tid == 0) a.dbg[241] = clock64();
   __syncthreads();
-  if (a.dbg && blockIdx.x == 0 && tid == 0) a.dbg[242] = clock64();
   if (warp == WARP_MMA) tmem_dealloc(tmem, 512);
 }
 
@@ -1376,16 +1120,16 @@ int launch_reduce_splits(const float* part, float* out, long long count, int spl
 
 int cell_backward_tc(const regt_args* a, const Layout& L, cudaStream_t st) {
   REGT_CHECK(a->precision == REGT_PREC_BF16,
-             "the tensor-core backward is built for precision bf16 only (tf32x3 is forward-only); use fp32 or bf16 to train");
+             "the tensor-core cell backward is built for precision bf16 only");
   REGT_CHECK(a->H == 64 && a->mode != REGT_MODE_TGCN, "tensor-core backward: hidden=64, TemporalGCN / RegionalTemporalGCN only");
   constexpr int HH = 64;
-  using Cfg = TcCfg<FMT_BF16, HH>;
+  using Cfg = TcCfg<HH>;
   const int slots = num_sms();
   TcArgs k = make_tcargs(a, L, slots);
   k.img = L.tc_img_b;
   const int grid = min(min(slots, k.items), TC_MAX_CTAS);
   const size_t smem = 1024 + ((Cfg::BWD_IMG + 1023) & ~1023) + 6 * Cfg::A_TILE + 2 * 4 * TC_ROWS * 16 +
-                      3 * PlaneIO<FMT_BF16, HH>::TILE_BYTES + TC_ROWS * HH * 4;
+                      3 * PlaneIO<__nv_bfloat16, HH>::TILE_BYTES + TC_ROWS * HH * 4;
   REGT_CUDA(cudaFuncSetAttribute(k_cell_bwd_tc<HH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   // the head's partial sums (left by the tensor-core head in regt_head_forward) are reduced beside the cell backward
   const bool head_sum = head_tc_usable(a);

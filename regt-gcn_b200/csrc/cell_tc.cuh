@@ -7,31 +7,25 @@ namespace regt {
 
 constexpr int TC_ROWS = 128;  // rows (b,n) per tile = UMMA M = TMEM lanes
 
-// Byte layout of the per-step weight image (built by k_pack_tc, copied verbatim to shared memory).
-// NSPLIT = 2 for tf32x3 (hi | lo tiles), 1 for bf16.
-template <int FMT, int HH>
+// Byte layout of the per-step weight image (built by k_pack_tc, copied verbatim to shared memory): bf16 operand tiles.
+template <int HH>
 struct TcCfg {
-  static constexpr int ES = (FMT == tc::FMT_TF32) ? 4 : 2;       // operand element size
-  static constexpr int NSPLIT = (FMT == tc::FMT_TF32) ? 2 : 1;
-  static constexpr int UK = (FMT == tc::FMT_TF32) ? 8 : 16;      // K per MMA
+  static constexpr int ES = 2;                                     // operand element size (bf16)
+  static constexpr int UK = 16;                                    // K per MMA
   static constexpr int KBYTES = HH * ES;                          // bytes along K of the H-wide part
   static constexpr int A_TILE = TC_ROWS * KBYTES;                 // one [128 x HH] SW128 tile
-  static constexpr int AS_TILE = 2 * TC_ROWS * 16;                // chunk tile, 2 chunks (one k-step)
   // forward weights (B operands, K-major): rows = output features
   static constexpr int WZR_H = 2 * HH * KBYTES;
   static constexpr int WZR_S = 2 * (2 * HH) * 16;
   static constexpr int WC_H = HH * KBYTES;
   static constexpr int WC_S = 2 * HH * 16;
   // regional combine on the tensor core: B0[n][k] = (M0 | M1[0]) (K = 16 = X | U), chunk tile of HH rows
-  static constexpr int W0 = (FMT == tc::FMT_TF32 ? 4 : 2) * HH * 16;
-  static constexpr int FWD_SPLIT = WZR_H + WZR_S + WC_H + WC_S + W0;   // per split, all multiples of 1024
+  static constexpr int W0 = 2 * HH * 16;
   static constexpr int OFF_W0 = WZR_H + WZR_S + WC_H + WC_S;
-  // small per-row operand tile of the forward ([chunk][row][16 B]): S (+pad) | X | U
-  static constexpr int SMF_CHUNKS = (FMT == tc::FMT_TF32) ? 6 : 4;
-  static constexpr int SMF_TILE = SMF_CHUNKS * TC_ROWS * 16;
+  static constexpr int FWD_W = OFF_W0 + W0;                       // all parts multiples of 1024
+  // small per-row operand tile of the forward ([chunk][row][16 B]): S (+pad) | X | U, double-buffered
+  static constexpr int SMF_TILE = 4 * TC_ROWS * 16;
   static constexpr int SMF_XU_CHUNK = 2;                           // first chunk of the X | U part
-  static constexpr bool PIPE = (FMT == tc::FMT_BF16);             // double-buffer the small tile
-  static constexpr int FWD_W = NSPLIT * FWD_SPLIT;
   // fp32 constants after the tiles
   static constexpr int C_CZR = 0, C_CC = 2 * HH, C_C0 = 3 * HH, C_M0 = 4 * HH, C_M1 = 4 * HH + 8 * HH,
                        C_PROBS = 4 * HH + 16 * HH, C_FLOATS = 4 * HH + 16 * HH + 64;
@@ -39,8 +33,7 @@ struct TcCfg {
   // backward weights (B operands of the data gradients, K-major over the gate index n):
   //   Bt_g[k][n] = linear_g.weight[n][HH + k]      rows = k (hidden input index), K = n
   static constexpr int BT = HH * KBYTES;
-  static constexpr int BWD_SPLIT = 3 * BT + W0;
-  static constexpr int BWD_W = NSPLIT * BWD_SPLIT;
+  static constexpr int BWD_W = 3 * BT + W0;
   static constexpr int BWD_IMG = BWD_W + C_FLOATS * 4;
   static_assert(KBYTES % 128 == 0, "H-wide operand must be whole 128-byte swizzle blocks");
 };
@@ -60,7 +53,6 @@ struct TcArgs {
   float* dhp;              // d h_pre plane [T][nqt][H/4][128][4] (regional wgrad of M1)
   float* wpart;            // [grid][...] per-CTA weight-gradient partials
   float* dprobs_part;      // [grid][T]
-  long long* dbg;          // optional phase timestamps (REGT_TC_DEBUG)
 };
 
 }  // namespace regt

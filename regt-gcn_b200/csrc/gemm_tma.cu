@@ -1,10 +1,9 @@
-// TMA-fed 3xTF32 GEMMs (second generation of gemm_tc.cu: same contracts, same accuracy).
+// TMA-fed 3xTF32 GEMMs.
 //
-// gemm_tc.cu's loader warps pull their operands through registers, one chunk ahead: ~36 KB in flight per SM, and the
-// kernels ran latency-bound (20-35 % of their HBM / tensor roofline).  Here a single producer thread keeps whole
-// pipeline stages in flight with cp.async.bulk.tensor (TMA, SWIZZLE_128B boxes landing directly in the UMMA
-// operand layout), converter warps do the tf32 hi/lo split in shared memory, one thread issues the tcgen05 MMAs
-// into TMEM, and epilogue warps drain the accumulators.
+// A single producer thread keeps whole pipeline stages in flight with cp.async.bulk.tensor (TMA, SWIZZLE_128B boxes
+// landing directly in the UMMA operand layout), converter warps do the tf32 hi/lo split in shared memory, one thread issues
+// the tcgen05 MMAs into TMEM, and epilogue warps drain the accumulators.  (Loader warps that pulled the operands through
+// registers, one chunk ahead, kept ~36 KB in flight per SM and ran latency-bound at 20-35 % of the HBM / tensor roofline.)
 //
 //   gemm_nt : C[M][N] = A[M][K] . Bt[N][K]^T
 //             A chunks [128 rows][32 k] arrive as fp32; the converters overwrite them with hi = tf32(a) and write
@@ -21,11 +20,6 @@
 
 namespace regt {
 using namespace tc;
-
-int launch_gemm_nt_tf32x3(const float* A, long long lda, const float* Bt, long long ldb, float* C, long long ldc, long long M,
-                          int N, int K, cudaStream_t st);
-int launch_gemm_tn_tf32x3(const float* A, long long lda, const float* B, long long ldb, float* Cp, long long M, int K, int N,
-                          int splits, cudaStream_t st, const float* B2, long long ldb2, float* Cp2, long long c2_split, int relu_b);
 
 namespace {
 constexpr int KC = 32;               // contraction chunk: 32 fp32 = one 128-byte swizzle row
@@ -339,14 +333,8 @@ constexpr int TN_CV = 2 * TILE + 2 * TN_BT;   // A hi | A lo | B hi | B lo
 // chained into one accumulator (measured ~2e-8 relative per MMA).  A row contraction chains 12 MMAs per chunk over up to
 // 10^5 rows, so the TMEM accumulator is drained into fp32 registers (round-to-nearest adds) every TN_GROUP chunks; two
 // accumulators alternate so the drain of group g runs under the MMAs of group g + 1.
-#ifndef REGT_TN_GROUP
-#define REGT_TN_GROUP 8
-#endif
-constexpr int TN_GROUP = REGT_TN_GROUP;
-#ifndef REGT_TN_ACC
-#define REGT_TN_ACC 256
-#endif
-constexpr int TN_ACC = REGT_TN_ACC;           // TMEM column stride between the two accumulators (each 128 + 32 feature columns wide)
+constexpr int TN_GROUP = 8;
+constexpr int TN_ACC = 256;                   // TMEM column stride between the two accumulators (each 128 + 32 feature columns wide)
 static_assert(TN_NR * TN_RAW + TN_NC * TN_CV <= SMEM_BUDGET, "gemm_tn stages exceed shared memory");
 
 __global__ void __launch_bounds__(TN_THREADS, 1) k_gemm_tn_tma(const __grid_constant__ TnArgs a) {
@@ -437,7 +425,6 @@ __global__ void __launch_bounds__(TN_THREADS, 1) k_gemm_tn_tma(const __grid_cons
         for (int c = 0; c < 4; ++c) bv[c] = make_float4(fmaxf(bv[c].x, 0.f), fmaxf(bv[c].y, 0.f), fmaxf(bv[c].z, 0.f), fmaxf(bv[c].w, 0.f));
       }
       if (n2) fv = *reinterpret_cast<const float4*>(rw + 8 * TN_BOX + lane * 128 + ((warp ^ (lane & 7)) << 4));
-#if !defined(REGT_TN_LATE)
       {   // The raw stage is refilled by TMA once all 256 threads have arrived, and an mbarrier arrive does NOT wait for
           // this thread's earlier shared-memory loads to return (observed on B200: the tail loads of a warp read the
           // NEXT chunk's bytes).  A branch on the loaded values forces their completion before the arrive issues.
@@ -447,7 +434,6 @@ __global__ void __launch_bounds__(TN_THREADS, 1) k_gemm_tn_tma(const __grid_cons
         if (dep == 0x7FC0DEADu) __nanosleep(1);
         mbar_arrive(&bar_rfree[rs]);
       }
-#endif
       if (kc >= TN_NC) mbar_wait(&bar_empty[cs], (uint32_t)((kc / TN_NC - 1) & 1));
       // the MMAs of chunks <= kc - TN_NC have completed: group g is whole once (g + 1) * TN_GROUP - 1 <= kc - TN_NC
       if (kc >= TN_GROUP + TN_NC - 1 && (kc - (TN_NC - 1)) % TN_GROUP == 0) {
@@ -487,9 +473,6 @@ __global__ void __launch_bounds__(TN_THREADS, 1) k_gemm_tn_tma(const __grid_cons
       }
       fence_proxy_async();
       mbar_arrive(&bar_full[cs]);
-#if defined(REGT_TN_LATE)
-      mbar_arrive(&bar_rfree[rs]);
-#endif
     }
     // ---- epilogue: remaining groups, then the partial tile -> Cp[z] (an empty split contributes zeros) ----
     const int ngroups = (nchunks + TN_GROUP - 1) / TN_GROUP;
@@ -513,17 +496,10 @@ __global__ void __launch_bounds__(TN_THREADS, 1) k_gemm_tn_tma(const __grid_cons
     for (int kc = 0; kc < nchunks; ++kc) {
       const int s = kc % TN_NC;
       const int g = kc / TN_GROUP, buf = g & 1, kg0 = kc % TN_GROUP;
-#if defined(REGT_TN_SERIAL)
-      if (kg0 == 0 && g >= 1) {   // diagnostic: no MMA while the previous group is being drained
-        mbar_wait(&bar_acc_free[(g - 1) & 1], (uint32_t)(((g - 1) / 2) & 1));
-        tc_fence_after();
-      }
-#else
       if (kg0 == 0 && g >= 2) {   // the converters have drained this accumulator's previous group (g - 2)
         mbar_wait(&bar_acc_free[buf], (uint32_t)((g / 2 - 1) & 1));
         tc_fence_after();
       }
-#endif
       mbar_wait(&bar_full[s], (uint32_t)((kc / TN_NC) & 1));
       tc_fence_after();
       if (lane == 0) {
@@ -774,27 +750,17 @@ __global__ void __launch_bounds__(TN_THREADS, 1) k_gemm_kt(const __grid_constant
   __syncthreads();
   if (warp == TN_W_MMA) tmem_dealloc(tmem, 512);
 }
-
-bool legacy_forced() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("REGT_GEMM_LEGACY");
-    v = (e && e[0] == '1') ? 1 : 0;
-  }
-  return v == 1;
-}
 }  // namespace
 
 size_t gemm_nt_scratch_floats(int N, int K) { return (size_t)2 * ((N + 127) / 128 * 128) * ((K + KC - 1) / KC * KC); }
 
-// C[M][N] = A[M][K] . Bt[N][K]^T ; `scratch` (gemm_nt_scratch_floats(N, K) floats) receives the hi / lo images of Bt.
-// Falls back to the register-fed kernel when the TMA preconditions do not hold.
+// C[M][N] = A[M][K] . Bt[N][K]^T for any M >= 1 (TMA zero-fills the rows of the last tile past M; they are not stored);
+// `scratch` (gemm_nt_scratch_floats(N, K) floats) receives the hi / lo images of Bt.
 int launch_gemm_nt_tma(const float* A, long long lda, const float* Bt, long long ldb, float* C, long long ldc, long long M, int N,
                        int K, float* scratch, cudaStream_t st) {
-  if (legacy_forced() || !scratch || M < 128 || N % 16 != 0 || K % 4 != 0 || lda % 4 != 0 || ((uintptr_t)A % 16) != 0 ||
-      ((uintptr_t)scratch % 16) != 0)
-    return launch_gemm_nt_tf32x3(A, lda, Bt, ldb, C, ldc, M, N, K, st);
-  REGT_CHECK(A && Bt && C && N > 0 && K > 0 && ldc % 4 == 0 && ((uintptr_t)C % 16) == 0, "gemm_nt_tma: bad operands");
+  REGT_CHECK(A && Bt && C && scratch && M >= 1 && N > 0 && N % 16 == 0 && K > 0 && K % 4 == 0 && ldc % 4 == 0 &&
+                 ((uintptr_t)C % 16) == 0 && ((uintptr_t)scratch % 16) == 0,
+             "gemm_nt_tma: bad operands (M=%lld N=%d K=%d)", M, N, K);
   const int Np = (N + 127) / 128 * 128, Kp = (K + KC - 1) / KC * KC, nchunks = Kp / KC;
   float* hi = scratch;
   float* lo = scratch + (size_t)Np * Kp;
@@ -825,7 +791,7 @@ int launch_gemm_nt_tma(const float* A, long long lda, const float* Bt, long long
 int launch_gemm_tn_tma(const float* A, long long lda, long long M, int Ktot, int nseg, const int* seg_k0, const int* seg_b,
                        float* const* seg_C, const float* const* Bs, const long long* ldbs, int N, int splits, const float* B2,
                        long long ldb2, float* C2, long long c2_split, cudaStream_t st, int relu_b) {
-  REGT_CHECK(A && nseg >= 1 && nseg <= 4 && Ktot % 32 == 0 && N % 32 == 0 && splits > 0 && M >= 32, "gemm_tn_tma: bad shape");
+  REGT_CHECK(A && nseg >= 1 && nseg <= 4 && Ktot % 32 == 0 && N % 32 == 0 && splits > 0 && M >= 1, "gemm_tn_tma: bad shape");
   REGT_CHECK(!B2 || (C2 && ldb2 % 4 == 0), "gemm_tn_tma: bad second operand");
   TnArgs a{};
   if (tmap_2d(&a.ta, A, Ktot, M, lda, 32, "gemm_tn_tma(A)")) return -1;
@@ -899,12 +865,9 @@ int launch_gemm_kt(const float* AT, long long ntile, int Ktot, int nseg, const i
   return 0;
 }
 
-// drop-in for launch_gemm_tn_tf32x3 (single segment); falls back when the TMA preconditions do not hold
-int launch_gemm_tn_auto(const float* A, long long lda, const float* B, long long ldb, float* Cp, long long M, int K, int N, int splits,
-                        cudaStream_t st, const float* B2, long long ldb2, float* Cp2, long long c2_split, int relu_b) {
-  const bool ok = !legacy_forced() && M >= 32 && K % 32 == 0 && N % 32 == 0 && lda % 4 == 0 && ((uintptr_t)A % 16) == 0 &&
-                  (N == 0 || (ldb % 4 == 0 && ((uintptr_t)B % 16) == 0)) && (!B2 || ((uintptr_t)B2 % 16) == 0);
-  if (!ok) return launch_gemm_tn_tf32x3(A, lda, B, ldb, Cp, M, K, N, splits, st, B2, ldb2, Cp2, c2_split, relu_b);
+// the single-segment form of launch_gemm_tn_tma: Cp[z][K][N] = partials of A[:, :K]^T . B (no B when N == 0)
+int launch_gemm_tn(const float* A, long long lda, const float* B, long long ldb, float* Cp, long long M, int K, int N, int splits,
+                   cudaStream_t st, const float* B2, long long ldb2, float* Cp2, long long c2_split, int relu_b) {
   const int k0 = 0, sb = N > 0 ? 0 : -1;
   float* cs[1] = {Cp};
   const float* bs[2] = {B, nullptr};
@@ -921,7 +884,7 @@ extern "C" int regt_debug_gemm_nt_tma(const float* A, int64_t lda, const float* 
 }
 extern "C" int regt_debug_gemm_tn_tma(const float* A, int64_t lda, const float* B, int64_t ldb, float* Cp, int64_t M, int32_t K,
                                       int32_t N, int32_t splits, const float* B2, int64_t ldb2, float* Cp2, regt_stream_t stream) {
-  return regt::launch_gemm_tn_auto(A, lda, B, ldb, Cp, M, K, N, splits, (cudaStream_t)stream, B2, ldb2, Cp2, 0, 0);
+  return regt::launch_gemm_tn(A, lda, B, ldb, Cp, M, K, N, splits, (cudaStream_t)stream, B2, ldb2, Cp2, 0, 0);
 }
 // four-segment form used by the cell backward: A = D [M][4H]; segments z|r (B = h), h~ (B = hR), h_pre (B2 only)
 extern "C" int regt_debug_gemm_tn_multi(const float* A, int64_t lda, int64_t M, int32_t H, const float* B0, const float* B1,

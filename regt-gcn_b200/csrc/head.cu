@@ -485,8 +485,8 @@ int head_forward_fp32(const regt_args* a, const Layout& L, cudaStream_t st) {
   return 0;
 }
 
-int launch_gemm_tn_auto(const float* A, long long lda, const float* B, long long ldb, float* Cp, long long M, int K, int N, int splits,
-                        cudaStream_t st, const float* B2, long long ldb2, float* Cp2, long long c2_split, int relu_b);
+int launch_gemm_tn(const float* A, long long lda, const float* B, long long ldb, float* Cp, long long M, int K, int N, int splits,
+                   cudaStream_t st, const float* B2, long long ldb2, float* Cp2, long long c2_split, int relu_b);
 // out[r] (+)= sum over splits of Cp2[s][r][col]   (one column of a [splits][rows][32] partial array)
 __global__ void k_pick_col(const float* __restrict__ Cp2, int splits, int rows, int col, int acc, float* __restrict__ out) {
   const int r = threadIdx.x;
@@ -536,7 +536,7 @@ int head_backward_fp32(const regt_args* a, const Layout& L, cudaStream_t st) {
     const int s1 = (int)max(1ll, min((long long)cdiv(148, cdiv(H, 128)), BN / 256));
     float* p1 = part;                                    // [s1][128][H]
     float* p2 = part + (size_t)s1 * HEAD_HID * H;        // [s1][128][32]
-    if (launch_gemm_tn_auto(L.d_a1, HEAD_HID, a->out_hidden, H, p1, BN, HEAD_HID, H, s1, st, L.Feat, 32, p2, 0, 1)) return -1;
+    if (launch_gemm_tn(L.d_a1, HEAD_HID, a->out_hidden, H, p1, BN, HEAD_HID, H, s1, st, L.Feat, 32, p2, 0, 1)) return -1;
     if (launch_reduce_splits(p1, a->g.head_w1, (long long)HEAD_HID * H, s1, a->accumulate, st)) return -1;
     k_pick_col<<<1, HEAD_HID, 0, st>>>(p2, s1, HEAD_HID, 16, a->accumulate, a->g.head_b1);
     REGT_LAUNCHED("k_pick_col", st);

@@ -12,16 +12,14 @@
 //             dW1, db1 = d_a1^T [relu(hid) | 1]             gemm_tn (tensor cores, as before)
 //             dW2, (colsum a1) = a1^T [d_out | 1]           gemm_tn, feature-plane operand only
 //             db2 = colsum d_out                            k_colsum
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace regt {
 
 int launch_gemm_nt_tma(const float* A, long long lda, const float* Bt, long long ldb, float* C, long long ldc, long long M, int N,
                        int K, float* scratch, cudaStream_t st);
-int launch_gemm_tn_auto(const float* A, long long lda, const float* B, long long ldb, float* Cp, long long M, int K, int N, int splits,
-                        cudaStream_t st, const float* B2, long long ldb2, float* Cp2, long long c2_split, int relu_b);
+int launch_gemm_tn(const float* A, long long lda, const float* B, long long ldb, float* Cp, long long M, int K, int N, int splits,
+                   cudaStream_t st, const float* B2, long long ldb2, float* Cp2, long long c2_split, int relu_b);
 int launch_reduce_splits(const float* part, float* out, long long count, int splits, int accumulate, cudaStream_t st);
 int launch_colsum(const float* A, int lda, int C, long long rows, int splits, float* part, cudaStream_t st);
 
@@ -186,8 +184,7 @@ __global__ void k_hf_pick_col(const float* __restrict__ Cp2, int splits, int row
 }  // namespace
 
 bool head_f_usable(const regt_args* a) {
-  static const bool off = getenv("REGT_HEAD_FFMA") && getenv("REGT_HEAD_FFMA")[0] == '1';
-  return !off && a->precision == REGT_PREC_TF32X3 && a->H % 32 == 0 && a->O <= HF_O && (long long)a->B * a->N >= 128 && a->out;
+  return a->precision == REGT_PREC_TF32X3 && a->H % 32 == 0 && a->O <= HF_O && (long long)a->B * a->N >= 128 && a->out;
 }
 
 int head_forward_f(const regt_args* a, const Layout& L, cudaStream_t st) {
@@ -225,13 +222,13 @@ int head_backward_f(const regt_args* a, const Layout& L, cudaStream_t st, int g_
   const int s1 = (int)max(1ll, min((long long)cdiv(148, cdiv(H, 128)), BN / 256));
   float* p1 = part;                                    // [s1][128][H]    d_a1^T relu(hid)
   float* p2 = part + (size_t)s1 * HEAD_HID * H;        // [s1][128][32]   d_a1^T [. | 1]  -> column 16 = db1
-  if (launch_gemm_tn_auto(L.d_a1, HEAD_HID, a->out_hidden, H, p1, BN, HEAD_HID, H, s1, st, L.hf_do32, 32, p2, 0, 1)) return -1;
+  if (launch_gemm_tn(L.d_a1, HEAD_HID, a->out_hidden, H, p1, BN, HEAD_HID, H, s1, st, L.hf_do32, 32, p2, 0, 1)) return -1;
   if (launch_reduce_splits(p1, a->g.head_w1, (long long)HEAD_HID * H, s1, a->accumulate, st)) return -1;
   k_hf_pick_col<<<1, HEAD_HID, 0, st>>>(p2, s1, HEAD_HID, 16, a->accumulate, a->g.head_b1);
   REGT_LAUNCHED("k_hf_pick_col", st);
   const int s2 = (int)max(1ll, min(148ll, BN / 256));
   float* p3 = part;                                    // [s2][128][32]   a1^T [d_out | 1]
-  if (launch_gemm_tn_auto(L.a1, HEAD_HID, nullptr, 0, nullptr, BN, HEAD_HID, 0, s2, st, L.hf_do32, 32, p3, 0, 0)) return -1;
+  if (launch_gemm_tn(L.a1, HEAD_HID, nullptr, 0, nullptr, BN, HEAD_HID, 0, s2, st, L.hf_do32, 32, p3, 0, 0)) return -1;
   k_hf_dw2<<<cdiv(O * HEAD_HID, 256), 256, 0, st>>>(p3, s2, O, a->accumulate, a->g.head_w2);
   REGT_LAUNCHED("k_hf_dw2", st);
   const int s3 = (int)max(1ll, min(128ll, BN / 128));

@@ -69,7 +69,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_head_tc(HeadTcArgs a) {
   const int O = a.O;
 
   if (tid == 0) {
-    mbar_init(&bar_a0, NEPI_WARPS * ARRIVALS_PER_WARP); mbar_init(&bar_a1, NEPI_WARPS * ARRIVALS_PER_WARP); mbar_init(&bar_a2, NEPI_WARPS * ARRIVALS_PER_WARP); mbar_init(&bar_a3, NEPI_WARPS * ARRIVALS_PER_WARP);
+    mbar_init(&bar_a0, NEPI); mbar_init(&bar_a1, NEPI); mbar_init(&bar_a2, NEPI); mbar_init(&bar_a3, NEPI);
     mbar_init(&bar_m1, 1); mbar_init(&bar_m2, 1); mbar_init(&bar_m3, 1); mbar_init(&bar_m4, 1); mbar_init(&bar_w, 1);
     fence_barrier_init();
   }
@@ -158,7 +158,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_head_tc(HeadTcArgs a) {
       }
       fence_proxy_async();
       tc_fence_before();
-      mbar_arrive_warp(&bar_a0);
+      mbar_arrive(&bar_a0);
 
       // ---- P1: a1 = relu(a1_pre + b1), 64 columns ----
       uint32_t amask[2];
@@ -186,7 +186,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_head_tc(HeadTcArgs a) {
       }
       fence_proxy_async();
       tc_fence_before();
-      mbar_arrive_warp(&bar_a1);
+      mbar_arrive(&bar_a1);
 
       // ---- P2: out, loss, d_out (8 of the 16 padded outputs per thread) ----
       mbar_wait(&bar_m2, ph);
@@ -215,7 +215,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_head_tc(HeadTcArgs a) {
       }
       fence_proxy_async();
       tc_fence_before();
-      mbar_arrive_warp(&bar_a2);
+      mbar_arrive(&bar_a2);
 
       // ---- P3: d a1 = da1_pre * (a1 > 0), 64 columns ----
       mbar_wait(&bar_m3, ph);
@@ -237,7 +237,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_head_tc(HeadTcArgs a) {
       }
       fence_proxy_async();
       tc_fence_before();
-      mbar_arrive_warp(&bar_a3);
+      mbar_arrive(&bar_a3);
 
       // ---- P4: G = G_pre * (hid > 0) (+ d_hidden), 32 columns, tiled layout [qt][HH/4][128][4] ----
       mbar_wait(&bar_m4, ph);

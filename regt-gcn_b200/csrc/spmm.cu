@@ -8,8 +8,6 @@
 //
 // One warp per output row; lane c owns float4 #c of the row (128-bit loads/stores, fully
 // coalesced 384 B per neighbour); edge metadata is read once per warp (uniform address).
-#include <stdlib.h>
-
 #include <vector>
 
 #include "common.cuh"
@@ -324,17 +322,12 @@ int launch_feat_tc(const regt_graph_plan& p, const float* x, int B, int xN, int 
   return 0;
 }
 
-// staged-kernel geometry for rows of `width` floats with `ctas` resident CTAs per SM: row capacity of a block, staged edges
-static inline void spmm_geometry(int width, int ctas, int* nb_cap, int* emax) {
-  *emax = SPMM_EDGES_PER_SM / ctas;
-  *nb_cap = ((227 * 1024) / ctas - 2048 - *emax * 16 - 64) / (width * 4 + 4) / 8 * 8;
-}
-static inline int spmm_ctas() {
-  // resident CTAs per SM.  One 1024-thread CTA with the whole shared memory measured fastest on config 5 (3.07 TB/s against
-  // 2.67 with two CTAs of half the rows: the larger block keeps more neighbours staged, which matters more than overlapping
-  // one CTA's block load with the other's gather).  (REGT_SPMM_CTAS = 1..4: test hook)
-  static const int ctas_env = getenv("REGT_SPMM_CTAS") ? atoi(getenv("REGT_SPMM_CTAS")) : 1;
-  return (ctas_env >= 1 && ctas_env <= 4) ? ctas_env : 1;
+// staged-kernel geometry for rows of `width` floats: row capacity of a block, staged edges.  One 1024-thread CTA per SM with
+// the whole shared memory measured fastest on config 5 (3.07 TB/s against 2.67 with two CTAs of half the rows: the larger
+// block keeps more neighbours staged, which matters more than overlapping one CTA's block load with the other's gather).
+static inline void spmm_geometry(int width, int* nb_cap, int* emax) {
+  *emax = SPMM_EDGES_PER_SM;
+  *nb_cap = (227 * 1024 - 2048 - *emax * 16 - 64) / (width * 4 + 4) / 8 * 8;
 }
 
 int launch_spmm_impl(const int32_t* rowptr, const int32_t* col, const float* val, const float* x, float* y, int B,
@@ -343,15 +336,12 @@ int launch_spmm_impl(const int32_t* rowptr, const int32_t* col, const float* val
   if (B == 0 || n_out == 0) return 0;
   // staged variant: output row r <-> node r (square operator, possibly with halo columns behind the rows), blocks of
   // NB nodes = up to 192 KB of shared memory; small problems keep the plain warp-per-row kernel (less than one wave)
-  static const bool no_blk = getenv("REGT_SPMM_PLAIN") && getenv("REGT_SPMM_PLAIN")[0] == '1';
-  // resident CTAs per SM: each gets its share of the 227 KB, minus the staged CSR slice.  (REGT_SPMM_CTAS = 1, 2, 3, 4: test hook)
-  const int ctas = spmm_ctas();
   const int row_bytes = width * 4;
   int emax, NB;
-  spmm_geometry(width, ctas, &NB, &emax);
+  spmm_geometry(width, &NB, &emax);
   REGT_CHECK(!blk_ptr || (NB >= 32 && n_out == n_in && nblk_p > 0 && ((uintptr_t)x % 16) == 0),
              "spmm: a partition needs a square operator, 16-byte aligned x and rows that fit the staged kernel (width %d)", width);
-  if (blk_ptr || (!no_blk && n_out <= n_in && NB >= 32 && (long long)B * n_out >= 4096 && ((uintptr_t)x % 16) == 0)) {
+  if (blk_ptr || (n_out <= n_in && NB >= 32 && (long long)B * n_out >= 4096 && ((uintptr_t)x % 16) == 0)) {
     int nblk = nblk_p;
     if (!blk_ptr) {
       NB = min(NB, (n_out + 7) / 8 * 8);
@@ -366,17 +356,9 @@ int launch_spmm_impl(const int32_t* rowptr, const int32_t* col, const float* val
       if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sms <= 0) sms = 148;
     }
     const long long items = (long long)B * nblk;
-    const int grid = (int)min(items, (long long)ctas * sms);
-#define REGT_SPMM_LAUNCH(NT, MINB)                                                                                                 \
-  do {                                                                                                                             \
-    REGT_CUDA(cudaFuncSetAttribute(k_spmm_blk<NT, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                 \
-    k_spmm_blk<NT, MINB><<<grid, NT, smem, st>>>(rowptr, col, val, (const float4*)x, (float4*)y, B, n_out, n_in, width / 4, NB, nblk, blk_ptr); \
-  } while (0)
-    if (ctas == 1) REGT_SPMM_LAUNCH(1024, 1);
-    else if (ctas == 3) REGT_SPMM_LAUNCH(320, 3);
-    else if (ctas == 4) REGT_SPMM_LAUNCH(256, 4);
-    else REGT_SPMM_LAUNCH(512, 2);
-#undef REGT_SPMM_LAUNCH
+    const int grid = (int)min(items, (long long)sms);
+    REGT_CUDA(cudaFuncSetAttribute(k_spmm_blk<1024, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k_spmm_blk<1024, 1><<<grid, 1024, smem, st>>>(rowptr, col, val, (const float4*)x, (float4*)y, B, n_out, n_in, width / 4, NB, nblk, blk_ptr);
     REGT_LAUNCHED("k_spmm_blk", st);
     return 0;
   }
@@ -472,7 +454,7 @@ extern "C" int regt_scatter_rows(const float* src, const int64_t* idx, float* ds
 extern "C" int32_t regt_spmm_partition_capacity(int32_t N, int32_t width) {
   if (N <= 0 || width <= 0 || width % 4) return 0;
   int nb, emax;
-  regt::spmm_geometry(width, regt::spmm_ctas(), &nb, &emax);
+  regt::spmm_geometry(width, &nb, &emax);
   if (nb < 32) return 0;                                // rows too wide for the staged kernel: no partition
   return N + 2;                                         // worst case: one block per row (rows with more edges than a block stages)
 }
@@ -482,7 +464,7 @@ extern "C" int regt_spmm_partition(const int32_t* rowptr, const int32_t* col, in
   REGT_CHECK(regt_spmm_partition_capacity(N, width) > 0, "spmm_partition: N %d / width %d not supported by the staged kernel", N, width);
   cudaStream_t st = (cudaStream_t)stream;
   int nb, emax;
-  regt::spmm_geometry(width, regt::spmm_ctas(), &nb, &emax);
+  regt::spmm_geometry(width, &nb, &emax);
   std::vector<int32_t> rp((size_t)N + 1);
   REGT_CUDA(cudaMemcpyAsync(rp.data(), rowptr, sizeof(int32_t) * ((size_t)N + 1), cudaMemcpyDeviceToHost, st));
   REGT_CUDA(cudaStreamSynchronize(st));
@@ -502,7 +484,7 @@ extern "C" int regt_debug_spmm_partition_host(const int32_t* rowptr, const int32
                                               int32_t* nblk_out, int32_t* cap_out) {
   REGT_CHECK(rowptr && col && blk_ptr && nblk_out && N > 0 && width > 0 && width % 4 == 0, "spmm_partition_host: bad arguments");
   int nb, emax;
-  regt::spmm_geometry(width, regt::spmm_ctas(), &nb, &emax);
+  regt::spmm_geometry(width, &nb, &emax);
   REGT_CHECK(nb >= 32, "spmm_partition_host: rows of %d floats do not fit the staged kernel", width);
   std::vector<int32_t> rp(rowptr, rowptr + N + 1), cj(col, col + rowptr[N]), blk;
   *nblk_out = regt::spmm_partition_host(rp, cj, N, nb, emax, &blk);

@@ -28,20 +28,6 @@ __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
   asm volatile("{\n\t.reg .b64 st;\n\tmbarrier.arrive.shared::cta.b64 st, [%0];\n\t}" ::"r"(smem_u32(bar)) : "memory");
 }
-// one arrival per WARP: every lane has fenced its own writes; lane 0 arrives after the warp converges.
-// (hundreds of per-thread arrivals on one mbarrier serialise on the same shared-memory word)
-#ifndef REGT_WARP_ARRIVE
-#define REGT_WARP_ARRIVE 0   // A/B on B200: per-thread arrivals are not slower (159.5 vs 160.8 us per step)
-#endif
-constexpr int ARRIVALS_PER_WARP = REGT_WARP_ARRIVE ? 1 : 32;   // mbar_init count = warps * ARRIVALS_PER_WARP
-__device__ __forceinline__ void mbar_arrive_warp(uint64_t* bar) {
-#if REGT_WARP_ARRIVE
-  __syncwarp();
-  if ((threadIdx.x & 31) == 0) mbar_arrive(bar);
-#else
-  mbar_arrive(bar);
-#endif
-}
 __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
   asm volatile("{\n\t.reg .b64 st;\n\tmbarrier.arrive.expect_tx.shared::cta.b64 st, [%0], %1;\n\t}" ::"r"(smem_u32(bar)),
                "r"(bytes)

@@ -67,9 +67,6 @@ _lib = None
 
 
 def lib_path() -> str:
-    alt = os.environ.get("REGT_B200_LIB")   # experiment builds (csrc/build.py build_variant)
-    if alt:
-        return alt
     return os.path.normpath(os.path.join(_HERE, "..", "lib", "libregt_b200.so"))
 
 
@@ -153,13 +150,6 @@ def load() -> C.CDLL:
     lib.regt_rmsprop_step.argtypes = [vp, vp, vp, C.c_int64, C.c_float, C.c_float, C.c_float, C.c_float, vp]
     lib.regt_eval_metrics.restype = C.c_int
     lib.regt_eval_metrics.argtypes = [vp, vp, C.c_int32, C.c_int64, C.c_double, vp, vp]
-    lib.regt_debug_gemm_nt.restype = C.c_int
-    lib.regt_debug_gemm_nt.argtypes = [vp, C.c_int64, vp, C.c_int64, vp, C.c_int64, C.c_int64, C.c_int32, C.c_int32, vp]
-    lib.regt_debug_gemm_tn.restype = C.c_int
-    lib.regt_debug_gemm_tn.argtypes = [vp, C.c_int64, vp, C.c_int64, vp, C.c_int64, C.c_int32, C.c_int32, C.c_int32, vp]
-    lib.regt_debug_gemm_tn2.restype = C.c_int
-    lib.regt_debug_gemm_tn2.argtypes = [vp, C.c_int64, vp, C.c_int64, vp, C.c_int64, C.c_int32, C.c_int32, C.c_int32,
-                                        vp, C.c_int64, vp, vp]
     lib.regt_debug_gemm_nt_tma.restype = C.c_int
     lib.regt_debug_gemm_nt_tma.argtypes = [vp, C.c_int64, vp, C.c_int64, vp, C.c_int64, C.c_int64, C.c_int32, C.c_int32, vp, vp]
     lib.regt_debug_gemm_tn_tma.restype = C.c_int

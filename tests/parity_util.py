@@ -24,6 +24,21 @@ def is_dead(model_name: str, key: str) -> bool:
     return model_name == "TemporalGCN" and key.startswith("tgnn.linear.")
 
 
+def profiled(fn):
+    """run ``fn`` with the library's launch recorder on; returns (fn's result, names of the kernels it launched)."""
+    from regt_b200 import _lib
+    lib = _lib.load()
+    torch.cuda.synchronize()
+    lib.regt_profile(1, torch.cuda.current_stream().cuda_stream)
+    try:
+        res = fn()
+        torch.cuda.synchronize()
+        names = {n for n, _ in _lib.profile_read()}
+    finally:
+        lib.regt_profile(0, None)
+    return res, names
+
+
 def build_oracle(w, dtype=torch.float64, seed=1234):
     from oracle import regt_oracle as O
     torch.manual_seed(0)

@@ -5,7 +5,7 @@ import numpy as np
 import pytest
 import torch
 
-from parity_util import W, build_cuda, is_dead, oracle_step, relerr, to_dev
+from parity_util import W, build_cuda, is_dead, oracle_step, profiled, relerr, to_dev
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-5
@@ -21,7 +21,15 @@ def _cases():
     c.append((W.make_workload(1), 1))      # TPIMS, reference defaults H=256 R=5
     c.append((W.make_workload(2), 2))      # METR-LA shape, sub-batch
     c.append((W.make_workload(3), 1))      # PEMS-BAY shape, H=256 R=12, sub-batch
+    # fewer than 32 rows B*N*T, run at tf32x3 (_precision): the GEMM-by-GEMM cell of cell_g.cu with less than one TMA box
+    # of rows, through the merged four-segment weight-gradient launch (H = 256) and the single-segment one (H = 32)
+    c.append((W.tiny_workload("RegionalTemporalGCN", N=7, T=2, H=256, O=2, R=2, B=2, seed=25), 2))
+    c.append((W.tiny_workload("TemporalGCN", N=5, T=3, H=32, O=2, R=0, B=2, seed=26), 2))
     return c
+
+
+def _precision(w, B):
+    return "tf32x3" if B * w.N * w.T < 32 else "fp32"
 
 
 def _compare(w, B, cuda_out, cuda_hid, cuda_loss, cuda_grads, ref):
@@ -43,7 +51,8 @@ def _compare(w, B, cuda_out, cuda_hid, cuda_loss, cuda_grads, ref):
 @pytest.mark.parametrize("w,B", _cases(), ids=lambda v: v.name if hasattr(v, "name") else str(v))
 def test_autograd_path_matches_oracle(w, B):
     ref = oracle_step(w, B)
-    m = build_cuda(w, ref["state"])
+    prec = _precision(w, B)
+    m = build_cuda(w, ref["state"], precision=prec)
     x, y = w.inputs(B)
     x, y = x.cuda(), y.cuda()
     out, hid = m(x, *to_dev(w.graph_args(), "cuda"))
@@ -53,12 +62,16 @@ def test_autograd_path_matches_oracle(w, B):
     _compare(w, B, out, hid, loss, grads, ref)
 
 
-@pytest.mark.parametrize("w,B", _cases()[:5] + _cases()[6:8], ids=lambda v: v.name if hasattr(v, "name") else str(v))
+@pytest.mark.parametrize("w,B", _cases()[:5] + _cases()[6:8] + _cases()[9:], ids=lambda v: v.name if hasattr(v, "name") else str(v))
 def test_fused_step_matches_oracle(w, B):
     ref = oracle_step(w, B)
-    m = build_cuda(w, ref["state"])
+    prec = _precision(w, B)
+    m = build_cuda(w, ref["state"], precision=prec)
     x, y = w.inputs(B)
-    loss, out, hid = m.fused_step(x.cuda(), y.cuda(), *to_dev(w.graph_args(), "cuda"))
+    (loss, out, hid), names = profiled(lambda: m.fused_step(x.cuda(), y.cuda(), *to_dev(w.graph_args(), "cuda")))
+    if prec == "tf32x3":
+        for k in ("k_gemm_nt_tma_ts", "k_gemm_tn_tma"):
+            assert k in names, (k, sorted(names))
     grads = {k: p.grad for k, p in m.named_parameters()}
     _compare(w, B, out, hid, loss, grads, ref)
     # a second call accumulates (run.py:190: grads accumulate over snapshots until optimizer.step)

@@ -18,27 +18,12 @@ import functools
 import pytest
 import torch
 
-from parity_util import W, build_cuda, build_oracle, is_dead, oracle_step, relerr, to_dev, twin_limits
+from parity_util import W, build_cuda, build_oracle, is_dead, oracle_step, profiled, relerr, to_dev, twin_limits
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-5
 ATT_TOL = 1e-4
 FUSED = ("k_cell_fwd_f", "k_cell_bwd_f")
-
-
-def _profiled(fn):
-    """run ``fn`` with the library's launch recorder on; returns (fn's result, names of the kernels it launched)."""
-    from regt_b200 import _lib
-    lib = _lib.load()
-    torch.cuda.synchronize()
-    lib.regt_profile(1, torch.cuda.current_stream().cuda_stream)
-    try:
-        res = fn()
-        torch.cuda.synchronize()
-        names = {n for n, _ in _lib.profile_read()}
-    finally:
-        lib.regt_profile(0, None)
-    return res, names
 
 
 def _profiled_autograd(forward, loss_of):
@@ -47,7 +32,7 @@ def _profiled_autograd(forward, loss_of):
     node switch the recorder on and off around it there."""
     from regt_b200 import _lib
     lib = _lib.load()
-    (out, hid), names = _profiled(forward)
+    (out, hid), names = profiled(forward)
 
     def pre(grad_outputs):
         lib.regt_profile(1, torch.cuda.current_stream().cuda_stream)
@@ -126,7 +111,7 @@ def test_micro_batched_step_matches_oracle(key, mb):
     x, y = x.cuda(), y.cuda()
     g = to_dev(w.graph_args(), "cuda")
     m = build_cuda(w, ref["state"], precision="tf32x3")
-    (loss, out, hid), names = _profiled(lambda: m.fused_step(x, y, *g, micro_batch=mb or B))
+    (loss, out, hid), names = profiled(lambda: m.fused_step(x, y, *g, micro_batch=mb or B))
     for k in FUSED + ("k_wgrad_m1_kt", "k_chain", "k_hf_mid"):
         assert k in names, (k, sorted(names))
     _check(w, ref, lims, loss, out, hid, _grads(m), f"{key}/mb={mb}")
@@ -154,8 +139,8 @@ def test_grouped_dm1_contraction_matches_oracle(key):
     assert bper > 1 and B % bper != 0, (B, w.R, bper, nbg)      # the case still exercises what it is named for
     x, y = w.inputs(B)
     m = build_cuda(w, ref["state"], precision="tf32x3")
-    (loss, out, hid), names = _profiled(lambda: m.fused_step(x.cuda(), y.cuda(), *to_dev(w.graph_args(), "cuda"),
-                                                             micro_batch=B))
+    (loss, out, hid), names = profiled(lambda: m.fused_step(x.cuda(), y.cuda(), *to_dev(w.graph_args(), "cuda"),
+                                                            micro_batch=B))
     for k in FUSED + ("k_wgrad_m1_kt",):
         assert k in names, (k, sorted(names))
     _check(w, ref, lims, loss, out, hid, _grads(m), key)
@@ -203,7 +188,7 @@ def test_graph_replay_matches_eager_and_follows_inplace_updates():
     # the graph's content is first seen through other tensors (as after the reference's per-snapshot .to(device)): the
     # capture below must still find the plan by the identity of ``g`` without hashing or building it on the device
     m.fused_step(xs, ys, *[t.clone() for t in g], micro_batch=4)
-    _, names = _profiled(step)                      # eager warm-up: creates .grad, the workspace and the plan
+    _, names = profiled(step)                      # eager warm-up: creates .grad, the workspace and the plan
     for k in FUSED + ("k_wgrad_m1_kt", "k_hf_mid"):
         assert k in names, (k, sorted(names))
     s = torch.cuda.Stream()
@@ -291,6 +276,9 @@ _POISON_CASES = {
                                FUSED + ("k_wgrad_m1_kt", "k_hf_mid")),
     "unfused_h128": (lambda: W.tiny_workload("RegionalTemporalGCN", N=700, T=4, H=128, O=4, R=5, B=3, seed=9), 3,
                      "tf32x3", "fused", "1", ("k_g_zr", "k_g_b1")),
+    # 2 * 20 * 3 = 120 rows: fewer than one 128-row tile of the GEMMs (TMA reads the rows past M as zeros)
+    "unfused_h128_one_partial_tile": (lambda: W.tiny_workload("RegionalTemporalGCN", N=20, T=3, H=128, O=4, R=3, B=2, seed=10), 2,
+                                      "tf32x3", "fused", "1", ("k_g_zr", "k_gemm_nt_tma_ts", "k_gemm_tn_tma")),
     "fp32_h64": (lambda: W.tiny_workload("RegionalTemporalGCN", N=300, T=6, H=64, O=5, R=7, B=3, seed=31, k_intra=4), 3,
                  "fp32", "fused", "0", ("k_cell_fwd", "k_cell_bwd")),
     "bf16_h64": (lambda: W.tiny_workload("TemporalGCN", N=150, T=12, H=64, O=12, R=0, B=3, seed=7, k_intra=5), 3,
@@ -322,7 +310,7 @@ def _run_on_workspace(w, B, precision, path, poison):
 
     if path == "fused":
         m._ws = ws_for(y=y, fuse_head=True)
-        (loss, out, hid), names = _profiled(lambda: m.fused_step(x, y, *g, micro_batch=B))
+        (loss, out, hid), names = profiled(lambda: m.fused_step(x, y, *g, micro_batch=B))
         return (loss, out, hid), _grads(m), names
     if path == "inference":
         def fwd():
@@ -330,7 +318,7 @@ def _run_on_workspace(w, B, precision, path, poison):
                                     workspace=ws_for(inference=True))
             engine.run_forward(st, True)
             return st.out, st.out_hidden
-        (out, hid), names = _profiled(fwd)
+        (out, hid), names = profiled(fwd)
         return (None, out, hid), {}, names
 
     def fwd_bwd():
@@ -340,7 +328,7 @@ def _run_on_workspace(w, B, precision, path, poison):
         grads = {k: torch.empty_like(t) for k, t in params.items()}
         engine.run_backward(st, grads, d_out, None, False, True)
         return st.out, st.out_hidden, grads
-    (out, hid, grads), names = _profiled(fwd_bwd)
+    (out, hid, grads), names = profiled(fwd_bwd)
     return (None, out, hid), grads, names
 
 
@@ -387,7 +375,7 @@ def test_fused_period_counts_match_oracle(model, T):
     lims, _ = twin_limits(w, B, ref)
     m = build_cuda(w, ref["state"], precision="auto")       # the default picks the fused kernels up to 64 periods
     x, y = w.inputs(B)
-    (loss, out, hid), names = _profiled(lambda: m.fused_step(x.cuda(), y.cuda(), *to_dev(w.graph_args(), "cuda")))
+    (loss, out, hid), names = profiled(lambda: m.fused_step(x.cuda(), y.cuda(), *to_dev(w.graph_args(), "cuda")))
     for k in FUSED + ("k_f_sum_dpp",):
         assert k in names, (k, sorted(names))
     grads = _grads(m)
@@ -407,7 +395,7 @@ def test_65_periods_auto_runs_fp32_kernels():
     m = build_cuda(w, ref["state"], precision="auto")
     x, y = w.inputs(2)
     g = to_dev(w.graph_args(), "cuda")
-    (loss, out, hid), names = _profiled(lambda: m.fused_step(x.cuda(), y.cuda(), *g))
+    (loss, out, hid), names = profiled(lambda: m.fused_step(x.cuda(), y.cuda(), *g))
     assert "k_cell_fwd" in names and "k_cell_bwd" in names, sorted(names)
     assert not names & {"k_cell_fwd_f", "k_cell_bwd_f", "k_g_zr"}, sorted(names)
     _check(w, ref, lims, loss, out, hid, _grads(m), "T=65/auto")
@@ -448,7 +436,7 @@ def test_head_output_width(O, H, path):
     x, y = w.inputs(B)
     x, y = x.cuda(), y.cuda()
     if path == "fused_step":
-        res, names = _profiled(lambda: m.fused_step(x, y, *to_dev(w.graph_args(), "cuda")))
+        res, names = profiled(lambda: m.fused_step(x, y, *to_dev(w.graph_args(), "cuda")))
     else:
         res, names = _profiled_autograd(lambda: m(x, *to_dev(w.graph_args(), "cuda")),
                                         lambda out, hid: ((out - y) ** 2).mean(dim=(1, 2)).sum())
@@ -466,7 +454,7 @@ def test_head_row_threshold(N):
     w, B, ref, lims = _head_case(4, 128, N=N, B=1)
     m = build_cuda(w, ref["state"], precision="tf32x3")
     x, y = w.inputs(B)
-    (loss, out, hid), names = _profiled(lambda: m.fused_step(x.cuda(), y.cuda(), *to_dev(w.graph_args(), "cuda")))
+    (loss, out, hid), names = profiled(lambda: m.fused_step(x.cuda(), y.cuda(), *to_dev(w.graph_args(), "cuda")))
     assert ("k_hf_mid" in names) == (N >= 128), sorted(names)
     _check(w, ref, lims, loss, out, hid, _grads(m), f"B*N={N}")
 

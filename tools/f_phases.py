@@ -22,8 +22,8 @@ for _ in range(2):
 torch.cuda.synchronize()
 buf = (C.c_longlong * (3 * 16 * 12))()
 _lib.check(_lib.load().regt_debug_f_timestamps(buf), "timestamps")
-names = {0: ["wait z-gate MMAs", "E1z (sigmoid, save Z, acc)", "wait r-gate MMAs", "E1r (sigmoid, save R, h*R -> A)", "Pcompute(next) [REGT_F_PRE]",
-             "wait candidate MMAs", "Pstore(next) (+Pcompute if not PRE)", "E2 (tanh, save H~, acc)"],
+names = {0: ["wait z-gate MMAs", "E1z (sigmoid, save Z, acc)", "wait r-gate MMAs", "E1r (sigmoid, save R, h*R -> A)", "Pcompute(next)",
+             "wait candidate MMAs", "Pstore(next)", "E2 (tanh, save H~, acc)"],
          1: ["E0 (recompute h, planes, Dz Dc h hR out, Dc -> A)", "wait M1 (dHR)", "Dz -> A", "E1 (Dr, t1)", "wait M2z", "Dr -> A", "wait M2r",
              "E2 (d h_pre out)"]}
 for which, title in ((0, "forward k_cell_fwd_f"), (1, "backward k_cell_bwd_f")):
