@@ -293,7 +293,10 @@ int regt_profile_read(char* names, size_t names_len, float* ms, int max_n);
  *   gemm_tn_multi: the four-gate-block form of the cell backward, A = D [M][4H]
  *   gemm_kt: the same contraction over transposed tiles A^T [ntile][4H][128], B^T [ntile][H][128], F^T [ntile][32][128]
  *            (what the fused cell backward of cell_f.cu writes); H = 128 or 64
- *   umma_selftest: one 128 x N x K MMA on operand tiles written by CUDA-core threads (fmt 1 = bf16, 2 = tf32)         */
+ *   umma_selftest: one 128 x N x K MMA on operand tiles written by CUDA-core threads (fmt 1 = bf16, 2 = tf32)
+ *   tc_split: how the bf16 kernels of cell_tc.cu / head_tc.cu split B*N rows over T periods on this device, written to
+ *             out[7] = {128-row tiles nqt, periods per item tp, period chunks ntc = T / tp, items = nqt * ntc,
+ *             forward grid, backward grid, k_head_tc grid} (tests/test_gpu_bf16_edges.py states its preconditions so)   */
 int regt_debug_gemm_nt_tma(const float* A, int64_t lda, const float* Bt, int64_t ldb, float* C, int64_t ldc, int64_t M,
                            int32_t N, int32_t K, float* scratch, regt_stream_t stream);
 int regt_debug_gemm_tn_tma(const float* A, int64_t lda, const float* B, int64_t ldb, float* Cp, int64_t M, int32_t K,
@@ -307,6 +310,7 @@ int regt_debug_spmm_partition_host(const int32_t* rowptr, const int32_t* col, in
 int regt_debug_f_timestamps(long long* out);   /* phase clocks of the fused 3xTF32 cell kernels (REGT_F_DEBUG), [3][16][12]: forward epilogue, backward epilogue, forward MMA warp */
 int regt_debug_umma_selftest(int fmt, int variant, const float* A, const float* B, float* D, int N, int K,
                              regt_stream_t stream);
+int regt_debug_tc_split(int32_t B, int32_t N, int32_t T, int32_t* out);
 
 #ifdef __cplusplus
 }

@@ -610,6 +610,7 @@ static int choose_tp(int nqt, int T, int slots) {
 
 bool head_fusable(const regt_args* a);
 bool head_tc_usable(const regt_args* a);
+int head_tc_grid(const regt_args* a);
 int launch_head_grad_reduce(const regt_args* a, const Layout& L, cudaStream_t st);
 int tc_num_chunks(const regt_args* a) {
   const int BN = a->B * a->N, nqt = (BN + TC_ROWS - 1) / TC_ROWS;
@@ -632,6 +633,9 @@ static TcArgs make_tcargs(const regt_args* a, const Layout& L, int slots) {
   k.G = L.G; k.dhp = L.dhp_p; k.wpart = L.tc_wpart; k.dprobs_part = L.tc_dpp;
   return k;
 }
+// persistent grids: one CTA per SM at most; the backward's per-CTA weight-gradient partials hold TC_MAX_CTAS
+static int tc_fwd_grid(const TcArgs& k, int slots) { return min(slots, k.items); }
+static int tc_bwd_grid(const TcArgs& k, int slots) { return min(tc_fwd_grid(k, slots), TC_MAX_CTAS); }
 
 template <int HH>
 static int run_fwd_tc(const regt_args* a, const Layout& L, cudaStream_t st, bool forked) {
@@ -646,7 +650,7 @@ static int run_fwd_tc(const regt_args* a, const Layout& L, cudaStream_t st, bool
   TcArgs k = make_tcargs(a, L, slots);
   const size_t smem = 1024 + ((Cfg::FWD_IMG + 1023) & ~1023) + Cfg::A_TILE + 2 * Cfg::SMF_TILE;
   REGT_CUDA(cudaFuncSetAttribute(k_cell_fwd_tc<HH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const int grid = min(slots, k.items);
+  const int grid = tc_fwd_grid(k, slots);
   k_cell_fwd_tc<HH><<<grid, NTHREADS, smem, st>>>(k);
   REGT_LAUNCHED("k_cell_fwd_tc", st);
   if (!head_fusable(a)) {  // otherwise the fused head sums the partials while loading its tiles
@@ -1127,7 +1131,7 @@ int cell_backward_tc(const regt_args* a, const Layout& L, cudaStream_t st) {
   const int slots = num_sms();
   TcArgs k = make_tcargs(a, L, slots);
   k.img = L.tc_img_b;
-  const int grid = min(min(slots, k.items), TC_MAX_CTAS);
+  const int grid = tc_bwd_grid(k, slots);
   const size_t smem = 1024 + ((Cfg::BWD_IMG + 1023) & ~1023) + 6 * Cfg::A_TILE + 2 * 4 * TC_ROWS * 16 +
                       3 * PlaneIO<__nv_bfloat16, HH>::TILE_BYTES + TC_ROWS * HH * 4;
   REGT_CUDA(cudaFuncSetAttribute(k_cell_bwd_tc<HH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1153,3 +1157,17 @@ int cell_backward_tc(const regt_args* a, const Layout& L, cudaStream_t st) {
 }
 
 }  // namespace regt
+
+// TEST HOOK: the work split the bf16 kernels use for B snapshots of N nodes over T periods, from the code that launches
+// them: out = {nqt, tp, ntc, items, forward grid, backward grid, k_head_tc grid}
+extern "C" int regt_debug_tc_split(int32_t B, int32_t N, int32_t T, int32_t* out) {
+  REGT_CHECK(B > 0 && N > 0 && T > 0 && out, "regt_debug_tc_split: B, N, T must be positive and out non-NULL");
+  regt_args a{};
+  a.B = B; a.N = N; a.T = T;
+  const int slots = regt::num_sms();
+  const regt::TcArgs k = regt::make_tcargs(&a, regt::Layout{}, slots);
+  const int32_t v[7] = {k.nqt, k.tp, k.ntc, k.items, regt::tc_fwd_grid(k, slots), regt::tc_bwd_grid(k, slots),
+                        regt::head_tc_grid(&a)};
+  for (int i = 0; i < 7; ++i) out[i] = v[i];
+  return 0;
+}

@@ -412,8 +412,17 @@ __global__ void __launch_bounds__(256) k_head_grad_reduce(const float* __restric
   if (dst) dst[j] = acc ? dst[j] + s : s;
 }
 
+// k_head_fused keeps both weight layouts, the dW2 accumulator and four row tiles in shared memory
+static size_t head_fused_smem(int H, int O) {
+  const int OP = (O + 3) & ~3;
+  return ((size_t)2 * HEAD_HID * H + HEAD_HID * OP + 2 * O * HEAD_HID + TMH * (H + 4) + 2 * TMH * (HEAD_HID + 4) +
+          TMH * (OP + 4)) * sizeof(float);
+}
+// H = 64 fits up to O = 44 in the 227 KB a block may use (O = 45 would need 229 KB), H = 32 every O up to 64; wider
+// heads run k_head_fwd / k_head_bwd
 bool head_fusable(const regt_args* a) {
-  return a->fuse_head && a->y && a->d_out && a->loss && (a->H == 64 || a->H == 32) && a->O <= 64;
+  return a->fuse_head && a->y && a->d_out && a->loss && (a->H == 64 || a->H == 32) && a->O <= 64 &&
+         head_fused_smem(a->H, a->O) <= 227 * 1024;
 }
 static int head_fused_grid(const regt_args* a) {
   const long long BN = (long long)a->B * a->N;
@@ -453,9 +462,8 @@ int head_forward_fp32(const regt_args* a, const Layout& L, cudaStream_t st) {
   if (head_f_usable(a)) return head_forward_f(a, L, st);      // tf32x3: the 128-wide GEMMs on the tensor cores (head_f.cu)
   if (head_fusable(a)) {
     HeadK k = make_headk(a, L, nullptr, nullptr);
-    const int grid = head_fused_grid(a), ntiles = cdiv(k.BN, TMH), OP = (O + 3) & ~3;
-    const size_t smem = ((size_t)2 * HEAD_HID * H + HEAD_HID * OP + 2 * O * HEAD_HID + TMH * (H + 4) +
-                         2 * TMH * (HEAD_HID + 4) + TMH * (OP + 4)) * sizeof(float);
+    const int grid = head_fused_grid(a), ntiles = cdiv(k.BN, TMH);
+    const size_t smem = head_fused_smem(H, O);
     if (H == 64) {
       REGT_CUDA(cudaFuncSetAttribute(k_head_fused<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       k_head_fused<64><<<grid, 256, smem, st>>>(k, L.hpart, ntiles);

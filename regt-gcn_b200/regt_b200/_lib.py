@@ -165,6 +165,8 @@ def load() -> C.CDLL:
     lib.regt_debug_f_timestamps.argtypes = [vp]
     lib.regt_debug_umma_selftest.restype = C.c_int
     lib.regt_debug_umma_selftest.argtypes = [C.c_int, C.c_int, vp, vp, vp, C.c_int, C.c_int, vp]
+    lib.regt_debug_tc_split.restype = C.c_int
+    lib.regt_debug_tc_split.argtypes = [C.c_int32, C.c_int32, C.c_int32, c_i32p]
     _lib = lib
     return lib
 

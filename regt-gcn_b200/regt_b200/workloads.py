@@ -116,7 +116,7 @@ def _regional_graph(N: int, R: int, k_intra: int, n_cross: int, seed: int):
         reg_ea.append(torch.from_numpy(w))
     region_of = np.concatenate([np.full(len(n), r) for r, n in enumerate(regions)])
     cs, cd = [], []
-    while len(cs) < n_cross:
+    while R > 1 and len(cs) < n_cross:     # one region: there is no cross-region edge to draw
         s, d = int(rng.integers(N)), int(rng.integers(N))
         if region_of[s] != region_of[d]:
             cs.append(s); cd.append(d)

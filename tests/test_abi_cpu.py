@@ -42,6 +42,30 @@ def test_library_exports_nothing_undeclared():
     assert not undeclared, f"exported but not declared in include/regt_b200.h: {undeclared}"
 
 
+def test_tc_split_hook():
+    """regt_debug_tc_split (the work split of the bf16 kernels) is consistent in itself and, with 148 SMs (a B200, or
+    the count assumed without a device), gives the splits tests/test_gpu_bf16_edges.py is built around."""
+    from regt_b200 import _lib
+    lib = _lib.load()
+
+    def split(B, N, T):
+        o = (C.c_int32 * 7)()
+        _lib.check(lib.regt_debug_tc_split(B, N, T, o), "regt_debug_tc_split")
+        return list(o)
+
+    shapes = {(64, 207, 12): [104, 3, 4, 416], (3, 207, 12): [5, 1, 12, 60], (64, 592, 12): [296, 12, 1, 296],
+              (32, 592, 12): [148, 12, 1, 148], (16, 592, 12): [74, 6, 2, 148], (8, 592, 12): [37, 3, 4, 148]}
+    slots = split(64, 592, 12)[4]
+    for (B, N, T), want in shapes.items():
+        nqt, tp, ntc, items, fwd, bwd, head = split(B, N, T)
+        assert nqt == -(-B * N // 128) and T % tp == 0 and ntc == T // tp and items == nqt * ntc
+        assert fwd == min(slots, items) and bwd == min(fwd, 160) and head == min(148, nqt)
+        if slots == 148:
+            assert [nqt, tp, ntc, items] == want, (B, N, T)
+    with pytest.raises(RuntimeError, match="must be positive"):
+        _lib.check(lib.regt_debug_tc_split(0, 207, 12, (C.c_int32 * 7)()), "regt_debug_tc_split")
+
+
 def test_ctypes_structs_mirror_header():
     from regt_b200 import _lib
     src = open(HEADER).read()

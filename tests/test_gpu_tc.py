@@ -1,6 +1,9 @@
 """Tensor-core (tcgen05) precision modes of the cell against the fp64 oracle.
 tf32x3 (generic 3xTF32 GEMM path, any hidden % 32 == 0): fp32-equivalent accuracy (1e-5 normwise); bf16 (fused H=64 kernels): stated tolerance 2e-2 activations / loss,
-5e-2 gradients (bf16 operands have an 8-bit mantissa; accumulation is fp32)."""
+5e-2 gradients (bf16 operands have an 8-bit mantissa; accumulation is fp32).
+Every bf16 case here has one work item per CTA, one period per item and at most 12 outputs; test_gpu_bf16_edges.py
+covers the rest: several items and head tiles per CTA, 1 < tp < T, the bench's shape and graph replay, every head
+kernel, the autograd surface, 1 to 64 periods, many regions and one."""
 import pytest
 import torch
 
