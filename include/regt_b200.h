@@ -296,7 +296,10 @@ int regt_profile_read(char* names, size_t names_len, float* ms, int max_n);
  *   umma_selftest: one 128 x N x K MMA on operand tiles written by CUDA-core threads (fmt 1 = bf16, 2 = tf32)
  *   tc_split: how the bf16 kernels of cell_tc.cu / head_tc.cu split B*N rows over T periods on this device, written to
  *             out[7] = {128-row tiles nqt, periods per item tp, period chunks ntc = T / tp, items = nqt * ntc,
- *             forward grid, backward grid, k_head_tc grid} (tests/test_gpu_bf16_edges.py states its preconditions so)   */
+ *             forward grid, backward grid, k_head_tc grid} (tests/test_gpu_bf16_edges.py states its preconditions so)
+ *   route: which cell and head kernels the entry points run for these arguments (no CUDA call, no workspace needed),
+ *          out[4] = {cell: 0 fp32, 1 unfused tf32x3, 2 fused tf32x3, 3 bf16; head: 0 row kernels k_head_fwd / k_head_bwd,
+ *          1 k_head_fused, 2 tf32x3 head, 3 k_head_tc; G written as tiles; bf16 forward leaves out_hidden partials}   */
 int regt_debug_gemm_nt_tma(const float* A, int64_t lda, const float* Bt, int64_t ldb, float* C, int64_t ldc, int64_t M,
                            int32_t N, int32_t K, float* scratch, regt_stream_t stream);
 int regt_debug_gemm_tn_tma(const float* A, int64_t lda, const float* B, int64_t ldb, float* Cp, int64_t M, int32_t K,
@@ -311,6 +314,7 @@ int regt_debug_f_timestamps(long long* out);   /* phase clocks of the fused 3xTF
 int regt_debug_umma_selftest(int fmt, int variant, const float* A, const float* B, float* D, int N, int K,
                              regt_stream_t stream);
 int regt_debug_tc_split(int32_t B, int32_t N, int32_t T, int32_t* out);
+int regt_debug_route(const regt_args* args, int32_t* out);
 
 #ifdef __cplusplus
 }

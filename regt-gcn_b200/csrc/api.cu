@@ -1,25 +1,36 @@
-// C-ABI entry points of the cell + head (include/regt_b200.h) and the workspace layout.
+// C-ABI entry points of the cell + head (include/regt_b200.h), the choice of their kernels and the workspace layout.
+#include <stdlib.h>
+
 #include "common.cuh"
 
 namespace regt {
 
 constexpr int F = REGT_F;
 
-int cell_forward_fp32(const regt_args* a, const Layout& L, cudaStream_t st);
-int cell_backward_fp32(const regt_args* a, const Layout& L, cudaStream_t st);
-int head_forward_fp32(const regt_args* a, const Layout& L, cudaStream_t st);
-int head_backward_fp32(const regt_args* a, const Layout& L, cudaStream_t st);
-int cell_forward_tc(const regt_args* a, const Layout& L, cudaStream_t st);
-int cell_backward_tc(const regt_args* a, const Layout& L, cudaStream_t st);
-int cell_forward_g(const regt_args* a, const Layout& L, cudaStream_t st);
-int cell_backward_g(const regt_args* a, const Layout& L, cudaStream_t st);
-int cell_forward_f(const regt_args* a, const Layout& L, cudaStream_t st);
-int cell_backward_f(const regt_args* a, const Layout& L, cudaStream_t st);
-size_t cell_backward_x_scratch_bytes(const regt_args* a, const regt_xgrad_plan* xp);
-int cell_backward_x(const regt_args* a, const Layout& L, const regt_xgrad_plan* xp, float* d_x, void* scratch, cudaStream_t st);
+Route route_of(const regt_args* a) {
+  const char* e = getenv("REGT_UNFUSED");
+  const bool unfused = e && e[0] == '1';
+  const bool tf32x3 = a->precision == REGT_PREC_TF32X3, bf16 = a->precision == REGT_PREC_BF16;
+  const bool fused_step = a->fuse_head && a->y && a->d_out && a->loss;   // forward, loss and head gradients in one step
+  Route r{};
+  r.cell = bf16 ? CellPath::Bf16
+                : !tf32x3 ? CellPath::Fp32 : (!unfused && cell_f_fits(a)) ? CellPath::Tf32x3Fused : CellPath::Tf32x3Unfused;
+  if (bf16 && fused_step && head_tc_fits(a->H, a->O))
+    r.head = HeadPath::Bf16;
+  else if (tf32x3 && a->H % 32 == 0 && head_f_fits(a->O) && (long long)a->B * a->N >= 128 && a->out)
+    r.head = HeadPath::Tf32x3;
+  else if (fused_step && head_fused_fits(a->H, a->O))
+    r.head = HeadPath::FusedFfma;
+  else
+    r.head = HeadPath::Rows;
+  r.g_tiled = r.cell == CellPath::Tf32x3Fused || r.cell == CellPath::Bf16;
+  r.hid_partials = r.cell == CellPath::Bf16 && (r.head == HeadPath::Bf16 || r.head == HeadPath::FusedFfma);
+  return r;
+}
 
 Layout make_layout(const regt_args* a, void* base) {
   Layout L{};
+  L.route = route_of(a);
   Carver c(base);
   const size_t H = a->H, T = a->T, R = a->plan.R > 0 ? a->plan.R : 1, O = a->O;
   const size_t BN = (size_t)a->B * a->N, rows = BN * T;
@@ -35,8 +46,7 @@ Layout make_layout(const regt_args* a, void* base) {
   L.probs = c.take<float>(T);
   L.S = c.take<float>(BN * F * T);
   L.U = c.take<float>((size_t)a->B * (nseg ? nseg : 1) * F * T);
-  const bool tcp = a->precision == REGT_PREC_BF16;   // fused tcgen05 kernels (tile-layout planes); tf32x3 uses the fp32 planes
-  if (cell_f_usable(a)) {
+  if (L.route.cell == CellPath::Tf32x3Fused) {
     // fused 3xTF32 cell (cell_f.cu): three saved planes in tile layout; the backward kernel writes the gate-gradient
     // blocks D and h, h*R as TRANSPOSED tiles [T*nqt][cols][128 rows] for the weight-gradient contraction (gemm_kt)
     const size_t nqt = (BN + 127) / 128, rowsP = T * nqt * 128;
@@ -53,7 +63,7 @@ Layout make_layout(const regt_args* a, void* base) {
     L.Feat = c.take<float>(inf ? 4 : nqt * 128 * 32);      // the head's ones column (row major, BNp rows)
     L.FeatT = c.take<float>(inf ? 4 : rowsP * 32);
     L.tc_dpp = c.take<float>(2 * (T * TC_MAX_CTAS + 64));   // fp64 attention-gradient partials
-  } else if (!tcp) {
+  } else if (L.route.cell != CellPath::Bf16) {   // fp32 and unfused tf32x3: row-major planes
     L.h = c.take<float>(rows * H);
     L.Z = c.take<float>(rows * H);
     L.Rg = c.take<float>(rows * H);
@@ -63,7 +73,7 @@ Layout make_layout(const regt_args* a, void* base) {
     L.D = c.take<float>(rows * 4 * H);
     L.Feat = c.take<float>(a->precision == REGT_PREC_TF32X3 ? rows * 32 : 4);
     L.bsplit = c.take<float>(a->precision == REGT_PREC_TF32X3 ? gemm_nt_scratch_floats((int)H, 2 * (int)H) : 4);
-  } else {
+  } else {   // bf16 fused tcgen05 kernels: tile-layout planes
     const size_t nqt = (BN + 127) / 128, plane = T * nqt * 128 * H;
     L.tc_img_f = c.take<unsigned char>(TC_IMG_BYTES);
     L.tc_img_b = c.take<unsigned char>(TC_IMG_BYTES);
@@ -136,29 +146,35 @@ extern "C" size_t regt_workspace_bytes(const regt_args* a) {
 extern "C" int regt_cell_forward(const regt_args* a) {
   if (validate(a, "regt_cell_forward")) return -1;
   REGT_CHECK(a->x && a->out_hidden, "regt_cell_forward: x / out_hidden is NULL");
+  if (a->precision == REGT_PREC_TF32X3)
+    REGT_CHECK(a->H % 32 == 0, "precision tf32x3 needs hidden %% 32 == 0 (got %d); use precision fp32", a->H);
   Layout L = make_layout(a, a->workspace);
   cudaStream_t st = (cudaStream_t)a->stream;
   prof_mark("<begin>", st);
-  if (a->precision == REGT_PREC_FP32) return cell_forward_fp32(a, L, st);
-  if (a->precision == REGT_PREC_TF32X3) {
-    REGT_CHECK(a->H % 32 == 0, "precision tf32x3 needs hidden %% 32 == 0 (got %d); use precision fp32", a->H);
-    return cell_f_usable(a) ? cell_forward_f(a, L, st) : cell_forward_g(a, L, st);
+  switch (L.route.cell) {
+    case CellPath::Fp32: return cell_forward_fp32(a, L, st);
+    case CellPath::Tf32x3Unfused: return cell_forward_g(a, L, st);
+    case CellPath::Tf32x3Fused: return cell_forward_f(a, L, st);
+    case CellPath::Bf16: return cell_forward_tc(a, L, st);
   }
-  return cell_forward_tc(a, L, st);
+  return -1;
 }
 
 extern "C" int regt_cell_backward(const regt_args* a) {
   if (validate(a, "regt_cell_backward")) return -1;
   REGT_CHECK(!a->inference, "regt_cell_backward: the forward ran with inference=1 (no activations were saved)");
+  if (a->precision == REGT_PREC_TF32X3)
+    REGT_CHECK(a->H % 32 == 0, "precision tf32x3 needs hidden %% 32 == 0 (got %d); use precision fp32", a->H);
   Layout L = make_layout(a, a->workspace);
   cudaStream_t st = (cudaStream_t)a->stream;
   prof_mark("<begin>", st);
-  if (a->precision == REGT_PREC_FP32) return cell_backward_fp32(a, L, st);
-  if (a->precision == REGT_PREC_TF32X3) {
-    REGT_CHECK(a->H % 32 == 0, "precision tf32x3 needs hidden %% 32 == 0 (got %d); use precision fp32", a->H);
-    return cell_f_usable(a) ? cell_backward_f(a, L, st) : cell_backward_g(a, L, st);
+  switch (L.route.cell) {
+    case CellPath::Fp32: return cell_backward_fp32(a, L, st);
+    case CellPath::Tf32x3Unfused: return cell_backward_g(a, L, st);
+    case CellPath::Tf32x3Fused: return cell_backward_f(a, L, st);
+    case CellPath::Bf16: return cell_backward_tc(a, L, st);
   }
-  return cell_backward_tc(a, L, st);
+  return -1;
 }
 
 static int validate_x(const regt_args* a, const regt_xgrad_plan* xp, const char* who) {
@@ -196,7 +212,7 @@ extern "C" int regt_head_forward(const regt_args* a) {
   REGT_CHECK(a->out_hidden && a->out, "regt_head_forward: out_hidden / out is NULL");
   Layout L = make_layout(a, a->workspace);
   prof_mark("<begin>", (cudaStream_t)a->stream);
-  return head_forward_fp32(a, L, (cudaStream_t)a->stream);
+  return head_forward(a, L, (cudaStream_t)a->stream);
 }
 
 extern "C" int regt_head_backward(const regt_args* a) {
@@ -204,5 +220,16 @@ extern "C" int regt_head_backward(const regt_args* a) {
   REGT_CHECK(!a->inference, "regt_head_backward: the forward ran with inference=1 (no activations were saved)");
   Layout L = make_layout(a, a->workspace);
   prof_mark("<begin>", (cudaStream_t)a->stream);
-  return head_backward_fp32(a, L, (cudaStream_t)a->stream);
+  return head_backward(a, L, (cudaStream_t)a->stream);
+}
+
+// TEST HOOK: the kernels route_of picks for these arguments, out = {cell, head, g_tiled, hid_partials} (CellPath, HeadPath)
+extern "C" int regt_debug_route(const regt_args* a, int32_t* out) {
+  REGT_CHECK(a && out, "regt_debug_route: args and out must be non-NULL");
+  const Route r = route_of(a);
+  out[0] = (int32_t)r.cell;
+  out[1] = (int32_t)r.head;
+  out[2] = r.g_tiled;
+  out[3] = r.hid_partials;
+  return 0;
 }

@@ -728,10 +728,6 @@ int launch_colsum(const float* A, int lda, int C, long long rows, int splits, fl
 // ------------------------------------------------------------------------------------------
 // host-side orchestration of the fp32 path
 // ------------------------------------------------------------------------------------------
-int launch_spmm_rows(const int32_t* rowptr, const int32_t* col, const float* val, const float* x, float* y, int B,
-                     int n_out, int n_in, int width, cudaStream_t st);
-int launch_prep(const regt_args* a, const Layout& L, cudaStream_t st);
-int launch_chain(const regt_args* a, const Layout& L, cudaStream_t st);
 
 static CellK make_cellk(const regt_args* a, const Layout& L) {
   CellK k{};
@@ -763,8 +759,8 @@ static int run_bwd(const CellK& k, cudaStream_t st) {
   return 0;
 }
 
-// dM1[r] = sum over the (node, region r) segments of dhp^T U  -- shared with cell_g.cu; dhp = rows of `ldd` floats
-int launch_wgrad_m1_from(const regt_args* a, const Layout& L, const float* dhp, long long ldd, cudaStream_t st, int period_major,
+// dM1[r] = sum over the (node, region r) segments of dhp^T U; dhp = rows of `ldd` floats
+static int launch_wgrad_m1_from(const regt_args* a, const Layout& L, const float* dhp, long long ldd, cudaStream_t st, int period_major,
                          long long BNp) {
   const int H = a->H, T = a->T, R = a->plan.R;
   const long long nsg = a->plan.nseg;
@@ -824,7 +820,7 @@ int launch_wgrad_m1(const regt_args* a, const Layout& L, cudaStream_t st) {
 }
 
 // F-wide weight gradients (dP_g = D_g^T S, dM0 = D_3^T X, biases = column sums, dM1 per region)
-int launch_fwide_wgrads(const regt_args* a, const Layout& L, int splits, cudaStream_t st) {
+static int launch_fwide_wgrads(const regt_args* a, const Layout& L, int splits, cudaStream_t st) {
   const int H = a->H, T = a->T, R = a->plan.R;
   const long long rows = (long long)a->B * a->N * T;
   float* part = L.part;
@@ -836,18 +832,6 @@ int launch_fwide_wgrads(const regt_args* a, const Layout& L, int splits, cudaStr
   REGT_LAUNCHED("k_skinny_reduce", st);
   if (a->mode != REGT_MODE_TGCN && launch_wgrad_m1(a, L, st)) return -1;
   return 0;
-}
-
-int launch_attn_accum(const float* Hn, const float* probs, int T, int H, long long BN, float* out_hidden, cudaStream_t st) {
-  k_attn_accum<<<cdiv(BN * (H / 4), 256), 256, 0, st>>>(Hn, probs, T, H, BN, out_hidden);
-  REGT_LAUNCHED("k_attn_accum", st);
-  return 0;
-}
-int launch_dprobs(const float* G, const float* Hn, int T, int H, long long BN, float* part, float* dprobs, cudaStream_t st) {
-  const int nblk = 128;
-  k_dprobs<<<nblk, 256, 0, st>>>(G, Hn, T, H, BN, part);
-  REGT_LAUNCHED("k_dprobs", st);
-  return launch_reduce_splits(part, dprobs, T, nblk, 0, st);
 }
 
 int cell_forward_fp32(const regt_args* a, const Layout& L, cudaStream_t st) {

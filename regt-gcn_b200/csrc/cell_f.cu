@@ -1251,14 +1251,6 @@ FArgs make_fargs(const regt_args* a, const Layout& L) {
   k.G = L.G; k.D = L.D; k.hpl = L.h; k.hRpl = L.hR; k.dpp = reinterpret_cast<double*>(L.tc_dpp);
   return k;
 }
-int num_sms_f() {
-  static int n = 0;
-  if (n == 0) {
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = 148;
-  }
-  return n;
-}
 
 template <int HH>
 int run_fwd(const regt_args* a, const Layout& L, cudaStream_t st) {
@@ -1276,7 +1268,7 @@ int run_fwd_kernel(const regt_args* a, const Layout& L, cudaStream_t st) {
   FArgs k = make_fargs<HH>(a, L);
   k.img = L.tc_img_f;
   REGT_CUDA(cudaFuncSetAttribute(k_cell_fwd_f<HH>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM));
-  const int grid = min(num_sms_f(), k.nqt);
+  const int grid = min(sm_count(), k.nqt);
   REGT_CHECK(grid <= TC_MAX_CTAS, "fused forward: grid %d exceeds the per-CTA scratch tiles", grid);
   k_cell_fwd_f<HH><<<grid, NTHR, C::SMEM, st>>>(k);
   REGT_LAUNCHED("k_cell_fwd_f", st);
@@ -1287,29 +1279,13 @@ int run_bwd_kernel(const regt_args* a, const Layout& L, cudaStream_t st, int* gr
   using C = FCfg<HH>;
   FArgs k = make_fargs<HH>(a, L);
   k.img = L.tc_img_b;
-  const int grid = min(num_sms_f(), k.nqt);
+  const int grid = min(sm_count(), k.nqt);
   REGT_CHECK(grid <= TC_MAX_CTAS, "fused backward: grid %d exceeds the partial buffers", grid);
   REGT_CUDA(cudaFuncSetAttribute(k_cell_bwd_f<HH>, cudaFuncAttributeMaxDynamicSharedMemorySize, BCfg<HH>::SMEM));
   k_cell_bwd_f<HH><<<grid, NTHR, BCfg<HH>::SMEM, st>>>(k);
   REGT_LAUNCHED("k_cell_bwd_f", st);
   *grid_out = grid;
   return 0;
-}
-}  // namespace
-
-bool cell_f_usable(const regt_args* a) {
-  const char* e = getenv("REGT_UNFUSED");      // "1": the GEMM-by-GEMM path of cell_g.cu (kept for H = 256 and as the A/B baseline)
-  const bool off = e && e[0] == '1';
-  return !off && a->precision == REGT_PREC_TF32X3 && (a->H == 128 || a->H == 64) && a->mode != REGT_MODE_TGCN && a->T <= 64;
-}
-int launch_pack_f(const regt_args* a, const Layout& L, cudaStream_t st) {
-  return a->H == 128 ? run_fwd<128>(a, L, st) : run_fwd<64>(a, L, st);
-}
-int launch_cell_fwd_f(const regt_args* a, const Layout& L, cudaStream_t st) {
-  return a->H == 128 ? run_fwd_kernel<128>(a, L, st) : run_fwd_kernel<64>(a, L, st);
-}
-int launch_cell_bwd_f(const regt_args* a, const Layout& L, cudaStream_t st, int* grid) {
-  return a->H == 128 ? run_bwd_kernel<128>(a, L, st, grid) : run_bwd_kernel<64>(a, L, st, grid);
 }
 int launch_feat_f(const regt_args* a, const Layout& L, cudaStream_t st) {
   const int BN = a->B * a->N, nqt = (BN + TC_ROWS - 1) / TC_ROWS, BNp = nqt * TC_ROWS;
@@ -1318,6 +1294,64 @@ int launch_feat_f(const regt_args* a, const Layout& L, cudaStream_t st) {
   k_ones_f<<<cdiv((long long)BNp * 8, 256), 256, 0, st>>>(BN, BNp, L.Feat);
   REGT_LAUNCHED("k_ones_f", st);
   return 0;
+}
+}  // namespace
+
+bool cell_f_fits(const regt_args* a) { return (a->H == 128 || a->H == 64) && a->mode != REGT_MODE_TGCN && a->T <= 64; }
+
+int cell_forward_f(const regt_args* a, const Layout& L, cudaStream_t st) {
+  // features (graph + x) and collapsed weights (parameters) are independent: two streams
+  cudaStream_t side = fork_side(st);
+  cudaStream_t fs = side ? side : st;
+  if (launch_feat_tc(a->plan, a->x, a->B, a->x_rows > 0 ? a->x_rows : a->N, a->T, L.Xt, L.S, L.U, fs)) return -1;
+  if (!a->inference && launch_feat_f(a, L, fs)) return -1;   // feature plane of the weight-gradient contractions (cell and head backward)
+  if (launch_prep(a, L, st)) return -1;
+  if (a->H == 128 ? run_fwd<128>(a, L, st) : run_fwd<64>(a, L, st)) return -1;
+  if (side && join_side(st)) return -1;
+  return a->H == 128 ? run_fwd_kernel<128>(a, L, st) : run_fwd_kernel<64>(a, L, st);
+}
+
+int cell_backward_f(const regt_args* a, const Layout& L, cudaStream_t st) {
+  const int H = a->H, T = a->T;
+  const long long BN = (long long)a->B * a->N, nqt = (BN + 127) / 128, ntile = nqt * T;
+  int grid = 0;
+  if (H == 128 ? run_bwd_kernel<128>(a, L, st, &grid) : run_bwd_kernel<64>(a, L, st, &grid)) return -1;
+  if (launch_f_sum_dpp(reinterpret_cast<const double*>(L.tc_dpp), grid, T, L.dprobs, st)) return -1;
+  // weight gradients: ONE row contraction over the transposed gate-gradient tiles D^T [tile][4H][128] (z | r against h,
+  // h~ against h*R, h_pre against the feature tile only; every block also against [S | X | 1]), rows = K
+  float* part = L.part;
+  const int mtiles = 4 * H / 128;
+  const int splits = (int)max(1ll, min((long long)min(WGRAD_SPLITS, cdiv(148, mtiles)), ntile / 4));
+  float* pB = part;                                          // [splits][2H][H]  dB_z | dB_r
+  float* pBh = pB + (size_t)splits * 2 * H * H;              // [splits][H][H]   dB_h
+  float* pF = pBh + (size_t)splits * H * H;                  // [splits][4H][32] D^T Feat
+  const long long fsplit = 4ll * H * 32;
+  {
+    // segments start at multiples of 128 columns.  H = 128: z|r (2 tiles), h~, h_pre.  H = 64: tile 0 = z|r, tile 1 = h~ | h_pre
+    // (its rows 64.. are contracted against h*R too and dropped: only the feature columns of h_pre are kept)
+    int k0[3], k1[3], sb[3];
+    float* cs[3];
+    int ns;
+    if (H == 128) {
+      ns = 3;
+      k0[0] = 0; k1[0] = 256; sb[0] = 0; cs[0] = pB;
+      k0[1] = 256; k1[1] = 384; sb[1] = 1; cs[1] = pBh;
+      k0[2] = 384; k1[2] = 512; sb[2] = -1; cs[2] = nullptr;
+    } else {
+      ns = 2;
+      k0[0] = 0; k1[0] = 128; sb[0] = 0; cs[0] = pB;
+      k0[1] = 128; k1[1] = 192; sb[1] = 1; cs[1] = pBh;
+    }
+    const float* bs[2] = {L.h, L.hR};
+    if (launch_gemm_kt(L.D, ntile, 4 * H, ns, k0, k1, sb, cs, bs, H, splits, L.FeatT, pF, fsplit, st)) return -1;
+  }
+  if (launch_reduce_splits(pB, L.dB, 2ll * H * H, splits, 0, st)) return -1;
+  if (launch_reduce_splits(pBh, L.dB + (size_t)2 * H * H, (long long)H * H, splits, 0, st)) return -1;
+  if (launch_fw_scatter(pF, splits, H, L, st)) return -1;
+  if (a->plan.nseg > 0) {   // dM1[r]: per-region sums over the (node, region) segments
+    if (launch_wgrad_m1_kt(a, L, st)) return -1;
+  }
+  return launch_chain(a, L, st);
 }
 
 }  // namespace regt

@@ -28,22 +28,6 @@ namespace regt {
 
 constexpr int F = REGT_F;
 
-int launch_prep(const regt_args* a, const Layout& L, cudaStream_t st);
-int launch_chain(const regt_args* a, const Layout& L, cudaStream_t st);
-int launch_spmm_rows(const int32_t* rowptr, const int32_t* col, const float* val, const float* x, float* y, int B,
-                     int n_out, int n_in, int width, cudaStream_t st);
-int launch_gemm_nt_tma(const float* A, long long lda, const float* Bt, long long ldb, float* C, long long ldc, long long M, int N,
-                       int K, float* scratch, cudaStream_t st);
-int launch_gemm_tn_tma(const float* A, long long lda, long long M, int Ktot, int nseg, const int* seg_k0, const int* seg_b,
-                       float* const* seg_C, const float* const* Bs, const long long* ldbs, int N, int splits, const float* B2,
-                       long long ldb2, float* C2, long long c2_split, cudaStream_t st, int relu_b);
-int launch_gemm_tn(const float* A, long long lda, const float* B, long long ldb, float* Cp, long long M, int K, int N, int splits,
-                   cudaStream_t st, const float* B2, long long ldb2, float* Cp2, long long c2_split, int relu_b);
-int launch_attn_accum(const float* Hn, const float* probs, int T, int H, long long BN, float* out_hidden, cudaStream_t st);
-int launch_dprobs(const float* G, const float* Hn, int T, int H, long long BN, float* part, float* dprobs, cudaStream_t st);
-int launch_fwide_wgrads(const regt_args* a, const Layout& L, int splits, cudaStream_t st);
-int launch_wgrad_m1(const regt_args* a, const Layout& L, cudaStream_t st);
-
 namespace {
 struct GK {
   long long rows;
@@ -369,7 +353,17 @@ GK make_gk(const regt_args* a, const Layout& L) {
   } while (0)
 }  // namespace
 
-bool cell_g_usable(const regt_args* a) { return a->precision == REGT_PREC_TF32X3 && a->H % 32 == 0; }
+// shared with the fused backward of cell_f.cu
+int launch_f_sum_dpp(const double* part, int nparts, int T, float* dprobs, cudaStream_t st) {
+  k_f_sum_dpp<<<1, 64, 0, st>>>(part, nparts, T, dprobs);
+  REGT_LAUNCHED("k_f_sum_dpp", st);
+  return 0;
+}
+int launch_fw_scatter(const float* Cp, int splits, int H, const Layout& L, cudaStream_t st) {
+  k_g_fw_scatter<<<cdiv(4ll * H * 32, 32), dim3(32, 8), 0, st>>>(Cp, splits, H, L.dP, L.dcg, L.dM0, L.dc0);
+  REGT_LAUNCHED("k_g_fw_scatter", st);
+  return 0;
+}
 
 int cell_forward_g(const regt_args* a, const Layout& L, cudaStream_t st) {
   const int H = a->H, T = a->T;
@@ -416,8 +410,7 @@ int cell_backward_g(const regt_args* a, const Layout& L, cudaStream_t st) {
   k.dp_part = dpp;
   k_g_b1<<<nb1, 256, 0, st>>>(k);
   REGT_LAUNCHED("k_g_b1", st);
-  k_f_sum_dpp<<<1, 64, 0, st>>>(dpp, nb1, T, L.dprobs);
-  REGT_LAUNCHED("k_f_sum_dpp", st);
+  if (launch_f_sum_dpp(dpp, nb1, T, L.dprobs, st)) return -1;
   if (launch_gemm_nt_tma(L.D + 2 * H, 4 * H, BhT, H, L.Hn, H, rows, H, H, L.bsplit, st)) return -1;            // dHR = Dh . B_h
   G_LAUNCH(k_g_b2, "k_g_b2");
   if (launch_gemm_nt_tma(L.D, 4 * H, BzrT, 2 * H, L.D + 3 * H, 4 * H, rows, H, 2 * H, L.bsplit, st)) return -1;   // dhg
@@ -447,83 +440,9 @@ int cell_backward_g(const regt_args* a, const Layout& L, cudaStream_t st) {
   }
   if (launch_reduce_splits(pB, L.dB, 2ll * H * H, splits, 0, st)) return -1;
   if (launch_reduce_splits(pBh, L.dB + (size_t)2 * H * H, (long long)H * H, splits, 0, st)) return -1;
-  k_g_fw_scatter<<<cdiv(4ll * H * 32, 32), dim3(32, 8), 0, st>>>(pF, splits, H, L.dP, L.dcg, L.dM0, L.dc0);
-  REGT_LAUNCHED("k_g_fw_scatter", st);
+  if (launch_fw_scatter(pF, splits, H, L, st)) return -1;
   if (a->mode != REGT_MODE_TGCN) {   // dM1[r]: per-region sums over the (node, region) segments
     if (launch_wgrad_m1(a, L, st)) return -1;
-  }
-  return launch_chain(a, L, st);
-}
-
-// ------------------------------------------------------------------------------------------
-// fused 3xTF32 cell (kernels in cell_f.cu): hidden 128 / 64
-// ------------------------------------------------------------------------------------------
-int launch_feat_tc(const regt_graph_plan& p, const float* x, int B, int xN, int T, float* Xt, float* St, float* Ut, cudaStream_t st);
-int launch_pack_f(const regt_args* a, const Layout& L, cudaStream_t st);
-int launch_cell_fwd_f(const regt_args* a, const Layout& L, cudaStream_t st);
-int launch_cell_bwd_f(const regt_args* a, const Layout& L, cudaStream_t st, int* grid);
-int launch_feat_f(const regt_args* a, const Layout& L, cudaStream_t st);
-int launch_wgrad_m1_from(const regt_args* a, const Layout& L, const float* dhp, long long ldd, cudaStream_t st, int period_major,
-                         long long BNp);
-
-int cell_forward_f(const regt_args* a, const Layout& L, cudaStream_t st) {
-  // features (graph + x) and collapsed weights (parameters) are independent: two streams
-  cudaStream_t side = fork_side(st);
-  cudaStream_t fs = side ? side : st;
-  if (launch_feat_tc(a->plan, a->x, a->B, a->x_rows > 0 ? a->x_rows : a->N, a->T, L.Xt, L.S, L.U, fs)) return -1;
-  if (!a->inference && launch_feat_f(a, L, fs)) return -1;   // feature plane of the weight-gradient contractions (cell and head backward)
-  if (launch_prep(a, L, st)) return -1;
-  if (launch_pack_f(a, L, st)) return -1;
-  if (side && join_side(st)) return -1;
-  return launch_cell_fwd_f(a, L, st);
-}
-
-int launch_gemm_kt(const float* AT, long long ntile, int Ktot, int nseg, const int* seg_k0, const int* seg_k1, const int* seg_b,
-                   float* const* seg_C, const float* const* BTs, int N, int splits, const float* FT, float* C2, long long c2_split,
-                   cudaStream_t st);
-int launch_wgrad_m1_kt(const regt_args* a, const Layout& L, cudaStream_t st);
-
-int cell_backward_f(const regt_args* a, const Layout& L, cudaStream_t st) {
-  const int H = a->H, T = a->T;
-  const long long BN = (long long)a->B * a->N, nqt = (BN + 127) / 128, ntile = nqt * T;
-  int grid = 0;
-  if (launch_cell_bwd_f(a, L, st, &grid)) return -1;
-  k_f_sum_dpp<<<1, 64, 0, st>>>(reinterpret_cast<const double*>(L.tc_dpp), grid, T, L.dprobs);
-  REGT_LAUNCHED("k_f_sum_dpp", st);
-  // weight gradients: ONE row contraction over the transposed gate-gradient tiles D^T [tile][4H][128] (z | r against h,
-  // h~ against h*R, h_pre against the feature tile only; every block also against [S | X | 1]), rows = K
-  float* part = L.part;
-  const int mtiles = 4 * H / 128;
-  const int splits = (int)max(1ll, min((long long)min(WGRAD_SPLITS, cdiv(148, mtiles)), ntile / 4));
-  float* pB = part;                                          // [splits][2H][H]  dB_z | dB_r
-  float* pBh = pB + (size_t)splits * 2 * H * H;              // [splits][H][H]   dB_h
-  float* pF = pBh + (size_t)splits * H * H;                  // [splits][4H][32] D^T Feat
-  const long long fsplit = 4ll * H * 32;
-  {
-    // segments start at multiples of 128 columns.  H = 128: z|r (2 tiles), h~, h_pre.  H = 64: tile 0 = z|r, tile 1 = h~ | h_pre
-    // (its rows 64.. are contracted against h*R too and dropped: only the feature columns of h_pre are kept)
-    int k0[3], k1[3], sb[3];
-    float* cs[3];
-    int ns;
-    if (H == 128) {
-      ns = 3;
-      k0[0] = 0; k1[0] = 256; sb[0] = 0; cs[0] = pB;
-      k0[1] = 256; k1[1] = 384; sb[1] = 1; cs[1] = pBh;
-      k0[2] = 384; k1[2] = 512; sb[2] = -1; cs[2] = nullptr;
-    } else {
-      ns = 2;
-      k0[0] = 0; k1[0] = 128; sb[0] = 0; cs[0] = pB;
-      k0[1] = 128; k1[1] = 192; sb[1] = 1; cs[1] = pBh;
-    }
-    const float* bs[2] = {L.h, L.hR};
-    if (launch_gemm_kt(L.D, ntile, 4 * H, ns, k0, k1, sb, cs, bs, H, splits, L.FeatT, pF, fsplit, st)) return -1;
-  }
-  if (launch_reduce_splits(pB, L.dB, 2ll * H * H, splits, 0, st)) return -1;
-  if (launch_reduce_splits(pBh, L.dB + (size_t)2 * H * H, (long long)H * H, splits, 0, st)) return -1;
-  k_g_fw_scatter<<<cdiv(4ll * H * 32, 32), dim3(32, 8), 0, st>>>(pF, splits, H, L.dP, L.dcg, L.dM0, L.dc0);
-  REGT_LAUNCHED("k_g_fw_scatter", st);
-  if (a->plan.nseg > 0) {   // dM1[r]: per-region sums over the (node, region) segments
-    if (launch_wgrad_m1_kt(a, L, st)) return -1;
   }
   return launch_chain(a, L, st);
 }

@@ -576,21 +576,6 @@ __global__ void k_hid_reduce(const float* __restrict__ part, int ntc, int nqt, i
 // ------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------
-int launch_spmm_rows(const int32_t* rowptr, const int32_t* col, const float* val, const float* x, float* y, int B,
-                     int n_out, int n_in, int width, cudaStream_t st);
-int launch_prep(const regt_args* a, const Layout& L, cudaStream_t st);
-int launch_feat_tc(const regt_graph_plan& p, const float* x, int B, int xN, int T, float* Xt, float* St, float* Ut, cudaStream_t st);
-
-static int num_sms() {
-  static int n = 0;
-  if (n == 0) {
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0)
-      n = 148;
-  }
-  return n;
-}
-
 // periods per work item: maximise SM utilisation of the last wave, prefer longer chunks
 static int choose_tp(int nqt, int T, int slots) {
   int best = 1;
@@ -608,13 +593,9 @@ static int choose_tp(int nqt, int T, int slots) {
   return best;
 }
 
-bool head_fusable(const regt_args* a);
-bool head_tc_usable(const regt_args* a);
-int head_tc_grid(const regt_args* a);
-int launch_head_grad_reduce(const regt_args* a, const Layout& L, cudaStream_t st);
 int tc_num_chunks(const regt_args* a) {
   const int BN = a->B * a->N, nqt = (BN + TC_ROWS - 1) / TC_ROWS;
-  return a->T / choose_tp(nqt, a->T, num_sms());
+  return a->T / choose_tp(nqt, a->T, sm_count());
 }
 
 static TcArgs make_tcargs(const regt_args* a, const Layout& L, int slots) {
@@ -646,14 +627,14 @@ static int run_fwd_tc(const regt_args* a, const Layout& L, cudaStream_t st, bool
                                                   a->p.lin_w[0], a->p.lin_w[1], a->p.lin_w[2], L.tc_img_f, L.tc_img_b);
   REGT_LAUNCHED("k_pack_tc", st);
   if (forked && join_side(st)) return -1;   // the feature builder ran beside the weight collapse
-  const int slots = num_sms();
+  const int slots = sm_count();
   TcArgs k = make_tcargs(a, L, slots);
   const size_t smem = 1024 + ((Cfg::FWD_IMG + 1023) & ~1023) + Cfg::A_TILE + 2 * Cfg::SMF_TILE;
   REGT_CUDA(cudaFuncSetAttribute(k_cell_fwd_tc<HH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int grid = tc_fwd_grid(k, slots);
   k_cell_fwd_tc<HH><<<grid, NTHREADS, smem, st>>>(k);
   REGT_LAUNCHED("k_cell_fwd_tc", st);
-  if (!head_fusable(a)) {  // otherwise the fused head sums the partials while loading its tiles
+  if (!L.route.hid_partials) {  // otherwise the head sums the partials while loading its tiles
     const long long count = (long long)k.BN * HH;
     k_hid_reduce<<<cdiv(count / 4, 256), 256, 0, st>>>(L.hid_part, k.ntc, k.nqt, HH, k.BN, a->out_hidden);
     REGT_LAUNCHED("k_hid_reduce", st);
@@ -1119,16 +1100,13 @@ __global__ void __launch_bounds__(HH) k_wgrad_m1_tc(const float* __restrict__ dh
   for (int f = 0; f < F; ++f) o[f] = acc[f];
 }
 
-int launch_chain(const regt_args* a, const Layout& L, cudaStream_t st);
-int launch_reduce_splits(const float* part, float* out, long long count, int splits, int accumulate, cudaStream_t st);
-
 int cell_backward_tc(const regt_args* a, const Layout& L, cudaStream_t st) {
   REGT_CHECK(a->precision == REGT_PREC_BF16,
              "the tensor-core cell backward is built for precision bf16 only");
   REGT_CHECK(a->H == 64 && a->mode != REGT_MODE_TGCN, "tensor-core backward: hidden=64, TemporalGCN / RegionalTemporalGCN only");
   constexpr int HH = 64;
   using Cfg = TcCfg<HH>;
-  const int slots = num_sms();
+  const int slots = sm_count();
   TcArgs k = make_tcargs(a, L, slots);
   k.img = L.tc_img_b;
   const int grid = tc_bwd_grid(k, slots);
@@ -1136,7 +1114,7 @@ int cell_backward_tc(const regt_args* a, const Layout& L, cudaStream_t st) {
                       3 * PlaneIO<__nv_bfloat16, HH>::TILE_BYTES + TC_ROWS * HH * 4;
   REGT_CUDA(cudaFuncSetAttribute(k_cell_bwd_tc<HH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   // the head's partial sums (left by the tensor-core head in regt_head_forward) are reduced beside the cell backward
-  const bool head_sum = head_tc_usable(a);
+  const bool head_sum = L.route.head == HeadPath::Bf16;
   cudaStream_t side = head_sum ? fork_side(st) : nullptr;
   if (head_sum && launch_head_grad_reduce(a, L, side ? side : st)) return -1;
   k_cell_bwd_tc<HH><<<grid, NTHREADS, smem, st>>>(k);
@@ -1164,7 +1142,7 @@ extern "C" int regt_debug_tc_split(int32_t B, int32_t N, int32_t T, int32_t* out
   REGT_CHECK(B > 0 && N > 0 && T > 0 && out, "regt_debug_tc_split: B, N, T must be positive and out non-NULL");
   regt_args a{};
   a.B = B; a.N = N; a.T = T;
-  const int slots = regt::num_sms();
+  const int slots = regt::sm_count();
   const regt::TcArgs k = regt::make_tcargs(&a, regt::Layout{}, slots);
   const int32_t v[7] = {k.nqt, k.tp, k.ntc, k.items, regt::tc_fwd_grid(k, slots), regt::tc_bwd_grid(k, slots),
                         regt::head_tc_grid(&a)};

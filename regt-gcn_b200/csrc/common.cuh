@@ -70,8 +70,41 @@ struct Carver {
 
 __device__ __forceinline__ float sigmoidf_(float v) { return 1.0f / (1.0f + expf(-v)); }
 
+// offset of G[q][n] (gradient wrt out_hidden): row major, or the [qt][H/4][128][4] tiles the fused cell backwards read
+__device__ __forceinline__ size_t g_off(long long q, int n, int H, int tiled) {
+  return tiled ? ((((size_t)(q >> 7) * (H >> 2) + (n >> 2)) * 128 + (size_t)(q & 127)) * 4 + (n & 3)) : ((size_t)q * H + n);
+}
+
+// multiprocessor count of the current device (148 when it cannot be read)
+inline int sm_count() {
+  static int n = 0;
+  if (n == 0) {
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = 148;
+  }
+  return n;
+}
+
+// ---- which cell and head kernels a call runs (route_of, api.cu) ----------------------
+enum class CellPath { Fp32, Tf32x3Unfused, Tf32x3Fused, Bf16 };   // cell.cu, cell_g.cu, cell_f.cu, cell_tc.cu
+enum class HeadPath { Rows, FusedFfma, Tf32x3, Bf16 };             // k_head_fwd / k_head_bwd, k_head_fused, head_f.cu, k_head_tc
+struct Route {
+  CellPath cell;
+  HeadPath head;
+  bool g_tiled;        // G is written as tiles (g_off): the fused tf32x3 and bf16 cell backwards read it so
+  bool hid_partials;   // the bf16 forward leaves per-chunk partials of out_hidden and the head sums them (no k_hid_reduce)
+};
+// reads REGT_UNFUSED ("1": the GEMM-by-GEMM tf32x3 cell of cell_g.cu wherever the fused one would run); no CUDA calls
+Route route_of(const regt_args* a);
+// the shapes each implementation is built for, with no knowledge of the other paths
+bool cell_f_fits(const regt_args* a);   // fused tf32x3 cell: hidden 64 / 128, not the bare TGCN cell, <= 64 periods
+bool head_fused_fits(int H, int O);     // k_head_fused: hidden 32 / 64, <= 64 outputs, within a block's shared memory
+bool head_tc_fits(int H, int O);        // k_head_tc: hidden 64, <= 16 outputs
+bool head_f_fits(int O);                // k_hf_mid: <= 16 outputs
+
 // ---- workspace layout shared by forward / backward (cell.cu, head.cu, api.cu) -------
 struct Layout {
+  Route route;   // the kernels of this call: the layout below and every launcher follow it
   // collapsed weights (rebuilt every forward: parameters change between steps)
   float* Wzr;    // [F+H][2H]   rows 0..F-1: (A_g W_g)^T, rows F..: B_g^T ; cols 0..H-1 z, H..2H-1 r
   float* Wc;     // [F+H][H]
@@ -132,13 +165,67 @@ struct Layout {
 constexpr int TC_MAX_CTAS = 160;
 constexpr int TC_IMG_BYTES = 160 * 1024;
 constexpr int F_IMG_BYTES = 432 * 1024;   // fused 3xTF32 cell (cell_f.cu): 12 ring stages of 32 KB + F-wide weights + constants at H = 128
-bool cell_f_usable(const regt_args* a);
-bool head_f_usable(const regt_args* a);   // precision tf32x3, hidden % 32 == 0, output_dim <= 16, >= 128 rows   // precision tf32x3, hidden 128 / 64, not the bare TGCN cell
 
 Layout make_layout(const regt_args* a, void* base);
-size_t gemm_nt_scratch_floats(int N, int K);
 
 constexpr int HEAD_HID = 128;  // hidden_dim of the decoder MLP (models/RegionalTemporalGCN.py:19)
 constexpr int WGRAD_SPLITS = 64;
+
+// ---- host functions one file calls in another ----------------------------------------
+// cell and head of each path (api.cu dispatches on Layout::route)
+int cell_forward_fp32(const regt_args* a, const Layout& L, cudaStream_t st);    // cell.cu
+int cell_backward_fp32(const regt_args* a, const Layout& L, cudaStream_t st);
+int cell_forward_g(const regt_args* a, const Layout& L, cudaStream_t st);       // cell_g.cu
+int cell_backward_g(const regt_args* a, const Layout& L, cudaStream_t st);
+int cell_forward_f(const regt_args* a, const Layout& L, cudaStream_t st);       // cell_f.cu
+int cell_backward_f(const regt_args* a, const Layout& L, cudaStream_t st);
+int cell_forward_tc(const regt_args* a, const Layout& L, cudaStream_t st);      // cell_tc.cu
+int cell_backward_tc(const regt_args* a, const Layout& L, cudaStream_t st);
+size_t cell_backward_x_scratch_bytes(const regt_args* a, const regt_xgrad_plan* xp);   // input_grad.cu
+int cell_backward_x(const regt_args* a, const Layout& L, const regt_xgrad_plan* xp, float* d_x, void* scratch, cudaStream_t st);
+int head_forward(const regt_args* a, const Layout& L, cudaStream_t st);         // head.cu
+int head_backward(const regt_args* a, const Layout& L, cudaStream_t st);
+int head_forward_f(const regt_args* a, const Layout& L, cudaStream_t st);       // head_f.cu
+int head_backward_f(const regt_args* a, const Layout& L, cudaStream_t st);
+int head_forward_tc(const regt_args* a, const Layout& L, cudaStream_t st);      // head_tc.cu
+
+// weights.cu: collapsed weights before the cell, chain rule back to the parameters after it
+int launch_prep(const regt_args* a, const Layout& L, cudaStream_t st);
+int launch_chain(const regt_args* a, const Layout& L, cudaStream_t st);
+// spmm.cu: F-wide SpMM on rows of `width` floats; period-major Xt / St / Ut of the tensor-core cells
+int launch_spmm_rows(const int32_t* rowptr, const int32_t* col, const float* val, const float* x, float* y, int B,
+                     int n_out, int n_in, int width, cudaStream_t st);
+int launch_feat_tc(const regt_graph_plan& p, const float* x, int B, int xN, int T, float* Xt, float* St, float* Ut, cudaStream_t st);
+// cell.cu
+struct TNBatch;   // gemm_simt.cuh
+int launch_wgrad_tn(const TNBatch& batch, long long rows, int splits, cudaStream_t st);   // split-K C = A^T B per problem of the batch
+// out[i] (+)= sum_s part[s*count + i]
+int launch_reduce_splits(const float* part, float* out, long long count, int splits, int accumulate, cudaStream_t st);
+// part[s][c] = sum over the rows of split s of A[r*lda + c]
+int launch_colsum(const float* A, int lda, int C, long long rows, int splits, float* part, cudaStream_t st);
+int launch_wgrad_m1(const regt_args* a, const Layout& L, cudaStream_t st);      // dM1 per region from the row-major gate gradients
+int launch_wgrad_m1_kt(const regt_args* a, const Layout& L, cudaStream_t st);   // ... from the transposed tiles of the fused backward
+// cell_g.cu: d probs from the fused backward's fp64 partials; F-wide weight gradients from the [splits][4H][32] partials of D^T Feat
+int launch_f_sum_dpp(const double* part, int nparts, int T, float* dprobs, cudaStream_t st);
+int launch_fw_scatter(const float* Cp, int splits, int H, const Layout& L, cudaStream_t st);
+// gemm_tma.cu: TMA-fed 3xTF32 GEMMs
+size_t gemm_nt_scratch_floats(int N, int K);
+int launch_gemm_nt_tma(const float* A, long long lda, const float* Bt, long long ldb, float* C, long long ldc, long long M, int N,
+                       int K, float* scratch, cudaStream_t st);
+int launch_gemm_tn(const float* A, long long lda, const float* B, long long ldb, float* Cp, long long M, int K, int N, int splits,
+                   cudaStream_t st, const float* B2, long long ldb2, float* Cp2, long long c2_split, int relu_b);
+int launch_gemm_tn_tma(const float* A, long long lda, long long M, int Ktot, int nseg, const int* seg_k0, const int* seg_b,
+                       float* const* seg_C, const float* const* Bs, const long long* ldbs, int N, int splits, const float* B2,
+                       long long ldb2, float* C2, long long c2_split, cudaStream_t st, int relu_b);
+int launch_gemm_kt(const float* AT, long long ntile, int Ktot, int nseg, const int* seg_k0, const int* seg_k1, const int* seg_b,
+                   float* const* seg_C, const float* const* BTs, int N, int splits, const float* FT, float* C2, long long c2_split,
+                   cudaStream_t st);
+// head.cu / head_tc.cu: the fused heads' per-CTA partials and their cross-CTA sum
+int head_part_stride_host(int H, int O);
+int launch_head_grad_reduce(const regt_args* a, const Layout& L, cudaStream_t st);
+int launch_head_dw1_tf32x3(const regt_args* a, const Layout& L, const float* ones, cudaStream_t st);
+int head_tc_grid(const regt_args* a);
+// cell_tc.cu: period chunks of the bf16 forward (the partials of out_hidden it leaves)
+int tc_num_chunks(const regt_args* a);
 
 }  // namespace regt

@@ -111,10 +111,4 @@ struct TNBatch {
   int nprob;
 };
 
-int launch_wgrad_tn(const TNBatch& batch, long long rows, int splits, cudaStream_t st);
-// out[i] (+)= sum_s part[s*count + i]
-int launch_reduce_splits(const float* part, float* out, long long count, int splits, int accumulate, cudaStream_t st);
-// part[s][c] = sum over the rows of split s of A[r*lda + c]
-int launch_colsum(const float* A, int lda, int C, long long rows, int splits, float* part, cudaStream_t st);
-
 }  // namespace regt

@@ -77,15 +77,6 @@ int tmap_2d(CUtensorMap* m, const float* base, long long cols, long long rows, l
   REGT_CHECK(r == CUDA_SUCCESS, "%s: cuTensorMapEncodeTiled failed (%d) cols=%lld rows=%lld ld=%lld", who, (int)r, cols, rows, ld);
   return 0;
 }
-int sm_count() {
-  static int sms = 0;
-  if (sms == 0) {
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sms <= 0)
-      sms = 148;
-  }
-  return sms;
-}
 
 // ------------------------------------------------------------------------------------------
 // dense hi / lo images of a weight operand: hi[n][k] = tf32(B[n][k]), lo = B - hi, zero-padded to [Np][Kp]

@@ -20,9 +20,6 @@ struct HeadK {
   float* hid_out;         // where the summed out_hidden goes when hid_part is used
   int g_tiled;            // 1: G is written as [qt][H/4][128][4] tiles (tensor-core backward), 0: row-major
 };
-__device__ __forceinline__ size_t g_off(long long q, int n, int H, int tiled) {
-  return tiled ? ((((size_t)(q >> 7) * (H >> 2) + (n >> 2)) * 128 + (size_t)(q & 127)) * 4 + (n & 3)) : ((size_t)q * H + n);
-}
 
 __global__ void k_head_transpose(const float* __restrict__ w1, const float* __restrict__ w2, int H, int O,
                                  float* __restrict__ W1t, float* __restrict__ W2t) {
@@ -420,21 +417,12 @@ static size_t head_fused_smem(int H, int O) {
 }
 // H = 64 fits up to O = 44 in the 227 KB a block may use (O = 45 would need 229 KB), H = 32 every O up to 64; wider
 // heads run k_head_fwd / k_head_bwd
-bool head_fusable(const regt_args* a) {
-  return a->fuse_head && a->y && a->d_out && a->loss && (a->H == 64 || a->H == 32) && a->O <= 64 &&
-         head_fused_smem(a->H, a->O) <= 227 * 1024;
-}
+bool head_fused_fits(int H, int O) { return (H == 64 || H == 32) && O <= 64 && head_fused_smem(H, O) <= 227 * 1024; }
 static int head_fused_grid(const regt_args* a) {
   const long long BN = (long long)a->B * a->N;
   return (int)min((long long)HP_MAX_CTAS, (BN + TMH - 1) / TMH);
 }
 
-bool head_fusable(const regt_args* a);
-int tc_num_chunks(const regt_args* a);
-// tcgen05 head (head_tc.cu): bf16 precision, hidden 64, output_dim <= 16
-bool head_tc_usable(const regt_args* a);
-int head_tc_grid(const regt_args* a);
-int head_forward_tc(const regt_args* a, const Layout& L, cudaStream_t st, bool cell_left_partials);
 int head_part_stride_host(int H, int O) { return head_part_stride(H, O); }
 static HeadK make_headk(const regt_args* a, const Layout& L, float* W1t, float* W2t) {
   HeadK k{};
@@ -444,8 +432,8 @@ static HeadK make_headk(const regt_args* a, const Layout& L, float* W1t, float* 
   k.w1 = a->p.head_w1; k.w2 = a->p.head_w2; k.d_hidden = a->d_hidden;
   k.a1 = L.a1; k.out = a->out; k.d_out = a->d_out; k.loss_part = L.part; k.d_a1 = L.d_a1; k.G = L.G;
   k.hid_part = nullptr; k.ntc = 0; k.hid_out = a->out_hidden;
-  k.g_tiled = a->precision == REGT_PREC_BF16 || cell_f_usable(a);   // the fused tcgen05 backward kernels read G tiles
-  if (a->precision == REGT_PREC_BF16 && head_fusable(a)) {  // the cell left per-chunk partials (see cell_tc.cu)
+  k.g_tiled = L.route.g_tiled;
+  if (L.route.hid_partials) {  // the cell left per-chunk partials (see cell_tc.cu)
     k.hid_part = L.hid_part;
     k.ntc = tc_num_chunks(a);
     k.nqt = (int)((k.BN + 127) / 128);
@@ -453,26 +441,26 @@ static HeadK make_headk(const regt_args* a, const Layout& L, float* W1t, float* 
   return k;
 }
 
-int head_forward_f(const regt_args* a, const Layout& L, cudaStream_t st);
-int head_backward_f(const regt_args* a, const Layout& L, cudaStream_t st, int g_tiled);
-
-int head_forward_fp32(const regt_args* a, const Layout& L, cudaStream_t st) {
+int head_forward(const regt_args* a, const Layout& L, cudaStream_t st) {
   const int H = a->H, O = a->O;
-  if (head_tc_usable(a)) return head_forward_tc(a, L, st, true);
-  if (head_f_usable(a)) return head_forward_f(a, L, st);      // tf32x3: the 128-wide GEMMs on the tensor cores (head_f.cu)
-  if (head_fusable(a)) {
-    HeadK k = make_headk(a, L, nullptr, nullptr);
-    const int grid = head_fused_grid(a), ntiles = cdiv(k.BN, TMH);
-    const size_t smem = head_fused_smem(H, O);
-    if (H == 64) {
-      REGT_CUDA(cudaFuncSetAttribute(k_head_fused<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      k_head_fused<64><<<grid, 256, smem, st>>>(k, L.hpart, ntiles);
-    } else {
-      REGT_CUDA(cudaFuncSetAttribute(k_head_fused<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      k_head_fused<32><<<grid, 256, smem, st>>>(k, L.hpart, ntiles);
+  switch (L.route.head) {
+    case HeadPath::Bf16: return head_forward_tc(a, L, st);
+    case HeadPath::Tf32x3: return head_forward_f(a, L, st);   // the 128-wide GEMMs on the tensor cores (head_f.cu)
+    case HeadPath::FusedFfma: {
+      HeadK k = make_headk(a, L, nullptr, nullptr);
+      const int grid = head_fused_grid(a), ntiles = cdiv(k.BN, TMH);
+      const size_t smem = head_fused_smem(H, O);
+      if (H == 64) {
+        REGT_CUDA(cudaFuncSetAttribute(k_head_fused<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        k_head_fused<64><<<grid, 256, smem, st>>>(k, L.hpart, ntiles);
+      } else {
+        REGT_CUDA(cudaFuncSetAttribute(k_head_fused<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        k_head_fused<32><<<grid, 256, smem, st>>>(k, L.hpart, ntiles);
+      }
+      REGT_LAUNCHED("k_head_fused", st);
+      return 0;   // loss and head gradients are finalised by k_head_grad_reduce in regt_head_backward
     }
-    REGT_LAUNCHED("k_head_fused", st);
-    return 0;   // loss and head gradients are finalised by k_head_grad_reduce in regt_head_backward
+    case HeadPath::Rows: break;
   }
   // transposed head weights live at the tail of the split-K scratch's first page
   float* W1t = L.part + L.part_floats - ((size_t)H * HEAD_HID + (size_t)HEAD_HID * O);
@@ -493,8 +481,6 @@ int head_forward_fp32(const regt_args* a, const Layout& L, cudaStream_t st) {
   return 0;
 }
 
-int launch_gemm_tn(const float* A, long long lda, const float* B, long long ldb, float* Cp, long long M, int K, int N, int splits,
-                   cudaStream_t st, const float* B2, long long ldb2, float* Cp2, long long c2_split, int relu_b);
 // out[r] (+)= sum over splits of Cp2[s][r][col]   (one column of a [splits][rows][32] partial array)
 __global__ void k_pick_col(const float* __restrict__ Cp2, int splits, int rows, int col, int acc, float* __restrict__ out) {
   const int r = threadIdx.x;
@@ -504,30 +490,44 @@ __global__ void k_pick_col(const float* __restrict__ Cp2, int splits, int rows, 
   out[r] = acc ? out[r] + s : s;
 }
 
+// dW1 = d_a1^T relu(hid) and, in the same pass over d_a1, db1 on the tensor cores (TMA-fed 3xTF32 row contraction): db1 is
+// column 16 of d_a1^T ones, where `ones` is a [>= BN][32] plane whose column 16 is all ones, split over the rows to fill the SMs
+int launch_head_dw1_tf32x3(const regt_args* a, const Layout& L, const float* ones, cudaStream_t st) {
+  const int H = a->H;
+  const long long BN = (long long)a->B * a->N;
+  const int s1 = (int)max(1ll, min((long long)cdiv(148, cdiv(H, 128)), BN / 256));
+  float* p1 = L.part;                                  // [s1][128][H]    d_a1^T relu(hid)
+  float* p2 = L.part + (size_t)s1 * HEAD_HID * H;      // [s1][128][32]   d_a1^T ones  -> column 16 = db1
+  if (launch_gemm_tn(L.d_a1, HEAD_HID, a->out_hidden, H, p1, BN, HEAD_HID, H, s1, st, ones, 32, p2, 0, 1)) return -1;
+  if (launch_reduce_splits(p1, a->g.head_w1, (long long)HEAD_HID * H, s1, a->accumulate, st)) return -1;
+  k_pick_col<<<1, HEAD_HID, 0, st>>>(p2, s1, HEAD_HID, 16, a->accumulate, a->g.head_b1);
+  REGT_LAUNCHED("k_pick_col", st);
+  return 0;
+}
+
 int launch_head_grad_reduce(const regt_args* a, const Layout& L, cudaStream_t st) {
   const int H = a->H, O = a->O;
   const int stride = head_part_stride(H, O), n = HEAD_HID * H + O * HEAD_HID + HEAD_HID + O;
-  k_head_grad_reduce<<<cdiv(n + 1, 32), dim3(32, 8), 0, st>>>(L.hpart, stride, head_tc_usable(a) ? head_tc_grid(a) : head_fused_grid(a),
-                                                            H, O, a->accumulate, a->g.head_w1, a->g.head_w2, a->g.head_b1,
-                                                            a->g.head_b2, a->loss);
+  const int ncta = L.route.head == HeadPath::Bf16 ? head_tc_grid(a) : head_fused_grid(a);
+  k_head_grad_reduce<<<cdiv(n + 1, 32), dim3(32, 8), 0, st>>>(L.hpart, stride, ncta, H, O, a->accumulate, a->g.head_w1,
+                                                            a->g.head_w2, a->g.head_b1, a->g.head_b2, a->loss);
   REGT_LAUNCHED("k_head_grad_reduce", st);
   return 0;
 }
 
-int head_backward_fp32(const regt_args* a, const Layout& L, cudaStream_t st) {
+int head_backward(const regt_args* a, const Layout& L, cudaStream_t st) {
   const int H = a->H, O = a->O;
   const long long BN = (long long)a->B * a->N;
-  if (!head_f_usable(a) && head_fusable(a)) {  // everything but the cross-CTA sum already happened in head_forward
-    // tensor-core step: the sum runs beside the cell backward (launch_head_grad_reduce from cell_backward_tc)
-    if (head_tc_usable(a)) return 0;
-    return launch_head_grad_reduce(a, L, st);
-  }
+  // fused heads: everything but the cross-CTA sum already happened in head_forward; the bf16 step runs that sum beside
+  // the cell backward (launch_head_grad_reduce from cell_backward_tc)
+  if (L.route.head == HeadPath::Bf16) return 0;
+  if (L.route.head == HeadPath::FusedFfma) return launch_head_grad_reduce(a, L, st);
   if (!a->d_out) {  // only out_hidden carries gradient
-    k_copy_or_zero<<<cdiv(BN * H, 256), 256, 0, st>>>(a->d_hidden, L.G, BN * H, H, a->precision == REGT_PREC_BF16 || cell_f_usable(a));
+    k_copy_or_zero<<<cdiv(BN * H, 256), 256, 0, st>>>(a->d_hidden, L.G, BN * H, H, L.route.g_tiled);
     REGT_LAUNCHED("k_copy_or_zero", st);
     return 0;
   }
-  if (head_f_usable(a)) return head_backward_f(a, L, st, a->precision == REGT_PREC_BF16 || cell_f_usable(a));
+  if (L.route.head == HeadPath::Tf32x3) return head_backward_f(a, L, st);
   HeadK k = make_headk(a, L, nullptr, nullptr);
   const int nblk = cdiv(BN, TMH);
   const size_t smem = ((size_t)TMH * (O + 1) + TMH * (HEAD_HID + 1) + KT * TN + 4) * sizeof(float);
@@ -539,15 +539,8 @@ int head_backward_fp32(const regt_args* a, const Layout& L, cudaStream_t st) {
   const int splits = (int)max(1ll, min(128ll, BN / 128));
   float* part = L.part;
   if (a->precision == REGT_PREC_TF32X3 && H % 32 == 0 && BN >= 128) {
-    // tensor cores (TMA-fed 3xTF32 row contraction): dW1 = d_a1^T relu(hid) and, in the same pass over d_a1, its column sums
-    // (column 16 of the cell's feature plane is all ones; its first BN rows serve as the second operand)
-    const int s1 = (int)max(1ll, min((long long)cdiv(148, cdiv(H, 128)), BN / 256));
-    float* p1 = part;                                    // [s1][128][H]
-    float* p2 = part + (size_t)s1 * HEAD_HID * H;        // [s1][128][32]
-    if (launch_gemm_tn(L.d_a1, HEAD_HID, a->out_hidden, H, p1, BN, HEAD_HID, H, s1, st, L.Feat, 32, p2, 0, 1)) return -1;
-    if (launch_reduce_splits(p1, a->g.head_w1, (long long)HEAD_HID * H, s1, a->accumulate, st)) return -1;
-    k_pick_col<<<1, HEAD_HID, 0, st>>>(p2, s1, HEAD_HID, 16, a->accumulate, a->g.head_b1);
-    REGT_LAUNCHED("k_pick_col", st);
+    // dW1, db1 on the tensor cores: column 16 of the cell's feature plane is all ones, its first BN rows are the operand
+    if (launch_head_dw1_tf32x3(a, L, L.Feat, st)) return -1;
     TNBatch tb{};
     tb.nprob = 1;
     tb.p[0] = TNProb{a->d_out, L.a1, part, O, HEAD_HID, O, HEAD_HID, 0};

@@ -16,13 +16,6 @@
 
 namespace regt {
 
-int launch_gemm_nt_tma(const float* A, long long lda, const float* Bt, long long ldb, float* C, long long ldc, long long M, int N,
-                       int K, float* scratch, cudaStream_t st);
-int launch_gemm_tn(const float* A, long long lda, const float* B, long long ldb, float* Cp, long long M, int K, int N, int splits,
-                   cudaStream_t st, const float* B2, long long ldb2, float* Cp2, long long c2_split, int relu_b);
-int launch_reduce_splits(const float* part, float* out, long long count, int splits, int accumulate, cudaStream_t st);
-int launch_colsum(const float* A, int lda, int C, long long rows, int splits, float* part, cudaStream_t st);
-
 namespace {
 __global__ void __launch_bounds__(256) k_hf_relu(const float4* __restrict__ hid, float4* __restrict__ rh, long long n4) {
   const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
@@ -139,9 +132,6 @@ __global__ void __launch_bounds__(256) k_hf_da1(const float* __restrict__ a1, co
   dO32[q * 32 + lane] = lane < O ? dv : (lane == 16 ? 1.0f : 0.f);
 }
 
-__device__ __forceinline__ size_t g_off_f(long long q, int n, int H, int tiled) {
-  return tiled ? ((((size_t)(q >> 7) * (H >> 2) + (n >> 2)) * 128 + (size_t)(q & 127)) * 4 + (n & 3)) : ((size_t)q * H + n);
-}
 // G = Gpre * (hid > 0) + d_hidden, four columns per thread
 __global__ void __launch_bounds__(256) k_hf_gmask(const float4* __restrict__ gpre, const float4* __restrict__ hid, const float4* __restrict__ dh,
                                                   long long BN, int H, int tiled, float* __restrict__ G) {
@@ -156,7 +146,7 @@ __global__ void __launch_bounds__(256) k_hf_gmask(const float4* __restrict__ gpr
     const float4 d = __ldg(dh + i);
     v.x += d.x; v.y += d.y; v.z += d.z; v.w += d.w;
   }
-  *reinterpret_cast<float4*>(G + g_off_f(q, n, H, tiled)) = v;
+  *reinterpret_cast<float4*>(G + g_off(q, n, H, tiled)) = v;
 }
 // W1t[k][m] = w1[m][k]   (K-major operand of the data-gradient GEMM)
 __global__ void k_hf_w1t(const float* __restrict__ w1, int H, float* __restrict__ W1t) {
@@ -174,18 +164,9 @@ __global__ void k_hf_dw2(const float* __restrict__ C2, int splits, int O, int ac
   for (int z = 0; z < splits; ++z) s += C2[((size_t)z * HEAD_HID + n) * 32 + o];
   dW2[i] = acc ? dW2[i] + s : s;
 }
-__global__ void k_hf_pick_col(const float* __restrict__ Cp2, int splits, int rows, int col, int acc, float* __restrict__ out) {
-  const int r = threadIdx.x;
-  if (r >= rows || !out) return;
-  float s = 0.f;
-  for (int z = 0; z < splits; ++z) s += Cp2[((size_t)z * rows + r) * 32 + col];
-  out[r] = acc ? out[r] + s : s;
-}
 }  // namespace
 
-bool head_f_usable(const regt_args* a) {
-  return a->precision == REGT_PREC_TF32X3 && a->H % 32 == 0 && a->O <= HF_O && (long long)a->B * a->N >= 128 && a->out;
-}
+bool head_f_fits(int O) { return O <= HF_O; }
 
 int head_forward_f(const regt_args* a, const Layout& L, cudaStream_t st) {
   const int H = a->H, O = a->O;
@@ -204,7 +185,7 @@ int head_forward_f(const regt_args* a, const Layout& L, cudaStream_t st) {
   return 0;
 }
 
-int head_backward_f(const regt_args* a, const Layout& L, cudaStream_t st, int g_tiled) {
+int head_backward_f(const regt_args* a, const Layout& L, cudaStream_t st) {
   const int H = a->H, O = a->O;
   const long long BN = (long long)a->B * a->N;
   k_hf_da1<<<cdiv(BN, 8), 256, 0, st>>>(L.a1, a->p.head_w2, a->d_out, BN, O, L.d_a1, L.hf_do32);
@@ -215,17 +196,11 @@ int head_backward_f(const regt_args* a, const Layout& L, cudaStream_t st, int g_
   // Gpre[q][k] = sum_n d_a1[q][n] W1[n][k]
   if (launch_gemm_nt_tma(L.d_a1, HEAD_HID, W1t, HEAD_HID, L.hf_rh, H, BN, H, HEAD_HID, L.hf_split, st)) return -1;
   k_hf_gmask<<<cdiv(BN * (H / 4), 256), 256, 0, st>>>(reinterpret_cast<const float4*>(L.hf_rh), reinterpret_cast<const float4*>(a->out_hidden),
-                                                      reinterpret_cast<const float4*>(a->d_hidden), BN, H, g_tiled, L.G);
+                                                      reinterpret_cast<const float4*>(a->d_hidden), BN, H, L.route.g_tiled, L.G);
   REGT_LAUNCHED("k_hf_gmask", st);
   // weight gradients: row contractions on the tensor cores, split over the rows so that the grid fills the SMs
   float* part = L.part;
-  const int s1 = (int)max(1ll, min((long long)cdiv(148, cdiv(H, 128)), BN / 256));
-  float* p1 = part;                                    // [s1][128][H]    d_a1^T relu(hid)
-  float* p2 = part + (size_t)s1 * HEAD_HID * H;        // [s1][128][32]   d_a1^T [. | 1]  -> column 16 = db1
-  if (launch_gemm_tn(L.d_a1, HEAD_HID, a->out_hidden, H, p1, BN, HEAD_HID, H, s1, st, L.hf_do32, 32, p2, 0, 1)) return -1;
-  if (launch_reduce_splits(p1, a->g.head_w1, (long long)HEAD_HID * H, s1, a->accumulate, st)) return -1;
-  k_hf_pick_col<<<1, HEAD_HID, 0, st>>>(p2, s1, HEAD_HID, 16, a->accumulate, a->g.head_b1);
-  REGT_LAUNCHED("k_hf_pick_col", st);
+  if (launch_head_dw1_tf32x3(a, L, L.hf_do32, st)) return -1;   // [d_out | 1]: column 16 is the ones column
   const int s2 = (int)max(1ll, min(148ll, BN / 256));
   float* p3 = part;                                    // [s2][128][32]   a1^T [d_out | 1]
   if (launch_gemm_tn(L.a1, HEAD_HID, nullptr, 0, nullptr, BN, HEAD_HID, 0, s2, st, L.hf_do32, 32, p3, 0, 0)) return -1;

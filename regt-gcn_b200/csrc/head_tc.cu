@@ -388,25 +388,21 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_head_tc(HeadTcArgs a) {
   if (warp == WARP_MMA) tmem_dealloc(tmem, 512);
 }
 
-bool head_tc_usable(const regt_args* a) {
-  return a->precision == REGT_PREC_BF16 && a->fuse_head && a->y && a->d_out && a->loss && a->H == HH && a->O <= OP;
-}
+bool head_tc_fits(int H, int O) { return H == HH && O <= OP; }
 int head_tc_grid(const regt_args* a) {
   const long long BN = (long long)a->B * a->N;
   return (int)min((long long)148, (BN + TC_ROWS - 1) / TC_ROWS);
 }
-int head_part_stride_host(int H, int O);
-int tc_num_chunks(const regt_args* a);
-
-int head_forward_tc(const regt_args* a, const Layout& L, cudaStream_t st, bool cell_left_partials) {
+// the bf16 cell left per-chunk partials of out_hidden (Route::hid_partials): summed here while loading the tiles
+int head_forward_tc(const regt_args* a, const Layout& L, cudaStream_t st) {
   HeadTcArgs k{};
   k.BN = (long long)a->B * a->N;
   k.O = a->O;
   k.nqt = (int)((k.BN + TC_ROWS - 1) / TC_ROWS);
   k.scale = 1.0f / ((float)(a->loss_nodes > 0 ? a->loss_nodes : a->N) * (float)a->O);
   k.w1 = a->p.head_w1; k.w2 = a->p.head_w2; k.b1 = a->p.head_b1; k.b2 = a->p.head_b2;
-  k.hid_part = cell_left_partials ? L.hid_part : nullptr;
-  k.ntc = cell_left_partials ? tc_num_chunks(a) : 0;
+  k.hid_part = L.hid_part;
+  k.ntc = tc_num_chunks(a);
   k.hid_in = a->out_hidden; k.hid_out = a->out_hidden;
   k.y = a->y; k.d_hidden = a->d_hidden;
   k.out = a->out; k.d_out = a->d_out; k.G = L.G; k.hpart = L.hpart;

@@ -19,9 +19,6 @@ namespace regt {
 
 constexpr int F = REGT_F;
 
-int launch_spmm_rows(const int32_t* rowptr, const int32_t* col, const float* val, const float* x, float* y, int B,
-                     int n_out, int n_in, int width, cudaStream_t st);
-
 struct XgK {
   const float* D;          // gate-gradient plane (layout: TILED below)
   const float *Wzr, *Wc;   // collapsed gate weights; rows 0..F-1 are (A_g W_g)^T
@@ -171,7 +168,7 @@ size_t cell_backward_x_scratch_bytes(const regt_args* a, const regt_xgrad_plan* 
 int cell_backward_x(const regt_args* a, const Layout& L, const regt_xgrad_plan* xp, float* d_x, void* scratch, cudaStream_t st) {
   const int H = a->H, T = a->T, R = a->plan.R > 0 ? a->plan.R : 1;
   const XgScratch S = xg_scratch(a, xp, scratch);
-  const bool tiled = a->precision == REGT_PREC_TF32X3 && cell_f_usable(a);
+  const bool tiled = L.route.cell == CellPath::Tf32x3Fused;   // D as the fused backward's transposed tiles
   XgK k{};
   k.D = L.D; k.Wzr = L.Wzr; k.Wc = L.Wc; k.M0t = L.M0t; k.M1h = S.M1h;
   k.seg_ptr = a->plan.nseg > 0 ? a->plan.seg_ptr : nullptr;

@@ -167,6 +167,8 @@ def load() -> C.CDLL:
     lib.regt_debug_umma_selftest.argtypes = [C.c_int, C.c_int, vp, vp, vp, C.c_int, C.c_int, vp]
     lib.regt_debug_tc_split.restype = C.c_int
     lib.regt_debug_tc_split.argtypes = [C.c_int32, C.c_int32, C.c_int32, c_i32p]
+    lib.regt_debug_route.restype = C.c_int
+    lib.regt_debug_route.argtypes = [C.POINTER(Args), c_i32p]
     _lib = lib
     return lib
 

@@ -66,6 +66,61 @@ def test_tc_split_hook():
         _lib.check(lib.regt_debug_tc_split(0, 207, 12, (C.c_int32 * 7)()), "regt_debug_tc_split")
 
 
+_FP32, _TF32X3, _BF16 = 0, 1, 2
+_REGIONAL, _TGCN = 1, 2
+_CELL = {"fp32": 0, "unfused": 1, "fused": 2, "bf16": 3}
+_HEAD = {"rows": 0, "fused_ffma": 1, "tf32x3": 2, "bf16": 3}
+# (precision, H, O, B*N, T, mode, fused training step, REGT_UNFUSED) -> (cell, head, G tiled, out_hidden partials)
+_ROUTES = [
+    ((_BF16, 64, 16, 256, 12, _REGIONAL, True, None), ("bf16", "bf16", 1, 1)),
+    ((_BF16, 64, 17, 256, 12, _REGIONAL, True, None), ("bf16", "fused_ffma", 1, 1)),
+    ((_BF16, 64, 44, 256, 12, _REGIONAL, True, None), ("bf16", "fused_ffma", 1, 1)),
+    ((_BF16, 64, 45, 256, 12, _REGIONAL, True, None), ("bf16", "rows", 1, 0)),     # k_head_fused needs 229 KB of shared memory
+    ((_BF16, 64, 65, 256, 12, _REGIONAL, True, None), ("bf16", "rows", 1, 0)),
+    ((_BF16, 64, 16, 256, 12, _REGIONAL, False, None), ("bf16", "rows", 1, 0)),
+    ((_BF16, 64, 17, 256, 12, _REGIONAL, False, None), ("bf16", "rows", 1, 0)),
+    ((_BF16, 64, 44, 256, 12, _REGIONAL, False, None), ("bf16", "rows", 1, 0)),
+    ((_BF16, 64, 45, 256, 12, _REGIONAL, False, None), ("bf16", "rows", 1, 0)),
+    ((_BF16, 64, 65, 256, 12, _REGIONAL, False, None), ("bf16", "rows", 1, 0)),
+    ((_BF16, 64, 16, 256, 12, _REGIONAL, True, "1"), ("bf16", "bf16", 1, 1)),
+    ((_TF32X3, 128, 16, 256, 12, _REGIONAL, True, None), ("fused", "tf32x3", 1, 0)),
+    ((_TF32X3, 128, 17, 256, 12, _REGIONAL, True, None), ("fused", "rows", 1, 0)),
+    ((_TF32X3, 128, 16, 127, 12, _REGIONAL, True, None), ("fused", "rows", 1, 0)),
+    ((_TF32X3, 128, 16, 128, 12, _REGIONAL, True, None), ("fused", "tf32x3", 1, 0)),
+    ((_TF32X3, 64, 16, 127, 12, _REGIONAL, True, None), ("fused", "fused_ffma", 1, 0)),
+    ((_TF32X3, 256, 16, 256, 12, _REGIONAL, True, None), ("unfused", "tf32x3", 0, 0)),
+    ((_TF32X3, 128, 16, 256, 65, _REGIONAL, True, None), ("unfused", "tf32x3", 0, 0)),
+    ((_TF32X3, 128, 16, 256, 12, _TGCN, True, None), ("unfused", "tf32x3", 0, 0)),
+    ((_TF32X3, 128, 16, 256, 12, _REGIONAL, True, "1"), ("unfused", "tf32x3", 0, 0)),
+    ((_TF32X3, 64, 17, 256, 12, _REGIONAL, True, "1"), ("unfused", "fused_ffma", 0, 0)),
+    ((_FP32, 32, 12, 256, 12, _REGIONAL, True, None), ("fp32", "fused_ffma", 0, 0)),
+    ((_FP32, 64, 12, 256, 12, _REGIONAL, True, None), ("fp32", "fused_ffma", 0, 0)),
+    ((_FP32, 128, 12, 256, 12, _REGIONAL, True, None), ("fp32", "rows", 0, 0)),
+    ((_FP32, 64, 12, 256, 12, _REGIONAL, False, None), ("fp32", "rows", 0, 0)),
+]
+
+
+@pytest.mark.parametrize("case,want", _ROUTES)
+def test_route_table(case, want, monkeypatch):
+    """regt_debug_route: which cell and head kernels the entry points run, decided on the host without a GPU.  A fused
+    training step passes fuse_head with y, d_out and loss; outside one fuse_head is 0."""
+    from regt_b200 import _lib
+    lib = _lib.load()
+    prec, H, O, BN, T, mode, step, unfused = case
+    if unfused is None:
+        monkeypatch.delenv("REGT_UNFUSED", raising=False)
+    else:
+        monkeypatch.setenv("REGT_UNFUSED", unfused)
+    a = _lib.Args()
+    a.B, a.N, a.T, a.H, a.O, a.mode, a.precision, a.fuse_head = 1, BN, T, H, O, mode, prec, int(step)
+    a.plan.N = BN
+    a.y, a.loss, a.d_out, a.out = 0x1000, 0x2000, 0x3000, 0x4000   # never dereferenced
+    o = (C.c_int32 * 4)()
+    _lib.check(lib.regt_debug_route(C.byref(a), o), "regt_debug_route")
+    cell, head, g_tiled, partials = want
+    assert list(o) == [_CELL[cell], _HEAD[head], g_tiled, partials]
+
+
 def test_ctypes_structs_mirror_header():
     from regt_b200 import _lib
     src = open(HEADER).read()

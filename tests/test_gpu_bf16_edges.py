@@ -357,7 +357,7 @@ _HEADS = {16: (("k_head_tc",), ("k_head_fused", "k_hid_reduce", "k_head_fwd")),
 def test_head_width(O):
     """on a tp > 1 shape (two partial chunks of out_hidden): O <= 16 -> k_head_tc; 17..44 -> k_head_fused, which sums
     the cell's chunks itself while loading its tiles; from 45 on, k_head_fused's weights and tiles exceed the 227 KB of
-    shared memory a block may use at hidden 64 (O = 64 asked for 260 KB and failed to launch before head_fusable checked
+    shared memory a block may use at hidden 64 (O = 64 asked for 260 KB and failed to launch before head_fused_fits checked
     it): k_hid_reduce, then k_head_fwd / k_head_bwd."""
     key = f"width_{O}"
     w, B, ref = _oracle(key)

@@ -450,7 +450,7 @@ def test_head_output_width(O, H, path):
 
 @pytest.mark.parametrize("N", [127, 128])
 def test_head_row_threshold(N):
-    """head_f_usable takes the tensor-core head from B*N = 128 rows on; 127 rows run the FFMA head.  Both meet the oracle."""
+    """route_of (api.cu) takes the tensor-core head from B*N = 128 rows on; 127 rows run the FFMA head.  Both meet the oracle."""
     w, B, ref, lims = _head_case(4, 128, N=N, B=1)
     m = build_cuda(w, ref["state"], precision="tf32x3")
     x, y = w.inputs(B)
