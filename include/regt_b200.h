@@ -28,7 +28,7 @@ extern "C" {
 #endif
 
 #define REGT_VERSION 100 /* 0.1.0 */
-#define REGT_F 8         /* node features; fixed by the reference (run.py:116) */
+#define REGT_F 8         /* the kernels' feature width, and the largest regt_args.F (the reference uses 8, run.py:116) */
 
 /* precision of the H x H contractions */
 #define REGT_PREC_FP32 0  /* FFMA, fp32 everywhere (parity mode, all shapes)            */
@@ -161,7 +161,8 @@ typedef struct regt_args {
                           /*    the fused kernels save no activations (the workspace shrinks accordingly) and     */
                           /*    regt_head_backward / regt_cell_backward must not follow                           */
   regt_graph_plan plan;
-  const float* x;         /* [B,x_rows,F,T] f32, T innermost (load_dataset.py:456)        */
+  const float* x;         /* [B,x_rows,F,T] f32, T innermost (load_dataset.py:456); 16-byte aligned at F = REGT_F,  */
+                          /*    4-byte aligned suffices below (x is then read with scalar loads only)             */
   const float* y;         /* [B,N,O] or NULL: if set head_forward also writes loss, d_out  */
   const float* h_ext;     /* REGT_MODE_TGCN: [B,N,T,H] state or NULL (= zeros)            */
   regt_params p;          /* parameters                                                   */
@@ -175,6 +176,10 @@ typedef struct regt_args {
   void* workspace;        /* regt_workspace_bytes(args) bytes, preserved fwd -> bwd       */
   size_t workspace_bytes;
   regt_stream_t stream;
+  int32_t F;              /* features per node of x, 1..REGT_F; 0 means REGT_F.  x, conv_w, cheb_w0 / cheb_w1 and    */
+                          /*    their gradients have this width; the kernels work at REGT_F with the features and   */
+                          /*    weight columns F..REGT_F-1 written as zeros, so the result is that of the REGT_F-wide */
+                          /*    model on zero-padded x and weights                                                  */
 } regt_args;
 
 size_t regt_workspace_bytes(const regt_args* a);
@@ -225,7 +230,7 @@ typedef struct regt_xgrad_plan {
 size_t regt_xgrad_plan_workspace_bytes(const regt_graph_plan* p);
 int regt_xgrad_plan_build(const regt_graph_plan* p, int32_t* rowptr, int32_t* col, float* val, void* workspace,
                           size_t workspace_bytes, regt_stream_t stream);
-/* d_x [B,N,F,T] f32 (overwritten) = gradient wrt x of the loss whose gradients the preceding
+/* d_x [B,N,F,T] f32 (F = regt_args.F; overwritten) = gradient wrt x of the loss whose gradients the preceding
  * regt_cell_backward (same args, same workspace) consumed.  Reads the workspace, allocates nothing:
  * scratch is at least regt_cell_backward_x_scratch_bytes(a, xp) bytes (256-byte aligned).
  * Refused: precision bf16 (its kernels keep no D plane), region shards (x_rows != N: halo rows

@@ -116,13 +116,22 @@ Layout make_layout(const regt_args* a, void* base) {
   L.hpart = c.take<float>((size_t)148 * (HEAD_HID * H + O * HEAD_HID + HEAD_HID + O + 8));
   L.part = c.take<float>(pf);
   L.part_floats = pf;
-  L.m1cp = c.take<int32_t>(R + 2);
+  if (feat_in(a) < F && (L.route.cell == CellPath::Fp32 || L.route.cell == CellPath::Tf32x3Unfused))
+    L.xw = c.take<float>((size_t)a->B * (a->x_rows > 0 ? a->x_rows : a->N) * F * T);
+  L.m1cp = c.take<int32_t>(R + 2);   // last: tests locate it from the end of the workspace
   L.total = align_up(c.off, 256);
   return L;
 }
 
+static int check_features(const regt_args* a, const char* who) {
+  REGT_CHECK(a->F >= 0 && a->F <= REGT_F, "%s: F=%d node features; the kernels take 1..%d (0 means %d)", who, a->F, REGT_F,
+             REGT_F);
+  return 0;
+}
+
 static int validate(const regt_args* a, const char* who) {
   REGT_CHECK(a != nullptr, "%s: args is NULL", who);
+  if (check_features(a, who)) return -1;
   REGT_CHECK(a->B > 0 && a->N > 0 && a->T > 0 && a->O > 0, "%s: bad dims B=%d N=%d T=%d O=%d", who, a->B, a->N, a->T, a->O);
   REGT_CHECK(a->H >= 8 && a->H % 8 == 0 && a->H <= 1024, "%s: H=%d must be a multiple of 8 in [8,1024]", who, a->H);
   REGT_CHECK(a->mode >= 0 && a->mode <= 2, "%s: bad mode %d", who, a->mode);
@@ -139,7 +148,7 @@ static int validate(const regt_args* a, const char* who) {
 using namespace regt;
 
 extern "C" size_t regt_workspace_bytes(const regt_args* a) {
-  if (!a) return 0;
+  if (!a || check_features(a, "regt_workspace_bytes")) return 0;
   return make_layout(a, nullptr).total;
 }
 
@@ -179,6 +188,7 @@ extern "C" int regt_cell_backward(const regt_args* a) {
 
 static int validate_x(const regt_args* a, const regt_xgrad_plan* xp, const char* who) {
   REGT_CHECK(a != nullptr, "%s: args is NULL", who);
+  if (check_features(a, who)) return -1;
   REGT_CHECK(a->precision != REGT_PREC_BF16, "%s: precision bf16 keeps no gate-gradient plane; use fp32 or tf32x3", who);
   REGT_CHECK(a->x_rows == 0 || a->x_rows == a->N,
              "%s: region shards (x_rows=%d != N=%d) are not supported: their halo rows belong to other ranks", who, a->x_rows, a->N);

@@ -733,7 +733,7 @@ static CellK make_cellk(const regt_args* a, const Layout& L) {
   CellK k{};
   k.rows = a->B * a->N * a->T;
   k.N = a->N; k.xN = a->x_rows > 0 ? a->x_rows : a->N; k.T = a->T; k.H = a->H; k.nseg = a->plan.nseg; k.mode = a->mode;
-  k.x = a->x; k.S = L.S; k.U = L.U; k.h_ext = a->h_ext;
+  k.x = x_wide(a, L); k.S = L.S; k.U = L.U; k.h_ext = a->h_ext;
   k.seg_ptr = a->plan.seg_ptr; k.seg_reg = a->plan.seg_reg;
   k.M0t = L.M0t; k.M1t = L.M1t; k.c0 = L.c0; k.Wzr = L.Wzr; k.Wc = L.Wc; k.czr = L.czr; k.cc = L.cc; k.probs = L.probs;
   k.h = L.h; k.Z = L.Z; k.Rg = L.Rg; k.Hc = L.Hc; k.hR = L.hR; k.Hn = L.Hn;
@@ -826,7 +826,7 @@ static int launch_fwide_wgrads(const regt_args* a, const Layout& L, int splits, 
   float* part = L.part;
   const int ncol = (a->mode == REGT_MODE_TGCN) ? 3 * H : 4 * H;
   long long chunk = (rows + splits - 1) / splits;
-  k_wgrad_skinny<<<dim3(cdiv(ncol, 128), splits), 128, 0, st>>>(L.D, L.S, a->x, a->N, a->x_rows > 0 ? a->x_rows : a->N, H, T, rows, ncol, chunk, part);
+  k_wgrad_skinny<<<dim3(cdiv(ncol, 128), splits), 128, 0, st>>>(L.D, L.S, x_wide(a, L), a->N, a->x_rows > 0 ? a->x_rows : a->N, H, T, rows, ncol, chunk, part);
   REGT_LAUNCHED("k_wgrad_skinny", st);
   k_skinny_reduce<<<cdiv((long long)ncol * (F + 1), 256), 256, 0, st>>>(part, splits, H, ncol, L.dP, L.dcg, L.dM0, L.dc0);
   REGT_LAUNCHED("k_skinny_reduce", st);
@@ -839,10 +839,11 @@ int cell_forward_fp32(const regt_args* a, const Layout& L, cudaStream_t st) {
   const long long BN = (long long)a->B * a->N;
   const int xN = a->x_rows > 0 ? a->x_rows : a->N;
   if (launch_prep(a, L, st)) return -1;
+  if (launch_widen_x(a, L, st)) return -1;
   // F-wide SpMM: S = A_hat X on rows of F*T floats; U per (node, region) segment
-  if (launch_spmm_rows(a->plan.g_rowptr, a->plan.g_col, a->plan.g_val, a->x, L.S, a->B, a->N, xN, F * T, st)) return -1;
+  if (launch_spmm_rows(a->plan.g_rowptr, a->plan.g_col, a->plan.g_val, x_wide(a, L), L.S, a->B, a->N, xN, F * T, st)) return -1;
   if (a->mode != REGT_MODE_TGCN && a->plan.nseg > 0) {
-    if (launch_spmm_rows(a->plan.seg_eptr, a->plan.c_col, a->plan.c_val, a->x, L.U, a->B, a->plan.nseg, xN, F * T, st))
+    if (launch_spmm_rows(a->plan.seg_eptr, a->plan.c_col, a->plan.c_val, x_wide(a, L), L.U, a->B, a->plan.nseg, xN, F * T, st))
       return -1;
   }
   CellK k = make_cellk(a, L);

@@ -1303,7 +1303,7 @@ int cell_forward_f(const regt_args* a, const Layout& L, cudaStream_t st) {
   // features (graph + x) and collapsed weights (parameters) are independent: two streams
   cudaStream_t side = fork_side(st);
   cudaStream_t fs = side ? side : st;
-  if (launch_feat_tc(a->plan, a->x, a->B, a->x_rows > 0 ? a->x_rows : a->N, a->T, L.Xt, L.S, L.U, fs)) return -1;
+  if (launch_feat_tc(a->plan, a->x, feat_in(a), a->B, a->x_rows > 0 ? a->x_rows : a->N, a->T, L.Xt, L.S, L.U, fs)) return -1;
   if (!a->inference && launch_feat_f(a, L, fs)) return -1;   // feature plane of the weight-gradient contractions (cell and head backward)
   if (launch_prep(a, L, st)) return -1;
   if (a->H == 128 ? run_fwd<128>(a, L, st) : run_fwd<64>(a, L, st)) return -1;

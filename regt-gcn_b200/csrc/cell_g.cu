@@ -337,7 +337,7 @@ GK make_gk(const regt_args* a, const Layout& L) {
   GK k{};
   k.rows = (long long)a->B * a->N * a->T;
   k.N = a->N; k.xN = a->x_rows > 0 ? a->x_rows : a->N; k.T = a->T; k.H = a->H; k.nseg = a->plan.nseg; k.mode = a->mode;
-  k.x = a->x; k.S = L.S; k.U = L.U; k.h_ext = a->h_ext;
+  k.x = x_wide(a, L); k.S = L.S; k.U = L.U; k.h_ext = a->h_ext;
   k.seg_ptr = a->plan.seg_ptr; k.seg_reg = a->plan.seg_reg;
   k.M0t = L.M0t; k.M1t = L.M1t; k.c0 = L.c0; k.Wzr = L.Wzr; k.Wc = L.Wc; k.czr = L.czr; k.cc = L.cc; k.probs = L.probs;
   k.G = L.G;
@@ -371,9 +371,10 @@ int cell_forward_g(const regt_args* a, const Layout& L, cudaStream_t st) {
   const int xN = a->x_rows > 0 ? a->x_rows : a->N;
   REGT_CHECK(T <= 64, "precision tf32x3 supports up to 64 periods (got %d)", T);
   if (launch_prep(a, L, st)) return -1;
-  if (launch_spmm_rows(a->plan.g_rowptr, a->plan.g_col, a->plan.g_val, a->x, L.S, a->B, a->N, xN, F * T, st)) return -1;
+  if (launch_widen_x(a, L, st)) return -1;
+  if (launch_spmm_rows(a->plan.g_rowptr, a->plan.g_col, a->plan.g_val, x_wide(a, L), L.S, a->B, a->N, xN, F * T, st)) return -1;
   if (a->mode != REGT_MODE_TGCN && a->plan.nseg > 0) {
-    if (launch_spmm_rows(a->plan.seg_eptr, a->plan.c_col, a->plan.c_val, a->x, L.U, a->B, a->plan.nseg, xN, F * T, st))
+    if (launch_spmm_rows(a->plan.seg_eptr, a->plan.c_col, a->plan.c_val, x_wide(a, L), L.U, a->B, a->plan.nseg, xN, F * T, st))
       return -1;
   }
   GK k = make_gk(a, L);

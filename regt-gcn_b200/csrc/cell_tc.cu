@@ -648,7 +648,7 @@ int cell_forward_tc(const regt_args* a, const Layout& L, cudaStream_t st) {
   REGT_CHECK(a->T <= 64, "tensor-core path supports up to 64 periods");
   // features (graph + x) and collapsed weights (parameters) are independent: two streams
   cudaStream_t side = fork_side(st);
-  if (launch_feat_tc(a->plan, a->x, a->B, a->x_rows > 0 ? a->x_rows : a->N, a->T, L.Xt, L.S, L.U, side ? side : st)) return -1;
+  if (launch_feat_tc(a->plan, a->x, feat_in(a), a->B, a->x_rows > 0 ? a->x_rows : a->N, a->T, L.Xt, L.S, L.U, side ? side : st)) return -1;
   if (launch_prep(a, L, st)) return -1;
   return run_fwd_tc<64>(a, L, st, side != nullptr);
 }

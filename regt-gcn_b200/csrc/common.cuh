@@ -160,6 +160,8 @@ struct Layout {
   float* hid_part;           // [T (max t-chunks)][nqt][H/4][128][4]
   float* tc_wpart;           // [TC_MAX_CTAS][TC_WPART_FLOATS]
   float* tc_dpp;             // [T * nqt] attention-gradient partials
+  float* xw;                 // [B][x_rows][REGT_F][T]  x widened with zero features (fp32 / unfused tf32x3 paths when the
+                             // caller's F < REGT_F; written by every forward, read by its backward), else NULL
   size_t total;
 };
 constexpr int TC_MAX_CTAS = 160;
@@ -167,6 +169,11 @@ constexpr int TC_IMG_BYTES = 160 * 1024;
 constexpr int F_IMG_BYTES = 432 * 1024;   // fused 3xTF32 cell (cell_f.cu): 12 ring stages of 32 KB + F-wide weights + constants at H = 128
 
 Layout make_layout(const regt_args* a, void* base);
+
+// features per node of the caller's x and [H, F] parameters (regt_args.F, 0 = REGT_F)
+inline int feat_in(const regt_args* a) { return a->F > 0 ? a->F : REGT_F; }
+// x as the FFMA and unfused tf32x3 kernels read it: REGT_F features per row
+inline const float* x_wide(const regt_args* a, const Layout& L) { return L.xw ? L.xw : a->x; }
 
 constexpr int HEAD_HID = 128;  // hidden_dim of the decoder MLP (models/RegionalTemporalGCN.py:19)
 constexpr int WGRAD_SPLITS = 64;
@@ -195,7 +202,11 @@ int launch_chain(const regt_args* a, const Layout& L, cudaStream_t st);
 // spmm.cu: F-wide SpMM on rows of `width` floats; period-major Xt / St / Ut of the tensor-core cells
 int launch_spmm_rows(const int32_t* rowptr, const int32_t* col, const float* val, const float* x, float* y, int B,
                      int n_out, int n_in, int width, cudaStream_t st);
-int launch_feat_tc(const regt_graph_plan& p, const float* x, int B, int xN, int T, float* Xt, float* St, float* Ut, cudaStream_t st);
+// x [B][xN][Fin][T]; Xt / St / Ut rows are REGT_F wide (features Fin.. are zeros)
+int launch_feat_tc(const regt_graph_plan& p, const float* x, int Fin, int B, int xN, int T, float* Xt, float* St, float* Ut,
+                   cudaStream_t st);
+// L.xw = x with zero features Fin..REGT_F-1 (no launch when L.xw is NULL)
+int launch_widen_x(const regt_args* a, const Layout& L, cudaStream_t st);
 // cell.cu
 struct TNBatch;   // gemm_simt.cuh
 int launch_wgrad_tn(const TNBatch& batch, long long rows, int splits, cudaStream_t st);   // split-K C = A^T B per problem of the batch

@@ -10,7 +10,7 @@
 //      contiguous -- one 32-byte sector per thread and period.
 //   2. the transposed operator (regt_xgrad_plan) on the F*T-wide rows of G with the F-wide SpMM of the forward
 //      (launch_spmm_rows, n_in = 2N + nseg > n_out = N): sequential CSR order, no atomics -> bit-reproducible.
-//   3. k_xg_layout: [B][N][T][F] -> x's layout [B][N][F][T].
+//   3. k_xg_layout: [B][N][T][F] -> x's layout [B][N][Fin][T] (the caller's Fin <= F features; the padded ones are dropped).
 // Keeping the period inside the SpMM row (width F*T, as in the forward) keeps the SpMM kernels' lanes busy; rows of F = 8
 // floats would use 2 of a warp's 32 lanes.
 #include "common.cuh"
@@ -140,12 +140,12 @@ __global__ void __launch_bounds__(128) k_xg_contract(XgK k) {
   }
 }
 
-// dx[q][f][t] = Y[q][t][f]
-__global__ void k_xg_layout(const float* __restrict__ Y, int T, long long total, float* __restrict__ dx) {
+// dx[q][f][t] = Y[q][t][f] for the caller's Fin features (dx [B*N][Fin][T]; the padded ones are dropped)
+__global__ void k_xg_layout(const float* __restrict__ Y, int Fin, int T, long long total, float* __restrict__ dx) {
   const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
   if (i >= total) return;
-  const long long q = i / ((long long)F * T);
-  const int rem = (int)(i - q * F * T), f = rem / T, t = rem - f * T;
+  const long long q = i / ((long long)Fin * T);
+  const int rem = (int)(i - q * Fin * T), f = rem / T, t = rem - f * T;
   dx[i] = __ldg(Y + (q * T + t) * F + f);
 }
 
@@ -191,8 +191,8 @@ int cell_backward_x(const regt_args* a, const Layout& L, const regt_xgrad_plan* 
   }
   REGT_LAUNCHED("k_xg_contract", st);
   if (launch_spmm_rows(xp->rowptr, xp->col, xp->val, S.G, S.Y, a->B, a->N, xp->n_src, F * T, st)) return -1;
-  const long long total = k.BN * F * T;
-  k_xg_layout<<<cdiv(total, 256), 256, 0, st>>>(S.Y, T, total, d_x);
+  const long long total = k.BN * feat_in(a) * T;
+  k_xg_layout<<<cdiv(total, 256), 256, 0, st>>>(S.Y, feat_in(a), T, total, d_x);
   REGT_LAUNCHED("k_xg_layout", st);
   return 0;
 }

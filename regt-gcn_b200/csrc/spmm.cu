@@ -245,10 +245,12 @@ __global__ void __launch_bounds__(NT, MINB) k_spmm_blk(const int32_t* __restrict
 // feature row between them (48-byte runs per feature), the edge metadata of a row is a broadcast load, and each
 // thread writes its own 32-byte output row -- no shuffles, no staging, ~4x fewer instructions than the warp-per-row
 // gather (which spent its time on issue slots and three dependent memory rounds at 37 % occupancy).  Sums stay in
-// sequential CSR order (bit-identical to the stand-alone SpMM).
+// sequential CSR order (bit-identical to the stand-alone SpMM).  x has FIN <= F features per node (row stride FIN*T): only
+// those are gathered, the output rows stay F wide with zeros in FIN..F-1.
 #ifndef REGT_FEAT_MINB
 #define REGT_FEAT_MINB 4
 #endif
+template <int FIN>
 __global__ void __launch_bounds__(256, REGT_FEAT_MINB) k_feat_tc(const int32_t* __restrict__ g_rowptr, const int32_t* __restrict__ g_col,
                                                  const float* __restrict__ g_val, const int32_t* __restrict__ seg_eptr,
                                                  const int32_t* __restrict__ c_col, const float* __restrict__ c_val,
@@ -268,16 +270,16 @@ __global__ void __launch_bounds__(256, REGT_FEAT_MINB) k_feat_tc(const int32_t* 
   const int* rowptr = is_seg ? seg_eptr : g_rowptr;
   const int* col = is_seg ? c_col : g_col;
   const float* val = is_seg ? c_val : g_val;
-  const int W = F * T;
+  const int W = FIN * T;
   const float* xb = x + (size_t)b * xN * W + t;    // element (node, f) of this sample and period: xb[node * W + f * T]
   const int e0 = __ldg(rowptr + r), e1 = __ldg(rowptr + r + 1);
   float acc[F];
 #pragma unroll
-  for (int f = 0; f < F; ++f) acc[f] = 0.f;
+  for (int f = 0; f < F; ++f) acc[f] = 0.f;       // features FIN.. stay zero
   int e = e0;
   for (; e + 4 <= e1; e += 4) {   // four edges' loads in flight, accumulated in CSR order
     int c4[4];
-    float v4[4], xv[4][F];
+    float v4[4], xv[4][FIN];
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
       c4[u] = __ldg(col + e + u);
@@ -287,18 +289,18 @@ __global__ void __launch_bounds__(256, REGT_FEAT_MINB) k_feat_tc(const int32_t* 
     for (int u = 0; u < 4; ++u) {
       const float* xr = xb + (size_t)c4[u] * W;
 #pragma unroll
-      for (int f = 0; f < F; ++f) xv[u][f] = __ldg(xr + f * T);
+      for (int f = 0; f < FIN; ++f) xv[u][f] = __ldg(xr + f * T);
     }
 #pragma unroll
     for (int u = 0; u < 4; ++u)
 #pragma unroll
-      for (int f = 0; f < F; ++f) acc[f] = fmaf(v4[u], xv[u][f], acc[f]);
+      for (int f = 0; f < FIN; ++f) acc[f] = fmaf(v4[u], xv[u][f], acc[f]);
   }
   for (; e < e1; ++e) {
     const float v = __ldg(val + e);
     const float* xr = xb + (size_t)__ldg(col + e) * W;
 #pragma unroll
-    for (int f = 0; f < F; ++f) acc[f] = fmaf(v, __ldg(xr + f * T), acc[f]);
+    for (int f = 0; f < FIN; ++f) acc[f] = fmaf(v, __ldg(xr + f * T), acc[f]);
   }
   float4* d = reinterpret_cast<float4*>((is_seg ? Ut : St) + ((size_t)t * (is_seg ? BS : BN) + w) * F);
   d[0] = make_float4(acc[0], acc[1], acc[2], acc[3]);
@@ -307,18 +309,50 @@ __global__ void __launch_bounds__(256, REGT_FEAT_MINB) k_feat_tc(const int32_t* 
     const float* xr = xb + (size_t)r * W;
     float sx[F];
 #pragma unroll
-    for (int f = 0; f < F; ++f) sx[f] = __ldg(xr + f * T);
+    for (int f = 0; f < F; ++f) sx[f] = f < FIN ? __ldg(xr + f * T) : 0.f;
     float4* dx = reinterpret_cast<float4*>(Xt + ((size_t)t * BN + w) * F);
     dx[0] = make_float4(sx[0], sx[1], sx[2], sx[3]);
     dx[1] = make_float4(sx[4], sx[5], sx[6], sx[7]);
   }
 }
 
-int launch_feat_tc(const regt_graph_plan& p, const float* x, int B, int xN, int T, float* Xt, float* St, float* Ut, cudaStream_t st) {
+int launch_feat_tc(const regt_graph_plan& p, const float* x, int Fin, int B, int xN, int T, float* Xt, float* St, float* Ut,
+                   cudaStream_t st) {
   const long long threads = ((long long)B * p.N + (long long)B * p.nseg) * T;
-  k_feat_tc<<<cdiv(threads, 256), 256, 0, st>>>(p.g_rowptr, p.g_col, p.g_val, p.seg_eptr, p.c_col, p.c_val, x, B, p.N, xN, p.nseg, T, Xt,
-                                                St, Ut);
+  auto kern = k_feat_tc<8>;
+  switch (Fin) {
+    case 1: kern = k_feat_tc<1>; break;
+    case 2: kern = k_feat_tc<2>; break;
+    case 3: kern = k_feat_tc<3>; break;
+    case 4: kern = k_feat_tc<4>; break;
+    case 5: kern = k_feat_tc<5>; break;
+    case 6: kern = k_feat_tc<6>; break;
+    case 7: kern = k_feat_tc<7>; break;
+    case 8: break;
+    default: REGT_CHECK(false, "feat_tc: %d node features, the kernels take 1..%d", Fin, REGT_F);
+  }
+  kern<<<cdiv(threads, 256), 256, 0, st>>>(p.g_rowptr, p.g_col, p.g_val, p.seg_eptr, p.c_col, p.c_val, x, B, p.N, xN, p.nseg, T, Xt, St,
+                                           Ut);
   REGT_LAUNCHED("k_feat_tc", st);
+  return 0;
+}
+
+// xw[q][f][t] = f < Fin ? x[q][f][t] : 0 for every row q of x (halo rows included): the FFMA and unfused tf32x3 kernels
+// read x through several launches at REGT_F features per row.  Scalar loads: x needs 4-byte alignment only.
+__global__ void k_widen_x(const float* __restrict__ x, int Fin, int T, long long total, float* __restrict__ xw) {
+  constexpr int F = REGT_F;
+  const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (i >= total) return;
+  const long long q = i / ((long long)F * T);
+  const int rem = (int)(i - q * F * T), f = rem / T, t = rem - f * T;
+  xw[i] = f < Fin ? __ldg(x + (q * Fin + f) * T + t) : 0.f;
+}
+
+int launch_widen_x(const regt_args* a, const Layout& L, cudaStream_t st) {
+  if (!L.xw) return 0;
+  const long long total = (long long)a->B * (a->x_rows > 0 ? a->x_rows : a->N) * REGT_F * a->T;
+  k_widen_x<<<cdiv(total, 256), 256, 0, st>>>(a->x, feat_in(a), a->T, total, L.xw);
+  REGT_LAUNCHED("k_widen_x", st);
   return 0;
 }
 

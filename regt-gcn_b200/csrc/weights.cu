@@ -9,11 +9,18 @@
 //   M0  = (sum_r L_r) W0,  M1[r] = L_r W1,  c0 = (sum_r L_r) b + b_lin
 // These are tiny (H*H*F flops); they run as plain one-thread-per-output kernels with fp64
 // accumulation so the collapse adds no rounding of its own.
+//
+// The parameters conv_w / cheb_w0 / cheb_w1 are [H, Fin] with the caller's Fin <= F (regt_args.F); everything collapsed
+// is F wide.  Columns Fin..F-1 of the collapsed weights are written as zeros, and the chain rule reads the missing
+// parameter columns as zeros and writes only the Fin real ones: the F-wide arithmetic of a zero-padded model.
 #include "common.cuh"
 
 namespace regt {
 
 constexpr int F = REGT_F;
+
+// element (m, f) of an [H, Fin] parameter, 0 for the padded columns f >= Fin
+__device__ __forceinline__ float wcol(const float* w, int m, int f, int Fin) { return f < Fin ? w[(size_t)m * Fin + f] : 0.f; }
 
 __global__ void k_lsum(const float* __restrict__ comb_w, int H, int R, float* __restrict__ Lsum) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -29,7 +36,7 @@ __global__ void k_lsum(const float* __restrict__ comb_w, int H, int R, float* __
 // slices are combined with a shuffle tree (the step waits on this kernel, so its latency -- a chain
 // of H dependent loads from cold HBM per output in a one-thread-per-output form -- matters).
 constexpr int PG = 8;
-__global__ void __launch_bounds__(256) k_prep(regt_params p, int H, int R, int T, int mode, const float* __restrict__ Lsum,
+__global__ void __launch_bounds__(256) k_prep(regt_params p, int H, int Fin, int R, int T, int mode, const float* __restrict__ Lsum,
                                               float* __restrict__ Wzr, float* __restrict__ Wc, float* __restrict__ czr,
                                               float* __restrict__ cc, float* __restrict__ M0t, float* __restrict__ M1t,
                                               float* __restrict__ c0, float* __restrict__ probs) {
@@ -45,11 +52,11 @@ __global__ void __launch_bounds__(256) k_prep(regt_params p, int H, int R, int T
     int g = (int)(i / ((F + H) * H));
     int rem = (int)(i % ((F + H) * H));
     int k = rem / H, j = rem % H;  // j fastest: coalesced writes
-    if (k < F) {
+    if (k < Fin) {
       const float* A = p.lin_w[g] + (size_t)j * 2 * H;
       const float* W = p.conv_w[g];
-      for (int m = m0; m < m1; ++m) s += (double)__ldg(A + m) * (double)__ldg(W + m * F + k);
-    } else if (sub == 0) {
+      for (int m = m0; m < m1; ++m) s += (double)__ldg(A + m) * (double)__ldg(W + m * Fin + k);
+    } else if (k >= F && sub == 0) {   // k in [Fin, F): zero column
       s = p.lin_w[g][(size_t)j * 2 * H + H + (k - F)];
     }
     dst = (g < 2) ? Wzr + (size_t)k * 2 * H + g * H + j : Wc + (size_t)k * H + j;
@@ -70,21 +77,23 @@ __global__ void __launch_bounds__(256) k_prep(regt_params p, int H, int R, int T
     }
   } else if ((i -= nC) < nM0) {
     int f = (int)(i / H), j = (int)(i % H);
-    if (mode == REGT_MODE_REGIONAL) {
-      for (int m = m0; m < m1; ++m) s += (double)__ldg(Lsum + (size_t)j * H + m) * (double)__ldg(p.cheb_w0 + m * F + f);
+    if (f >= Fin) {   // padded column: 0
+    } else if (mode == REGT_MODE_REGIONAL) {
+      for (int m = m0; m < m1; ++m) s += (double)__ldg(Lsum + (size_t)j * H + m) * (double)__ldg(p.cheb_w0 + m * Fin + f);
     } else if (sub == 0) {
-      s = p.cheb_w0[j * F + f];
+      s = p.cheb_w0[j * Fin + f];
     }
     dst = M0t + i;
   } else if ((i -= nM0) < nM1) {
     int r = (int)(i / (F * H));
     int rem = (int)(i % (F * H));
     int f = rem / H, j = rem % H;
-    if (mode == REGT_MODE_REGIONAL) {
+    if (f >= Fin) {   // padded column: 0
+    } else if (mode == REGT_MODE_REGIONAL) {
       const float* L = p.comb_w + (size_t)j * R * H + (size_t)r * H;
-      for (int m = m0; m < m1; ++m) s += (double)__ldg(L + m) * (double)__ldg(p.cheb_w1 + m * F + f);
+      for (int m = m0; m < m1; ++m) s += (double)__ldg(L + m) * (double)__ldg(p.cheb_w1 + m * Fin + f);
     } else if (sub == 0) {
-      s = p.cheb_w1[j * F + f];
+      s = p.cheb_w1[j * Fin + f];
     }
     dst = M1t + i;
   } else if ((i -= nM1) < nc0) {
@@ -117,7 +126,7 @@ int launch_prep(const regt_args* a, const Layout& L, cudaStream_t st) {
     REGT_LAUNCHED("k_lsum", st);
   }
   long long n = (long long)3 * (F + H) * H + 3 * H + (long long)F * H + (long long)R * F * H + H + 1;
-  k_prep<<<cdiv(n * PG, 256), 256, 0, st>>>(a->p, H, R, a->T, a->mode, L.Lsum, L.Wzr, L.Wc, L.czr, L.cc, L.M0t, L.M1t, L.c0,
+  k_prep<<<cdiv(n * PG, 256), 256, 0, st>>>(a->p, H, feat_in(a), R, a->T, a->mode, L.Lsum, L.Wzr, L.Wc, L.czr, L.cc, L.M0t, L.M1t, L.c0,
                                       L.probs);
   REGT_LAUNCHED("k_prep", st);
   return 0;
@@ -131,13 +140,13 @@ __device__ __forceinline__ void put(float* dst, size_t i, double v, int acc) {
   dst[i] = acc ? dst[i] + (float)v : (float)v;
 }
 
-__global__ void k_chain(regt_params p, regt_params g, int H, int R, int T, int mode, int acc,
+__global__ void k_chain(regt_params p, regt_params g, int H, int Fin, int R, int T, int mode, int acc,
                         const float* __restrict__ Lsum, const float* __restrict__ probs,
                         const float* __restrict__ dB, const float* __restrict__ dP, const float* __restrict__ dcg,
                         const float* __restrict__ dM0, const float* __restrict__ dM1, const float* __restrict__ dc0,
                         const float* __restrict__ dprobs) {
   long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-  const long long nLW = (long long)3 * H * 2 * H, nLB = 3 * H, nCW = (long long)3 * H * F, nCB = 3 * H;
+  const long long nLW = (long long)3 * H * 2 * H, nLB = 3 * H, nCW = (long long)3 * H * Fin, nCB = 3 * H;
   if (i < nLW) {  // linear_g.weight [H,2H] = [dA_g | dB_g]
     int gI = (int)(i / ((long long)H * 2 * H));
     int rem = (int)(i % ((long long)H * 2 * H));
@@ -145,7 +154,7 @@ __global__ void k_chain(regt_params p, regt_params g, int H, int R, int T, int m
     double v;
     if (c < H) {
       v = (double)dcg[gI * H + j] * (double)p.conv_b[gI][c];
-      for (int f = 0; f < F; ++f) v += (double)dP[((size_t)gI * H + j) * F + f] * (double)p.conv_w[gI][c * F + f];
+      for (int f = 0; f < F; ++f) v += (double)dP[((size_t)gI * H + j) * F + f] * (double)wcol(p.conv_w[gI], c, f, Fin);
     } else {
       v = dB[((size_t)gI * H + j) * H + (c - H)];
     }
@@ -159,13 +168,13 @@ __global__ void k_chain(regt_params p, regt_params g, int H, int R, int T, int m
     return;
   }
   i -= nLB;
-  if (i < nCW) {  // conv_g.lin.weight [H,F] = A_g^T dP_g
-    int gI = (int)(i / (H * F));
-    int rem = (int)(i % (H * F));
-    int m = rem / F, f = rem % F;
+  if (i < nCW) {  // conv_g.lin.weight [H,Fin] = A_g^T dP_g (the real columns)
+    int gI = (int)(i / (H * Fin));
+    int rem = (int)(i % (H * Fin));
+    int m = rem / Fin, f = rem % Fin;
     double v = 0.0;
     for (int j = 0; j < H; ++j) v += (double)p.lin_w[gI][(size_t)j * 2 * H + m] * (double)dP[((size_t)gI * H + j) * F + f];
-    put(g.conv_w[gI], (size_t)m * F + f, v, acc);
+    put(g.conv_w[gI], (size_t)m * Fin + f, v, acc);
     return;
   }
   i -= nCW;
@@ -187,11 +196,11 @@ __global__ void k_chain(regt_params p, regt_params g, int H, int R, int T, int m
   }
   i -= T;
   if (mode == REGT_MODE_TGCN) return;
-  const long long nW0 = (long long)H * F;
-  if (i < 2 * nW0) {  // cheb lins.0 / lins.1 weights
+  const long long nW0 = (long long)H * Fin;
+  if (i < 2 * nW0) {  // cheb lins.0 / lins.1 weights [H,Fin]
     int which = (int)(i / nW0);
     int rem = (int)(i % nW0);
-    int m = rem / F, f = rem % F;
+    int m = rem / Fin, f = rem % Fin;
     double v = 0.0;
     if (mode == REGT_MODE_REGIONAL) {
       if (which == 0) {
@@ -202,7 +211,7 @@ __global__ void k_chain(regt_params p, regt_params g, int H, int R, int T, int m
     } else {
       v = which == 0 ? dM0[(size_t)m * F + f] : dM1[(size_t)m * F + f];
     }
-    put(which == 0 ? g.cheb_w0 : g.cheb_w1, (size_t)m * F + f, v, acc);
+    put(which == 0 ? g.cheb_w0 : g.cheb_w1, (size_t)m * Fin + f, v, acc);
     return;
   }
   i -= 2 * nW0;
@@ -231,18 +240,18 @@ __global__ void k_chain(regt_params p, regt_params g, int H, int R, int T, int m
     int r = rem / H, m = rem % H;
     double v = (double)dc0[j] * (double)p.cheb_b[m];
     for (int f = 0; f < F; ++f) {
-      v += (double)dM0[(size_t)j * F + f] * (double)p.cheb_w0[m * F + f];
-      v += (double)dM1[((size_t)r * H + j) * F + f] * (double)p.cheb_w1[m * F + f];
+      v += (double)dM0[(size_t)j * F + f] * (double)wcol(p.cheb_w0, m, f, Fin);
+      v += (double)dM1[((size_t)r * H + j) * F + f] * (double)wcol(p.cheb_w1, m, f, Fin);
     }
     put(g.comb_w, (size_t)i, v, acc);
   }
 }
 
 // cheb lins.1 weight of the regional model: d W1[m][f] = sum_r sum_j L_r[j][m] * dM1[r][j][f]  (R*H terms per output)
-__global__ void __launch_bounds__(256) k_chain_w1(const float* __restrict__ comb_w, const float* __restrict__ dM1, int H, int R,
-                                                  int acc, float* __restrict__ g_w1) {
+__global__ void __launch_bounds__(256) k_chain_w1(const float* __restrict__ comb_w, const float* __restrict__ dM1, int H, int Fin,
+                                                  int R, int acc, float* __restrict__ g_w1) {
   __shared__ double red[256];
-  const int m = blockIdx.x / F, f = blockIdx.x % F;
+  const int m = blockIdx.x / Fin, f = blockIdx.x % Fin;
   double v = 0.0;
   for (int i = threadIdx.x; i < R * H; i += 256) {   // i = r*H + j ; fixed strided order, then a fixed tree
     const int r = i / H, j = i - r * H;
@@ -254,18 +263,18 @@ __global__ void __launch_bounds__(256) k_chain_w1(const float* __restrict__ comb
     if (threadIdx.x < d) red[threadIdx.x] += red[threadIdx.x + d];
     __syncthreads();
   }
-  if (threadIdx.x == 0 && g_w1) g_w1[(size_t)m * F + f] = acc ? g_w1[(size_t)m * F + f] + (float)red[0] : (float)red[0];
+  if (threadIdx.x == 0 && g_w1) g_w1[(size_t)m * Fin + f] = acc ? g_w1[(size_t)m * Fin + f] + (float)red[0] : (float)red[0];
 }
 
 int launch_chain(const regt_args* a, const Layout& L, cudaStream_t st) {
-  const int H = a->H, R = a->plan.R;
-  long long n = (long long)3 * H * 2 * H + 3 * H + (long long)3 * H * F + 3 * H + a->T + 2ll * H * F + H + H +
+  const int H = a->H, R = a->plan.R, Fin = feat_in(a);
+  long long n = (long long)3 * H * 2 * H + 3 * H + (long long)3 * H * Fin + 3 * H + a->T + 2ll * H * Fin + H + H +
                 (long long)H * R * H;
-  k_chain<<<cdiv(n, 256), 256, 0, st>>>(a->p, a->g, H, R, a->T, a->mode, a->accumulate, L.Lsum, L.probs, L.dB, L.dP,
+  k_chain<<<cdiv(n, 256), 256, 0, st>>>(a->p, a->g, H, Fin, R, a->T, a->mode, a->accumulate, L.Lsum, L.probs, L.dB, L.dP,
                                        L.dcg, L.dM0, L.dM1, L.dc0, L.dprobs);
   REGT_LAUNCHED("k_chain", st);
   if (a->mode == REGT_MODE_REGIONAL) {
-    k_chain_w1<<<H * F, 256, 0, st>>>(a->p.comb_w, L.dM1, H, R, a->accumulate, a->g.cheb_w1);
+    k_chain_w1<<<H * Fin, 256, 0, st>>>(a->p.comb_w, L.dM1, H, Fin, R, a->accumulate, a->g.cheb_w1);
     REGT_LAUNCHED("k_chain_w1", st);
   }
   return 0;

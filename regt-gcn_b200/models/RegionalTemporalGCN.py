@@ -11,7 +11,8 @@ import torch
 import torch.nn as nn
 
 from regt_b200 import _lib
-from regt_b200.module_base import ChebConvParams, RegTModelBase, split_regional_args, tgcn_param_dict
+from regt_b200.module_base import (ChebConvParams, RegTModelBase, check_node_features, split_regional_args,
+                                   tgcn_param_dict)
 from regt_b200.plan import get_plan
 from models.utils import TGCN
 
@@ -43,6 +44,7 @@ class RegionalTemporalGCN(RegTModelBase):
     def __init__(self, node_features, num_nodes, periods, output_dim, hidden: int = 256, n_regions: int = 5,
                  precision: str = "auto"):
         super().__init__()
+        check_node_features(node_features)
         self.tgnn = RegionalA3TGCN(in_channels=node_features, out_channels=hidden, num_nodes=num_nodes,
                                    periods=periods, n_regions=n_regions)
         self.output_dim = output_dim

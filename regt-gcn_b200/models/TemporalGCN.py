@@ -8,7 +8,7 @@ import torch
 import torch.nn as nn
 
 from regt_b200 import _lib
-from regt_b200.module_base import ChebConvParams, RegTModelBase, tgcn_param_dict
+from regt_b200.module_base import ChebConvParams, RegTModelBase, check_node_features, tgcn_param_dict
 from regt_b200.plan import get_plan
 from models.utils import TGCN
 
@@ -31,6 +31,7 @@ class TemporalGCN(RegTModelBase):
 
     def __init__(self, node_features, periods, output_dim, hidden: int = 256, precision: str = "auto"):
         super().__init__()
+        check_node_features(node_features)
         self.tgnn = A3TGCN(in_channels=node_features, out_channels=hidden, periods=periods)
         self.output_dim = output_dim
         self._hidden, self.precision = hidden, precision

@@ -10,7 +10,7 @@ import torch
 import torch.nn as nn
 
 from regt_b200 import _lib, engine
-from regt_b200.module_base import GCNConvParams, tgcn_param_dict
+from regt_b200.module_base import GCNConvParams, check_node_features, tgcn_param_dict
 from regt_b200.plan import get_plan
 
 
@@ -24,6 +24,7 @@ class TGCN(nn.Module):
             raise NotImplementedError("Current baseblock %s is not supported." % (baseblock))
         if improved or not add_self_loops:
             raise NotImplementedError("only improved=False, add_self_loops=True (the reference's use) is built")
+        check_node_features(in_channels)
         self.in_channels, self.out_channels = in_channels, out_channels
         self.improved, self.cached, self.add_self_loops, self.baseblock = improved, cached, add_self_loops, baseblock
         self.precision = precision

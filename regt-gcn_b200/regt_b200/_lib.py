@@ -45,7 +45,7 @@ class Args(C.Structure):
                 ("x", vp), ("y", vp), ("h_ext", vp),
                 ("p", Params), ("g", Params),
                 ("out_hidden", vp), ("out", vp), ("loss", vp), ("d_out", vp), ("d_hidden", vp), ("d_h_ext", vp),
-                ("workspace", vp), ("workspace_bytes", C.c_size_t), ("stream", vp)]
+                ("workspace", vp), ("workspace_bytes", C.c_size_t), ("stream", vp), ("F", C.c_int32)]
 
 
 MODE_A3TGCN, MODE_REGIONAL, MODE_TGCN = 0, 1, 2

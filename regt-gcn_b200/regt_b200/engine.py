@@ -12,7 +12,7 @@ import torch
 from . import _lib
 from .plan import GraphPlanTensors
 
-F_IN = 8
+F_IN = 8         # the kernels' feature width (REGT_F): node_features may be 1..F_IN
 HEAD_HID = 128
 
 # canonical order of the parameter tensors handed to the autograd Function
@@ -34,16 +34,24 @@ def keys_for(mode: int, head: bool):
     return k
 
 
-def _check(t: torch.Tensor, name: str, device) -> torch.Tensor:
+def _check(t: torch.Tensor, name: str, device, align: int = 16) -> torch.Tensor:
     if not t.is_cuda:
         raise RuntimeError(f"regt_b200: {name} must be a CUDA tensor (no CPU fallback exists); got {t.device}")
     if t.device != device:
         raise RuntimeError(f"regt_b200: {name} is on {t.device}, expected {device}")
     if t.dtype != torch.float32:
         raise TypeError(f"regt_b200: {name} must be float32, got {t.dtype}")
-    if not t.is_contiguous() or t.data_ptr() % 16:
-        raise RuntimeError(f"regt_b200: {name} must be contiguous and 16-byte aligned")
+    if not t.is_contiguous() or t.data_ptr() % align:
+        raise RuntimeError(f"regt_b200: {name} must be contiguous and {align}-byte aligned")
     return t
+
+
+def check_features(F: int, param_width: int) -> None:
+    """x's feature count F against the kernels' range and the [H, F] parameters' width."""
+    if not 1 <= F <= F_IN:
+        raise ValueError(f"regt_b200: node_features must be 1..{F_IN} (the kernels' feature width is {F_IN}), got {F}")
+    if F != param_width:
+        raise ValueError(f"regt_b200: x has {F} features per node, the model's parameters were built for {param_width}")
 
 
 def _fill_params(dst: _lib.Params, tensors: Dict[str, Optional[torch.Tensor]]) -> None:
@@ -83,11 +91,11 @@ def build_state(mode: int, precision: int, plan: GraphPlanTensors, x: torch.Tens
     node count of the full graph, so the per-rank losses and gradients add up to the unsharded ones."""
     lib = _lib.load()
     dev = x.device
-    _check(x, "x", dev)
     B, x_rows, Fx, T = x.shape
+    # F < F_IN: the kernels read x with scalar loads, and a micro-batch slice of x need not start on 16 bytes
+    _check(x, "x", dev, 16 if Fx == F_IN else 4)
     N = plan.N
-    if Fx != F_IN:
-        raise ValueError(f"regt_b200: node_features must be {F_IN} (reference run.py:116), got {Fx}")
+    check_features(Fx, params["conv_w0"].shape[1])
     if x_rows < N or (x_rows != N and x_rows != N + getattr(plan, "n_halo", 0)):
         raise ValueError(f"regt_b200: x has {x_rows} nodes, graph plan has {N} (+{getattr(plan, 'n_halo', 0)} halo)")
     st = StepState()
@@ -97,6 +105,7 @@ def build_state(mode: int, precision: int, plan: GraphPlanTensors, x: torch.Tens
     a.fuse_head = 1 if (fuse_head and head and y is not None) else 0
     a.inference = 1 if inference else 0
     a.x_rows = x_rows
+    a.F = Fx
     a.loss_nodes = int(loss_nodes) if loss_nodes else 0
     a.plan = plan.c_struct()
     a.x = x.data_ptr()
@@ -131,24 +140,25 @@ def build_state(mode: int, precision: int, plan: GraphPlanTensors, x: torch.Tens
     return st
 
 
-def workspace_bytes(mode: int, precision: int, plan: GraphPlanTensors, B: int, x_rows: int, T: int, H: int, O: int) -> int:
+def workspace_bytes(mode: int, precision: int, plan: GraphPlanTensors, B: int, x_rows: int, T: int, H: int, O: int,
+                    F: int = F_IN) -> int:
     """bytes ``build_state`` will ask for at batch B (saved planes scale with B*N*T*H): used to size micro-batches."""
     a = _lib.Args()
     a.B, a.N, a.T, a.H, a.O = B, plan.N, T, H, O
-    a.mode, a.precision, a.x_rows = mode, precision, x_rows
+    a.mode, a.precision, a.x_rows, a.F = mode, precision, x_rows, F
     a.fuse_head = 1
     a.plan = plan.c_struct()
     return int(_lib.load().regt_workspace_bytes(C.byref(a)))
 
 
 def auto_micro_batch(mode: int, precision: int, plan: GraphPlanTensors, B: int, x_rows: int, T: int, H: int, O: int,
-                     have: int = 0) -> int:
+                     have: int = 0, F: int = F_IN) -> int:
     """largest divisor of B whose workspace fits 70 % of the free device memory (plus what a cached workspace of
     ``have`` bytes already holds); SURVEY 8d: cfg 4/5 save 63 / 157 GB of planes at full B, so they micro-batch inside the step."""
     free, _ = torch.cuda.mem_get_info()
     budget = int(0.7 * (free + have))
     for mb in sorted({d for d in range(1, B + 1) if B % d == 0}, reverse=True):
-        if workspace_bytes(mode, precision, plan, mb, x_rows, T, H, O) <= budget:
+        if workspace_bytes(mode, precision, plan, mb, x_rows, T, H, O, F) <= budget:
             return mb
     return 1
 

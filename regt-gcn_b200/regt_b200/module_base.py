@@ -12,6 +12,13 @@ from . import _lib, engine
 from .plan import get_plan
 
 
+def check_node_features(F: int) -> None:
+    """constructor check: the kernels work at ``engine.F_IN`` features per node and take any narrower input."""
+    if not 1 <= F <= engine.F_IN:
+        raise ValueError(f"node_features must be an int in 1..{engine.F_IN} (the kernels' feature width is "
+                         f"{engine.F_IN}), got {F!r}")
+
+
 def _glorot(rows: int, cols: int) -> nn.Parameter:
     a = math.sqrt(6.0 / (rows + cols))
     return nn.Parameter(torch.empty(rows, cols).uniform_(-a, a))
@@ -138,7 +145,7 @@ class RegTModelBase(nn.Module):
             if getattr(self, "_mb_key", None) != key:
                 ws = getattr(self, "_ws", None)
                 self._mb = engine.auto_micro_batch(self._mode, prec, plan, B, xb.shape[1], xb.shape[3], self._hidden,
-                                                   self.output_dim, 0 if ws is None else ws.numel())
+                                                   self.output_dim, 0 if ws is None else ws.numel(), xb.shape[2])
                 self._mb_key = key
             mb = self._mb
         loss = None

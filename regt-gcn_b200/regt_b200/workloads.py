@@ -17,7 +17,7 @@ from typing import List, Optional
 import numpy as np
 import torch
 
-F_IN = 8  # node features, fixed by the reference (run.py:116 ``node_features=8``)
+F_IN = 8  # node features of the reference's data (run.py:116 ``node_features=8``), the default of every workload
 
 
 @dataclass
@@ -35,6 +35,7 @@ class Workload:
     edge_attr: Optional[torch.Tensor]            # f32 [E] (TemporalGCN only)
     reg_edge_index: List[torch.Tensor] = field(default_factory=list)
     reg_edge_attr: List[torch.Tensor] = field(default_factory=list)
+    F: int = F_IN                                # node features of x (1..8)
 
     @property
     def E(self) -> int:
@@ -48,7 +49,7 @@ class Workload:
         """x [B,N,F,T] ~ U[0,1), y [B,N,O] ~ U[0,1) (MinMax-scaled features, load_dataset.py:430)."""
         B = self.B if B is None else B
         g = torch.Generator().manual_seed(self.seed * 1000 + seed_offset)
-        x = torch.rand(B, self.N, F_IN, self.T, generator=g, dtype=torch.float32)
+        x = torch.rand(B, self.N, self.F, self.T, generator=g, dtype=torch.float32)
         y = torch.rand(B, self.N, self.O, generator=g, dtype=torch.float32)
         return x, y
 
@@ -59,7 +60,7 @@ class Workload:
         return (self.edge_index, *self.reg_edge_index, *self.reg_edge_attr)
 
     def describe(self) -> dict:
-        return dict(workload=self.name, model=self.model, B=self.B, N=self.N, T=self.T, F=F_IN,
+        return dict(workload=self.name, model=self.model, B=self.B, N=self.N, T=self.T, F=self.F,
                     H=self.H, O=self.O, R=self.R, E=self.E, E_reg=self.E_reg, seed=self.seed)
 
 
@@ -183,7 +184,7 @@ def cfg5_shaped(N: int = 2560, T: int = 2, B: int = 2, H: int = 128, R: int = 25
 
 
 def tiny_workload(model: str, N: int, T: int, H: int, O: int, R: int, B: int, seed: int,
-                  k_intra: int = 3, n_cross: int = 4, adversarial: bool = False) -> Workload:
+                  k_intra: int = 3, n_cross: int = 4, adversarial: bool = False, F: int = F_IN) -> Workload:
     """small seeded cases for parity tests.  ``adversarial`` adds what SURVEY section 4 asks for:
     existing self-loops (with weights), duplicate edges, isolated nodes, zero out-degree
     nodes, asymmetric weights, and a node that appears in two regional lists."""
@@ -205,7 +206,7 @@ def tiny_workload(model: str, N: int, T: int, H: int, O: int, R: int, B: int, se
             perm = rng.permutation(ei.shape[1])
             ei, ea = ei[:, perm], ea[perm]
         return Workload(f"tiny_tgcn_N{N}_H{H}_s{seed}", model, B, N, T, H, O, 0, seed,
-                        torch.from_numpy(ei), torch.from_numpy(ea))
+                        torch.from_numpy(ei), torch.from_numpy(ea), F=F)
     full, rei, rea = _regional_graph(N, R, k_intra, n_cross, seed)
     if adversarial and N >= 8 and R >= 2:
         # a self-loop inside list 0, a duplicate edge in list 1, and an edge of list 1 that
@@ -222,14 +223,14 @@ def tiny_workload(model: str, N: int, T: int, H: int, O: int, R: int, B: int, se
         last = len(rei) - 1
         keep = (rei[last][0] != N - 1) & (rei[last][1] != N - 1)
         rei[last], rea[last] = rei[last][:, keep], rea[last][keep]
-    return Workload(f"tiny_regional_N{N}_R{R}_H{H}_s{seed}", model, B, N, T, H, O, R, seed, full, None, rei, rea)
+    return Workload(f"tiny_regional_N{N}_R{R}_H{H}_s{seed}", model, B, N, T, H, O, R, seed, full, None, rei, rea, F=F)
 
 
 # ------------------------------------------------------------------------------------------
 # algorithmic work (SURVEY 8(d) formulas; "the formulas are the contract")
 # ------------------------------------------------------------------------------------------
 def param_count(w: Workload) -> int:
-    H, F, O, T, R = w.H, F_IN, w.O, w.T, w.R
+    H, F, O, T, R = w.H, w.F, w.O, w.T, w.R
     tgcn = 3 * (H * F + H) + 3 * (2 * H * H + H)
     cheb = 2 * H * F + H
     head = 128 * H + 128 + O * 128 + O
@@ -239,7 +240,7 @@ def param_count(w: Workload) -> int:
 
 def alg_bytes_per_step(w: Workload, B: Optional[int] = None) -> int:
     B = w.B if B is None else B
-    N, T, H, O, F = w.N, w.T, w.H, w.O, F_IN
+    N, T, H, O, F = w.N, w.T, w.H, w.O, w.F
     E, Er = w.E, (w.E_reg if w.R else w.E)
     G = ((N + 1) * 4 + (E + N) * 8) + ((N + 1) * 4 + Er * 8)
     return B * N * (2 * T * F * 4 + 2 * T * 4 * H * 4 + 2 * (H + O) * 4) + 3 * param_count(w) * 4 + 2 * G
@@ -247,11 +248,11 @@ def alg_bytes_per_step(w: Workload, B: Optional[int] = None) -> int:
 
 def fwd_flops_per_step(w: Workload, B: Optional[int] = None) -> int:
     B = w.B if B is None else B
-    N, T, H, O, F = w.N, w.T, w.H, w.O, F_IN
+    N, T, H, O, F = w.N, w.T, w.H, w.O, w.F
     E, Er = w.E, (w.E_reg if w.R else w.E)
     return 2 * B * T * N * (3 * (F + H) * H + 2 * F * H) + 2 * B * N * (128 * H + 128 * O) + 2 * B * T * ((E + N) + Er) * F
 
 
 def spmm_bytes(w: Workload, B: Optional[int] = None) -> int:
     B = w.B if B is None else B
-    return 2 * B * w.T * w.N * F_IN * 4 + (w.N + 1) * 4 + (w.E + w.N) * 8
+    return 2 * B * w.T * w.N * w.F * 4 + (w.N + 1) * 4 + (w.E + w.N) * 8
