@@ -33,7 +33,8 @@ extern "C" {
 /* precision of the H x H contractions */
 #define REGT_PREC_FP32 0  /* FFMA, fp32 everywhere (parity mode, all shapes)            */
 #define REGT_PREC_TF32X3 1 /* tcgen05 kind::tf32, 3-pass split: fp32-equivalent accuracy  */
-#define REGT_PREC_BF16 2  /* tcgen05 kind::f16 bf16 operands, fp32 accumulate            */
+#define REGT_PREC_BF16 2  /* tcgen05 kind::f16 bf16 operands, fp32 accumulate: the fused cell at hidden 64
+                             (not the bare TGCN cell), the single-pass bf16 GEMMs at every other hidden % 32 == 0 */
 
 typedef void* regt_stream_t; /* cudaStream_t */
 
@@ -290,12 +291,14 @@ int regt_profile_read(char* names, size_t names_len, float* ms, int max_n);
 
 /* ---- TEST HOOKS ------------------------------------------------------------------------------------------------
  * Not part of the reference-facing boundary: no reference call site maps to these.  They expose the internal
- * tensor-core building blocks (3xTF32 GEMMs of gemm_tma.cu, the hand-built UMMA operand layouts of
+ * tensor-core building blocks (3xTF32 and bf16 GEMMs of gemm_tma.cu, the hand-built UMMA operand layouts of
  * tc_common.cuh) to tests/test_gpu_gemm.py and tests/test_gpu_umma.py so that each is pinned against an fp64 matmul on
  * its own.  Integrators do not bind them.
  *   gemm_nt_tma:  C[M][N]   = A[M][K] . Bt[N][K]^T                    (scratch: 2 * ceil128(N) * ceil32(K) floats)
  *   gemm_tn_tma:  Cp[z]     = sum over the rows of split z of A[r][:K]^T . B[r][:N]      (+ a second, 32-wide operand B2)
- *   gemm_tn_multi: the four-gate-block form of the cell backward, A = D [M][4H]
+ *   gemm_nt_bf16, gemm_tn_bf16: the same two products with both operands rounded to bf16 once (single-pass kind::f16,
+ *                 fp32 accumulate), same arguments; gemm_nt_bf16 needs ceil128(N) * ceil64(K) / 2 floats of scratch
+ *   gemm_tn_multi: the four-gate-block form of the cell backward, A = D [M][4H] (gemm_tn_multi_bf16: its bf16 form)
  *   gemm_kt: the same contraction over transposed tiles A^T [ntile][4H][128], B^T [ntile][H][128], F^T [ntile][32][128]
  *            (what the fused cell backward of cell_f.cu writes); H = 128 or 64
  *   umma_selftest: one 128 x N x K MMA on operand tiles written by CUDA-core threads (fmt 1 = bf16, 2 = tf32)
@@ -303,14 +306,21 @@ int regt_profile_read(char* names, size_t names_len, float* ms, int max_n);
  *             out[7] = {128-row tiles nqt, periods per item tp, period chunks ntc = T / tp, items = nqt * ntc,
  *             forward grid, backward grid, k_head_tc grid} (tests/test_gpu_bf16_edges.py states its preconditions so)
  *   route: which cell and head kernels the entry points run for these arguments (no CUDA call, no workspace needed),
- *          out[4] = {cell: 0 fp32, 1 unfused tf32x3, 2 fused tf32x3, 3 bf16; head: 0 row kernels k_head_fwd / k_head_bwd,
+ *          out[4] = {cell: 0 fp32, 1 unfused tf32x3, 2 fused tf32x3, 3 fused bf16, 4 GEMM-by-GEMM bf16;
+ *          head: 0 row kernels k_head_fwd / k_head_bwd,
  *          1 k_head_fused, 2 tf32x3 head, 3 k_head_tc; G written as tiles; bf16 forward leaves out_hidden partials}   */
 int regt_debug_gemm_nt_tma(const float* A, int64_t lda, const float* Bt, int64_t ldb, float* C, int64_t ldc, int64_t M,
                            int32_t N, int32_t K, float* scratch, regt_stream_t stream);
 int regt_debug_gemm_tn_tma(const float* A, int64_t lda, const float* B, int64_t ldb, float* Cp, int64_t M, int32_t K,
                            int32_t N, int32_t splits, const float* B2, int64_t ldb2, float* Cp2, regt_stream_t stream);
+int regt_debug_gemm_nt_bf16(const float* A, int64_t lda, const float* Bt, int64_t ldb, float* C, int64_t ldc, int64_t M,
+                            int32_t N, int32_t K, float* scratch, regt_stream_t stream);
+int regt_debug_gemm_tn_bf16(const float* A, int64_t lda, const float* B, int64_t ldb, float* Cp, int64_t M, int32_t K,
+                            int32_t N, int32_t splits, const float* B2, int64_t ldb2, float* Cp2, regt_stream_t stream);
 int regt_debug_gemm_tn_multi(const float* A, int64_t lda, int64_t M, int32_t H, const float* B0, const float* B1,
                              float* C0, float* C1, int32_t splits, const float* B2, float* C2, regt_stream_t stream);
+int regt_debug_gemm_tn_multi_bf16(const float* A, int64_t lda, int64_t M, int32_t H, const float* B0, const float* B1,
+                                  float* C0, float* C1, int32_t splits, const float* B2, float* C2, regt_stream_t stream);
 int regt_debug_gemm_kt(const float* AT, int64_t ntile, int32_t H, const float* B0T, const float* B1T, const float* FT,
                        float* C0, float* C1, float* C2, int32_t splits, regt_stream_t stream);
 int regt_debug_spmm_partition_host(const int32_t* rowptr, const int32_t* col, int32_t N, int32_t width, int32_t* blk_ptr,

@@ -13,9 +13,11 @@ Route route_of(const regt_args* a) {
   const bool tf32x3 = a->precision == REGT_PREC_TF32X3, bf16 = a->precision == REGT_PREC_BF16;
   const bool fused_step = a->fuse_head && a->y && a->d_out && a->loss;   // forward, loss and head gradients in one step
   Route r{};
-  r.cell = bf16 ? CellPath::Bf16
+  // bf16: the fused H = 64 cell where it is built for the shape (REGT_UNFUSED does not apply: it names the tf32x3 cells),
+  // else the GEMM-by-GEMM cell on the single-pass bf16 GEMMs
+  r.cell = bf16 ? (cell_tc_fits(a) ? CellPath::Bf16 : CellPath::Bf16Gemm)
                 : !tf32x3 ? CellPath::Fp32 : (!unfused && cell_f_fits(a)) ? CellPath::Tf32x3Fused : CellPath::Tf32x3Unfused;
-  if (bf16 && fused_step && head_tc_fits(a->H, a->O))
+  if (r.cell == CellPath::Bf16 && fused_step && head_tc_fits(a->H, a->O))   // k_head_tc's partials are summed by the fused cell backward
     r.head = HeadPath::Bf16;
   else if (tf32x3 && a->H % 32 == 0 && head_f_fits(a->O) && (long long)a->B * a->N >= 128 && a->out)
     r.head = HeadPath::Tf32x3;
@@ -63,7 +65,8 @@ Layout make_layout(const regt_args* a, void* base) {
     L.Feat = c.take<float>(inf ? 4 : nqt * 128 * 32);      // the head's ones column (row major, BNp rows)
     L.FeatT = c.take<float>(inf ? 4 : rowsP * 32);
     L.tc_dpp = c.take<float>(2 * (T * TC_MAX_CTAS + 64));   // fp64 attention-gradient partials
-  } else if (L.route.cell != CellPath::Bf16) {   // fp32 and unfused tf32x3: row-major planes
+  } else if (L.route.cell != CellPath::Bf16) {   // fp32 and the GEMM-by-GEMM cells (tf32x3, bf16): row-major planes
+    const bool gemm_cell = L.route.cell != CellPath::Fp32;
     L.h = c.take<float>(rows * H);
     L.Z = c.take<float>(rows * H);
     L.Rg = c.take<float>(rows * H);
@@ -71,8 +74,10 @@ Layout make_layout(const regt_args* a, void* base) {
     L.hR = c.take<float>(rows * H);
     L.Hn = c.take<float>(rows * H);
     L.D = c.take<float>(rows * 4 * H);
-    L.Feat = c.take<float>(a->precision == REGT_PREC_TF32X3 ? rows * 32 : 4);
-    L.bsplit = c.take<float>(a->precision == REGT_PREC_TF32X3 ? gemm_nt_scratch_floats((int)H, 2 * (int)H) : 4);
+    L.Feat = c.take<float>(gemm_cell ? rows * 32 : 4);
+    L.bsplit = c.take<float>(L.route.cell == CellPath::Tf32x3Unfused ? gemm_nt_scratch_floats((int)H, 2 * (int)H)
+                             : L.route.cell == CellPath::Bf16Gemm  ? gemm_nt_bf16_scratch_floats((int)H, 2 * (int)H)
+                                                                   : 4);
   } else {   // bf16 fused tcgen05 kernels: tile-layout planes
     const size_t nqt = (BN + 127) / 128, plane = T * nqt * 128 * H;
     L.tc_img_f = c.take<unsigned char>(TC_IMG_BYTES);
@@ -116,7 +121,7 @@ Layout make_layout(const regt_args* a, void* base) {
   L.hpart = c.take<float>((size_t)148 * (HEAD_HID * H + O * HEAD_HID + HEAD_HID + O + 8));
   L.part = c.take<float>(pf);
   L.part_floats = pf;
-  if (feat_in(a) < F && (L.route.cell == CellPath::Fp32 || L.route.cell == CellPath::Tf32x3Unfused))
+  if (feat_in(a) < F && (L.route.cell == CellPath::Fp32 || L.route.cell == CellPath::Tf32x3Unfused || L.route.cell == CellPath::Bf16Gemm))
     L.xw = c.take<float>((size_t)a->B * (a->x_rows > 0 ? a->x_rows : a->N) * F * T);
   L.m1cp = c.take<int32_t>(R + 2);   // last: tests locate it from the end of the workspace
   L.total = align_up(c.off, 256);
@@ -126,6 +131,15 @@ Layout make_layout(const regt_args* a, void* base) {
 static int check_features(const regt_args* a, const char* who) {
   REGT_CHECK(a->F >= 0 && a->F <= REGT_F, "%s: F=%d node features; the kernels take 1..%d (0 means %d)", who, a->F, REGT_F,
              REGT_F);
+  return 0;
+}
+
+// the GEMM-by-GEMM tensor-core cells run the H x H contractions in 32-column boxes
+static int check_tc_width(const regt_args* a) {
+  if (a->precision == REGT_PREC_TF32X3)
+    REGT_CHECK(a->H % 32 == 0, "precision tf32x3 needs hidden %% 32 == 0 (got %d); use precision fp32", a->H);
+  if (a->precision == REGT_PREC_BF16)
+    REGT_CHECK(a->H % 32 == 0, "precision bf16 needs hidden %% 32 == 0 (got %d); use precision fp32", a->H);
   return 0;
 }
 
@@ -155,8 +169,7 @@ extern "C" size_t regt_workspace_bytes(const regt_args* a) {
 extern "C" int regt_cell_forward(const regt_args* a) {
   if (validate(a, "regt_cell_forward")) return -1;
   REGT_CHECK(a->x && a->out_hidden, "regt_cell_forward: x / out_hidden is NULL");
-  if (a->precision == REGT_PREC_TF32X3)
-    REGT_CHECK(a->H % 32 == 0, "precision tf32x3 needs hidden %% 32 == 0 (got %d); use precision fp32", a->H);
+  if (check_tc_width(a)) return -1;
   Layout L = make_layout(a, a->workspace);
   cudaStream_t st = (cudaStream_t)a->stream;
   prof_mark("<begin>", st);
@@ -165,6 +178,7 @@ extern "C" int regt_cell_forward(const regt_args* a) {
     case CellPath::Tf32x3Unfused: return cell_forward_g(a, L, st);
     case CellPath::Tf32x3Fused: return cell_forward_f(a, L, st);
     case CellPath::Bf16: return cell_forward_tc(a, L, st);
+    case CellPath::Bf16Gemm: return cell_forward_g(a, L, st);
   }
   return -1;
 }
@@ -172,8 +186,7 @@ extern "C" int regt_cell_forward(const regt_args* a) {
 extern "C" int regt_cell_backward(const regt_args* a) {
   if (validate(a, "regt_cell_backward")) return -1;
   REGT_CHECK(!a->inference, "regt_cell_backward: the forward ran with inference=1 (no activations were saved)");
-  if (a->precision == REGT_PREC_TF32X3)
-    REGT_CHECK(a->H % 32 == 0, "precision tf32x3 needs hidden %% 32 == 0 (got %d); use precision fp32", a->H);
+  if (check_tc_width(a)) return -1;
   Layout L = make_layout(a, a->workspace);
   cudaStream_t st = (cudaStream_t)a->stream;
   prof_mark("<begin>", st);
@@ -182,6 +195,7 @@ extern "C" int regt_cell_backward(const regt_args* a) {
     case CellPath::Tf32x3Unfused: return cell_backward_g(a, L, st);
     case CellPath::Tf32x3Fused: return cell_backward_f(a, L, st);
     case CellPath::Bf16: return cell_backward_tc(a, L, st);
+    case CellPath::Bf16Gemm: return cell_backward_g(a, L, st);
   }
   return -1;
 }

@@ -1,6 +1,7 @@
-// REGT_PREC_TF32X3 for any hidden width that is a multiple of 32: the regional temporal GCN cell with
-// every H x H contraction on the sm_100a tensor cores through the generic 3xTF32 GEMMs of gemm_tma.cu
-// (fp32-equivalent accuracy), forward AND backward.  Unlike the fused H = 64 kernels of cell_tc.cu the
+// REGT_PREC_TF32X3 and REGT_PREC_BF16 for any hidden width that is a multiple of 32: the regional temporal GCN
+// cell with every H x H contraction on the sm_100a tensor cores through the generic GEMMs of gemm_tma.cu, forward AND
+// backward -- 3xTF32 (fp32-equivalent accuracy) or single-pass bf16 (Route::cell Bf16Gemm, the bf16 tolerance), the
+// only part of this file that depends on the precision.  The elementwise passes and saved planes are fp32 in both.  Unlike the fused H = 64 kernels of cell_tc.cu the
 // gate pre-activations make one round trip through HBM, which is what lets the same code serve H = 128
 // (configs 4, 5) and H = 256 (configs 1, 3): no weight set has to fit one SM's shared memory or TMEM.
 //
@@ -365,11 +366,15 @@ int launch_fw_scatter(const float* Cp, int splits, int H, const Layout& L, cudaS
   return 0;
 }
 
+// the GEMMs of this call: 3xTF32 or single-pass bf16
+static GemmKind gemm_kind(const Layout& L) { return L.route.cell == CellPath::Bf16Gemm ? GemmKind::Bf16 : GemmKind::Tf32x3; }
+
 int cell_forward_g(const regt_args* a, const Layout& L, cudaStream_t st) {
   const int H = a->H, T = a->T;
   const long long BN = (long long)a->B * a->N;
   const int xN = a->x_rows > 0 ? a->x_rows : a->N;
-  REGT_CHECK(T <= 64, "precision tf32x3 supports up to 64 periods (got %d)", T);
+  const GemmKind gk = gemm_kind(L);
+  REGT_CHECK(T <= 64, "precision %s supports up to 64 periods (got %d)", gk == GemmKind::Bf16 ? "bf16" : "tf32x3", T);
   if (launch_prep(a, L, st)) return -1;
   if (launch_widen_x(a, L, st)) return -1;
   if (launch_spmm_rows(a->plan.g_rowptr, a->plan.g_col, a->plan.g_val, x_wide(a, L), L.S, a->B, a->N, xN, F * T, st)) return -1;
@@ -389,9 +394,9 @@ int cell_forward_g(const regt_args* a, const Layout& L, cudaStream_t st) {
   // warps -- was built and measured in round 1: slower, 200 -> 231 ms at config 4.  The fused cell of cell_f.cu is the
   // route that removes these round trips for H = 128.)
   for (int g = 0; g < 2; ++g)
-    if (launch_gemm_nt_tma(L.h, H, a->p.lin_w[g] + H, 2 * H, L.D + (size_t)g * H, 4 * H, k.rows, H, H, L.bsplit, st)) return -1;
+    if (launch_gemm_nt_tma(L.h, H, a->p.lin_w[g] + H, 2 * H, L.D + (size_t)g * H, 4 * H, k.rows, H, H, L.bsplit, st, gk)) return -1;
   G_LAUNCH(k_g_zr, "k_g_zr");
-  if (launch_gemm_nt_tma(L.hR, H, a->p.lin_w[2] + H, 2 * H, L.D + 2 * H, 4 * H, k.rows, H, H, L.bsplit, st)) return -1;
+  if (launch_gemm_nt_tma(L.hR, H, a->p.lin_w[2] + H, 2 * H, L.D + 2 * H, 4 * H, k.rows, H, H, L.bsplit, st, gk)) return -1;
   k_g_c<<<cdiv(BN * (H / 4), 256), 256, 0, st>>>(k);
   REGT_LAUNCHED("k_g_c", st);
   return 0;
@@ -401,6 +406,7 @@ int cell_backward_g(const regt_args* a, const Layout& L, cudaStream_t st) {
   const int H = a->H, T = a->T;
   const long long BN = (long long)a->B * a->N, rows = BN * T;
   GK k = make_gk(a, L);
+  const GemmKind gk = gemm_kind(L);
   float* part = L.part;
   float* BhT = part;                       // [H][H]   scratch until the weight-gradient partials take over
   float* BzrT = part + (size_t)H * H;      // [H][2H]
@@ -412,9 +418,9 @@ int cell_backward_g(const regt_args* a, const Layout& L, cudaStream_t st) {
   k_g_b1<<<nb1, 256, 0, st>>>(k);
   REGT_LAUNCHED("k_g_b1", st);
   if (launch_f_sum_dpp(dpp, nb1, T, L.dprobs, st)) return -1;
-  if (launch_gemm_nt_tma(L.D + 2 * H, 4 * H, BhT, H, L.Hn, H, rows, H, H, L.bsplit, st)) return -1;            // dHR = Dh . B_h
+  if (launch_gemm_nt_tma(L.D + 2 * H, 4 * H, BhT, H, L.Hn, H, rows, H, H, L.bsplit, st, gk)) return -1;            // dHR = Dh . B_h
   G_LAUNCH(k_g_b2, "k_g_b2");
-  if (launch_gemm_nt_tma(L.D, 4 * H, BzrT, 2 * H, L.D + 3 * H, 4 * H, rows, H, 2 * H, L.bsplit, st)) return -1;   // dhg
+  if (launch_gemm_nt_tma(L.D, 4 * H, BzrT, 2 * H, L.D + 3 * H, 4 * H, rows, H, 2 * H, L.bsplit, st, gk)) return -1;   // dhg
   G_LAUNCH(k_g_b3, "k_g_b3");
   // H x H weight gradients on the tensor cores (contraction over the rows)
   // ... and, in the SAME pass over D, the F-wide gradients and biases D^T . [S | X | 1] (second, 32-column operand:
@@ -433,11 +439,11 @@ int cell_backward_g(const regt_args* a, const Layout& L, cudaStream_t st) {
     float* cs[3] = {pB, pBh, nullptr};
     const float* bs[2] = {L.h, L.hR};
     const long long lds[2] = {H, H};
-    if (launch_gemm_tn_tma(L.D, 4 * H, rows, 4 * H, 3, k0, sb, cs, bs, lds, H, splits, L.Feat, 32, pF, fsplit, st, 0)) return -1;
+    if (launch_gemm_tn_tma(L.D, 4 * H, rows, 4 * H, 3, k0, sb, cs, bs, lds, H, splits, L.Feat, 32, pF, fsplit, st, 0, gk)) return -1;
   } else {
-    if (launch_gemm_tn(L.D, 4 * H, L.h, H, pB, rows, 2 * H, H, splits, st, L.Feat, 32, pF, fsplit, 0)) return -1;
-    if (launch_gemm_tn(L.D + 2 * H, 4 * H, L.hR, H, pBh, rows, H, H, splits, st, L.Feat, 32, pF + (size_t)2 * H * 32, fsplit, 0)) return -1;
-    if (launch_gemm_tn(L.D + 3 * H, 4 * H, nullptr, 0, nullptr, rows, H, 0, splits, st, L.Feat, 32, pF + (size_t)3 * H * 32, fsplit, 0)) return -1;
+    if (launch_gemm_tn(L.D, 4 * H, L.h, H, pB, rows, 2 * H, H, splits, st, L.Feat, 32, pF, fsplit, 0, gk)) return -1;
+    if (launch_gemm_tn(L.D + 2 * H, 4 * H, L.hR, H, pBh, rows, H, H, splits, st, L.Feat, 32, pF + (size_t)2 * H * 32, fsplit, 0, gk)) return -1;
+    if (launch_gemm_tn(L.D + 3 * H, 4 * H, nullptr, 0, nullptr, rows, H, 0, splits, st, L.Feat, 32, pF + (size_t)3 * H * 32, fsplit, 0, gk)) return -1;
   }
   if (launch_reduce_splits(pB, L.dB, 2ll * H * H, splits, 0, st)) return -1;
   if (launch_reduce_splits(pBh, L.dB + (size_t)2 * H * H, (long long)H * H, splits, 0, st)) return -1;

@@ -642,6 +642,8 @@ static int run_fwd_tc(const regt_args* a, const Layout& L, cudaStream_t st, bool
   return 0;
 }
 
+bool cell_tc_fits(const regt_args* a) { return a->H == 64 && a->mode != REGT_MODE_TGCN; }
+
 int cell_forward_tc(const regt_args* a, const Layout& L, cudaStream_t st) {
   REGT_CHECK(a->H == 64, "the fused bf16 tensor-core kernels are built for hidden=64 (got %d); use precision tf32x3 or fp32", a->H);
   REGT_CHECK(a->mode != REGT_MODE_TGCN, "tensor-core precisions do not cover the bare TGCN cell; use precision fp32");

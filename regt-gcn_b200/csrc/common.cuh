@@ -86,7 +86,8 @@ inline int sm_count() {
 }
 
 // ---- which cell and head kernels a call runs (route_of, api.cu) ----------------------
-enum class CellPath { Fp32, Tf32x3Unfused, Tf32x3Fused, Bf16 };   // cell.cu, cell_g.cu, cell_f.cu, cell_tc.cu
+// cell.cu, cell_g.cu, cell_f.cu, cell_tc.cu, and cell_g.cu on the single-pass bf16 GEMMs (every hidden % 32 == 0 width)
+enum class CellPath { Fp32, Tf32x3Unfused, Tf32x3Fused, Bf16, Bf16Gemm };
 enum class HeadPath { Rows, FusedFfma, Tf32x3, Bf16 };             // k_head_fwd / k_head_bwd, k_head_fused, head_f.cu, k_head_tc
 struct Route {
   CellPath cell;
@@ -98,6 +99,7 @@ struct Route {
 Route route_of(const regt_args* a);
 // the shapes each implementation is built for, with no knowledge of the other paths
 bool cell_f_fits(const regt_args* a);   // fused tf32x3 cell: hidden 64 / 128, not the bare TGCN cell, <= 64 periods
+bool cell_tc_fits(const regt_args* a);  // fused bf16 cell: hidden 64, not the bare TGCN cell
 bool head_fused_fits(int H, int O);     // k_head_fused: hidden 32 / 64, <= 64 outputs, within a block's shared memory
 bool head_tc_fits(int H, int O);        // k_head_tc: hidden 64, <= 16 outputs
 bool head_f_fits(int O);                // k_hf_mid: <= 16 outputs
@@ -139,7 +141,7 @@ struct Layout {
   float* hf_loss;    // per-block loss partials
   size_t hf_loss_floats;
   float* FeatT;  // fused tf32x3 cell: transposed feature tiles [T*nqt][32][128] (cell_f.cu)
-  float* bsplit; // tf32x3: hi | lo images of the weight operand of the current gate GEMM (gemm_tma.cu)
+  float* bsplit; // GEMM-by-GEMM cell: hi | lo (tf32x3) or bf16 image of the weight operand of the current gate GEMM (gemm_tma.cu)
   // collapsed-weight gradients
   float* dB;     // [3][H][H]   dB_z, dB_r, dB_h
   float* dP;     // [3][H][F]
@@ -219,15 +221,18 @@ int launch_wgrad_m1_kt(const regt_args* a, const Layout& L, cudaStream_t st);   
 // cell_g.cu: d probs from the fused backward's fp64 partials; F-wide weight gradients from the [splits][4H][32] partials of D^T Feat
 int launch_f_sum_dpp(const double* part, int nparts, int T, float* dprobs, cudaStream_t st);
 int launch_fw_scatter(const float* Cp, int splits, int H, const Layout& L, cudaStream_t st);
-// gemm_tma.cu: TMA-fed 3xTF32 GEMMs
-size_t gemm_nt_scratch_floats(int N, int K);
+// gemm_tma.cu: TMA-fed 3xTF32 GEMMs and their single-pass bf16 forms
+enum class GemmKind { Tf32x3, Bf16 };
+size_t gemm_nt_scratch_floats(int N, int K);        // hi | lo images of the weight operand (Tf32x3)
+size_t gemm_nt_bf16_scratch_floats(int N, int K);   // its bf16 image (Bf16)
 int launch_gemm_nt_tma(const float* A, long long lda, const float* Bt, long long ldb, float* C, long long ldc, long long M, int N,
-                       int K, float* scratch, cudaStream_t st);
+                       int K, float* scratch, cudaStream_t st, GemmKind kind = GemmKind::Tf32x3);
 int launch_gemm_tn(const float* A, long long lda, const float* B, long long ldb, float* Cp, long long M, int K, int N, int splits,
-                   cudaStream_t st, const float* B2, long long ldb2, float* Cp2, long long c2_split, int relu_b);
+                   cudaStream_t st, const float* B2, long long ldb2, float* Cp2, long long c2_split, int relu_b,
+                   GemmKind kind = GemmKind::Tf32x3);
 int launch_gemm_tn_tma(const float* A, long long lda, long long M, int Ktot, int nseg, const int* seg_k0, const int* seg_b,
                        float* const* seg_C, const float* const* Bs, const long long* ldbs, int N, int splits, const float* B2,
-                       long long ldb2, float* C2, long long c2_split, cudaStream_t st, int relu_b);
+                       long long ldb2, float* C2, long long c2_split, cudaStream_t st, int relu_b, GemmKind kind = GemmKind::Tf32x3);
 int launch_gemm_kt(const float* AT, long long ntile, int Ktot, int nseg, const int* seg_k0, const int* seg_k1, const int* seg_b,
                    float* const* seg_C, const float* const* BTs, int N, int splits, const float* FT, float* C2, long long c2_split,
                    cudaStream_t st);

@@ -1,4 +1,4 @@
-// TMA-fed 3xTF32 GEMMs.
+// TMA-fed 3xTF32 GEMMs, and their single-pass bf16 forms (below k_gemm_kt).
 //
 // A single producer thread keeps whole pipeline stages in flight with cp.async.bulk.tensor (TMA, SWIZZLE_128B boxes
 // landing directly in the UMMA operand layout), converter warps do the tf32 hi/lo split in shared memory, one thread issues
@@ -741,17 +741,454 @@ __global__ void __launch_bounds__(TN_THREADS, 1) k_gemm_kt(const __grid_constant
   __syncthreads();
   if (warp == TN_W_MMA) tmem_dealloc(tmem, 512);
 }
+
+// ------------------------------------------------------------------------------------------
+// Single-pass bf16 forms of gemm_nt and gemm_tn (precision bf16 on the GEMM-by-GEMM cell of cell_g.cu).  The operands
+// still arrive by TMA as fp32 and C stays fp32; the converters round each operand to bf16 once (round to nearest even)
+// instead of splitting it into tf32 hi / lo, and every K step is ONE kind::f16 MMA with fp32 accumulation in TMEM.
+// A 128-byte swizzle row holds 64 bf16 but only 32 fp32, so a chunk is KB = 64 contraction elements, fed by two 32-wide
+// fp32 boxes:
+//   gemm_nt: A chunk = two [128 rows][32 k] fp32 boxes -> one K-major SW128 bf16 tile [128 rows][64 k] (the layout of
+//            umma_selftest variant 0); the weight operand is packed ONCE per call into a dense bf16 image (k_pack_bf16)
+//            whose [128][64] TMA boxes land in that same layout, parked in shared memory (N <= 128, K <= 384) or streamed.
+//            A is read from SHARED memory, not TMEM: a converted tile is 16 KB (half the tf32 hi | lo pair), so four of
+//            them beside the raw stages still leave 3-4 stages = 96-128 KB of loads in flight (the TS kernel keeps 96 KB),
+//            and both operands then use the one bf16 layout umma_selftest pins; no test here pins the TMEM layout of a
+//            16-bit A operand.
+//   gemm_tn: raw boxes [64 rows][32 cols] fp32 and NO transpose: the contraction runs over the rows of the boxes, so each
+//            row is converted in place of position into MN-major SW128 bf16 tiles [cols / 64][64 rows][128 B] (the
+//            layout of umma_selftest variant 2; one 16-byte store per two 16-byte loads, where the tf32 converters issue
+//            eight 4-byte transposing stores).  The 32 columns of B2 follow the B columns of the tile as its last box.
+// Both keep the rules of the tf32 kernels: a raw stage is released only behind a branch on the values loaded from it,
+// and gemm_tn drains its accumulator into fp32 registers every TN_GROUP chunks.
+// ------------------------------------------------------------------------------------------
+constexpr int KB = 64;                        // bf16 contraction chunk: one 128-byte swizzle row
+constexpr int NB_SLOTS = 4;                   // converted A tiles of gemm_nt (shared memory)
+
+__device__ __forceinline__ uint4 pack8_bf16(const float4 u, const float4 v) {
+  return make_uint4(pack_bf16(u.x, u.y), pack_bf16(u.z, u.w), pack_bf16(v.x, v.y), pack_bf16(v.z, v.w));
+}
+
+// dense bf16 image of a weight operand: img[n][k] = bf16(B[n][k]), zero-padded to [Np][Kp]
+__global__ void k_pack_bf16(const float* __restrict__ B, long long ldb, int N, int K, int Np, int Kp, __nv_bfloat16* __restrict__ img) {
+  const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (i >= (long long)Np * Kp) return;
+  const int n = (int)(i / Kp), k = (int)(i - (long long)n * Kp);
+  img[i] = __float2bfloat16_rn((n < N && k < K) ? __ldg(B + (size_t)n * ldb + k) : 0.f);
+}
+
+struct NtBf16Args {
+  CUtensorMap ta, tb;   // A [M][K] fp32; Bt bf16 image [Np][Kp]
+  float* C;
+  long long M, ldc;
+  int N, K;
+  int resident;         // the bf16 image parked in shared memory for the whole kernel
+  int ns;               // pipeline stages
+};
+
+__global__ void __launch_bounds__(NT_THREADS, 1) k_gemm_nt_bf16(const __grid_constant__ NtBf16Args a) {
+  extern __shared__ __align__(1024) uint8_t smem_raw[];
+  uint8_t* sm = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
+  __shared__ uint64_t bar_tma[MAXS], bar_rfree[MAXS], bar_afull[NB_SLOTS], bar_afree[NB_SLOTS], bar_b, bar_acc_full[2], bar_acc_free[2];
+  __shared__ uint32_t tmem_base_s;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int ns = a.ns;
+  const int nchunks = (a.K + KB - 1) / KB;
+  const int ntn = (a.N + 127) / 128;
+  const long long ntiles = ((a.M + 127) / 128) * ntn;
+  const int stage_bytes = a.resident ? 2 * TILE : 3 * TILE;      // two raw fp32 A boxes ( | bf16 B tile when the weights stream)
+  uint8_t* bres = sm;
+  uint8_t* aslot = sm + (a.resident ? nchunks * TILE : 0);       // NB_SLOTS converted bf16 A tiles
+  uint8_t* stages = aslot + NB_SLOTS * TILE;
+  if (tid == 0) {
+    for (int s = 0; s < ns; ++s) {
+      mbar_init(&bar_tma[s], 1);
+      mbar_init(&bar_rfree[s], a.resident ? NT_CONV : NT_CONV + 1);   // streamed weights: + the commit of the MMAs that read them
+    }
+    for (int s = 0; s < NB_SLOTS; ++s) {
+      mbar_init(&bar_afull[s], NT_CONV);
+      mbar_init(&bar_afree[s], 1);
+    }
+    mbar_init(&bar_b, 1);
+    for (int b = 0; b < 2; ++b) {
+      mbar_init(&bar_acc_full[b], 1);
+      mbar_init(&bar_acc_free[b], 128);
+    }
+    fence_barrier_init();
+  }
+  if (warp == NT_W_MMA) tmem_alloc(&tmem_base_s, 256);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem = tmem_base_s;
+
+  if (warp < NT_W_TMA) {
+    // ---- converters: thread = (row of the tile, raw box `half` = k 32 half .. + 31 of the chunk); two 16-byte raw pieces
+    //      make one 16-byte piece of the bf16 row.  Reads and writes are 128-byte swizzled: conflict-free quarter-warps.
+    const int q = warp & 3, half = warp >> 2;
+    const int r = q * 32 + lane, sw = r & 7;
+    long long gc = 0;
+    for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+      for (int kc = 0; kc < nchunks; ++kc, ++gc) {
+        const int s = (int)(gc % ns), sl = (int)(gc % NB_SLOTS);
+        mbar_wait(&bar_tma[s], (uint32_t)((gc / ns) & 1));
+        uint4 p[4] = {make_uint4(0u, 0u, 0u, 0u), make_uint4(0u, 0u, 0u, 0u), make_uint4(0u, 0u, 0u, 0u), make_uint4(0u, 0u, 0u, 0u)};
+        if (kc * KB + 32 * half < a.K) {   // the box was loaded (a box wholly past K is not)
+          const uint8_t* rw = stages + (size_t)s * stage_bytes + half * TILE + r * 128;
+#pragma unroll
+          for (int c = 0; c < 4; ++c)
+            p[c] = pack8_bf16(*reinterpret_cast<const float4*>(rw + (((2 * c) ^ sw) << 4)),
+                              *reinterpret_cast<const float4*>(rw + (((2 * c + 1) ^ sw) << 4)));
+        }
+        // an arrive does not wait for this thread's loads (see k_gemm_tn_tma): it sits behind a branch on the loaded values
+        if ((p[0].x | p[1].x | p[2].x | p[3].x) == 0x7FC0DEADu) __nanosleep(1);
+        mbar_arrive(&bar_rfree[s]);
+        if (gc >= NB_SLOTS) mbar_wait(&bar_afree[sl], (uint32_t)((gc / NB_SLOTS - 1) & 1));
+        uint8_t* dst = aslot + (size_t)sl * TILE + r * 128;
+#pragma unroll
+        for (int c = 0; c < 4; ++c) *reinterpret_cast<uint4*>(dst + (((4 * half + c) ^ sw) << 4)) = p[c];
+        fence_proxy_async();
+        mbar_arrive(&bar_afull[sl]);
+      }
+    }
+  } else if (warp == NT_W_TMA) {
+    if (lane == 0) {
+      tmap_prefetch(&a.ta);
+      tmap_prefetch(&a.tb);
+      if (a.resident) {
+        mbar_arrive_expect_tx(&bar_b, (uint32_t)(nchunks * TILE));
+        for (int kc = 0; kc < nchunks; ++kc) tma_2d(bres + (size_t)kc * TILE, &a.tb, kc * KB, 0, &bar_b);
+      }
+      long long gc = 0;
+      for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+        const int m0 = (int)((tile / ntn) * 128), n0 = (int)(tile % ntn) * 128;
+        for (int kc = 0; kc < nchunks; ++kc, ++gc) {
+          const int s = (int)(gc % ns);
+          if (gc >= ns) mbar_wait(&bar_rfree[s], (uint32_t)((gc / ns - 1) & 1));
+          uint8_t* st = stages + (size_t)s * stage_bytes;
+          const bool second = kc * KB + 32 < a.K;
+          mbar_arrive_expect_tx(&bar_tma[s], (uint32_t)((1 + (second ? 1 : 0) + (a.resident ? 0 : 1)) * TILE));
+          tma_2d(st, &a.ta, kc * KB, m0, &bar_tma[s]);
+          if (second) tma_2d(st + TILE, &a.ta, kc * KB + 32, m0, &bar_tma[s]);
+          if (!a.resident) tma_2d(st + 2 * TILE, &a.tb, kc * KB, n0, &bar_tma[s]);
+        }
+      }
+    }
+  } else if (warp == NT_W_MMA) {
+    const uint32_t bres0 = smem_u32(bres), aslot0 = smem_u32(aslot), stage0 = smem_u32(stages);
+    if (a.resident) mbar_wait(&bar_b, 0);
+    long long gc = 0, li = 0;
+    for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++li) {
+      const int nt = min(128, a.N - (int)(tile % ntn) * 128);
+      const uint32_t idesc = make_idesc(FMT_BF16, 128, nt, 0, 0);
+      const int buf = (int)(li & 1);
+      if (li >= 2) {
+        mbar_wait(&bar_acc_free[buf], (uint32_t)((li / 2 - 1) & 1));
+        tc_fence_after();
+      }
+      for (int kc = 0; kc < nchunks; ++kc, ++gc) {
+        const int sl = (int)(gc % NB_SLOTS);
+        mbar_wait(&bar_afull[sl], (uint32_t)((gc / NB_SLOTS) & 1));
+        tc_fence_after();
+        if (lane == 0) {
+          const int s = (int)(gc % ns);
+          const uint32_t at = aslot0 + sl * TILE;
+          const uint32_t bt = a.resident ? bres0 + kc * TILE : stage0 + s * stage_bytes + 2 * TILE;
+#pragma unroll
+          for (int k = 0; k < KB / 16; ++k)
+            umma<FMT_BF16>(tmem + buf * 128, make_desc(at + k * 32, 16, 1024, LAYOUT_SW128), make_desc(bt + k * 32, 16, 1024, LAYOUT_SW128),
+                           idesc, (kc > 0 || k > 0) ? 1u : 0u);
+          umma_commit(&bar_afree[sl]);
+          if (!a.resident) umma_commit(&bar_rfree[s]);   // the streamed weight tile of this stage has been read
+          if (kc + 1 == nchunks) umma_commit(&bar_acc_full[buf]);
+        }
+        __syncwarp();
+      }
+    }
+    tc_fence_before();
+  } else {
+    // ---- epilogue warps: TMEM -> registers -> C (thread = row of the tile), as in k_gemm_nt_tma_ts ----
+    const int r = (warp & 3) * 32 + lane;
+    const uint32_t tlane = tmem + ((uint32_t)((warp & 3) * 32) << 16);
+    long long li = 0;
+    for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++li) {
+      const int buf = (int)(li & 1);
+      const int n0 = (int)(tile % ntn) * 128;
+      const int nt = min(128, a.N - n0);
+      const long long arow = (tile / ntn) * 128 + r;
+      const bool a_ok = arow < a.M;
+      float* cp = a.C + (a_ok ? arow : 0) * a.ldc + n0;
+      mbar_wait(&bar_acc_full[buf], (uint32_t)((li / 2) & 1));
+      tc_fence_after();
+      for (int c0 = 0; c0 < nt; c0 += 32) {
+        float v[32];
+        if (c0 + 32 <= nt) {
+          tmem_ld32(tlane + buf * 128 + c0, v);
+        } else {
+          float u[16];
+          tmem_ld16(tlane + buf * 128 + c0, u);
+#pragma unroll
+          for (int j = 0; j < 16; ++j) v[j] = u[j];
+        }
+        if (a_ok) {
+          const int w = min(32, nt - c0);
+#pragma unroll
+          for (int j = 0; j < 32; j += 4)
+            if (j < w) *reinterpret_cast<float4*>(cp + c0 + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
+        }
+      }
+      tc_fence_before();
+      mbar_arrive(&bar_acc_free[buf]);
+    }
+  }
+  __syncthreads();
+  if (warp == NT_W_MMA) tmem_dealloc(tmem, 256);
+}
+
+constexpr int TB_BOX = KB * 128;              // one [64 rows][32 cols] fp32 box
+constexpr int TB_RAW = 9 * TB_BOX;            // A: 4 boxes, B: 4 boxes, B2: 1 box
+constexpr int TB_BLK = KB * 128;              // one MN-major bf16 block: 64 columns x 64 rows
+constexpr int TB_AT = 2 * TB_BLK;             // converted A tile: 128 columns
+constexpr int TB_CV = TB_AT + 3 * TB_BLK;     // A | B tile of 128 + 32 feature columns
+static_assert(TN_NR * TB_RAW + TN_NC * TB_CV <= SMEM_BUDGET, "bf16 gemm_tn stages exceed shared memory");
+
+// raw box b (columns 32 b .. 32 b + 31 of its operand), quarter p of row `row`, converted: 8 bf16 for byte 16 p of the row
+__device__ __forceinline__ uint4 tb_piece(const uint8_t* rw_row, int b, int p, int sw, bool relu) {
+  const uint8_t* src = rw_row + b * TB_BOX;
+  float4 u = *reinterpret_cast<const float4*>(src + (((2 * p) ^ sw) << 4));
+  float4 v = *reinterpret_cast<const float4*>(src + (((2 * p + 1) ^ sw) << 4));
+  if (relu) {
+    u = make_float4(fmaxf(u.x, 0.f), fmaxf(u.y, 0.f), fmaxf(u.z, 0.f), fmaxf(u.w, 0.f));
+    v = make_float4(fmaxf(v.x, 0.f), fmaxf(v.y, 0.f), fmaxf(v.z, 0.f), fmaxf(v.w, 0.f));
+  }
+  return pack8_bf16(u, v);
+}
+// byte offset of column box b, quarter p of row `row` in an MN-major SW128 bf16 tile [blocks of 64 columns][64 rows][128 B]
+__device__ __forceinline__ uint32_t tb_off(int b, int p, int row) {
+  return (uint32_t)((b >> 1) * TB_BLK + row * 128 + ((((b & 1) * 4 + p) ^ (row & 7)) << 4));
+}
+
+__global__ void __launch_bounds__(TN_THREADS, 1) k_gemm_tn_bf16(const __grid_constant__ TnArgs a) {
+  extern __shared__ __align__(1024) uint8_t smem_raw[];
+  uint8_t* sm = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
+  __shared__ uint64_t bar_raw[TN_NR], bar_rfree[TN_NR], bar_full[TN_NC], bar_empty[TN_NC], bar_done, bar_acc_free[2];
+  __shared__ uint32_t tmem_base_s;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int kg = blockIdx.x * 128;   // first column of A of this tile
+  int si = 0;
+  for (int s = 1; s < a.nseg; ++s)
+    if (kg >= a.seg[s].k0) si = s;
+  const int sk0 = a.seg[si].k0, sk1 = a.seg[si].k1, sb = a.seg[si].b;
+  float* segC = a.seg[si].C;
+  const int n0 = blockIdx.y * 128;
+  const int kt = min(128, sk1 - kg);                                    // output rows of this tile (multiple of 32)
+  const int nt = sb >= 0 ? max(0, min(128, a.N - n0)) : 0;              // columns from the B operand (multiple of 32)
+  const int n2 = (blockIdx.y == 0) ? a.N2 : 0;                          // + the 32 feature columns on N tile 0
+  const int ntot = nt + n2;
+  const long long r0 = (long long)blockIdx.z * a.chunk, r1 = min(a.M, r0 + a.chunk);
+  const int nchunks = ntot > 0 ? (int)max(0ll, (r1 - r0 + KB - 1) / KB) : 0;
+  uint8_t* raw = sm;
+  uint8_t* cv = sm + TN_NR * TB_RAW;
+  if (tid == 0) {
+    for (int s = 0; s < TN_NR; ++s) {
+      mbar_init(&bar_raw[s], 1);
+      mbar_init(&bar_rfree[s], TN_CONV);
+    }
+    for (int s = 0; s < TN_NC; ++s) {
+      mbar_init(&bar_full[s], TN_CONV);
+      mbar_init(&bar_empty[s], 1);
+    }
+    mbar_init(&bar_done, 1);
+    mbar_init(&bar_acc_free[0], TN_CONV);
+    mbar_init(&bar_acc_free[1], TN_CONV);
+    fence_barrier_init();
+  }
+  if (warp == TN_W_MMA) tmem_alloc(&tmem_base_s, 512);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem = tmem_base_s;
+  const int ablk = kt / 32, bblk = nt / 32;   // boxes per chunk (the feature box, when present, is box bblk of B)
+
+  if (warp < TN_W_MMA) {
+    // ---- converters: thread = (row of the chunk tid % 64, 16-byte quarter tid / 64 of every box's bf16 row) ----
+    const int row = tid & 63, p = tid >> 6, sw = row & 7;
+    // accumulator draining as in k_gemm_tn_tma: row orow of the output tile, 16-column groups half, half + 2, ...
+    const int orow = (warp & 3) * 32 + lane, half = warp >> 2;
+    const uint32_t tlane = tmem + ((uint32_t)((warp & 3) * 32) << 16);
+    float acc[5][16];
+#pragma unroll
+    for (int i = 0; i < 5; ++i)
+#pragma unroll
+      for (int j = 0; j < 16; ++j) acc[i][j] = 0.f;
+    int drained = 0;
+    auto drain = [&](int buf) {
+      tc_fence_after();
+#pragma unroll
+      for (int i = 0; i < 5; ++i) {
+        const int c0 = half * 16 + 32 * i;
+        if (c0 < ntot) {
+          float v[16];
+          tmem_ld16(tlane + buf * TN_ACC + c0, v);
+#pragma unroll
+          for (int j = 0; j < 16; ++j) acc[i][j] += v[j];
+        }
+      }
+      tc_fence_before();
+      mbar_arrive(&bar_acc_free[buf]);
+    };
+    const uint4 zero = make_uint4(0u, 0u, 0u, 0u);
+    for (int kc = 0; kc < nchunks; ++kc) {
+      const int rs = kc % TN_NR, cs = kc % TN_NC;
+      mbar_wait(&bar_raw[rs], (uint32_t)((kc / TN_NR) & 1));
+      const uint8_t* rw = raw + rs * TB_RAW + row * 128;
+      uint4 av[4], bv[5];
+#pragma unroll
+      for (int b = 0; b < 4; ++b) {
+        av[b] = b < ablk ? tb_piece(rw, b, p, sw, false) : zero;
+        bv[b] = b < bblk ? tb_piece(rw, 4 + b, p, sw, a.relu_b != 0) : zero;
+      }
+      bv[4] = n2 ? tb_piece(rw, 8, p, sw, false) : zero;
+      {   // the raw stage is refilled once all 256 threads have arrived: the arrive sits behind a branch on the loaded
+          // values (see k_gemm_tn_tma)
+        const uint32_t dep = av[0].x | av[1].x | av[2].x | av[3].x | bv[0].x | bv[1].x | bv[2].x | bv[3].x | bv[4].x;
+        if (dep == 0x7FC0DEADu) __nanosleep(1);
+        mbar_arrive(&bar_rfree[rs]);
+      }
+      if (kc >= TN_NC) mbar_wait(&bar_empty[cs], (uint32_t)((kc / TN_NC - 1) & 1));
+      // the MMAs of chunks <= kc - TN_NC have completed: group g is whole once (g + 1) * TN_GROUP - 1 <= kc - TN_NC
+      if (kc >= TN_GROUP + TN_NC - 1 && (kc - (TN_NC - 1)) % TN_GROUP == 0) {
+        drain(drained & 1);
+        ++drained;
+      }
+      uint8_t* st = cv + cs * TB_CV;
+#pragma unroll
+      for (int b = 0; b < 4; ++b) {
+        *reinterpret_cast<uint4*>(st + tb_off(b, p, row)) = av[b];
+        if (b < bblk) *reinterpret_cast<uint4*>(st + TB_AT + tb_off(b, p, row)) = bv[b];
+      }
+      if (n2) *reinterpret_cast<uint4*>(st + TB_AT + tb_off(bblk, p, row)) = bv[4];
+      fence_proxy_async();
+      mbar_arrive(&bar_full[cs]);
+    }
+    // ---- epilogue: remaining groups, then the partial tile -> Cp[z] (an empty split contributes zeros) ----
+    const int ngroups = (nchunks + TN_GROUP - 1) / TN_GROUP;
+    if (nchunks > 0) mbar_wait(&bar_done, 0);
+    for (; drained < ngroups; ++drained) drain(drained & 1);
+    const bool row_ok = orow < kt;
+    float* cp = nt > 0 ? segC + ((size_t)blockIdx.z * (sk1 - sk0) + (kg - sk0) + (row_ok ? orow : 0)) * a.N + n0 : nullptr;
+    float* cp2 = n2 ? a.C2 + (size_t)blockIdx.z * a.c2_split + (size_t)(kg + (row_ok ? orow : 0)) * 32 : nullptr;
+#pragma unroll
+    for (int i = 0; i < 5; ++i) {
+      const int c0 = half * 16 + 32 * i;
+      if (c0 < ntot && row_ok) {
+        float* o = c0 < nt ? cp + c0 : cp2 + (c0 - nt);
+#pragma unroll
+        for (int j = 0; j < 16; j += 4) *reinterpret_cast<float4*>(o + j) = make_float4(acc[i][j], acc[i][j + 1], acc[i][j + 2], acc[i][j + 3]);
+      }
+    }
+  } else if (warp == TN_W_MMA) {
+    const uint32_t idesc = make_idesc(FMT_BF16, 128, max(ntot, 16), 1, 1);
+    const uint32_t base = smem_u32(cv);
+    for (int kc = 0; kc < nchunks; ++kc) {
+      const int s = kc % TN_NC;
+      const int g = kc / TN_GROUP, buf = g & 1, kg0 = kc % TN_GROUP;
+      if (kg0 == 0 && g >= 2) {   // the converters have drained this accumulator's previous group (g - 2)
+        mbar_wait(&bar_acc_free[buf], (uint32_t)((g / 2 - 1) & 1));
+        tc_fence_after();
+      }
+      mbar_wait(&bar_full[s], (uint32_t)((kc / TN_NC) & 1));
+      tc_fence_after();
+      if (lane == 0) {
+        const uint32_t at = base + s * TB_CV, bt = at + TB_AT;
+        // MN-major: LBO = stride of the 64-column blocks, SBO = stride of 8-row groups; a K step is 16 rows = 2 KB
+#pragma unroll
+        for (int k = 0; k < KB / 16; ++k)
+          umma<FMT_BF16>(tmem + buf * TN_ACC, make_desc(at + k * 2048, TB_BLK, 1024, LAYOUT_SW128),
+                         make_desc(bt + k * 2048, TB_BLK, 1024, LAYOUT_SW128), idesc, (kg0 > 0 || k > 0) ? 1u : 0u);
+        umma_commit(&bar_empty[s]);
+        if (kc + 1 == nchunks) umma_commit(&bar_done);
+      }
+      __syncwarp();
+    }
+    tc_fence_before();
+  } else {
+    // ---- producer ----
+    if (lane == 0 && nchunks > 0) {
+      tmap_prefetch(&a.ta);
+      if (sb >= 0) tmap_prefetch(&a.tb[sb]);
+      if (n2) tmap_prefetch(&a.tf);
+      const uint32_t bytes = (uint32_t)((ablk + bblk + (n2 ? 1 : 0)) * TB_BOX);
+      for (int kc = 0; kc < nchunks; ++kc) {
+        const int rs = kc % TN_NR;
+        if (kc >= TN_NR) mbar_wait(&bar_rfree[rs], (uint32_t)((kc / TN_NR - 1) & 1));
+        uint8_t* rw = raw + rs * TB_RAW;
+        const int row = (int)(r0 + (long long)kc * KB);
+        mbar_arrive_expect_tx(&bar_raw[rs], bytes);
+        for (int b = 0; b < ablk; ++b) tma_2d(rw + b * TB_BOX, &a.ta, kg + b * 32, row, &bar_raw[rs]);
+        for (int b = 0; b < bblk; ++b) tma_2d(rw + (4 + b) * TB_BOX, &a.tb[sb], n0 + b * 32, row, &bar_raw[rs]);
+        if (n2) tma_2d(rw + 8 * TB_BOX, &a.tf, 0, row, &bar_raw[rs]);
+      }
+    }
+  }
+  __syncthreads();
+  if (warp == TN_W_MMA) tmem_dealloc(tmem, 512);
+}
 }  // namespace
 
 size_t gemm_nt_scratch_floats(int N, int K) { return (size_t)2 * ((N + 127) / 128 * 128) * ((K + KC - 1) / KC * KC); }
+size_t gemm_nt_bf16_scratch_floats(int N, int K) { return (size_t)((N + 127) / 128 * 128) * ((K + KB - 1) / KB * KB) / 2; }
+
+// bf16 image [rows][cols] with pitch ld (elements); boxes of box_rows x 64 bf16 (one 128-byte swizzle row)
+static int tmap_2d_bf16(CUtensorMap* m, const __nv_bfloat16* base, long long cols, long long rows, long long ld, int box_rows,
+                        const char* who) {
+  EncodeFn enc = encoder();
+  REGT_CHECK(enc != nullptr, "%s: cuTensorMapEncodeTiled is not available from this driver", who);
+  REGT_CHECK(((uintptr_t)base % 16 == 0) && ld % 8 == 0, "%s: TMA operands need 16-byte aligned base and pitch", who);
+  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
+  cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
+  cuuint32_t box[2] = {KB, (cuuint32_t)box_rows};
+  cuuint32_t estr[2] = {1, 1};
+  const CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (void*)base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                         CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  REGT_CHECK(r == CUDA_SUCCESS, "%s: cuTensorMapEncodeTiled failed (%d) cols=%lld rows=%lld ld=%lld", who, (int)r, cols, rows, ld);
+  return 0;
+}
+
+// the bf16 form of launch_gemm_nt_tma; `scratch` (gemm_nt_bf16_scratch_floats(N, K) floats) receives the bf16 image of Bt
+static int launch_gemm_nt_bf16(const float* A, long long lda, const float* Bt, long long ldb, float* C, long long ldc, long long M,
+                               int N, int K, float* scratch, cudaStream_t st) {
+  const int Np = (N + 127) / 128 * 128, Kp = (K + KB - 1) / KB * KB, nchunks = Kp / KB;
+  __nv_bfloat16* img = reinterpret_cast<__nv_bfloat16*>(scratch);
+  k_pack_bf16<<<cdiv((long long)Np * Kp, 256), 256, 0, st>>>(Bt, ldb, N, K, Np, Kp, img);
+  REGT_LAUNCHED("k_pack_bf16", st);
+  NtBf16Args a{};
+  if (tmap_2d(&a.ta, A, K, M, lda, 128, "gemm_nt_bf16(A)")) return -1;
+  if (tmap_2d_bf16(&a.tb, img, Kp, Np, Kp, 128, "gemm_nt_bf16(B)")) return -1;
+  a.C = C; a.M = M; a.ldc = ldc; a.N = N; a.K = K;
+  // shared memory: the bf16 weights (parked when N <= 128 and they leave room for two stages) + NB_SLOTS converted A tiles
+  // + the stages of raw fp32 A chunks (and streamed bf16 weight tiles)
+  a.resident = (N <= 128 && (nchunks + NB_SLOTS + 2 * 2) * TILE <= SMEM_BUDGET) ? 1 : 0;
+  const int fixed = ((a.resident ? nchunks : 0) + NB_SLOTS) * TILE;
+  const int stage = a.resident ? 2 * TILE : 3 * TILE;
+  a.ns = min(MAXS, (SMEM_BUDGET - fixed) / stage);
+  const long long ntiles = (long long)cdiv(M, 128) * cdiv(N, 128);
+  const size_t smem = (size_t)fixed + (size_t)a.ns * stage + 1024;
+  REGT_CUDA(cudaFuncSetAttribute(k_gemm_nt_bf16, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k_gemm_nt_bf16<<<(int)min(ntiles, (long long)sm_count()), NT_THREADS, smem, st>>>(a);
+  REGT_LAUNCHED("k_gemm_nt_bf16", st);
+  return 0;
+}
 
 // C[M][N] = A[M][K] . Bt[N][K]^T for any M >= 1 (TMA zero-fills the rows of the last tile past M; they are not stored);
 // `scratch` (gemm_nt_scratch_floats(N, K) floats) receives the hi / lo images of Bt.
+// kind Bf16: the single-pass bf16 kernel (scratch: gemm_nt_bf16_scratch_floats(N, K) floats, the bf16 image of Bt).
 int launch_gemm_nt_tma(const float* A, long long lda, const float* Bt, long long ldb, float* C, long long ldc, long long M, int N,
-                       int K, float* scratch, cudaStream_t st) {
+                       int K, float* scratch, cudaStream_t st, GemmKind kind) {
   REGT_CHECK(A && Bt && C && scratch && M >= 1 && N > 0 && N % 16 == 0 && K > 0 && K % 4 == 0 && ldc % 4 == 0 &&
                  ((uintptr_t)C % 16) == 0 && ((uintptr_t)scratch % 16) == 0,
              "gemm_nt_tma: bad operands (M=%lld N=%d K=%d)", M, N, K);
+  if (kind == GemmKind::Bf16) return launch_gemm_nt_bf16(A, lda, Bt, ldb, C, ldc, M, N, K, scratch, st);
   const int Np = (N + 127) / 128 * 128, Kp = (K + KC - 1) / KC * KC, nchunks = Kp / KC;
   float* hi = scratch;
   float* lo = scratch + (size_t)Np * Kp;
@@ -778,14 +1215,16 @@ int launch_gemm_nt_tma(const float* A, long long lda, const float* Bt, long long
 // One launch of the row contraction over several column segments of A (each K-tile of 128 columns belongs to one segment):
 //   seg s: Cs[z][k1-k0][N] = partials of A[:, k0:k1]^T . B_s      (B_s = Bs[seg_b[s]], or none when seg_b[s] < 0)
 //   and, for every segment, C2[z][k0:k1][32] = partials of A[:, k0:k1]^T . B2.
-// Segment boundaries must be multiples of 128 unless there is a single segment.
+// Segment boundaries must be multiples of 128 unless there is a single segment.  kind Bf16: the single-pass bf16 kernel.
 int launch_gemm_tn_tma(const float* A, long long lda, long long M, int Ktot, int nseg, const int* seg_k0, const int* seg_b,
                        float* const* seg_C, const float* const* Bs, const long long* ldbs, int N, int splits, const float* B2,
-                       long long ldb2, float* C2, long long c2_split, cudaStream_t st, int relu_b) {
+                       long long ldb2, float* C2, long long c2_split, cudaStream_t st, int relu_b, GemmKind kind) {
   REGT_CHECK(A && nseg >= 1 && nseg <= 4 && Ktot % 32 == 0 && N % 32 == 0 && splits > 0 && M >= 1, "gemm_tn_tma: bad shape");
   REGT_CHECK(!B2 || (C2 && ldb2 % 4 == 0), "gemm_tn_tma: bad second operand");
+  const bool bf16 = kind == GemmKind::Bf16;
+  const int kc = bf16 ? KB : KC;   // rows per chunk = rows of a TMA box
   TnArgs a{};
-  if (tmap_2d(&a.ta, A, Ktot, M, lda, 32, "gemm_tn_tma(A)")) return -1;
+  if (tmap_2d(&a.ta, A, Ktot, M, lda, kc, "gemm_tn_tma(A)")) return -1;
   bool any_b = false;
   for (int s = 0; s < nseg; ++s) {
     a.seg[s].k0 = seg_k0[s];
@@ -799,22 +1238,30 @@ int launch_gemm_tn_tma(const float* A, long long lda, long long M, int Ktot, int
   for (int b = 0; b < 2; ++b) {
     bool used = false;
     for (int s = 0; s < nseg; ++s) used |= seg_b[s] == b;
-    if (used && tmap_2d(&a.tb[b], Bs[b], N, M, ldbs[b], 32, "gemm_tn_tma(B)")) return -1;
+    if (used && tmap_2d(&a.tb[b], Bs[b], N, M, ldbs[b], kc, "gemm_tn_tma(B)")) return -1;
   }
   REGT_CHECK(any_b || B2, "gemm_tn_tma: nothing to contract with");
-  if (B2 && tmap_2d(&a.tf, B2, 32, M, ldb2, 32, "gemm_tn_tma(B2)")) return -1;
+  if (B2 && tmap_2d(&a.tf, B2, 32, M, ldb2, kc, "gemm_tn_tma(B2)")) return -1;
   a.nseg = nseg;
   a.C2 = C2;
   a.c2_split = c2_split > 0 ? c2_split : (long long)Ktot * 32;
   a.M = M;
   long long chunk = (M + splits - 1) / splits;
-  a.chunk = (chunk + KC - 1) / KC * KC;
+  a.chunk = (chunk + kc - 1) / kc * kc;
   a.N = any_b ? N : 0;
   a.N2 = B2 ? 32 : 0;
   a.relu_b = relu_b;
+  const dim3 grid(cdiv(Ktot, 128), max(1, cdiv(a.N, 128)), splits);
+  if (bf16) {
+    const size_t smem = (size_t)TN_NR * TB_RAW + (size_t)TN_NC * TB_CV + 1024;
+    REGT_CUDA(cudaFuncSetAttribute(k_gemm_tn_bf16, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k_gemm_tn_bf16<<<grid, TN_THREADS, smem, st>>>(a);
+    REGT_LAUNCHED("k_gemm_tn_bf16", st);
+    return 0;
+  }
   const size_t smem = (size_t)TN_NR * TN_RAW + (size_t)TN_NC * TN_CV + 1024;
   REGT_CUDA(cudaFuncSetAttribute(k_gemm_tn_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  k_gemm_tn_tma<<<dim3(cdiv(Ktot, 128), max(1, cdiv(a.N, 128)), splits), TN_THREADS, smem, st>>>(a);
+  k_gemm_tn_tma<<<grid, TN_THREADS, smem, st>>>(a);
   REGT_LAUNCHED("k_gemm_tn_tma", st);
   return 0;
 }
@@ -858,12 +1305,12 @@ int launch_gemm_kt(const float* AT, long long ntile, int Ktot, int nseg, const i
 
 // the single-segment form of launch_gemm_tn_tma: Cp[z][K][N] = partials of A[:, :K]^T . B (no B when N == 0)
 int launch_gemm_tn(const float* A, long long lda, const float* B, long long ldb, float* Cp, long long M, int K, int N, int splits,
-                   cudaStream_t st, const float* B2, long long ldb2, float* Cp2, long long c2_split, int relu_b) {
+                   cudaStream_t st, const float* B2, long long ldb2, float* Cp2, long long c2_split, int relu_b, GemmKind kind) {
   const int k0 = 0, sb = N > 0 ? 0 : -1;
   float* cs[1] = {Cp};
   const float* bs[2] = {B, nullptr};
   const long long lds[2] = {ldb, 0};
-  return launch_gemm_tn_tma(A, lda, M, K, 1, &k0, &sb, cs, bs, lds, N, splits, B2, ldb2, Cp2, c2_split, st, relu_b);
+  return launch_gemm_tn_tma(A, lda, M, K, 1, &k0, &sb, cs, bs, lds, N, splits, B2, ldb2, Cp2, c2_split, st, relu_b, kind);
 }
 
 }  // namespace regt
@@ -877,6 +1324,16 @@ extern "C" int regt_debug_gemm_tn_tma(const float* A, int64_t lda, const float* 
                                       int32_t N, int32_t splits, const float* B2, int64_t ldb2, float* Cp2, regt_stream_t stream) {
   return regt::launch_gemm_tn(A, lda, B, ldb, Cp, M, K, N, splits, (cudaStream_t)stream, B2, ldb2, Cp2, 0, 0);
 }
+// the single-pass bf16 forms of the two hooks above (tests/test_gpu_bf16_widths.py); scratch: gemm_nt_bf16_scratch_floats(N, K)
+// floats, which the tf32 hook's scratch size covers
+extern "C" int regt_debug_gemm_nt_bf16(const float* A, int64_t lda, const float* Bt, int64_t ldb, float* C, int64_t ldc, int64_t M,
+                                       int32_t N, int32_t K, float* scratch, regt_stream_t stream) {
+  return regt::launch_gemm_nt_tma(A, lda, Bt, ldb, C, ldc, M, N, K, scratch, (cudaStream_t)stream, regt::GemmKind::Bf16);
+}
+extern "C" int regt_debug_gemm_tn_bf16(const float* A, int64_t lda, const float* B, int64_t ldb, float* Cp, int64_t M, int32_t K,
+                                       int32_t N, int32_t splits, const float* B2, int64_t ldb2, float* Cp2, regt_stream_t stream) {
+  return regt::launch_gemm_tn(A, lda, B, ldb, Cp, M, K, N, splits, (cudaStream_t)stream, B2, ldb2, Cp2, 0, 0, regt::GemmKind::Bf16);
+}
 // four-segment form used by the cell backward: A = D [M][4H]; segments z|r (B = h), h~ (B = hR), h_pre (B2 only)
 extern "C" int regt_debug_gemm_tn_multi(const float* A, int64_t lda, int64_t M, int32_t H, const float* B0, const float* B1,
                                         float* C0, float* C1, int32_t splits, const float* B2, float* C2, regt_stream_t stream) {
@@ -885,6 +1342,15 @@ extern "C" int regt_debug_gemm_tn_multi(const float* A, int64_t lda, int64_t M, 
   const float* bs[2] = {B0, B1};
   const long long lds[2] = {H, H};
   return regt::launch_gemm_tn_tma(A, lda, M, 4 * H, 3, k0, sb, cs, bs, lds, H, splits, B2, 32, C2, 0, (cudaStream_t)stream, 0);
+}
+extern "C" int regt_debug_gemm_tn_multi_bf16(const float* A, int64_t lda, int64_t M, int32_t H, const float* B0, const float* B1,
+                                             float* C0, float* C1, int32_t splits, const float* B2, float* C2, regt_stream_t stream) {
+  const int k0[3] = {0, 2 * H, 3 * H}, sb[3] = {0, 1, -1};
+  float* cs[3] = {C0, C1, nullptr};
+  const float* bs[2] = {B0, B1};
+  const long long lds[2] = {H, H};
+  return regt::launch_gemm_tn_tma(A, lda, M, 4 * H, 3, k0, sb, cs, bs, lds, H, splits, B2, 32, C2, 0, (cudaStream_t)stream, 0,
+                                  regt::GemmKind::Bf16);
 }
 // the transposed-tile form used by the fused cell backward: AT [ntile][4][4H][32]; B0T, B1T [ntile][4][H][32]; FT [ntile][4][32][32]
 extern "C" int regt_debug_gemm_kt(const float* AT, int64_t ntile, int32_t H, const float* B0T, const float* B1T, const float* FT,

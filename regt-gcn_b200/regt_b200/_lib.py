@@ -155,8 +155,14 @@ def load() -> C.CDLL:
     lib.regt_debug_gemm_tn_tma.restype = C.c_int
     lib.regt_debug_gemm_tn_tma.argtypes = [vp, C.c_int64, vp, C.c_int64, vp, C.c_int64, C.c_int32, C.c_int32, C.c_int32,
                                            vp, C.c_int64, vp, vp]
+    lib.regt_debug_gemm_nt_bf16.restype = C.c_int
+    lib.regt_debug_gemm_nt_bf16.argtypes = lib.regt_debug_gemm_nt_tma.argtypes
+    lib.regt_debug_gemm_tn_bf16.restype = C.c_int
+    lib.regt_debug_gemm_tn_bf16.argtypes = lib.regt_debug_gemm_tn_tma.argtypes
     lib.regt_debug_gemm_tn_multi.restype = C.c_int
     lib.regt_debug_gemm_tn_multi.argtypes = [vp, C.c_int64, C.c_int64, C.c_int32, vp, vp, vp, vp, C.c_int32, vp, vp, vp]
+    lib.regt_debug_gemm_tn_multi_bf16.restype = C.c_int
+    lib.regt_debug_gemm_tn_multi_bf16.argtypes = lib.regt_debug_gemm_tn_multi.argtypes
     lib.regt_debug_spmm_partition_host.restype = C.c_int
     lib.regt_debug_spmm_partition_host.argtypes = [vp, vp, C.c_int32, C.c_int32, vp, c_i32p, vp]
     lib.regt_debug_gemm_kt.restype = C.c_int
