@@ -170,8 +170,9 @@ typedef struct regt_args {
   regt_params g;          /* parameter gradients (same layouts; any may be NULL)          */
   float* out_hidden;      /* [B,N,H]  cell output (pre-ReLU), models/RegionalTemporalGCN.py:34 */
   float* out;             /* [B,N,O]                                                      */
-  float* loss;            /* [1]  sum_b mean_{n,o} (out-y)^2   (run.py:180)                */
-  float* d_out;           /* [B,N,O]  gradient of loss wrt out (in/out)                   */
+  float* loss;            /* [1]  sum_b mean_{n,o} l(out-y)  (run.py:180; l = loss_kind); with loss_masked the mean of  */
+                          /*    snapshot b runs over its valid targets only: sum_b [c_b > 0] sum_{n,o} m l / c_b        */
+  float* d_out;           /* [B,N,O]  gradient of loss wrt out (in/out); with loss_masked m l' / c_b (0 where c_b = 0)  */
   float* d_hidden;        /* [B,N,H]  extra gradient flowing into out_hidden, or NULL     */
   float* d_h_ext;         /* REGT_MODE_TGCN: [B,N,T,H] gradient wrt h_ext, or NULL        */
   void* workspace;        /* regt_workspace_bytes(args) bytes, preserved fwd -> bwd       */
@@ -181,7 +182,17 @@ typedef struct regt_args {
                           /*    their gradients have this width; the kernels work at REGT_F with the features and   */
                           /*    weight columns F..REGT_F-1 written as zeros, so the result is that of the REGT_F-wide */
                           /*    model on zero-padded x and weights                                                  */
+  int32_t loss_kind;      /* REGT_LOSS_*: l = (out-y)^2, l' = 2(out-y) (MSE, 0) or l = |out-y|, l' = sign(out-y) (MAE)  */
+  int32_t loss_masked;    /* 1: target y[b,n,o] is missing when it equals loss_null or is NaN; m = 0 there, else 1.     */
+                          /*    0: no mask (a NaN in y propagates).  The kernels run their unmasked MSE code unchanged  */
+                          /*    when loss_kind = 0 and loss_masked = 0                                                 */
+  float loss_null;        /* the value that marks a missing target (NaN: only NaNs are missing)                        */
+  const float* loss_count;/* [B] valid count c_b of each snapshot over ALL nodes of the graph (region shards: the full   */
+                          /*    graph's counts), or NULL: counted over rows [0,N) of y on the device                   */
 } regt_args;
+
+#define REGT_LOSS_MSE 0
+#define REGT_LOSS_MAE 1
 
 size_t regt_workspace_bytes(const regt_args* a);
 
@@ -273,6 +284,11 @@ int regt_rmsprop_step(float* params, const float* grads, float* square_avg, int6
                       float weight_decay, regt_stream_t stream);
 int regt_eval_metrics(const float* out, const float* y, int32_t B, int64_t n_per_snapshot, double q, double* sums,
                       regt_stream_t stream);
+/* regt_eval_metrics over the valid targets only (y != null_value and not NaN; null_value NaN: only NaNs are missing):
+ *   sums[b] = { valid count c_b, sum m|y-out|, sum m (y-out)^2, percentile q of the valid y_b, sum m|y-out| / percentile }
+ * as doubles [B][5]; a snapshot with c_b = 0 gives {0, 0, 0, NaN, NaN}.                                                   */
+int regt_eval_metrics_masked(const float* out, const float* y, int32_t B, int64_t n_per_snapshot, double q, float null_value,
+                             double* sums, regt_stream_t stream);
 
 int regt_version(void);
 const char* regt_last_error(void);

@@ -123,6 +123,11 @@ Layout make_layout(const regt_args* a, void* base) {
   L.part_floats = pf;
   if (feat_in(a) < F && (L.route.cell == CellPath::Fp32 || L.route.cell == CellPath::Tf32x3Unfused || L.route.cell == CellPath::Bf16Gemm))
     L.xw = c.take<float>((size_t)a->B * (a->x_rows > 0 ? a->x_rows : a->N) * F * T);
+  // whenever y is set, masked or not: changing a step's loss never grows (and so never re-allocates) its workspace
+  if (a->y) {
+    L.inv_c = c.take<float>(a->B);
+    L.lc_part = c.take<unsigned int>((size_t)a->B * LC_CHUNKS);
+  }
   L.m1cp = c.take<int32_t>(R + 2);   // last: tests locate it from the end of the workspace
   L.total = align_up(c.off, 256);
   return L;
@@ -149,6 +154,9 @@ static int validate(const regt_args* a, const char* who) {
   REGT_CHECK(a->B > 0 && a->N > 0 && a->T > 0 && a->O > 0, "%s: bad dims B=%d N=%d T=%d O=%d", who, a->B, a->N, a->T, a->O);
   REGT_CHECK(a->H >= 8 && a->H % 8 == 0 && a->H <= 1024, "%s: H=%d must be a multiple of 8 in [8,1024]", who, a->H);
   REGT_CHECK(a->mode >= 0 && a->mode <= 2, "%s: bad mode %d", who, a->mode);
+  REGT_CHECK(a->loss_kind == REGT_LOSS_MSE || a->loss_kind == REGT_LOSS_MAE, "%s: bad loss_kind %d (0 = MSE, 1 = MAE)", who,
+             a->loss_kind);
+  REGT_CHECK(!a->loss_masked || a->y, "%s: loss_masked needs y (the mask is read from the targets)", who);
   REGT_CHECK(a->x_rows == 0 || a->x_rows >= a->N, "%s: x_rows=%d must be 0 or >= N=%d", who, a->x_rows, a->N);
   REGT_CHECK(a->plan.N == a->N, "%s: plan built for %d nodes, args say %d", who, a->plan.N, a->N);
   REGT_CHECK((long long)a->B * a->N * a->T < (1ll << 31), "%s: B*N*T overflows int32 rows", who);

@@ -75,6 +75,38 @@ __device__ __forceinline__ size_t g_off(long long q, int n, int H, int tiled) {
   return tiled ? ((((size_t)(q >> 7) * (H >> 2) + (n >> 2)) * 128 + (size_t)(q & 127)) * 4 + (n & 3)) : ((size_t)q * H + n);
 }
 
+// ---- loss of the head kernels (regt_args.loss_kind / loss_masked / loss_null / loss_count) ---------------------------
+// Every head kernel is instantiated twice: LX = false is the unmasked MSE of run.py:180 with its arithmetic unchanged;
+// LX = true reads the loss kind and the mask from a LossX (uniform branches) and scales each row by its snapshot's
+// 1 / valid count.  Its loss is accumulated in two sums: `lu` for rows whose scale equals the unmasked one (multiplied
+// once at the end, as the unmasked kernel does) and `ls` for the others (scaled per element), so a mask that finds no
+// missing target gives the unmasked result bit for bit.
+struct LossX {
+  int mae;             // 0: (out - y)^2, 1: |out - y|
+  int masked;          // 1: a target equal to null_v, or NaN, is missing
+  float null_v;
+  const float* inv_c;  // [B] 1 / valid count of each snapshot (0 when it has none), or NULL: the unmasked scale
+  int N;               // rows per snapshot of this call: row q belongs to snapshot q / N
+};
+__device__ __forceinline__ float lossx_inv(const LossX& L, long long q, float scale) {
+  return L.inv_c ? __ldg(L.inv_c + q / L.N) : scale;
+}
+// one target: adds its loss to lu or ls and returns d_out = m * l'(out - y) * inv
+__device__ __forceinline__ float lossx_elem(const LossX& L, float v, float yv, float inv, float scale, float& lu, float& ls) {
+  const bool keep = !L.masked || (yv == yv && yv != L.null_v);
+  const float diff = keep ? v - yv : 0.f;
+  if (L.mae) {
+    const float l = fabsf(diff);
+    if (inv == scale) lu += l;
+    else ls = fmaf(l, inv, ls);
+    return (diff > 0.f ? 1.f : diff < 0.f ? -1.f : diff) * inv;   // sign, 0 at 0 (torch's abs backward); NaN stays NaN
+  }
+  if (inv == scale) lu = fmaf(diff, diff, lu);
+  else ls = fmaf(diff * diff, inv, ls);
+  return 2.0f * diff * inv;
+}
+inline bool loss_ext(const regt_args* a) { return a->y && (a->loss_kind != REGT_LOSS_MSE || a->loss_masked); }
+
 // multiprocessor count of the current device (148 when it cannot be read)
 inline int sm_count() {
   static int n = 0;
@@ -164,9 +196,12 @@ struct Layout {
   float* tc_dpp;             // [T * nqt] attention-gradient partials
   float* xw;                 // [B][x_rows][REGT_F][T]  x widened with zero features (fp32 / unfused tf32x3 paths when the
                              // caller's F < REGT_F; written by every forward, read by its backward), else NULL
+  float* inv_c;              // [B] 1 / valid count per snapshot (loss_masked), written by k_loss_inv; NULL without y
+  unsigned int* lc_part;     // [B][LC_CHUNKS] valid counts of each snapshot's chunks (k_loss_count); NULL without y
   size_t total;
 };
 constexpr int TC_MAX_CTAS = 160;
+constexpr int LC_CHUNKS = 64;     // most blocks k_loss_count gives one snapshot
 constexpr int TC_IMG_BYTES = 160 * 1024;
 constexpr int F_IMG_BYTES = 432 * 1024;   // fused 3xTF32 cell (cell_f.cu): 12 ring stages of 32 KB + F-wide weights + constants at H = 128
 
@@ -197,6 +232,7 @@ int head_backward(const regt_args* a, const Layout& L, cudaStream_t st);
 int head_forward_f(const regt_args* a, const Layout& L, cudaStream_t st);       // head_f.cu
 int head_backward_f(const regt_args* a, const Layout& L, cudaStream_t st);
 int head_forward_tc(const regt_args* a, const Layout& L, cudaStream_t st);      // head_tc.cu
+LossX make_lossx(const regt_args* a, const Layout& L);                          // head.cu: the LossX of an LX head kernel
 
 // weights.cu: collapsed weights before the cell, chain rule back to the parameters after it
 int launch_prep(const regt_args* a, const Layout& L, cudaStream_t st);

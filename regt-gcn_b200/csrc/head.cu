@@ -1,6 +1,7 @@
 // Decoder head of RegionalTemporalGCN / TemporalGCN and the call-site loss:
 //   out = linear2(relu(linear1(relu(out_hidden))))      models/RegionalTemporalGCN.py:35-38
 //   loss = sum_b mean_{n,o} (out - y)^2                 run.py:180 (one backward per snapshot)
+//          (or the MAE, or either over the valid targets only: LossX, common.cuh)
 // plus their autograd (run.py:190).  One row per (b, n); tiny next to the cell.
 #include "gemm_simt.cuh"
 
@@ -19,6 +20,7 @@ struct HeadK {
   int ntc, nqt;
   float* hid_out;         // where the summed out_hidden goes when hid_part is used
   int g_tiled;            // 1: G is written as [qt][H/4][128][4] tiles (tensor-core backward), 0: row-major
+  LossX lx;               // loss kind and mask of the LX instantiations
 };
 
 __global__ void k_head_transpose(const float* __restrict__ w1, const float* __restrict__ w2, int H, int O,
@@ -34,6 +36,7 @@ __global__ void k_head_transpose(const float* __restrict__ w1, const float* __re
   }
 }
 
+template <bool LX>
 __global__ void __launch_bounds__(TMH * 4) k_head_fwd(HeadK a) {
   constexpr int NT = TMH * 4;
   extern __shared__ __align__(16) float smem[];
@@ -66,7 +69,7 @@ __global__ void __launch_bounds__(TMH * 4) k_head_fwd(HeadK a) {
       }
     }
   }
-  float lsum = 0.f;
+  float lsum = 0.f, lsc = 0.f;
   const float scale = 1.0f / ((float)a.N * (float)O);
   for (int n0 = 0; n0 < O; n0 += TN) {
     float acc[4][4];
@@ -76,6 +79,8 @@ __global__ void __launch_bounds__(TMH * 4) k_head_fwd(HeadK a) {
     for (int i = 0; i < 4; ++i) {
       const long long q = q0 + ty * 4 + i;
       if (q >= a.BN) continue;
+      float inv = scale;
+      if constexpr (LX) inv = lossx_inv(a.lx, q, scale);
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
         const int n = n0 + tx * 4 + j;
@@ -83,16 +88,25 @@ __global__ void __launch_bounds__(TMH * 4) k_head_fwd(HeadK a) {
         const float v = acc[i][j] + __ldg(a.b2 + n);
         a.out[q * O + n] = v;
         if (a.y) {
-          const float diff = v - __ldg(a.y + q * O + n);
-          lsum = fmaf(diff, diff, lsum);
-          a.d_out[q * O + n] = 2.0f * diff * scale;
+          if constexpr (LX) {
+            a.d_out[q * O + n] = lossx_elem(a.lx, v, __ldg(a.y + q * O + n), inv, scale, lsum, lsc);
+          } else {
+            const float diff = v - __ldg(a.y + q * O + n);
+            lsum = fmaf(diff, diff, lsum);
+            a.d_out[q * O + n] = 2.0f * diff * scale;
+          }
         }
       }
     }
   }
   if (a.y) {
     lsum = block_sum(lsum, red);
-    if (tid == 0) a.loss_part[blockIdx.x] = lsum * scale;
+    if constexpr (LX) {
+      lsc = block_sum(lsc, red);
+      if (tid == 0) a.loss_part[blockIdx.x] = lsum * scale + lsc;
+    } else {
+      if (tid == 0) a.loss_part[blockIdx.x] = lsum * scale;
+    }
   }
 }
 
@@ -166,7 +180,7 @@ constexpr int HP_MAX_CTAS = 148;
 // multiple of 4 floats: the tensor-core head writes its dW1 partial with 16-byte stores
 __host__ __device__ inline int head_part_stride(int H, int O) { return (HEAD_HID * H + O * HEAD_HID + HEAD_HID + O + 4 + 3) & ~3; }
 
-template <int H>
+template <int H, bool LX>
 __global__ void __launch_bounds__(256, 1) k_head_fused(HeadK a, float* __restrict__ hpart, int ntiles) {
   constexpr int HJ = H / 16;             // dW1 columns per thread
   constexpr int LDA = H + 4, LD1 = HEAD_HID + 4;
@@ -202,7 +216,7 @@ __global__ void __launch_bounds__(256, 1) k_head_fused(HeadK a, float* __restric
   for (int i = 0; i < 8; ++i)
 #pragma unroll
     for (int j = 0; j < HJ; ++j) dw1[i][j] = 0.f;
-  float dbias = 0.f, lsum = 0.f;
+  float dbias = 0.f, lsum = 0.f, lsc = 0.f;
   const float scale = 1.0f / ((float)a.N * (float)O);
   __syncthreads();
 
@@ -272,6 +286,8 @@ __global__ void __launch_bounds__(256, 1) k_head_fused(HeadK a, float* __restric
       for (int i = 0; i < 4; ++i) {
         const int rl = ty * 4 + i;
         const long long q = q0 + rl;
+        float inv = scale;
+        if constexpr (LX) inv = q < a.BN ? lossx_inv(a.lx, q, scale) : scale;
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           const int n = n0 + tx * 4 + j;
@@ -280,9 +296,13 @@ __global__ void __launch_bounds__(256, 1) k_head_fused(HeadK a, float* __restric
           if (n < O && q < a.BN) {
             const float v = acc[i][j] + __ldg(a.b2 + n);
             a.out[q * O + n] = v;
-            const float diff = v - __ldg(a.y + q * O + n);
-            lsum = fmaf(diff, diff, lsum);
-            dv = 2.0f * diff * scale;
+            if constexpr (LX) {
+              dv = lossx_elem(a.lx, v, __ldg(a.y + q * O + n), inv, scale, lsum, lsc);
+            } else {
+              const float diff = v - __ldg(a.y + q * O + n);
+              lsum = fmaf(diff, diff, lsum);
+              dv = 2.0f * diff * scale;
+            }
             a.d_out[q * O + n] = dv;
           }
           Do[rl * LDO + n] = dv;
@@ -383,7 +403,12 @@ __global__ void __launch_bounds__(256, 1) k_head_fused(HeadK a, float* __restric
   if (tid < HEAD_HID) hp[HEAD_HID * H + O * HEAD_HID + tid] = dbias;
   else if (tid - HEAD_HID < O) hp[HEAD_HID * H + O * HEAD_HID + HEAD_HID + tid - HEAD_HID] = dbias;
   lsum = block_sum(lsum, red);
-  if (tid == 0) hp[HEAD_HID * H + O * HEAD_HID + HEAD_HID + O] = lsum * scale;
+  if constexpr (LX) {
+    lsc = block_sum(lsc, red);
+    if (tid == 0) hp[HEAD_HID * H + O * HEAD_HID + HEAD_HID + O] = lsum * scale + lsc;
+  } else {
+    if (tid == 0) hp[HEAD_HID * H + O * HEAD_HID + HEAD_HID + O] = lsum * scale;
+  }
 }
 
 // sums the per-CTA partials into the head gradients; the slot after the gradients is the loss
@@ -433,6 +458,7 @@ static HeadK make_headk(const regt_args* a, const Layout& L, float* W1t, float* 
   k.a1 = L.a1; k.out = a->out; k.d_out = a->d_out; k.loss_part = L.part; k.d_a1 = L.d_a1; k.G = L.G;
   k.hid_part = nullptr; k.ntc = 0; k.hid_out = a->out_hidden;
   k.g_tiled = L.route.g_tiled;
+  k.lx = make_lossx(a, L);
   if (L.route.hid_partials) {  // the cell left per-chunk partials (see cell_tc.cu)
     k.hid_part = L.hid_part;
     k.ntc = tc_num_chunks(a);
@@ -441,8 +467,65 @@ static HeadK make_headk(const regt_args* a, const Layout& L, float* W1t, float* 
   return k;
 }
 
+// valid targets among rows [0, N) of y, counted as integers (exact in any order): block (chunk, b) writes the count of
+// its slice of snapshot b to part[b][chunk]; k_loss_inv sums a snapshot's chunks and writes inv_c[b] = 1 / c_b (0 when
+// c_b = 0), or takes c_b from the caller's counts
+__global__ void __launch_bounds__(256) k_loss_count(const float* __restrict__ y, long long n, float null_v,
+                                                    unsigned int* __restrict__ part) {
+  __shared__ unsigned int red[8];
+  const float* yb = y + (size_t)blockIdx.y * n;
+  unsigned int k = 0;
+  for (long long i = blockIdx.x * 256ll + threadIdx.x; i < n; i += (long long)gridDim.x * 256) {
+    const float v = __ldg(yb + i);
+    k += (v == v && v != null_v) ? 1u : 0u;
+  }
+  for (int d = 16; d > 0; d >>= 1) k += __shfl_xor_sync(0xffffffffu, k, d);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = k;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    unsigned int s = 0;
+    for (int w = 0; w < 8; ++w) s += red[w];
+    part[(size_t)blockIdx.y * gridDim.x + blockIdx.x] = s;
+  }
+}
+__global__ void k_loss_inv(const unsigned int* __restrict__ part, int nchunks, const float* __restrict__ given, int B,
+                           float* __restrict__ inv_c) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  float c;
+  if (given) {
+    c = given[b];
+  } else {
+    unsigned long long k = 0;
+    for (int i = 0; i < nchunks; ++i) k += part[(size_t)b * nchunks + i];
+    c = (float)k;
+  }
+  inv_c[b] = c > 0.f ? 1.0f / c : 0.f;
+}
+
+LossX make_lossx(const regt_args* a, const Layout& L) {
+  LossX x{};
+  x.mae = a->loss_kind == REGT_LOSS_MAE;
+  x.masked = a->loss_masked != 0;
+  x.null_v = a->loss_null;
+  x.inv_c = a->loss_masked ? L.inv_c : nullptr;
+  x.N = a->N;
+  return x;
+}
+
 int head_forward(const regt_args* a, const Layout& L, cudaStream_t st) {
   const int H = a->H, O = a->O;
+  if (a->y && a->loss_masked) {
+    const long long n = (long long)a->N * O;
+    const int nchunks = (int)min((long long)LC_CHUNKS, (n + 2047) / 2048);
+    unsigned int* part = L.lc_part;
+    if (!a->loss_count) {
+      k_loss_count<<<dim3(nchunks, a->B), 256, 0, st>>>(a->y, n, a->loss_null, part);
+      REGT_LAUNCHED("k_loss_count", st);
+    }
+    k_loss_inv<<<cdiv(a->B, 128), 128, 0, st>>>(part, nchunks, a->loss_count, a->B, L.inv_c);
+    REGT_LAUNCHED("k_loss_inv", st);
+  }
   switch (L.route.head) {
     case HeadPath::Bf16: return head_forward_tc(a, L, st);
     case HeadPath::Tf32x3: return head_forward_f(a, L, st);   // the 128-wide GEMMs on the tensor cores (head_f.cu)
@@ -450,13 +533,10 @@ int head_forward(const regt_args* a, const Layout& L, cudaStream_t st) {
       HeadK k = make_headk(a, L, nullptr, nullptr);
       const int grid = head_fused_grid(a), ntiles = cdiv(k.BN, TMH);
       const size_t smem = head_fused_smem(H, O);
-      if (H == 64) {
-        REGT_CUDA(cudaFuncSetAttribute(k_head_fused<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_head_fused<64><<<grid, 256, smem, st>>>(k, L.hpart, ntiles);
-      } else {
-        REGT_CUDA(cudaFuncSetAttribute(k_head_fused<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_head_fused<32><<<grid, 256, smem, st>>>(k, L.hpart, ntiles);
-      }
+      auto kern = H == 64 ? (loss_ext(a) ? k_head_fused<64, true> : k_head_fused<64, false>)
+                          : (loss_ext(a) ? k_head_fused<32, true> : k_head_fused<32, false>);
+      REGT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      kern<<<grid, 256, smem, st>>>(k, L.hpart, ntiles);
       REGT_LAUNCHED("k_head_fused", st);
       return 0;   // loss and head gradients are finalised by k_head_grad_reduce in regt_head_backward
     }
@@ -471,8 +551,9 @@ int head_forward(const regt_args* a, const Layout& L, cudaStream_t st) {
   HeadK k = make_headk(a, L, W1t, W2t);
   const int nblk = cdiv(k.BN, TMH);
   const size_t smem = ((size_t)TMH * (H + 1) + TMH * (HEAD_HID + 1) + KT * TN) * sizeof(float);
-  REGT_CUDA(cudaFuncSetAttribute(k_head_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  k_head_fwd<<<nblk, TMH * 4, smem, st>>>(k);
+  auto kern = loss_ext(a) ? k_head_fwd<true> : k_head_fwd<false>;
+  REGT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<nblk, TMH * 4, smem, st>>>(k);
   REGT_LAUNCHED("k_head_fwd", st);
   if (a->y) {
     REGT_CHECK(a->loss && a->d_out, "head_forward: y given but loss/d_out is NULL");

@@ -5,7 +5,7 @@
 //   forward   rh = relu(hid)                                k_hf_relu
 //             a1pre = rh . W1^T                             gemm_nt (tensor cores)
 //             a1 = relu(a1pre + b1); out = a1 . W2^T + b2;  k_hf_mid   (warp per row; O <= 16 outputs through shuffles)
-//             loss = sum (out - y)^2 / (N O), d_out         (run.py:180)
+//             loss = sum (out - y)^2 / (N O), d_out         (run.py:180; or the MAE / a masked mean: LossX, common.cuh)
 //   backward  d_a1 = (d_out . W2) * (a1 > 0); [d_out | 1] plane     k_hf_da1   (warp per row)
 //             Gpre = d_a1 . W1                              gemm_nt (tensor cores)
 //             G = Gpre * (hid > 0) + d_hidden               k_hf_gmask (row major or the tile layout the fused cell reads)
@@ -26,10 +26,12 @@ __global__ void __launch_bounds__(256) k_hf_relu(const float4* __restrict__ hid,
 
 // warp per row; lane owns columns 4*lane .. 4*lane+3 of the 128-wide hidden layer
 constexpr int HF_O = 16;     // output_dim handled by the shuffle reductions
+template <bool LX>
 __global__ void __launch_bounds__(256) k_hf_mid(float* __restrict__ a1, const float* __restrict__ b1, const float* __restrict__ w2,
                                                 const float* __restrict__ b2, const float* __restrict__ y, long long BN, int O, float scale,
-                                                float* __restrict__ out, float* __restrict__ d_out, float* __restrict__ loss_part) {
-  __shared__ float red[8];
+                                                float* __restrict__ out, float* __restrict__ d_out, float* __restrict__ loss_part,
+                                                LossX lx) {
+  __shared__ float red[8], red2[8];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   float w[HF_O][4];
 #pragma unroll
@@ -38,7 +40,7 @@ __global__ void __launch_bounds__(256) k_hf_mid(float* __restrict__ a1, const fl
     w[o][0] = t.x; w[o][1] = t.y; w[o][2] = t.z; w[o][3] = t.w;
   }
   const float4 bb = __ldg(reinterpret_cast<const float4*>(b1) + lane);
-  float lsum = 0.f;
+  float lsum = 0.f, lsc = 0.f;
   // grid-stride over the rows (a bounded number of blocks: the loss partials are summed by one thread per output)
   for (long long q = blockIdx.x * 8ll + warp; q < BN; q += (long long)gridDim.x * 8) {
     const float4 p = reinterpret_cast<const float4*>(a1 + q * HEAD_HID)[lane];
@@ -90,9 +92,13 @@ __global__ void __launch_bounds__(256) k_hf_mid(float* __restrict__ a1, const fl
       const float v = mine + __ldg(b2 + o);
       out[q * O + o] = v;
       if (y) {
-        const float diff = v - __ldg(y + q * O + o);
-        lsum = fmaf(diff, diff, lsum);
-        d_out[q * O + o] = 2.0f * diff * scale;
+        if constexpr (LX) {
+          d_out[q * O + o] = lossx_elem(lx, v, __ldg(y + q * O + o), lossx_inv(lx, q, scale), scale, lsum, lsc);
+        } else {
+          const float diff = v - __ldg(y + q * O + o);
+          lsum = fmaf(diff, diff, lsum);
+          d_out[q * O + o] = 2.0f * diff * scale;
+        }
       }
     }
   }
@@ -100,12 +106,23 @@ __global__ void __launch_bounds__(256) k_hf_mid(float* __restrict__ a1, const fl
 #pragma unroll
     for (int d = 16; d > 0; d >>= 1) lsum += __shfl_xor_sync(0xffffffffu, lsum, d);
     if (lane == 0) red[warp] = lsum;
+    if constexpr (LX) {
+      for (int d = 16; d > 0; d >>= 1) lsc += __shfl_xor_sync(0xffffffffu, lsc, d);
+      if (lane == 0) red2[warp] = lsc;
+    }
     __syncthreads();
     if (threadIdx.x == 0) {
       float s = 0.f;
 #pragma unroll
       for (int i = 0; i < 8; ++i) s += red[i];
-      loss_part[blockIdx.x] = s * scale;
+      if constexpr (LX) {
+        float s2 = 0.f;
+#pragma unroll
+        for (int i = 0; i < 8; ++i) s2 += red2[i];
+        loss_part[blockIdx.x] = s * scale + s2;
+      } else {
+        loss_part[blockIdx.x] = s * scale;
+      }
     }
   }
 }
@@ -178,8 +195,9 @@ int head_forward_f(const regt_args* a, const Layout& L, cudaStream_t st) {
   const int nblk = (int)min((long long)cdiv(BN, 8), 1184ll);      // 8 blocks per SM, grid-stride
   REGT_CHECK(!a->y || (a->loss && a->d_out), "head_forward: y given but loss/d_out is NULL");
   REGT_CHECK(!a->y || (size_t)nblk <= L.hf_loss_floats, "head_forward: loss partial buffer too small");
-  k_hf_mid<<<nblk, 256, 0, st>>>(L.a1, a->p.head_b1, a->p.head_w2, a->p.head_b2, a->y, BN, O, 1.0f / ((float)Nl * (float)O), a->out,
-                                 a->d_out, L.hf_loss);
+  (loss_ext(a) ? k_hf_mid<true> : k_hf_mid<false>)<<<nblk, 256, 0, st>>>(
+      L.a1, a->p.head_b1, a->p.head_w2, a->p.head_b2, a->y, BN, O, 1.0f / ((float)Nl * (float)O), a->out, a->d_out, L.hf_loss,
+      make_lossx(a, L));
   REGT_LAUNCHED("k_hf_mid", st);
   if (a->y) return launch_reduce_splits(L.hf_loss, a->loss, 1, nblk, 0, st);
   return 0;

@@ -8,6 +8,7 @@
 //   P1  CUDA cores : a1 = relu(a1_pre + b1) -> A1 tile
 //   M2  tcgen05.mma: out[128x16] = A1[128x128] . W2^T                       (O <= 16, zero padded)
 //   P2  CUDA cores : out += b2 -> out; diff = out - y; loss; d_out = 2 diff / (N O) -> Do tile
+//                    (or the MAE / a masked mean: LossX, common.cuh, with a scale per row: a tile may span two snapshots)
 //   M3  tcgen05.mma: da1_pre[128x128] = Do[128x16] . W2     ;  dW2^T[128x16] += A1^T . Do   (over rows)
 //   P3  CUDA cores : d a1 = da1_pre * (a1 > 0) -> D1 tile
 //   M4  tcgen05.mma: G_pre[128x64] = D1[128x128] . W1       ;  dW1[128x64] += D1^T . A0 ; db1 += D1^T . 1
@@ -52,6 +53,7 @@ struct HeadTcArgs {
   const float* d_hidden;
   float *out, *d_out, *G, *hpart;
   int part_stride;
+  LossX lx;
 };
 
 __device__ __forceinline__ void put_bf16(uint8_t* base, uint32_t off, float v) {
@@ -59,6 +61,7 @@ __device__ __forceinline__ void put_bf16(uint8_t* base, uint32_t off, float v) {
 }
 }  // namespace
 
+template <bool LX>
 __global__ void __launch_bounds__(NTHREADS, 1) k_head_tc(HeadTcArgs a) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* sm = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -105,7 +108,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_head_tc(HeadTcArgs a) {
     const int r = (warp & 3) * 32 + lane;    // row of the tile = TMEM lane
     const int ch = warp >> 2;                // column half
     const uint32_t tlane = tmem + ((uint32_t)((warp & 3) * 32) << 16);
-    float lsum = 0.f, db2[8];
+    float lsum = 0.f, lsc = 0.f, db2[8];
 #pragma unroll
     for (int j = 0; j < 8; ++j) db2[j] = 0.f;
     for (int i = 0; i < n_my; ++i) {
@@ -194,6 +197,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_head_tc(HeadTcArgs a) {
       {
         float v[8], dv[8];
         tmem_ld8(tlane + C_OUT + ch * 8, v);
+        float inv = a.scale;
+        if constexpr (LX) inv = valid ? lossx_inv(a.lx, q, a.scale) : a.scale;
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
           const int n = ch * 8 + j;
@@ -201,9 +206,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_head_tc(HeadTcArgs a) {
           if (valid && n < O) {
             const float o = v[j] + cb[128 + n];
             a.out[q * O + n] = o;
-            const float diff = o - __ldg(a.y + q * O + n);
-            lsum = fmaf(diff, diff, lsum);
-            dv[j] = 2.0f * diff * a.scale;
+            if constexpr (LX) {
+              dv[j] = lossx_elem(a.lx, o, __ldg(a.y + q * O + n), inv, a.scale, lsum, lsc);
+            } else {
+              const float diff = o - __ldg(a.y + q * O + n);
+              lsum = fmaf(diff, diff, lsum);
+              dv[j] = 2.0f * diff * a.scale;
+            }
             a.d_out[q * O + n] = dv[j];
             db2[j] += dv[j];
           }
@@ -295,6 +304,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_head_tc(HeadTcArgs a) {
 #pragma unroll
     for (int d = 16; d > 0; d >>= 1) {
       lsum += __shfl_down_sync(0xffffffffu, lsum, d);
+      if constexpr (LX) lsc += __shfl_down_sync(0xffffffffu, lsc, d);
 #pragma unroll
       for (int j = 0; j < 8; ++j) db2[j] += __shfl_down_sync(0xffffffffu, db2[j], d);
     }
@@ -302,6 +312,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_head_tc(HeadTcArgs a) {
 #pragma unroll
       for (int j = 0; j < 8; ++j) red[warp][j] = db2[j];
       red[warp][8] = lsum;
+      if constexpr (LX) red[warp][9] = lsc;
     }
     asm volatile("bar.sync 1, %0;" ::"n"(NEPI) : "memory");
     if (tid < OP) {
@@ -312,7 +323,14 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_head_tc(HeadTcArgs a) {
       float s = 0.f;
 #pragma unroll
       for (int w8 = 0; w8 < NEPI_WARPS; ++w8) s += red[w8][8];
-      hp[n1 + n2 + 128 + O] = s * a.scale;
+      if constexpr (LX) {
+        float s2 = 0.f;
+#pragma unroll
+        for (int w8 = 0; w8 < NEPI_WARPS; ++w8) s2 += red[w8][9];
+        hp[n1 + n2 + 128 + O] = s * a.scale + s2;
+      } else {
+        hp[n1 + n2 + 128 + O] = s * a.scale;
+      }
     }
   } else {
     // ================= MMA issuer =================
@@ -407,9 +425,11 @@ int head_forward_tc(const regt_args* a, const Layout& L, cudaStream_t st) {
   k.y = a->y; k.d_hidden = a->d_hidden;
   k.out = a->out; k.d_out = a->d_out; k.G = L.G; k.hpart = L.hpart;
   k.part_stride = head_part_stride_host(a->H, a->O);
+  k.lx = make_lossx(a, L);
   const size_t smem = SMEM_BYTES + 1024;
-  REGT_CUDA(cudaFuncSetAttribute(k_head_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  k_head_tc<<<head_tc_grid(a), NTHREADS, smem, st>>>(k);
+  auto kern = loss_ext(a) ? k_head_tc<true> : k_head_tc<false>;
+  REGT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<head_tc_grid(a), NTHREADS, smem, st>>>(k);
   REGT_LAUNCHED("k_head_tc", st);
   return 0;
 }

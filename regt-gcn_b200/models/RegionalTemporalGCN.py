@@ -78,6 +78,7 @@ class RegionalTemporalGCN(RegTModelBase):
                     KYedge_attr, OHedge_attr, WIedge_attr) + tuple(more)
         return self._run(x, self._plan(x, edge_index, regional))
 
-    def fused_step(self, x, y, edge_index, *regional, micro_batch=None):
-        """forward + MSE loss + backward in one pass (run.py:178-190); grads accumulate in .grad."""
-        return self._fused_step(x, y, self._plan(x, edge_index, regional), micro_batch)
+    def fused_step(self, x, y, edge_index, *regional, micro_batch=None, loss="mse", null_value=None):
+        """forward + MSE loss + backward in one pass (run.py:178-190); grads accumulate in .grad.
+        ``loss="mae"``: mean absolute error; ``null_value``: targets equal to it (or NaN) are missing and left out."""
+        return self._fused_step(x, y, self._plan(x, edge_index, regional), micro_batch, loss=loss, null_value=null_value)

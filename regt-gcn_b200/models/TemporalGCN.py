@@ -56,6 +56,7 @@ class TemporalGCN(RegTModelBase):
         """x = node features for T time steps; returns (h [.,N,O], out_hidden [.,N,H])."""
         return self._run(x, self._plan(x, edge_index, edge_attr))
 
-    def fused_step(self, x, y, edge_index, edge_attr=None, micro_batch=None):
-        """forward + MSE loss + backward in one pass (run.py:188-190); grads accumulate in .grad."""
-        return self._fused_step(x, y, self._plan(x, edge_index, edge_attr), micro_batch)
+    def fused_step(self, x, y, edge_index, edge_attr=None, micro_batch=None, loss="mse", null_value=None):
+        """forward + MSE loss + backward in one pass (run.py:188-190); grads accumulate in .grad.
+        ``loss="mae"``: mean absolute error; ``null_value``: targets equal to it (or NaN) are missing and left out."""
+        return self._fused_step(x, y, self._plan(x, edge_index, edge_attr), micro_batch, loss=loss, null_value=null_value)

@@ -45,10 +45,13 @@ class Args(C.Structure):
                 ("x", vp), ("y", vp), ("h_ext", vp),
                 ("p", Params), ("g", Params),
                 ("out_hidden", vp), ("out", vp), ("loss", vp), ("d_out", vp), ("d_hidden", vp), ("d_h_ext", vp),
-                ("workspace", vp), ("workspace_bytes", C.c_size_t), ("stream", vp), ("F", C.c_int32)]
+                ("workspace", vp), ("workspace_bytes", C.c_size_t), ("stream", vp), ("F", C.c_int32),
+                ("loss_kind", C.c_int32), ("loss_masked", C.c_int32), ("loss_null", C.c_float), ("loss_count", vp)]
 
 
 MODE_A3TGCN, MODE_REGIONAL, MODE_TGCN = 0, 1, 2
+LOSS_MSE, LOSS_MAE = 0, 1
+LOSSES = {"mse": LOSS_MSE, "mae": LOSS_MAE}
 PREC_FP32, PREC_TF32X3, PREC_BF16 = 0, 1, 2
 PRECISIONS = {"fp32": PREC_FP32, "tf32x3": PREC_TF32X3, "bf16": PREC_BF16}
 
@@ -61,7 +64,7 @@ EXPORTS = ["regt_version", "regt_last_error", "regt_launch_count", "regt_plan_wo
            "regt_profile", "regt_profile_begin", "regt_profile_read",
            "regt_comm_region_bytes", "regt_comm_data_offset", "regt_comm_alloc", "regt_comm_free", "regt_comm_export",
            "regt_comm_import", "regt_comm_unimport", "regt_peer_allreduce_f32", "regt_peer_push_max_floats", "regt_comm_error",
-           "regt_window_gather", "regt_rmsprop_step", "regt_eval_metrics"]
+           "regt_window_gather", "regt_rmsprop_step", "regt_eval_metrics", "regt_eval_metrics_masked"]
 
 _lib = None
 
@@ -150,6 +153,8 @@ def load() -> C.CDLL:
     lib.regt_rmsprop_step.argtypes = [vp, vp, vp, C.c_int64, C.c_float, C.c_float, C.c_float, C.c_float, vp]
     lib.regt_eval_metrics.restype = C.c_int
     lib.regt_eval_metrics.argtypes = [vp, vp, C.c_int32, C.c_int64, C.c_double, vp, vp]
+    lib.regt_eval_metrics_masked.restype = C.c_int
+    lib.regt_eval_metrics_masked.argtypes = [vp, vp, C.c_int32, C.c_int64, C.c_double, C.c_float, vp, vp]
     lib.regt_debug_gemm_nt_tma.restype = C.c_int
     lib.regt_debug_gemm_nt_tma.argtypes = [vp, C.c_int64, vp, C.c_int64, vp, C.c_int64, C.c_int64, C.c_int32, C.c_int32, vp, vp]
     lib.regt_debug_gemm_tn_tma.restype = C.c_int

@@ -5,6 +5,7 @@ There is no CPU / eager fallback: non-CUDA tensors raise."""
 from __future__ import annotations
 
 import ctypes as C
+import math
 from typing import Dict, Optional, Sequence
 
 import torch
@@ -84,11 +85,14 @@ def build_state(mode: int, precision: int, plan: GraphPlanTensors, x: torch.Tens
                 params: Dict[str, torch.Tensor], y: Optional[torch.Tensor] = None,
                 h_ext: Optional[torch.Tensor] = None, head: bool = True,
                 workspace: Optional[torch.Tensor] = None, fuse_head: bool = False,
-                loss_nodes: Optional[int] = None, inference: bool = False) -> StepState:
+                loss_nodes: Optional[int] = None, inference: bool = False, loss_kind: int = _lib.LOSS_MSE,
+                null_value: Optional[float] = None, loss_count: Optional[torch.Tensor] = None) -> StepState:
     """x [B,N,F,T] float32 CUDA.  Allocates outputs + workspace and fills ``regt_args``.
     Region shards (shard.py): x is [B,x_rows,F,T] with x_rows >= plan.N -- the plan's N owned rows
     followed by halo rows that only the plan's column indices address -- and ``loss_nodes`` is the
-    node count of the full graph, so the per-rank losses and gradients add up to the unsharded ones."""
+    node count of the full graph, so the per-rank losses and gradients add up to the unsharded ones.
+    ``loss_kind`` / ``null_value`` pick the loss of the fused step (``check_loss``); ``loss_count`` [B] holds the valid
+    targets of each snapshot over the full graph (region shards), else the library counts them in ``y``."""
     lib = _lib.load()
     dev = x.device
     B, x_rows, Fx, T = x.shape
@@ -107,6 +111,15 @@ def build_state(mode: int, precision: int, plan: GraphPlanTensors, x: torch.Tens
     a.x_rows = x_rows
     a.F = Fx
     a.loss_nodes = int(loss_nodes) if loss_nodes else 0
+    a.loss_kind = loss_kind
+    if null_value is not None:
+        a.loss_masked, a.loss_null = 1, float(null_value)
+        if loss_count is not None:
+            _check(loss_count, "loss_count", dev, 4)
+            if tuple(loss_count.shape) != (B,):
+                raise ValueError(f"regt_b200: loss_count must be [B]=({B},), got {tuple(loss_count.shape)}")
+            a.loss_count = loss_count.data_ptr()
+            st.keep.append(loss_count)
     a.plan = plan.c_struct()
     a.x = x.data_ptr()
     for k in keys_for(mode, head):
@@ -138,6 +151,23 @@ def build_state(mode: int, precision: int, plan: GraphPlanTensors, x: torch.Tens
     st.workspace = workspace
     a.workspace, a.workspace_bytes = workspace.data_ptr(), workspace.numel()
     return st
+
+
+def check_loss(loss: str, null_value) -> int:
+    """``loss`` ("mse" or "mae") -> its ``REGT_LOSS_*`` code; ``null_value`` must be None (no mask) or a float (targets equal to
+    it, or NaN, are missing; ``float("nan")`` marks only NaNs)."""
+    if loss not in _lib.LOSSES:
+        raise ValueError(f"regt_b200: loss must be one of {sorted(_lib.LOSSES)}, got {loss!r}")
+    if null_value is not None and (isinstance(null_value, bool) or not isinstance(null_value, (int, float))):
+        raise ValueError(f"regt_b200: null_value must be None (no mask) or a float, got {null_value!r}")
+    return _lib.LOSSES[loss]
+
+
+def loss_counts(y: torch.Tensor, null_value: float) -> torch.Tensor:
+    """valid targets of each snapshot of ``y [B,N,O]`` (neither ``null_value`` nor NaN) as float32 [B]: the ``loss_count`` a
+    region shard passes, taken from the full graph's targets."""
+    missing = torch.isnan(y) if math.isnan(null_value) else (torch.isnan(y) | (y == null_value))
+    return (~missing).sum(dim=(1, 2)).to(torch.float32)
 
 
 def workspace_bytes(mode: int, precision: int, plan: GraphPlanTensors, B: int, x_rows: int, T: int, H: int, O: int,

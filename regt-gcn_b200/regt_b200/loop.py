@@ -6,6 +6,9 @@
   ``RMSprop`` step per epoch; no per-snapshot ``loss.cpu()`` (the losses stay on the device, one read at the end).
 * ``evaluate``        -- ``predict.py:142-194``: MAE, RMSE, MAPE normalised by each snapshot's 95th percentile, reduced on the
   device (``regt_eval_metrics``), one small D2H read per batch instead of three tensors per snapshot.
+
+Both take a ``null_value`` for series that mark a missing reading (METR-LA / PEMS-BAY: 0): the loss and the metrics then
+run over the valid targets only.
 """
 from __future__ import annotations
 
@@ -136,9 +139,10 @@ class FlatRMSprop:
 
 
 def train_epoch(model, windows: SlidingWindows, graph_args: Sequence, optimizer, first: int = 0, last: Optional[int] = None,
-                batch: int = 64, micro_batch: Optional[int] = None):
+                batch: int = 64, micro_batch: Optional[int] = None, loss: str = "mse", null_value: Optional[float] = None):
     """one epoch of run.py:163-199 over windows [first, last): gradients of every snapshot accumulate, ONE optimizer step.
-    Returns (last snapshot's loss -- what run.py:197 returns --, sum of the snapshot losses); both are device tensors."""
+    Returns (last snapshot's loss -- what run.py:197 returns --, sum of the snapshot losses); both are device tensors.
+    ``loss`` / ``null_value``: the loss of ``model.fused_step``."""
     last = len(windows) if last is None else last
     optimizer.zero_grad()
     total = torch.zeros(1, device=windows.data.device)
@@ -150,10 +154,10 @@ def train_epoch(model, windows: SlidingWindows, graph_args: Sequence, optimizer,
         tail = 1 if s1 == last else 0
         if s1 - tail > s0:
             x, y = windows.gather(torch.arange(s0, s1 - tail, device=windows.data.device))
-            total += model.fused_step(x, y, *graph_args, micro_batch=micro_batch)[0]
+            total += model.fused_step(x, y, *graph_args, micro_batch=micro_batch, loss=loss, null_value=null_value)[0]
         if tail:
             x, y = windows.gather(torch.arange(s1 - 1, s1, device=windows.data.device))
-            last_loss = model.fused_step(x, y, *graph_args)[0]
+            last_loss = model.fused_step(x, y, *graph_args, loss=loss, null_value=null_value)[0]
             total += last_loss
     optimizer.step()
     return last_loss, total
@@ -161,8 +165,9 @@ def train_epoch(model, windows: SlidingWindows, graph_args: Sequence, optimizer,
 
 @torch.no_grad()
 def evaluate(model, windows: SlidingWindows, graph_args: Sequence, first: int = 0, last: Optional[int] = None, batch: int = 64,
-             q: float = 95.0):
-    """predict.py:142-194 -> (MAE, RMSE, MAPE %) over windows [first, last)."""
+             q: float = 95.0, null_value: Optional[float] = None):
+    """predict.py:142-194 -> (MAE, RMSE, MAPE %) over windows [first, last).  ``null_value`` (a float): targets equal to it,
+    or NaN, are missing and left out of every metric and of the percentile (``regt_eval_metrics_masked``)."""
     lib = _lib.load()
     last = len(windows) if last is None else last
     dev = windows.data.device
@@ -173,17 +178,30 @@ def evaluate(model, windows: SlidingWindows, graph_args: Sequence, first: int = 
         x, y = windows.gather(torch.arange(s0, s1, device=dev))
         out = model(x, *graph_args)[0].contiguous()
         n = out[0].numel()
-        part = torch.empty(s1 - s0, 4, device=dev, dtype=torch.float64)
+        part = torch.empty(s1 - s0, 4 if null_value is None else 5, device=dev, dtype=torch.float64)
         with torch.cuda.device(dev):
-            _lib.check(lib.regt_eval_metrics(out.data_ptr(), y.contiguous().data_ptr(), s1 - s0, n, q, part.data_ptr(), _stream()),
-                       "regt_eval_metrics")
+            if null_value is None:
+                _lib.check(lib.regt_eval_metrics(out.data_ptr(), y.contiguous().data_ptr(), s1 - s0, n, q, part.data_ptr(),
+                                                 _stream()), "regt_eval_metrics")
+            else:
+                _lib.check(lib.regt_eval_metrics_masked(out.data_ptr(), y.contiguous().data_ptr(), s1 - s0, n, q, float(null_value),
+                                                        part.data_ptr(), _stream()), "regt_eval_metrics_masked")
         sums.append(part)
     return reduce_metrics(torch.cat(sums).cpu(), n)
 
 
 def reduce_metrics(sums: torch.Tensor, n: int):
     """per-snapshot [sum|e|, sum e^2, p95, sum|e|/p95] -> predict.py's return values: snapshots whose normalised errors
-    contain an inf (p95 == 0) are left out of the MAPE only (predict.py:167-169)."""
+    contain an inf (p95 == 0) are left out of the MAPE only (predict.py:167-169).  Masked sums [count, sum|e|, sum e^2, p95,
+    sum|e|/p95] (5 columns) are divided by the valid counts; snapshots without a valid target drop out."""
+    if sums.shape[1] == 5:
+        sums = sums[sums[:, 0] > 0]
+        cnt = float(sums[:, 0].sum())
+        if cnt == 0:
+            return float("nan"), float("nan"), float("nan")
+        keep = ~torch.isinf(sums[:, 4])
+        mape = float(sums[keep, 4].sum()) / float(sums[keep, 0].sum()) * 100 if bool(keep.any()) else float("nan")
+        return float(sums[:, 1].sum()) / cnt, math.sqrt(float(sums[:, 2].sum()) / cnt), mape
     S = sums.shape[0]
     mae = float(sums[:, 0].sum()) / (S * n)
     rmse = math.sqrt(float(sums[:, 1].sum()) / (S * n))

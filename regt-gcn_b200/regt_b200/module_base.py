@@ -118,10 +118,16 @@ class RegTModelBase(nn.Module):
 
     # ---- fused training step: forward + loss + backward in one pass, no autograd graph ----
     def _fused_step(self, x: torch.Tensor, y: torch.Tensor, plan, micro_batch: Optional[int] = None,
-                    loss_nodes: Optional[int] = None):
+                    loss_nodes: Optional[int] = None, loss: str = "mse", null_value: Optional[float] = None,
+                    loss_count: Optional[torch.Tensor] = None):
         """run.py:170-192 for a whole batch of snapshots: loss = sum_b mean((out_b-y_b)^2);
         gradients are ACCUMULATED into ``.grad`` (the reference accumulates over the epoch and
-        steps once, run.py:190-195).  Returns (loss [1] device tensor, out, out_hidden)."""
+        steps once, run.py:190-195).  Returns (loss [1] device tensor, out, out_hidden).
+
+        ``loss="mae"`` takes |out_b-y_b| instead.  ``null_value`` (a float) marks a target equal to it, or NaN, as missing:
+        each snapshot's mean then runs over its valid targets only, and a snapshot without one adds 0 and no gradient.
+        ``loss_count`` [B]: the valid targets per snapshot when ``y`` holds only part of the graph (region shards)."""
+        loss_kind = engine.check_loss(loss, null_value)
         xb, batched = self._as_batched(x)
         yb = y if batched else y.unsqueeze(0)
         xb = xb.to(torch.float32).contiguous()
@@ -148,23 +154,28 @@ class RegTModelBase(nn.Module):
                                                    self.output_dim, 0 if ws is None else ws.numel(), xb.shape[2])
                 self._mb_key = key
             mb = self._mb
-        loss = None
+        if loss_count is not None and null_value is not None:
+            loss_count = loss_count.reshape(-1).to(device=xb.device, dtype=torch.float32).contiguous()
+        else:
+            loss_count = None   # without counts the library counts each micro-batch's snapshots (whole snapshots: exact)
+        total = None
         outs, hids = [], []
         for b0 in range(0, B, mb):
             st = engine.build_state(self._mode, prec, plan, xb[b0:b0 + mb], self._hidden, self.output_dim,
                                     params, yb[b0:b0 + mb], None, True, getattr(self, "_ws", None), fuse_head=True,
-                                    loss_nodes=loss_nodes)
+                                    loss_nodes=loss_nodes, loss_kind=loss_kind, null_value=null_value,
+                                    loss_count=None if loss_count is None else loss_count[b0:b0 + mb])
             self._ws = st.workspace
             engine.run_forward(st, True)
             engine.run_backward(st, grads, st.d_out, None, True, True)
-            loss = st.loss if loss is None else loss + st.loss
+            total = st.loss if total is None else total + st.loss
             outs.append(st.out)
             hids.append(st.out_hidden)
         out = outs[0] if len(outs) == 1 else torch.cat(outs)
         hid = hids[0] if len(hids) == 1 else torch.cat(hids)
         if not batched:
             out, hid = out[0], hid[0]
-        return loss, out, hid
+        return total, out, hid
 
 
 def split_regional_args(regional: Sequence, R: int):

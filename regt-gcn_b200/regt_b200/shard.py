@@ -456,15 +456,28 @@ class RegionShardedModel:
         return gather_rows(x, self.perm), (None if y is None else gather_rows(y, self.own))
 
     def fused_step(self, x: torch.Tensor, y: torch.Tensor, micro_batch: Optional[int] = None,
-                   gather_outputs: bool = False, local_inputs=None, sync: bool = True):
+                   gather_outputs: bool = False, local_inputs=None, sync: bool = True, loss: str = "mse",
+                   null_value: Optional[float] = None, loss_count: Optional[torch.Tensor] = None):
         """forward + loss + backward on this rank's rows; gradients ACCUMULATE into the flat buffer
         behind ``.grad`` (run.py:190).  ``sync=True`` all-reduces that buffer in place right away, so
         it is for loops that zero the gradients every step; loops that accumulate over many
         snapshots and step once (the reference's epoch, run.py:190-195) pass ``sync=False`` and call
         ``sync_gradients()`` once before ``optimizer.step()`` -- the sum is linear, one all-reduce
-        per optimizer step is enough.  The loss rides in a slot of the same buffer."""
+        per optimizer step is enough.  The loss rides in a slot of the same buffer.
+
+        ``loss`` / ``null_value`` as in the model's ``fused_step``.  A masked mean divides by the valid targets of the FULL
+        graph, so the rank needs them: taken from the full ``y``, or passed as ``loss_count`` [B]
+        (``engine.loss_counts(y, null_value)``) by a caller that gives only ``local_inputs``."""
+        from . import engine
+        engine.check_loss(loss, null_value)
+        if null_value is not None and loss_count is None:
+            if y is None:
+                raise ValueError("regt_b200: a masked loss (null_value set) with local_inputs only needs loss_count= "
+                                 "(valid targets per snapshot over the full graph: engine.loss_counts(y, null_value))")
+            loss_count = engine.loss_counts(y, null_value)
         xl, yl = local_inputs if local_inputs is not None else self.local_inputs(x, y)
-        loss, out, hid = self.model._fused_step(xl, yl, self.plan, micro_batch, loss_nodes=self.shard.N)
+        loss, out, hid = self.model._fused_step(xl, yl, self.plan, micro_batch, loss_nodes=self.shard.N, loss=loss,
+                                                null_value=null_value, loss_count=loss_count)
         self.exchange.add_loss(loss)
         if sync:
             loss = self.sync_gradients()
