@@ -75,8 +75,8 @@ Layout make_layout(const regt_args* a, void* base) {
     L.Hn = c.take<float>(rows * H);
     L.D = c.take<float>(rows * 4 * H);
     L.Feat = c.take<float>(gemm_cell ? rows * 32 : 4);
-    L.bsplit = c.take<float>(L.route.cell == CellPath::Tf32x3Unfused ? gemm_nt_scratch_floats((int)H, 2 * (int)H)
-                             : L.route.cell == CellPath::Bf16Gemm  ? gemm_nt_bf16_scratch_floats((int)H, 2 * (int)H)
+    L.bsplit = c.take<float>(L.route.cell == CellPath::Tf32x3Unfused ? gemm_nt_scratch_floats((int)H, 2 * (int)H, GemmKind::Tf32x3)
+                             : L.route.cell == CellPath::Bf16Gemm  ? gemm_nt_scratch_floats((int)H, 2 * (int)H, GemmKind::Bf16)
                                                                    : 4);
   } else {   // bf16 fused tcgen05 kernels: tile-layout planes
     const size_t nqt = (BN + 127) / 128, plane = T * nqt * 128 * H;
@@ -94,7 +94,7 @@ Layout make_layout(const regt_args* a, void* base) {
   if (a->precision == REGT_PREC_TF32X3) {   // tensor-core head (head_f.cu)
     L.hf_rh = c.take<float>(BN * H);
     L.hf_do32 = c.take<float>(BN * 32);
-    L.hf_split = c.take<float>(max(gemm_nt_scratch_floats(HEAD_HID, (int)H), gemm_nt_scratch_floats((int)H, HEAD_HID)));
+    L.hf_split = c.take<float>(max(gemm_nt_scratch_floats(HEAD_HID, (int)H, GemmKind::Tf32x3), gemm_nt_scratch_floats((int)H, HEAD_HID, GemmKind::Tf32x3)));
     L.hf_loss_floats = BN / 8 + 2;
     L.hf_loss = c.take<float>(L.hf_loss_floats);
   }

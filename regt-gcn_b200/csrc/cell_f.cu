@@ -101,11 +101,6 @@ struct FArgs {
   int hpre_mma;                    // forward: h_pre on the tensor cores where the item allows it (TEST HOOK REGT_F_HPRE_MMA=0: CUDA cores)
 };
 
-__device__ __forceinline__ uint32_t tf32_rn_bits(float a) {
-  uint32_t u;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(u) : "f"(a));
-  return u;
-}
 __device__ __forceinline__ float sigm(float v) { return __fdividef(1.0f, 1.0f + __expf(-v)); }
 __device__ __forceinline__ float tanh_(float v) { return 1.0f - __fdividef(2.0f, 1.0f + __expf(2.0f * v)); }
 
@@ -115,7 +110,7 @@ __device__ __forceinline__ void put_a16(uint32_t tlane, int col, const float (&v
   uint32_t hi[16], lo[16];
 #pragma unroll
   for (int i = 0; i < 16; ++i) {
-    hi[i] = tf32_rn_bits(v[i]);
+    hi[i] = tf32_rn(v[i]);
     lo[i] = __float_as_uint(v[i] - __uint_as_float(hi[i]));
   }
   tmem_st16(tlane + col, hi);
@@ -126,7 +121,7 @@ __device__ __forceinline__ void put_a8(uint32_t tlane, int col, const float (&v)
   uint32_t hi[8], lo[8];
 #pragma unroll
   for (int i = 0; i < 8; ++i) {
-    hi[i] = tf32_rn_bits(v[i]);
+    hi[i] = tf32_rn(v[i]);
     lo[i] = __float_as_uint(v[i] - __uint_as_float(hi[i]));
   }
   tmem_st8(tlane + col, hi);
@@ -472,7 +467,7 @@ __global__ void __launch_bounds__(NTHR, 1) k_cell_fwd_f(FArgs a) {
               const int rg = pregs[j - 1];
               v = rg >= 0 ? __ldg(a.M1t + ((size_t)rg * F + kk) * HH + n) : 0.f;
             }
-            const float hi = __uint_as_float(tf32_rn_bits(v));
+            const float hi = __uint_as_float(tf32_rn(v));
             uint8_t* w0 = wp + j * 2 * C::SW_TILE + chunk_off(n, kk >> 2, HH) + (kk & 3) * 4;
             *reinterpret_cast<float*>(w0) = hi;
             *reinterpret_cast<float*>(w0 + C::SW_TILE) = v - hi;
@@ -497,7 +492,7 @@ __global__ void __launch_bounds__(NTHR, 1) k_cell_fwd_f(FArgs a) {
           float hi[8], lo[8];
 #pragma unroll
           for (int i = 0; i < 8; ++i) {
-            hi[i] = __uint_as_float(tf32_rn_bits(v[i]));
+            hi[i] = __uint_as_float(tf32_rn(v[i]));
             lo[i] = v[i] - hi[i];
           }
           const int j = ch == 1 ? 0 : (slot == 1 ? 2 : 1);      // k-step that receives this row's values
@@ -538,7 +533,7 @@ __global__ void __launch_bounds__(NTHR, 1) k_cell_fwd_f(FArgs a) {
         float hi[8], lo[8];
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
-          hi[i] = __uint_as_float(tf32_rn_bits(svn[i]));
+          hi[i] = __uint_as_float(tf32_rn(svn[i]));
           lo[i] = svn[i] - hi[i];
         }
 #pragma unroll
@@ -1151,7 +1146,7 @@ __device__ __forceinline__ void put_stage(uint8_t* img, int g, int n, int k, flo
   using C = FCfg<HH>;
   uint8_t* st = img + (size_t)(g * C::NCH + (k >> 5)) * C::STAGE;
   const uint32_t off = sw128_off(n, (k & 31) * 4, HH);
-  const float hi = __uint_as_float(tf32_rn_bits(v));
+  const float hi = __uint_as_float(tf32_rn(v));
   *reinterpret_cast<float*>(st + off) = hi;
   *reinterpret_cast<float*>(st + C::TILE + off) = v - hi;
 }
@@ -1181,7 +1176,7 @@ __global__ void k_pack_f(const float* __restrict__ Wzr, const float* __restrict_
     const float v = g < 2 ? Wzr[(size_t)f * 2 * HH + g * HH + n] : Wc[(size_t)f * HH + n];
     uint8_t* t0 = img_f + C::RING_IMG + (size_t)g * 2 * C::SW_TILE;
     const uint32_t off = chunk_off(n, f >> 2, HH) + (f & 3) * 4;
-    const float hi = __uint_as_float(tf32_rn_bits(v));
+    const float hi = __uint_as_float(tf32_rn(v));
     *reinterpret_cast<float*>(t0 + off) = hi;
     *reinterpret_cast<float*>(t0 + C::SW_TILE + off) = v - hi;
     return;

@@ -259,8 +259,7 @@ int launch_f_sum_dpp(const double* part, int nparts, int T, float* dprobs, cudaS
 int launch_fw_scatter(const float* Cp, int splits, int H, const Layout& L, cudaStream_t st);
 // gemm_tma.cu: TMA-fed 3xTF32 GEMMs and their single-pass bf16 forms
 enum class GemmKind { Tf32x3, Bf16 };
-size_t gemm_nt_scratch_floats(int N, int K);        // hi | lo images of the weight operand (Tf32x3)
-size_t gemm_nt_bf16_scratch_floats(int N, int K);   // its bf16 image (Bf16)
+size_t gemm_nt_scratch_floats(int N, int K, GemmKind kind);   // hi | lo images of the weight operand, or its bf16 image
 int launch_gemm_nt_tma(const float* A, long long lda, const float* Bt, long long ldb, float* C, long long ldc, long long M, int N,
                        int K, float* scratch, cudaStream_t st, GemmKind kind = GemmKind::Tf32x3);
 int launch_gemm_tn(const float* A, long long lda, const float* B, long long ldb, float* Cp, long long M, int K, int N, int splits,

@@ -234,6 +234,12 @@ __device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
 }
 // tf32 split: hi keeps the top 19 bits (what the tensor core reads), lo = exact remainder
 __device__ __forceinline__ float tf32_hi(float a) { return __uint_as_float(__float_as_uint(a) & 0xFFFFE000u); }
+// the bits of a rounded to tf32 (to nearest, ties away from zero)
+__device__ __forceinline__ uint32_t tf32_rn(float a) {
+  uint32_t u;
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(u) : "f"(a));
+  return u;
+}
 
 }  // namespace tc
 }  // namespace regt
