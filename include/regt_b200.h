@@ -189,6 +189,10 @@ typedef struct regt_args {
   float loss_null;        /* the value that marks a missing target (NaN: only NaNs are missing)                        */
   const float* loss_count;/* [B] valid count c_b of each snapshot over ALL nodes of the graph (region shards: the full   */
                           /*    graph's counts), or NULL: counted over rows [0,N) of y on the device                   */
+  int32_t head_only;      /* 1: the call runs the head (and loss) on a given out_hidden, with no cell: the workspace holds  */
+                          /*    no cell planes, regt_cell_* refuse the args, the head never runs k_head_tc, and the         */
+                          /*    gradient wrt out_hidden, G [B*N][H] row major, is left at the START of the workspace by     */
+                          /*    regt_head_backward (what regt_combine_backward reads).  0: the full step, as before        */
 } regt_args;
 
 #define REGT_LOSS_MSE 0
@@ -290,6 +294,25 @@ int regt_eval_metrics(const float* out, const float* y, int32_t B, int64_t n_per
 int regt_eval_metrics_masked(const float* out, const float* y, int32_t B, int64_t n_per_snapshot, double q, float null_value,
                              double* sums, regt_stream_t stream);
 
+/* ---- time steps shared across sliding windows (csrc/combine.cu; regt_b200/loop.py share_periods) --------------------
+ * The cell output of a period depends on that period's input alone (the hidden state is not carried across periods), so
+ * the cell output H'(tau) of time step tau is the same in every window that contains tau.  A pass over C consecutive
+ * windows runs the cell once per time step, S = C + T - 1 steps (regt_cell_forward at T = 1 over S "snapshots"), then
+ *   regt_combine_forward:  out_hidden[w] = sum_{t<T} p_t H'[w+t]        (w < C; summed in period order)
+ *   regt_combine_backward: Gs[tau]      = sum_{t<T, 0 <= tau-t < C} p_t G[tau-t]     (tau < S; in period order)
+ *                          dprobs_t     = sum_w <G[w], H'[w+t]>  (fp64 partials, summed in a fixed order)
+ *                          attention_grad[t] += p_t (dprobs_t - sum_s p_s dprobs_s)     (when attention_grad is set)
+ * p = softmax(attention [T]), computed as the cell kernels compute it.  Hs / Gs [S][width], out_hidden / G [C][width],
+ * width = N*H (a multiple of 4; 16-byte aligned rows).  Each element of Hs and G is read once when width fills the device;
+ * a narrower pass is split into chunks of windows (steps) that re-read T - 1 rows each.  Gs is the gradient wrt the
+ * step cell's out_hidden (regt_args.d_hidden of its regt_head_backward with d_out = NULL).
+ * scratch: at least regt_combine_scratch_bytes(T) bytes (backward only; 8-byte aligned).                               */
+size_t regt_combine_scratch_bytes(int32_t T);
+int regt_combine_forward(const float* attention, const float* Hs, int32_t S, int32_t C, int32_t T, int64_t width, float* out_hidden,
+                         regt_stream_t stream);
+int regt_combine_backward(const float* attention, const float* Hs, const float* G, int32_t S, int32_t C, int32_t T, int64_t width,
+                          float* Gs, float* attention_grad, void* scratch, size_t scratch_bytes, regt_stream_t stream);
+
 int regt_version(void);
 const char* regt_last_error(void);
 /* number of kernel launches issued by this library on the calling thread since the last
@@ -322,7 +345,7 @@ int regt_profile_read(char* names, size_t names_len, float* ms, int max_n);
  *             out[7] = {128-row tiles nqt, periods per item tp, period chunks ntc = T / tp, items = nqt * ntc,
  *             forward grid, backward grid, k_head_tc grid} (tests/test_gpu_bf16_edges.py states its preconditions so)
  *   route: which cell and head kernels the entry points run for these arguments (no CUDA call, no workspace needed),
- *          out[4] = {cell: 0 fp32, 1 unfused tf32x3, 2 fused tf32x3, 3 fused bf16, 4 GEMM-by-GEMM bf16;
+ *          out[4] = {cell: 0 fp32, 1 unfused tf32x3, 2 fused tf32x3, 3 fused bf16, 4 GEMM-by-GEMM bf16, 5 none (head_only);
  *          head: 0 row kernels k_head_fwd / k_head_bwd,
  *          1 k_head_fused, 2 tf32x3 head, 3 k_head_tc; G written as tiles; bf16 forward leaves out_hidden partials}   */
 int regt_debug_gemm_nt_tma(const float* A, int64_t lda, const float* Bt, int64_t ldb, float* C, int64_t ldc, int64_t M,

@@ -50,7 +50,8 @@ def main(argv=None):
     nd, _ = R.load_series(args, N)
     windows = SlidingWindows(nd.to(device), args.num_timesteps_in, args.num_timesteps_out)
     n_train = int(args.tr * len(windows))
-    mae, rmse, mape = evaluate(model, windows, graph, n_train, len(windows), batch=max(1, args.bs))    # predict.py:142-194
+    mae, rmse, mape = evaluate(model, windows, graph, n_train, len(windows), batch=max(1, args.bs),    # predict.py:142-194
+                               share_periods=args.share_periods)
     print(f"Test Results: RMSE: {rmse}, MAE: {mae}, MAPE: {mape}")                                     # predict.py:252
     return mae, rmse, mape
 

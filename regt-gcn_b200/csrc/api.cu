@@ -15,7 +15,9 @@ Route route_of(const regt_args* a) {
   Route r{};
   // bf16: the fused H = 64 cell where it is built for the shape (REGT_UNFUSED does not apply: it names the tf32x3 cells),
   // else the GEMM-by-GEMM cell on the single-pass bf16 GEMMs
-  r.cell = bf16 ? (cell_tc_fits(a) ? CellPath::Bf16 : CellPath::Bf16Gemm)
+  // head_only: no cell, so none of the cell couplings below applies (k_head_tc, tiled G, out_hidden partials)
+  r.cell = a->head_only ? CellPath::None
+         : bf16 ? (cell_tc_fits(a) ? CellPath::Bf16 : CellPath::Bf16Gemm)
                 : !tf32x3 ? CellPath::Fp32 : (!unfused && cell_f_fits(a)) ? CellPath::Tf32x3Fused : CellPath::Tf32x3Unfused;
   if (r.cell == CellPath::Bf16 && fused_step && head_tc_fits(a->H, a->O))   // k_head_tc's partials are summed by the fused cell backward
     r.head = HeadPath::Bf16;
@@ -30,10 +32,44 @@ Route route_of(const regt_args* a) {
   return r;
 }
 
+// head_only: what the head and the loss need, no cell planes.  G comes first, so that a caller (the period-sharing
+// combine backward) finds the gradient wrt out_hidden at the start of the workspace
+static Layout make_head_layout(const regt_args* a, Layout L, Carver& c) {
+  const size_t H = a->H, O = a->O, BN = (size_t)a->B * a->N, BNp = (BN + 127) / 128 * 128;
+  L.G = c.take<float>(BNp * H);
+  if (a->precision == REGT_PREC_TF32X3) {   // tensor-core head (head_f.cu)
+    L.hf_rh = c.take<float>(BN * H);
+    L.hf_do32 = c.take<float>(BN * 32);
+    L.hf_split = c.take<float>(max(gemm_nt_scratch_floats(HEAD_HID, (int)H, GemmKind::Tf32x3), gemm_nt_scratch_floats((int)H, HEAD_HID, GemmKind::Tf32x3)));
+    L.hf_loss_floats = BN / 8 + 2;
+    L.hf_loss = c.take<float>(L.hf_loss_floats);
+    // ones column of the row head's dW1 / db1 contraction.  Taken whichever head the route picks: the head calls of a
+    // pass (training, evaluation, the final window alone) route differently, and one workspace sized for the largest
+    // of them must hold every one
+    L.Feat = c.take<float>(BNp * 32);
+  }
+  L.a1 = c.take<float>(BN * HEAD_HID);
+  L.d_a1 = c.take<float>(BN * HEAD_HID);
+  size_t pf = (size_t)128 * (O * HEAD_HID + HEAD_HID * H);          // head split-K partials (<= 128 splits)
+  pf = max(pf, (size_t)152 * HEAD_HID * (H + 32));                   // head dW1 on the tensor cores (+ the 32-wide second operand)
+  pf = max(pf, BN / 64 + 2);                                         // loss partials
+  pf += H * HEAD_HID + HEAD_HID * O + 64;                            // transposed head weights (tail)
+  L.hpart = c.take<float>((size_t)148 * (HEAD_HID * H + O * HEAD_HID + HEAD_HID + O + 8));
+  L.part = c.take<float>(pf);
+  L.part_floats = pf;
+  if (a->y) {
+    L.inv_c = c.take<float>(a->B);
+    L.lc_part = c.take<unsigned int>((size_t)a->B * LC_CHUNKS);
+  }
+  L.total = align_up(c.off, 256);
+  return L;
+}
+
 Layout make_layout(const regt_args* a, void* base) {
   Layout L{};
   L.route = route_of(a);
   Carver c(base);
+  if (L.route.cell == CellPath::None) return make_head_layout(a, L, c);
   const size_t H = a->H, T = a->T, R = a->plan.R > 0 ? a->plan.R : 1, O = a->O;
   const size_t BN = (size_t)a->B * a->N, rows = BN * T;
   const size_t nseg = a->plan.nseg;
@@ -162,6 +198,7 @@ static int validate(const regt_args* a, const char* who) {
   REGT_CHECK((long long)a->B * a->N * a->T < (1ll << 31), "%s: B*N*T overflows int32 rows", who);
   REGT_CHECK(a->workspace && a->workspace_bytes >= regt_workspace_bytes(a), "%s: workspace missing or too small", who);
   REGT_CHECK(a->precision >= 0 && a->precision <= 2, "%s: bad precision %d", who, a->precision);
+  REGT_CHECK(a->head_only == 0 || a->head_only == 1, "%s: head_only must be 0 or 1 (got %d)", who, a->head_only);
   return 0;
 }
 
@@ -176,6 +213,7 @@ extern "C" size_t regt_workspace_bytes(const regt_args* a) {
 
 extern "C" int regt_cell_forward(const regt_args* a) {
   if (validate(a, "regt_cell_forward")) return -1;
+  REGT_CHECK(!a->head_only, "regt_cell_forward: head_only args run no cell (their workspace holds no cell planes)");
   REGT_CHECK(a->x && a->out_hidden, "regt_cell_forward: x / out_hidden is NULL");
   if (check_tc_width(a)) return -1;
   Layout L = make_layout(a, a->workspace);
@@ -193,6 +231,7 @@ extern "C" int regt_cell_forward(const regt_args* a) {
 
 extern "C" int regt_cell_backward(const regt_args* a) {
   if (validate(a, "regt_cell_backward")) return -1;
+  REGT_CHECK(!a->head_only, "regt_cell_backward: head_only args run no cell (their workspace holds no cell planes)");
   REGT_CHECK(!a->inference, "regt_cell_backward: the forward ran with inference=1 (no activations were saved)");
   if (check_tc_width(a)) return -1;
   Layout L = make_layout(a, a->workspace);
@@ -215,6 +254,7 @@ static int validate_x(const regt_args* a, const regt_xgrad_plan* xp, const char*
   REGT_CHECK(a->x_rows == 0 || a->x_rows == a->N,
              "%s: region shards (x_rows=%d != N=%d) are not supported: their halo rows belong to other ranks", who, a->x_rows, a->N);
   REGT_CHECK(!a->inference, "%s: the forward ran with inference=1 (no activations were saved)", who);
+  REGT_CHECK(!a->head_only, "%s: head_only args run no cell (their workspace holds no cell planes)", who);
   if (validate(a, who)) return -1;
   REGT_CHECK(xp && xp->N == a->N && xp->n_src == 2 * a->N + a->plan.nseg && xp->rowptr && xp->col && xp->val,
              "%s: transposed plan missing or built for another graph", who);
@@ -255,7 +295,8 @@ extern "C" int regt_head_backward(const regt_args* a) {
   return head_backward(a, L, (cudaStream_t)a->stream);
 }
 
-// TEST HOOK: the kernels route_of picks for these arguments, out = {cell, head, g_tiled, hid_partials} (CellPath, HeadPath)
+// TEST HOOK: the kernels route_of picks for these arguments, out = {cell, head, g_tiled, hid_partials} (CellPath, HeadPath;
+// cell 5 = none: head_only)
 extern "C" int regt_debug_route(const regt_args* a, int32_t* out) {
   REGT_CHECK(a && out, "regt_debug_route: args and out must be non-NULL");
   const Route r = route_of(a);

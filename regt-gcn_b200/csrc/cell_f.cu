@@ -1286,11 +1286,15 @@ int launch_feat_f(const regt_args* a, const Layout& L, cudaStream_t st) {
   const int BN = a->B * a->N, nqt = (BN + TC_ROWS - 1) / TC_ROWS, BNp = nqt * TC_ROWS;
   k_featT_f<<<a->T * nqt, 128, 0, st>>>(L.Xt, L.S, BN, nqt, L.FeatT);
   REGT_LAUNCHED("k_featT_f", st);
-  k_ones_f<<<cdiv((long long)BNp * 8, 256), 256, 0, st>>>(BN, BNp, L.Feat);
+  return launch_ones_f(BN, BNp, L.Feat, st);
+}
+}  // namespace
+
+int launch_ones_f(int BN, int BNp, float* Feat, cudaStream_t st) {
+  k_ones_f<<<cdiv((long long)BNp * 8, 256), 256, 0, st>>>(BN, BNp, Feat);
   REGT_LAUNCHED("k_ones_f", st);
   return 0;
 }
-}  // namespace
 
 bool cell_f_fits(const regt_args* a) { return (a->H == 128 || a->H == 64) && a->mode != REGT_MODE_TGCN && a->T <= 64; }
 

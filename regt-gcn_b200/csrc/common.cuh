@@ -70,6 +70,16 @@ struct Carver {
 
 __device__ __forceinline__ float sigmoidf_(float v) { return 1.0f / (1.0f + expf(-v)); }
 
+// softmax over the T learned period-attention scalars (models/RegionalTemporalGCN.py:134), one thread: what k_prep writes
+// to Layout::probs and what the period-sharing combine kernels (combine.cu) weight the time steps with
+__device__ __forceinline__ void attention_softmax(const float* att, int T, float* probs) {
+  float mx = -INFINITY;
+  for (int t = 0; t < T; ++t) mx = fmaxf(mx, att[t]);
+  double den = 0.0;
+  for (int t = 0; t < T; ++t) den += exp((double)att[t] - mx);
+  for (int t = 0; t < T; ++t) probs[t] = (float)(exp((double)att[t] - mx) / den);
+}
+
 // offset of G[q][n] (gradient wrt out_hidden): row major, or the [qt][H/4][128][4] tiles the fused cell backwards read
 __device__ __forceinline__ size_t g_off(long long q, int n, int H, int tiled) {
   return tiled ? ((((size_t)(q >> 7) * (H >> 2) + (n >> 2)) * 128 + (size_t)(q & 127)) * 4 + (n & 3)) : ((size_t)q * H + n);
@@ -119,7 +129,8 @@ inline int sm_count() {
 
 // ---- which cell and head kernels a call runs (route_of, api.cu) ----------------------
 // cell.cu, cell_g.cu, cell_f.cu, cell_tc.cu, and cell_g.cu on the single-pass bf16 GEMMs (every hidden % 32 == 0 width)
-enum class CellPath { Fp32, Tf32x3Unfused, Tf32x3Fused, Bf16, Bf16Gemm };
+// None: a head-only call (regt_args.head_only), which runs no cell
+enum class CellPath { Fp32, Tf32x3Unfused, Tf32x3Fused, Bf16, Bf16Gemm, None };
 enum class HeadPath { Rows, FusedFfma, Tf32x3, Bf16 };             // k_head_fwd / k_head_bwd, k_head_fused, head_f.cu, k_head_tc
 struct Route {
   CellPath cell;
@@ -127,6 +138,7 @@ struct Route {
   bool g_tiled;        // G is written as tiles (g_off): the fused tf32x3 and bf16 cell backwards read it so
   bool hid_partials;   // the bf16 forward leaves per-chunk partials of out_hidden and the head sums them (no k_hid_reduce)
 };
+// head_only: cell None, never k_head_tc, row-major G, no out_hidden partials.
 // reads REGT_UNFUSED ("1": the GEMM-by-GEMM tf32x3 cell of cell_g.cu wherever the fused one would run); no CUDA calls
 Route route_of(const regt_args* a);
 // the shapes each implementation is built for, with no knowledge of the other paths
@@ -161,7 +173,7 @@ struct Layout {
   float* Hn;     // H' (cell output per period)
   // head
   float* a1;     // [B*N][128]  relu(linear1(relu(hid)))
-  float* G;      // [B*N][H]    gradient wrt out_hidden
+  float* G;      // [B*N][H]    gradient wrt out_hidden (head_only: row major, at the start of the workspace)
   float* d_a1;   // [B*N][128]
   // backward planes
   float* D;      // [rows][4H]  d_pre_z | d_pre_r | d_pre_h | d_hpre
@@ -241,6 +253,8 @@ int launch_chain(const regt_args* a, const Layout& L, cudaStream_t st);
 int launch_spmm_rows(const int32_t* rowptr, const int32_t* col, const float* val, const float* x, float* y, int B,
                      int n_out, int n_in, int width, cudaStream_t st);
 // x [B][xN][Fin][T]; Xt / St / Ut rows are REGT_F wide (features Fin.. are zeros)
+// cell_f.cu: Feat [BNp][32] = 0 with column 16 = 1 in rows < BN (the ones column of the head's bias sums)
+int launch_ones_f(int BN, int BNp, float* Feat, cudaStream_t st);
 int launch_feat_tc(const regt_graph_plan& p, const float* x, int Fin, int B, int xN, int T, float* Xt, float* St, float* Ut,
                    cudaStream_t st);
 // L.xw = x with zero features Fin..REGT_F-1 (no launch when L.xw is NULL)

@@ -620,7 +620,9 @@ int head_backward(const regt_args* a, const Layout& L, cudaStream_t st) {
   const int splits = (int)max(1ll, min(128ll, BN / 128));
   float* part = L.part;
   if (a->precision == REGT_PREC_TF32X3 && H % 32 == 0 && BN >= 128) {
-    // dW1, db1 on the tensor cores: column 16 of the cell's feature plane is all ones, its first BN rows are the operand
+    // dW1, db1 on the tensor cores: column 16 of the cell's feature plane is all ones, its first BN rows are the operand.
+    // A head-only call ran no cell: it writes that plane itself
+    if (L.route.cell == CellPath::None && launch_ones_f((int)BN, (int)((BN + 127) / 128 * 128), L.Feat, st)) return -1;
     if (launch_head_dw1_tf32x3(a, L, L.Feat, st)) return -1;
     TNBatch tb{};
     tb.nprob = 1;

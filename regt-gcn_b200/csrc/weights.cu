@@ -106,12 +106,7 @@ __global__ void __launch_bounds__(256) k_prep(regt_params p, int H, int Fin, int
     }
     dst = c0 + j;
   } else if ((i -= nc0) == 0 && sub == 0) {
-    // softmax over the T learned scalars (models/RegionalTemporalGCN.py:134)
-    float mx = -INFINITY;
-    for (int t = 0; t < T; ++t) mx = fmaxf(mx, p.attention[t]);
-    double den = 0.0;
-    for (int t = 0; t < T; ++t) den += exp((double)p.attention[t] - mx);
-    for (int t = 0; t < T; ++t) probs[t] = (float)(exp((double)p.attention[t] - mx) / den);
+    attention_softmax(p.attention, T, probs);   // softmax over the T learned scalars (models/RegionalTemporalGCN.py:134)
   }
   // all 32 lanes reach this point: combine the PG slices (fixed tree: deterministic)
 #pragma unroll

@@ -69,6 +69,10 @@ class RegionalTemporalGCN(RegTModelBase):
         # the regional ChebConvs see the raw distances (RegionalTemporalGCN.py:128,136-148)
         return get_plan(N, x.device, edge_index, None, eis, eas)
 
+    def step_plan(self, x, edge_index, *regional):
+        """the graph plan ``fused_step`` runs on for these graph arguments (``loop.train_epoch(share_periods=True)``)"""
+        return self._plan(x, edge_index, regional)
+
     def forward(self, x, edge_index, IAedge_index=None, KSedge_index=None, KYedge_index=None, OHedge_index=None,
                 WIedge_index=None, IAedge_attr=None, KSedge_attr=None, KYedge_attr=None, OHedge_attr=None,
                 WIedge_attr=None, *more):

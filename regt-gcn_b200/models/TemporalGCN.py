@@ -52,6 +52,10 @@ class TemporalGCN(RegTModelBase):
         # edge_attr reaches BOTH the ChebConv and the gcn_norm of the TGCN (TemporalGCN.py:88-90)
         return get_plan(N, x.device, edge_index, edge_attr, [edge_index], [edge_attr])
 
+    def step_plan(self, x, edge_index, edge_attr=None):
+        """the graph plan ``fused_step`` runs on for these graph arguments (``loop.train_epoch(share_periods=True)``)"""
+        return self._plan(x, edge_index, edge_attr)
+
     def forward(self, x, edge_index, edge_attr=None):
         """x = node features for T time steps; returns (h [.,N,O], out_hidden [.,N,H])."""
         return self._run(x, self._plan(x, edge_index, edge_attr))

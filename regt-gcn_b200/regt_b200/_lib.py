@@ -46,7 +46,8 @@ class Args(C.Structure):
                 ("p", Params), ("g", Params),
                 ("out_hidden", vp), ("out", vp), ("loss", vp), ("d_out", vp), ("d_hidden", vp), ("d_h_ext", vp),
                 ("workspace", vp), ("workspace_bytes", C.c_size_t), ("stream", vp), ("F", C.c_int32),
-                ("loss_kind", C.c_int32), ("loss_masked", C.c_int32), ("loss_null", C.c_float), ("loss_count", vp)]
+                ("loss_kind", C.c_int32), ("loss_masked", C.c_int32), ("loss_null", C.c_float), ("loss_count", vp),
+                ("head_only", C.c_int32)]
 
 
 MODE_A3TGCN, MODE_REGIONAL, MODE_TGCN = 0, 1, 2
@@ -64,7 +65,8 @@ EXPORTS = ["regt_version", "regt_last_error", "regt_launch_count", "regt_plan_wo
            "regt_profile", "regt_profile_begin", "regt_profile_read",
            "regt_comm_region_bytes", "regt_comm_data_offset", "regt_comm_alloc", "regt_comm_free", "regt_comm_export",
            "regt_comm_import", "regt_comm_unimport", "regt_peer_allreduce_f32", "regt_peer_push_max_floats", "regt_comm_error",
-           "regt_window_gather", "regt_rmsprop_step", "regt_eval_metrics", "regt_eval_metrics_masked"]
+           "regt_window_gather", "regt_rmsprop_step", "regt_eval_metrics", "regt_eval_metrics_masked",
+           "regt_combine_scratch_bytes", "regt_combine_forward", "regt_combine_backward"]
 
 _lib = None
 
@@ -155,6 +157,12 @@ def load() -> C.CDLL:
     lib.regt_eval_metrics.argtypes = [vp, vp, C.c_int32, C.c_int64, C.c_double, vp, vp]
     lib.regt_eval_metrics_masked.restype = C.c_int
     lib.regt_eval_metrics_masked.argtypes = [vp, vp, C.c_int32, C.c_int64, C.c_double, C.c_float, vp, vp]
+    lib.regt_combine_scratch_bytes.restype = C.c_size_t
+    lib.regt_combine_scratch_bytes.argtypes = [C.c_int32]
+    lib.regt_combine_forward.restype = C.c_int
+    lib.regt_combine_forward.argtypes = [vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int64, vp, vp]
+    lib.regt_combine_backward.restype = C.c_int
+    lib.regt_combine_backward.argtypes = [vp, vp, vp, C.c_int32, C.c_int32, C.c_int32, C.c_int64, vp, vp, vp, C.c_size_t, vp]
     lib.regt_debug_gemm_nt_tma.restype = C.c_int
     lib.regt_debug_gemm_nt_tma.argtypes = [vp, C.c_int64, vp, C.c_int64, vp, C.c_int64, C.c_int64, C.c_int32, C.c_int32, vp, vp]
     lib.regt_debug_gemm_tn_tma.restype = C.c_int

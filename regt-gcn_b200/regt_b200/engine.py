@@ -86,13 +86,15 @@ def build_state(mode: int, precision: int, plan: GraphPlanTensors, x: torch.Tens
                 h_ext: Optional[torch.Tensor] = None, head: bool = True,
                 workspace: Optional[torch.Tensor] = None, fuse_head: bool = False,
                 loss_nodes: Optional[int] = None, inference: bool = False, loss_kind: int = _lib.LOSS_MSE,
-                null_value: Optional[float] = None, loss_count: Optional[torch.Tensor] = None) -> StepState:
+                null_value: Optional[float] = None, loss_count: Optional[torch.Tensor] = None,
+                out_hidden: Optional[torch.Tensor] = None) -> StepState:
     """x [B,N,F,T] float32 CUDA.  Allocates outputs + workspace and fills ``regt_args``.
     Region shards (shard.py): x is [B,x_rows,F,T] with x_rows >= plan.N -- the plan's N owned rows
     followed by halo rows that only the plan's column indices address -- and ``loss_nodes`` is the
     node count of the full graph, so the per-rank losses and gradients add up to the unsharded ones.
     ``loss_kind`` / ``null_value`` pick the loss of the fused step (``check_loss``); ``loss_count`` [B] holds the valid
-    targets of each snapshot over the full graph (region shards), else the library counts them in ``y``."""
+    targets of each snapshot over the full graph (region shards), else the library counts them in ``y``.
+    ``out_hidden``: a caller's [B,N,H] buffer for the cell output (else one is allocated)."""
     lib = _lib.load()
     dev = x.device
     B, x_rows, Fx, T = x.shape
@@ -136,7 +138,11 @@ def build_state(mode: int, precision: int, plan: GraphPlanTensors, x: torch.Tens
         _check(h_ext, "H", dev)
         a.h_ext = h_ext.data_ptr()
         st.keep.append(h_ext)
-    st.out_hidden = torch.empty(B, N, H, device=dev, dtype=torch.float32)
+    if out_hidden is not None:
+        _check(out_hidden, "out_hidden", dev)
+        if tuple(out_hidden.shape) != (B, N, H):
+            raise ValueError(f"regt_b200: out_hidden must be [B,N,H]={B, N, H}, got {tuple(out_hidden.shape)}")
+    st.out_hidden = torch.empty(B, N, H, device=dev, dtype=torch.float32) if out_hidden is None else out_hidden
     a.out_hidden = st.out_hidden.data_ptr()
     if head:
         st.out = torch.empty(B, N, O, device=dev, dtype=torch.float32)
@@ -151,6 +157,76 @@ def build_state(mode: int, precision: int, plan: GraphPlanTensors, x: torch.Tens
     st.workspace = workspace
     a.workspace, a.workspace_bytes = workspace.data_ptr(), workspace.numel()
     return st
+
+
+def _head_args(mode: int, precision: int, plan: GraphPlanTensors, B: int, T: int, H: int, O: int, F: int) -> _lib.Args:
+    a = _lib.Args()
+    a.B, a.N, a.T, a.H, a.O = B, plan.N, T, H, O
+    a.mode, a.precision, a.x_rows, a.F = mode, precision, plan.N, F
+    a.head_only = 1
+    a.plan = plan.c_struct()
+    return a
+
+
+def head_workspace_bytes(mode: int, precision: int, plan: GraphPlanTensors, B: int, T: int, H: int, O: int, F: int = F_IN) -> int:
+    """bytes of a head-only workspace that holds every head-only call over at most B snapshots: the training call (targets,
+    fused head) is the largest, since the head-only layout takes the same buffers whichever head the route picks"""
+    a = _head_args(mode, precision, plan, B, T, H, O, F)
+    a.fuse_head, a.y, a.out, a.d_out, a.loss = 1, 1, 1, 1, 1     # sizes only: never dereferenced
+    return int(_lib.load().regt_workspace_bytes(C.byref(a)))
+
+
+def build_head_state(mode: int, precision: int, plan: GraphPlanTensors, hid: torch.Tensor, T: int, O: int,
+                     params: Dict[str, torch.Tensor], out: torch.Tensor, workspace: torch.Tensor, y: Optional[torch.Tensor] = None,
+                     loss: Optional[torch.Tensor] = None, d_out: Optional[torch.Tensor] = None, train: bool = False,
+                     loss_kind: int = _lib.LOSS_MSE, null_value: Optional[float] = None) -> StepState:
+    """``head_only`` args: the decoder head (and, with y, the loss) on a given out_hidden ``hid`` [B,N,H], with no cell; T is
+    the model's period count (it sizes nothing).  ``train``: the fused head of a training step (needs y, loss, d_out); its
+    regt_head_backward leaves the gradient wrt ``hid`` at the start of ``workspace``.  All buffers are the caller's."""
+    lib = _lib.load()
+    dev = hid.device
+    B, N, H = hid.shape
+    F = params["conv_w0"].shape[1]
+    st = StepState()
+    a = st.args = _head_args(mode, precision, plan, B, T, H, O, F)
+    a.fuse_head = 1 if train else 0
+    a.inference = 0 if train else 1
+    a.loss_kind = loss_kind
+    if null_value is not None:
+        a.loss_masked, a.loss_null = 1, float(null_value)
+    for k in HEAD_KEYS:
+        _check(params[k], k, dev)
+    _fill_params(a.p, params)
+    st.out_hidden, st.out = _check(hid, "out_hidden", dev), _check(out, "out", dev)
+    a.out_hidden, a.out = hid.data_ptr(), out.data_ptr()
+    st.keep += [params, plan, hid, out]
+    if y is not None:
+        _check(y, "y", dev)
+        if tuple(y.shape) != (B, N, O) or tuple(out.shape) != (B, N, O):
+            raise ValueError(f"regt_b200: y and out must be [B,N,O]={B, N, O}, got {tuple(y.shape)}, {tuple(out.shape)}")
+        a.y, a.loss, a.d_out = y.data_ptr(), loss.data_ptr(), d_out.data_ptr()
+        st.y, st.loss, st.d_out = y, loss, d_out
+    nbytes = lib.regt_workspace_bytes(C.byref(a))
+    if workspace.numel() < nbytes:
+        raise RuntimeError(f"regt_b200: head workspace of {workspace.numel()} bytes, the call needs {nbytes}")
+    st.workspace = workspace
+    a.workspace, a.workspace_bytes = workspace.data_ptr(), workspace.numel()
+    return st
+
+
+def run_head(st: StepState, grads: Optional[Dict[str, torch.Tensor]] = None) -> None:
+    """regt_head_forward on head-only args; with ``grads`` (the head's .grad views) also regt_head_backward, which
+    accumulates into them and leaves the gradient wrt out_hidden at the start of the workspace"""
+    lib = _lib.load()
+    a = st.args
+    with torch.cuda.device(st.out.device):
+        a.stream = _stream()
+        _lib.check(lib.regt_head_forward(C.byref(a)), "regt_head_forward")
+        if grads is not None:
+            a.accumulate = 1
+            _fill_params(a.g, {k: grads[k] for k in HEAD_KEYS})
+            st.keep.append(grads)
+            _lib.check(lib.regt_head_backward(C.byref(a)), "regt_head_backward")
 
 
 def check_loss(loss: str, null_value) -> int:
@@ -171,12 +247,13 @@ def loss_counts(y: torch.Tensor, null_value: float) -> torch.Tensor:
 
 
 def workspace_bytes(mode: int, precision: int, plan: GraphPlanTensors, B: int, x_rows: int, T: int, H: int, O: int,
-                    F: int = F_IN) -> int:
+                    F: int = F_IN, inference: bool = False) -> int:
     """bytes ``build_state`` will ask for at batch B (saved planes scale with B*N*T*H): used to size micro-batches."""
     a = _lib.Args()
     a.B, a.N, a.T, a.H, a.O = B, plan.N, T, H, O
     a.mode, a.precision, a.x_rows, a.F = mode, precision, x_rows, F
     a.fuse_head = 1
+    a.inference = 1 if inference else 0
     a.plan = plan.c_struct()
     return int(_lib.load().regt_workspace_bytes(C.byref(a)))
 

@@ -116,6 +116,20 @@ class RegTModelBase(nn.Module):
             out, hid = out[0], hid[0]
         return out, hid
 
+    @staticmethod
+    def _grad_views(params: Dict[str, torch.Tensor]) -> Dict[str, torch.Tensor]:
+        """``.grad`` of every parameter, created (zeroed) where missing: the kernels accumulate into these"""
+        grads = {}
+        for k, p in params.items():
+            if p.grad is None:
+                owner = getattr(p, "_regt_grad_owner", None)   # a GradExchange / FlatRMSprop owns the flat buffer behind .grad
+                if owner is not None:
+                    owner.attach(p)
+                else:
+                    p.grad = torch.zeros_like(p)
+            grads[k] = p.grad
+        return grads
+
     # ---- fused training step: forward + loss + backward in one pass, no autograd graph ----
     def _fused_step(self, x: torch.Tensor, y: torch.Tensor, plan, micro_batch: Optional[int] = None,
                     loss_nodes: Optional[int] = None, loss: str = "mse", null_value: Optional[float] = None,
@@ -133,15 +147,7 @@ class RegTModelBase(nn.Module):
         xb = xb.to(torch.float32).contiguous()
         yb = yb.to(torch.float32).contiguous()
         params = self._param_dict()
-        grads = {}
-        for k, p in params.items():
-            if p.grad is None:
-                owner = getattr(p, "_regt_grad_owner", None)   # a GradExchange / FlatRMSprop owns the flat buffer behind .grad
-                if owner is not None:
-                    owner.attach(p)
-                else:
-                    p.grad = torch.zeros_like(p)
-            grads[k] = p.grad
+        grads = self._grad_views(params)
         B = xb.shape[0]
         prec = self._prec(xb.shape[3])
         if micro_batch:

@@ -50,6 +50,9 @@ def build_parser() -> argparse.ArgumentParser:
     # additive (reference defaults reproduce the reference)
     parser.add_argument("--hidden", default=256, type=int, help="hidden width (reference: 256)")
     parser.add_argument("--precision", default="auto", type=str, help="auto | fp32 | tf32x3 | bf16")
+    parser.add_argument("--share_periods", action="store_true",
+                        help="run the cell once per time step of a batch of windows and share it across them (exact in real "
+                             "arithmetic, sums in another order; off: every window runs its own periods)")
     parser.add_argument("--synthetic_steps", default=600, type=int, help="length of the synthetic series when no node_data.npy is found")
     return parser
 
@@ -107,8 +110,9 @@ def main(argv=None):
           f"precision={model.precision}; series: {src}; {n_train} train / {len(windows) - n_train} test snapshots")
     opt = FlatRMSprop(list(model.parameters()), lr=args.lr, weight_decay=args.decay, skip=model.dead_parameters())   # run.py:145
     for epoch in range(args.epochs + 1):                                               # run.py:230
-        last_loss, _ = train_epoch(model, windows, graph, opt, 0, n_train, batch=max(1, args.bs))
-        mae, rmse, _ = evaluate(model, windows, graph, n_train, len(windows), batch=max(1, args.bs))
+        last_loss, _ = train_epoch(model, windows, graph, opt, 0, n_train, batch=max(1, args.bs), share_periods=args.share_periods)
+        mae, rmse, _ = evaluate(model, windows, graph, n_train, len(windows), batch=max(1, args.bs),
+                                share_periods=args.share_periods)
         print("Train Loss: {:.4f}, Test RMSE: {:.4f}, MAE: {:.4f}".format(float(last_loss), rmse, rmse * rmse))      # run.py:236
         if epoch % 10 == 0:                                                            # run.py:242-243
             os.makedirs(ck_dir, exist_ok=True)
